@@ -11,11 +11,17 @@ carries a `bands8k` sub-record: BASELINE configs[4], one 7680x4320 frame over a 
 peer memory with a device-side completion (strong scaling).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload flythrough4k|...]
+                    [--dump-outputs DIR]
 
 Prints ONE JSON line (rank 0).  `value` is timed with CUDA events around K frames rendered into device memory
 (inputs resident in HBM); `e2e` times the same frames through the C-ABI call with a host output buffer (the D2H
 of every frame inside the timed region).  `--impl reference` times the UNMODIFIED reference
 (oracle/_ref/hmap_ref*, built from /root/reference by oracle/Makefile) on the host cores, on a bounded sample.
+
+`--dump-outputs DIR` writes rank 0's frame of the last timed step, as the caller of the timed path receives it, to
+DIR/frame.npy (float32 [n, channels]: the pixels at DIR/pixel_index.npy, float64 [n] row-major indices y*W + x, a fixed
+seeded sample of at most 2^21 pixels, every pixel of a smaller frame).  The inputs are seeded, so two builds run with
+the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -60,6 +66,23 @@ MIN_HEIGHT, MAX_HEIGHT = 0.0, 10.0
 SEED = 1234
 REF_SAMPLE_DIV = 4          # the CPU arms render every frame at W/4 x H/4 (1/16 as many rays, same cameras)
 SM_COUNT_FALLBACK = 148
+DUMP_MAX_PIXELS = 1 << 21   # --dump-outputs: 2^21 pixels x 4 channels in float32 + their float64 indices = 48 MiB
+DUMP_SEED = 20240601
+
+
+def dump_frame(dump_dir: str, frame) -> None:
+    """frame: uint8 [H, W, C] -> DIR/frame.npy (float32 [n, C]) and DIR/pixel_index.npy (float64 [n]), a fixed seeded
+    sample of the pixels in row-major order."""
+    import numpy as np
+
+    h, w, c = frame.shape
+    if h * w <= DUMP_MAX_PIXELS:
+        idx = np.arange(h * w)
+    else:
+        idx = np.sort(np.random.default_rng(DUMP_SEED).choice(h * w, size=DUMP_MAX_PIXELS, replace=False))
+    os.makedirs(dump_dir, exist_ok=True)
+    np.save(os.path.join(dump_dir, "frame.npy"), frame.reshape(h * w, c)[idx].astype(np.float32))
+    np.save(os.path.join(dump_dir, "pixel_index.npy"), idx.astype(np.float64))
 
 
 def camera(wl: dict, n: int) -> dict:
@@ -229,6 +252,8 @@ def reference_arm(args, wl) -> None:
     frame_ids = [(s * args.gpus) % wl["frames"] for s in range(args.steps)]
     with tempfile.TemporaryDirectory(prefix="hmrm_bench_", dir="/dev/shm" if os.path.isdir("/dev/shm") else None) as td:
         res = run_cpu_reference(wl, frame_ids, args.warmup, Path(td))
+    if args.dump_outputs:
+        dump_frame(args.dump_outputs, res["frames"][-1])
     rays = res["W"] * res["H"]
     total_ms = sum(res["ms"])
     value = rays * len(res["ms"]) / (total_ms * 1e-3) / 1e6
@@ -324,9 +349,10 @@ class Job:
         self.r.close()
 
 
-def measure(job: Job, steps: int, warmup: int, sampler, want_cpu: bool) -> dict | None:
+def measure(job: Job, steps: int, warmup: int, sampler, want_cpu: bool, dump_dir: str | None = None) -> dict | None:
     """Runs `steps` timed steps of job's workload (after `warmup`): device-resident value, e2e through the C ABI,
-    statistics, roofline inputs.  Returns the record on rank 0, None elsewhere."""
+    statistics, roofline inputs.  Returns the record on rank 0, None elsewhere.  With `dump_dir`, rank 0's frame of
+    the last device-resident timed step goes there (dump_frame)."""
     import numpy as np
 
     torch, dist, hmrm, binding, MG = job.torch, job.dist, job.hmrm, job.binding, job.MG
@@ -407,6 +433,11 @@ def measure(job: Job, steps: int, warmup: int, sampler, want_cpu: bool) -> dict 
     barrier()
     dev_ms = ev0.elapsed_time(ev1)
     dev_ms_own = dev_ms
+    last_frame = None
+    if dump_dir is not None and rank == 0:
+        # copied before keep_busy / the roofline pass render into outs[0] again
+        last = outs[(steps - 1) % n_flight]
+        last_frame = last.view(-1)[: H * W * job.channels].view(H, W, job.channels).cpu().numpy()
     keep_busy(0.4)
 
     # ---- e2e: the user's call — host output buffer, D2H inside the timed region ----
@@ -661,6 +692,8 @@ def measure(job: Job, steps: int, warmup: int, sampler, want_cpu: bool) -> dict 
             shared.unlink()
             if not ok_host:
                 raise SystemExit("bands e2e: the shared host frame differs from the frame rendered whole")
+    if last_frame is not None:
+        dump_frame(dump_dir, last_frame)
     return rec
 
 
@@ -689,6 +722,8 @@ def ours_arm(args, wl) -> None:
     local = int(os.environ.get("LOCAL_RANK", "0"))
     if world != args.gpus:
         raise SystemExit(f"--gpus {args.gpus} but WORLD_SIZE={world}: launch with torchrun --nproc-per-node {args.gpus}")
+    if args.dump_outputs and wl.get("mode") == "bands" and world > 1:
+        raise SystemExit("--dump-outputs: a band-split frame is assembled across the ranks; run it with --gpus 1")
     if not torch.cuda.is_available():
         raise SystemExit("bench.py needs a CUDA device; there is no CPU fallback")
     torch.cuda.set_device(local)
@@ -709,7 +744,8 @@ def ours_arm(args, wl) -> None:
         sampler.start()
 
     job = Job(hmrm, binding, MG, torch, dist, wl, args, rank, world, local, stream)
-    rec = measure(job, args.steps, args.warmup, sampler, want_cpu=(world == 1 and not args.no_cpu_baseline))
+    rec = measure(job, args.steps, args.warmup, sampler, want_cpu=(world == 1 and not args.no_cpu_baseline),
+                  dump_dir=args.dump_outputs)
     job.close()
 
     # ---- N > 1, default workload: BASELINE configs[4] (row bands of one 8K frame over the N GPUs) as a sub-record ----
@@ -784,6 +820,8 @@ def main() -> None:
     ap.add_argument("--bands-workload", choices=["bands8k", "smokebands"], default="bands8k")
     ap.add_argument("--bands-steps", type=int, default=96)
     ap.add_argument("--cpu-frames", type=int, default=2)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the frame of the last timed step to DIR/frame.npy + DIR/pixel_index.npy (see above)")
     ap.add_argument("--inflight", type=int, default=2, help="frames in flight in the device-resident timing (1..4)")
     ap.add_argument("--bands-inflight", type=int, default=4,
                     help="bands workloads: frames in flight (1..6; one stream and one peer buffer each); measured per 8K frame: "

@@ -24,6 +24,10 @@ def golden_frames():
     return np.load(GOLDEN / "frames.npz")
 
 
+def golden_replays() -> dict:
+    return json.loads((GOLDEN / "replays.json").read_text())
+
+
 def golden_kat() -> dict:
     return json.loads((GOLDEN / "kat.json").read_text())
 

@@ -23,6 +23,19 @@ def test_reference_arm_prints_contract_line(oracle):
     assert d["e2e"] == {"value": d["value"], "unit": "Mrays/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
 
 
+def test_reference_arm_dump_outputs(oracle, tmp_path):
+    """--dump-outputs: the last timed frame (160x90 RGBA8 at the reference arm's sample resolution), every pixel."""
+    import numpy as np
+
+    res = subprocess.run([sys.executable, str(ROOT / "bench.py"), "--impl", "reference", "--workload", "smoke",
+                          "--steps", "2", "--warmup", "1", "--dump-outputs", str(tmp_path)],
+                         capture_output=True, text=True, timeout=600, cwd=str(ROOT))
+    assert res.returncode == 0, res.stderr[-2000:]
+    frame, idx = np.load(tmp_path / "frame.npy"), np.load(tmp_path / "pixel_index.npy")
+    assert frame.dtype == np.float32 and frame.shape == (160 * 90, 4) and frame.max() <= 255 and frame[:, 3].any()
+    assert idx.dtype == np.float64 and np.array_equal(idx, np.arange(160 * 90))
+
+
 def test_reference_arm_on_other_ranks_is_silent(oracle):
     import os
 

@@ -1,6 +1,7 @@
 """CPU: the oracle (oracle/hmap_oracle.c) against the committed fixtures that were produced by the
-UNMODIFIED reference (tests/golden/make_golden.py), and — when oracle/_ref is present — against the
-reference build itself, live."""
+UNMODIFIED reference (tests/golden/make_golden.py) or recorded where it matched the reference
+(tests/golden/replays.json, tests/golden/make_golden_replays.py), and — when oracle/_ref is present — against
+the reference build itself, live."""
 import numpy as np
 import pytest
 
@@ -77,39 +78,48 @@ def test_cycle_interleave_and_row_band(oracle):
 
 @pytest.mark.parametrize("name", ["persp_basic", "spher_fine", "ortho_basic", "noise_lum_neg", "min_height_twice"])
 def test_oracle_matches_live_reference(oracle, name, tmp_path):
-    """Oracle A (unmodified reference under the fake SDL) rendered now, if it is built here."""
-    if not oracle.have_ref():
-        pytest.skip("oracle/_ref not built (needs /root/reference)")
+    """Oracle A (unmodified reference under the fake SDL): its stored frame (tests/golden/frames.npz), and both
+    builds rendered now where oracle/_ref is built."""
     scene = S.SCENE_BY_NAME[name]
     hm, cm = H.load_scene_maps(scene, oracle)
+    fb, _, _ = H.oracle_render_scene(oracle, scene, (hm, cm))
+    assert np.array_equal(H.golden_frames()[name], fb)
+    if not oracle.have_ref():
+        return
     oracle.write_png(tmp_path / "h.png", hm)
     oracle.write_png(tmp_path / "c.png", cm)
     kw = S.frame_kwargs(scene)
     cfg = oracle.config_text(kw, tmp_path / "h.png", tmp_path / "c.png", lum=scene["lum"])
     for binary in (oracle.REF_BIN, oracle.REF_BIN_O2):
         frames, _ = oracle.run_ref(cfg, scene["projection"], kw["width"], kw["height"], binary=binary)
-        fb, _, _ = H.oracle_render_scene(oracle, scene, (hm, cm))
         assert np.array_equal(frames[0], fb)
+
+
+FLY_SCENE = dict(S.SCENE_BY_NAME["persp_basic"], width=160, height=90)
+FLY_STATES = [dict(pos=(-0.6, 0.6, 3.2), hang_deg=-45.0), dict(pos=(-0.2, 0.9, 3.0), hang_deg=-60.0),
+              dict(pos=(0.4, 1.0, 2.8), hang_deg=-80.0)]
+
+
+def flythrough_oracle_frames(oracle, maps):
+    return [H.oracle_render_scene(oracle, dict(FLY_SCENE, **s), maps)[0] for s in FLY_STATES]
 
 
 def test_reference_scripted_flythrough_matches_oracle(oracle, tmp_path):
     """Console-driven camera changes in the unmodified reference (main/hmap.cpp:760-804) reproduce
-    per-frame oracle renders (each state rendered twice because of the one-frame look/up lag)."""
+    per-frame oracle renders (each state rendered twice because of the one-frame look/up lag): against the
+    reference's recorded frames, and rendered now where oracle/_ref is built."""
+    hm, cm = H.load_scene_maps(FLY_SCENE, oracle)
+    want = flythrough_oracle_frames(oracle, (hm, cm))
+    assert [H.sha(fb) for fb in want] == H.golden_replays()["flythrough"]
     if not oracle.have_ref():
-        pytest.skip("oracle/_ref not built (needs /root/reference)")
-    scene = dict(S.SCENE_BY_NAME["persp_basic"], width=160, height=90)
-    hm, cm = H.load_scene_maps(scene, oracle)
+        return
     oracle.write_png(tmp_path / "h.png", hm)
     oracle.write_png(tmp_path / "c.png", cm)
-    kw = S.frame_kwargs(scene)
-    cfg = oracle.config_text(kw, tmp_path / "h.png", tmp_path / "c.png", lum=scene["lum"])
-    states = [dict(pos=(-0.6, 0.6, 3.2), hang_deg=-45.0), dict(pos=(-0.2, 0.9, 3.0), hang_deg=-60.0),
-              dict(pos=(0.4, 1.0, 2.8), hang_deg=-80.0)]
-    script = ["pos %r %r %r hang %r" % (*s["pos"], s["hang_deg"]) for s in states]
+    kw = S.frame_kwargs(FLY_SCENE)
+    cfg = oracle.config_text(kw, tmp_path / "h.png", tmp_path / "c.png", lum=FLY_SCENE["lum"])
+    script = ["pos %r %r %r hang %r" % (*s["pos"], s["hang_deg"]) for s in FLY_STATES]
     frames, _ = oracle.run_ref(cfg, 1, kw["width"], kw["height"], script=script)
-    for s, got in zip(states, frames):
-        sc = dict(scene, **s)
-        fb, _, _ = H.oracle_render_scene(oracle, sc, (hm, cm))
+    for got, fb in zip(frames, want):
         assert np.array_equal(got, fb)
 
 
@@ -128,19 +138,25 @@ def random_scene(rng, i):
                     lum=tuple(float(v) for v in rng.uniform(-0.3, 1.2, size=3)), bg=tuple(int(v) for v in rng.integers(0, 256, size=3)))
 
 
-def test_oracle_matches_live_reference_on_random_scenes(oracle, tmp_path):
-    """The restatement against the unmodified reference, rendered now (only where oracle/_ref is built): 18 random
-    scenes beyond the committed golden frames."""
-    if not oracle.have_ref():
-        pytest.skip("oracle/_ref not built (needs /root/reference)")
+def random_scenes():
     rng = np.random.default_rng(424242)
-    for i in range(18):
-        scene = random_scene(rng, i)
+    return [random_scene(rng, i) for i in range(18)]
+
+
+def test_oracle_matches_live_reference_on_random_scenes(oracle, tmp_path):
+    """The restatement against the unmodified reference on 18 random scenes beyond the committed golden frames: against
+    the reference's recorded frames, and rendered now where oracle/_ref is built."""
+    recorded = H.golden_replays()["random_scenes"]
+    assert len(recorded) == 18
+    for scene, want_sha in zip(random_scenes(), recorded):
         hm, cm = H.load_scene_maps(scene, oracle)
+        fb, _, _ = H.oracle_render_scene(oracle, scene, (hm, cm))
+        assert H.sha(fb) == want_sha, scene
+        if not oracle.have_ref():
+            continue
         oracle.write_png(tmp_path / "h.png", hm)
         oracle.write_png(tmp_path / "c.png", cm)
         kw = S.frame_kwargs(scene)
         cfg = oracle.config_text(kw, tmp_path / "h.png", tmp_path / "c.png", lum=scene["lum"])
         frames, _ = oracle.run_ref(cfg, scene["projection"], kw["width"], kw["height"], binary=oracle.REF_BIN_O2)
-        fb, _, _ = H.oracle_render_scene(oracle, scene, (hm, cm))
         assert np.array_equal(frames[0], fb), scene
