@@ -39,11 +39,13 @@ from .binding import (  # noqa: F401
     get_ray,
     library_path,
     load_library,
+    pinned_empty,
+    png_bound,
 )
 
 __all__ = [
     "Renderer", "Frame", "Stats", "HmrmError", "load_library", "library_path", "deg2rad", "camera_basis",
-    "get_ray", "PERSPECTIVE", "SPHERICAL", "ORTHOGRAPHIC", "FP64_EXACT", "FP32_FAST", "TRAVERSAL_AUTO",
+    "get_ray", "png_bound", "pinned_empty", "PERSPECTIVE", "SPHERICAL", "ORTHOGRAPHIC", "FP64_EXACT", "FP32_FAST", "TRAVERSAL_AUTO",
     "TRAVERSAL_BRUTE", "TRAVERSAL_SKIP", "TRAVERSAL_PACK", "FLAG_STATS", "FLAG_STEP_INDEX", "FLAG_RAY_DUMP", "PIXEL_RGBA8", "PIXEL_RGB8",
     "LAYOUT_ROWMAJOR", "LAYOUT_TILE4", "LAYOUT_ZORDER",
 ]

@@ -94,6 +94,10 @@ PROTOTYPES = {
     "hmrm_render_async": (C.c_int, [C.c_void_p, C.POINTER(Frame), C.c_void_p]),
     "hmrm_wait": (C.c_int, [C.c_void_p]),
     "hmrm_wait_pending": (C.c_int, [C.c_void_p, C.c_int]),
+    "hmrm_png_bound": (C.c_size_t, [C.c_int32, C.c_int32, C.c_int32]),
+    "hmrm_render_png_async": (C.c_int, [C.c_void_p, C.POINTER(Frame), C.c_void_p, C.c_size_t, C.c_void_p]),
+    "hmrm_encode_png": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_size_t,
+                                  C.c_void_p]),
     "hmrm_get_stats": (C.c_int, [C.c_void_p, C.POINTER(Stats)]),
     "hmrm_get_step_index": (C.c_int, [C.c_void_p, C.c_void_p]),
     "hmrm_get_ray_dump": (C.c_int, [C.c_void_p, C.c_void_p]),
@@ -170,6 +174,20 @@ def get_ray(frame: Frame, w: float, h: float):
     if rc:
         raise HmrmError(rc, "hmrm_get_ray: invalid frame")
     return tuple(pos), tuple(d)
+
+
+def png_bound(width: int, height: int, channels: int) -> int:
+    """Worst-case PNG file size of a width x height x channels (3 | 4) frame (hmrm_png_bound); 0 for other shapes."""
+    return int(load_library().hmrm_png_bound(int(width), int(height), int(channels)))
+
+
+def _nbytes(a):
+    """Size in bytes of a numpy array or torch tensor; None for a raw address."""
+    if isinstance(a, np.ndarray):
+        return a.nbytes
+    if hasattr(a, "numel") and hasattr(a, "element_size"):
+        return int(a.numel()) * int(a.element_size())
+    return None
 
 
 def _ptr(a) -> int:
@@ -323,8 +341,54 @@ class Renderer:
         self._check(self._lib.hmrm_wait(self._h))
 
     def wait_pending(self, max_pending: int) -> None:
-        """Streaming: return once at most `max_pending` (0 or 1) frames of render_async are still in flight."""
+        """Streaming: return once at most `max_pending` (0..3) frames of render_async / render_png_async are still in flight."""
         self._check(self._lib.hmrm_wait_pending(self._h, max_pending))
+
+    # -- PNG frames, deflated on the device -------------------------------------------------------
+    def render_png_async(self, frame: Frame, out, size_out, capacity: int | None = None) -> None:
+        """hmrm_render_png_async: `out` (pinned host or device memory of png_bound bytes or more) receives the PNG file,
+        `size_out` (one uint64 in the same kinds of memory) its size, once wait / wait_pending covers the frame.
+        numpy arrays and torch tensors report their own sizes; a raw address needs `capacity`."""
+        if capacity is None:
+            capacity = _nbytes(out)
+            if capacity is None:
+                raise ValueError("render_png_async: pass capacity= with a raw output address")
+        size_bytes = _nbytes(size_out)
+        if size_bytes is not None and (size_bytes < 8 or str(getattr(size_out, "dtype", "")).split(".")[-1]
+                                       not in ("uint64", "int64")):
+            raise ValueError("render_png_async: size_out must hold one 64-bit integer")
+        self._check(self._lib.hmrm_render_png_async(self._h, C.byref(frame), _ptr(out), int(capacity), _ptr(size_out)))
+
+    def render_png(self, frame: Frame | None = None, **overrides) -> bytes:
+        """One frame as a complete PNG file (the decoded pixels are render()'s)."""
+        f = frame if frame is not None else self.frame(**overrides)
+        out, size = self._png_buffers(f.screen_width, f.screen_height, 3 if f.pixel_format == PIXEL_RGB8 else 4)
+        self.render_png_async(f, out, size)
+        self.wait()
+        return out[:int(size[0])].tobytes()
+
+    def encode_png(self, pixels: np.ndarray) -> bytes:
+        """[H, W, 3 | 4] uint8 pixels -> PNG file, encoded on this context's device."""
+        px = np.ascontiguousarray(pixels, dtype=np.uint8)
+        if px.ndim != 3 or px.shape[2] not in (3, 4):
+            raise ValueError("pixels must be [H, W, 3] or [H, W, 4] uint8")
+        h, w, ch = px.shape
+        out, size = self._png_buffers(w, h, ch)
+        self._check(self._lib.hmrm_encode_png(self._h, px.ctypes.data, w, h, ch, out.ctypes.data, out.nbytes,
+                                              size.ctypes.data))
+        return out[:int(size[0])].tobytes()
+
+    def _png_buffers(self, width: int, height: int, channels: int):
+        """Pinned file + size buffers, kept for the last shape: pinning ~33 MB per 4K call would cost more than the
+        encode."""
+        bound = png_bound(width, height, channels)
+        if bound == 0:
+            raise ValueError(f"no PNG of {width}x{height}x{channels}")
+        cached = getattr(self, "_png_cache", None)
+        if cached is None or cached[0].nbytes < bound:
+            cached = (pinned_empty((bound,)), pinned_empty((1,), dtype=np.uint64))
+            self._png_cache = cached
+        return cached
 
     def render_device(self, frame: Frame, d_out, stream=None) -> None:
         self._check(self._lib.hmrm_render_device(self._h, C.byref(frame), _ptr(d_out), _ptr(stream)))

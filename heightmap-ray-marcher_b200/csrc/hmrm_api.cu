@@ -25,6 +25,7 @@
 #include "k2_render_skip.cuh"
 #include "k2_render_lin.cuh"
 #include "k2_render_pack.cuh"
+#include "k3_png.cuh"
 #include "peer_sync.cuh"
 #include "render_params.h"
 #include "synth_fbm.h"
@@ -57,6 +58,16 @@ struct LaunchSlot {
 	size_t step_cap;             // pixels
 	double *d_ray_dump;          // HMRM_FLAG_RAY_DUMP output, [pixels][10]
 	size_t dump_cap;             // pixels
+};
+
+// K3 scratch of one ring slot: filtered stream, staged chunks, per-segment sizes / Adler-32 partials, piece offsets,
+// signature / IHDR / tail chunks.  Each slot has its own, so two frames in flight never share it.
+struct PngScratch {
+	uint8_t *filt, *stage, *meta;
+	PngSegInfo *info;
+	unsigned long long *offsets;
+	unsigned long long filt_cap;  // bytes of filtered stream
+	int seg_cap;                  // segments
 };
 
 } // namespace
@@ -118,6 +129,10 @@ struct hmrm_ctx {
 	bool copy_pending[kFrameRing];
 	int fb_format;               // pixel format of what the ring holds (a change re-zeroes it, like a new resolution)
 	int slot;                    // buffer of the most recent hmrm_render_async
+	// PNG encoding: scratch per ring slot, allocated by the first PNG frame that uses the slot
+	PngScratch png[kFrameRing];
+	uint8_t *d_png_in;           // hmrm_encode_png's device copy of the caller's pixels
+	size_t png_in_cap;
 
 	// per-launch resources, used round-robin so that up to kLaunchSlots kernels of this context may be in flight
 	LaunchSlot slots[kLaunchSlots];
@@ -746,6 +761,93 @@ int peer_arrive(hmrm_ctx *c, PeerCtrl *ctrl, const hmrm_frame *f, unsigned int u
 	return HMRM_OK;
 }
 
+// ---- PNG frames (K3, csrc/k3_png.cuh) ------------------------------------------------------------------------------
+void free_png_scratch(PngScratch &p) {
+	cudaFree(p.filt);
+	cudaFree(p.stage);
+	cudaFree(p.meta);
+	cudaFree(p.info);
+	cudaFree(p.offsets);
+	std::memset(&p, 0, sizeof p);
+}
+
+int ensure_png_scratch(hmrm_ctx *c, int slot, const PngShape &s) {
+	PngScratch &p = c->png[slot];
+	if (p.filt && p.filt_cap >= s.total && p.seg_cap >= s.nseg) return HMRM_OK;
+	// the slot's previous PNG frame may still be encoding from the buffers about to be replaced
+	if (c->copy_pending[slot]) HMRM_CUDA(c, cudaEventSynchronize(c->ev_copied[slot]));
+	free_png_scratch(p);
+	HMRM_CUDA(c, cudaMalloc(&p.filt, (size_t)s.total));
+	HMRM_CUDA(c, cudaMalloc(&p.stage, (size_t)s.nseg * kPngStageStride));
+	HMRM_CUDA(c, cudaMalloc(&p.meta, kPngMetaBytes));
+	HMRM_CUDA(c, cudaMalloc(&p.info, (size_t)s.nseg * sizeof(PngSegInfo)));
+	HMRM_CUDA(c, cudaMalloc(&p.offsets, ((size_t)s.nseg + 3) * sizeof(unsigned long long)));
+	p.filt_cap = s.total;
+	p.seg_cap = s.nseg;
+	return HMRM_OK;
+}
+
+// The address the device writes `p` through: device memory of the context's device as it is, pinned / registered host
+// memory through its mapping.  Pageable memory is refused with a status (the device cannot write it).
+int png_device_view(hmrm_ctx *c, void *p, const char *what, void **dev) {
+	cudaPointerAttributes a;
+	const cudaError_t e = cudaPointerGetAttributes(&a, p);
+	if (e != cudaSuccess) {
+		cudaGetLastError();
+		return fail(c, HMRM_ERR_INVALID, "%s: %s", what, cudaGetErrorString(e));
+	}
+	if (a.type == cudaMemoryTypeDevice) {
+		if (a.device != c->device)
+			return fail(c, HMRM_ERR_INVALID, "%s is memory of device %d, not of the context's device %d", what, a.device,
+			            c->device);
+		*dev = p;
+		return HMRM_OK;
+	}
+	if (a.type == cudaMemoryTypeHost && a.devicePointer) {
+		*dev = a.devicePointer;
+		return HMRM_OK;
+	}
+	return fail(c, HMRM_ERR_INVALID, "%s must be pinned or registered host memory, or device memory of device %d", what,
+	            c->device);
+}
+
+// validates png_out / capacity / png_bytes for a W x H x C file and resolves their device addresses
+int png_outputs(hmrm_ctx *c, const PngShape &s, uint8_t *png_out, size_t capacity, uint64_t *png_bytes, uint8_t **d_out,
+                unsigned long long **d_size) {
+	if (!png_out || !png_bytes) return fail(c, HMRM_ERR_INVALID, "png_out and png_bytes must not be NULL");
+	if ((uintptr_t)png_bytes % 8 != 0) return fail(c, HMRM_ERR_INVALID, "png_bytes must be 8-byte aligned");
+	const unsigned long long bound = png_bound(s);
+	if ((unsigned long long)capacity < bound)
+		return fail(c, HMRM_ERR_INVALID, "capacity %zu is below hmrm_png_bound = %llu", capacity, bound);
+	HMRM_CUDA(c, cudaSetDevice(c->device));
+	void *o = NULL, *z = NULL;
+	if (int rc = png_device_view(c, png_out, "png_out", &o)) return rc;
+	if (int rc = png_device_view(c, png_bytes, "png_bytes", &z)) return rc;
+	*d_out = (uint8_t *)o;
+	*d_size = (unsigned long long *)z;
+	return HMRM_OK;
+}
+
+// Enqueue the four K3 launches on `st`: d_img [H][W][C] -> PNG file at d_dst, its size at d_size.
+int enqueue_png(hmrm_ctx *c, int slot, const uint8_t *d_img, int W, int H, int C, uint8_t *d_dst,
+                unsigned long long *d_size, cudaStream_t st) {
+	PngShape s;
+	png_shape(W, H, C, &s);
+	if (int rc = ensure_png_scratch(c, slot, s)) return rc;
+	const PngScratch &p = c->png[slot];
+	k3_png_filter<<<H, 256, 0, st>>>(d_img, (int)s.row_bytes, C, p.filt);
+	// the byte one row up is a candidate distance while deflate can reach it
+	const int row_dist = s.row_bytes + 1 <= 32768ull ? (int)(s.row_bytes + 1) : 0;
+	k3_png_deflate<<<(s.nseg + kPngDeflateWarps - 1) / kPngDeflateWarps, kPngDeflateWarps * 32, 0, st>>>(
+		p.filt, s.total, s.nseg, C, row_dist, p.stage, p.info);
+	k3_png_finish<<<1, 1024, 0, st>>>(p.info, s.nseg, s.total, W, H, C, p.offsets, p.meta);
+	const unsigned long long words = png_bound(s) / 16 + 2;
+	const int blocks = (int)std::min((words + 255) / 256, (unsigned long long)c->num_sms * 16ull);
+	k3_png_gather<<<blocks, 256, 0, st>>>(p.offsets, s.nseg + 2, p.meta, p.stage, d_dst, d_size);
+	HMRM_CUDA(c, cudaGetLastError());
+	return HMRM_OK;
+}
+
 } // namespace
 
 extern "C" {
@@ -849,6 +951,9 @@ int hmrm_create(int device, hmrm_ctx **out) {
 	c->copy_stream = NULL;
 	c->slot = 0;
 	c->fb_format = HMRM_PIXEL_RGBA8;
+	std::memset(c->png, 0, sizeof c->png);
+	c->d_png_in = NULL;
+	c->png_in_cap = 0;
 
 	c->launch_next = c->launch_last = 0;
 	c->last_had_stats = c->last_had_step_index = c->last_had_ray_dump = c->timing_valid = false;
@@ -894,7 +999,9 @@ void hmrm_destroy(hmrm_ctx *c) {
 	cudaFree(c->d_htab);
 
 	if (c->copy_stream) cudaStreamSynchronize(c->copy_stream);
+	cudaFree(c->d_png_in);
 	for (int i = 0; i < kFrameRing; ++i) {
+		free_png_scratch(c->png[i]);
 		cudaFree(c->d_fb[i]);
 		if (c->ev_rendered[i]) cudaEventDestroy(c->ev_rendered[i]);
 		if (c->ev_copied[i]) cudaEventDestroy(c->ev_copied[i]);
@@ -1204,6 +1311,78 @@ int hmrm_render(hmrm_ctx *c, const hmrm_frame *f, uint8_t *rgba_out) {
 	int rc = hmrm_render_async(c, f, rgba_out);
 	if (rc) return rc;
 	return hmrm_wait(c);
+}
+
+size_t hmrm_png_bound(int32_t width, int32_t height, int32_t channels) {
+	PngShape s;
+	if (!png_shape(width, height, channels, &s)) return 0;
+	return (size_t)png_bound(s);
+}
+
+int hmrm_render_png_async(hmrm_ctx *c, const hmrm_frame *f, uint8_t *png_out, size_t capacity, uint64_t *png_bytes) {
+	if (!c) return HMRM_ERR_INVALID;
+	if (!f) return fail(c, HMRM_ERR_INVALID, "frame is NULL");
+	if (f->cycle_period != 1 || f->cycle != 0) return fail(c, HMRM_ERR_INVALID, "PNG frames are whole frames: cycle_period 1");
+	if (f->band_count > 1) return fail(c, HMRM_ERR_INVALID, "PNG frames are whole frames: band_count <= 1");
+	if (f->flags & (HMRM_FLAG_STEP_INDEX | HMRM_FLAG_RAY_DUMP))
+		return fail(c, HMRM_ERR_INVALID, "PNG frames do not record step indices or ray dumps");
+	if (f->row_begin != 0 || (f->row_end != 0 && f->row_end != f->screen_height))
+		return fail(c, HMRM_ERR_INVALID, "PNG frames are whole frames: row_begin 0, row_end 0 or screen_height");
+	if (f->pixel_format != HMRM_PIXEL_RGBA8 && f->pixel_format != HMRM_PIXEL_RGB8)
+		return fail(c, HMRM_ERR_INVALID, "unknown pixel_format %d", (int)f->pixel_format);
+	if (f->screen_width < 2 || f->screen_height < 2 || f->screen_width > 65536 || f->screen_height > 65536)
+		return fail(c, HMRM_ERR_INVALID, "resolution %dx%d outside [2,65536]", f->screen_width, f->screen_height);
+	const int C = f->pixel_format == HMRM_PIXEL_RGB8 ? 3 : 4;
+	PngShape s;
+	png_shape(f->screen_width, f->screen_height, C, &s);
+	uint8_t *d_out = NULL;
+	unsigned long long *d_size = NULL;
+	int rc = png_outputs(c, s, png_out, capacity, png_bytes, &d_out, &d_size);
+	if (rc) return rc;
+	if ((rc = ensure_framebuffer(c, f->screen_width, f->screen_height, f->pixel_format)) != HMRM_OK) return rc;
+	// the ring exactly as hmrm_render_async uses it for whole frames; the encoder takes the place of the copy-out
+	const int slot = (c->slot + 1) % kFrameRing;
+	if ((rc = ensure_png_scratch(c, slot, s)) != HMRM_OK) return rc;
+	uint32_t *fb = c->d_fb[slot];
+	cudaStream_t cs = c->ring_stream[slot];
+	if (c->copy_pending[slot]) HMRM_CUDA(c, cudaStreamWaitEvent(cs, c->ev_copied[slot], 0));
+	if ((rc = enqueue_render(c, f, fb, cs, true)) != HMRM_OK) return rc;
+	HMRM_CUDA(c, cudaEventRecord(c->ev_rendered[slot], cs));
+	HMRM_CUDA(c, cudaStreamWaitEvent(c->copy_stream, c->ev_rendered[slot], 0));
+	rc = enqueue_png(c, slot, (const uint8_t *)fb, f->screen_width, f->screen_height, C, d_out, d_size, c->copy_stream);
+	if (rc) return rc;
+	HMRM_CUDA(c, cudaEventRecord(c->ev_copied[slot], c->copy_stream));
+	c->copy_pending[slot] = true;
+	c->slot = slot;
+	return HMRM_OK;
+}
+
+int hmrm_encode_png(hmrm_ctx *c, const uint8_t *pixels, int32_t width, int32_t height, int32_t channels,
+                    uint8_t *png_out, size_t capacity, uint64_t *png_bytes) {
+	if (!c) return HMRM_ERR_INVALID;
+	if (!pixels) return fail(c, HMRM_ERR_INVALID, "pixels is NULL");
+	PngShape s;
+	if (!png_shape(width, height, channels, &s))
+		return fail(c, HMRM_ERR_INVALID, "image %dx%dx%d: need 1 <= width, height <= 65536 and 3 or 4 channels", width,
+		            height, channels);
+	uint8_t *d_out = NULL;
+	unsigned long long *d_size = NULL;
+	int rc = png_outputs(c, s, png_out, capacity, png_bytes, &d_out, &d_size);
+	if (rc) return rc;
+	// synchronous: whatever the context has in flight finishes first, then ring slot 0's scratch is free
+	if ((rc = drain(c)) != HMRM_OK) return rc;
+	const size_t bytes = (size_t)width * (size_t)height * (size_t)channels;
+	if (bytes > c->png_in_cap) {
+		cudaFree(c->d_png_in);
+		c->d_png_in = NULL;
+		c->png_in_cap = 0;
+		HMRM_CUDA(c, cudaMalloc(&c->d_png_in, bytes));
+		c->png_in_cap = bytes;
+	}
+	HMRM_CUDA(c, cudaMemcpyAsync(c->d_png_in, pixels, bytes, cudaMemcpyDefault, c->stream));
+	if ((rc = enqueue_png(c, 0, c->d_png_in, width, height, channels, d_out, d_size, c->stream)) != HMRM_OK) return rc;
+	HMRM_CUDA(c, cudaStreamSynchronize(c->stream));
+	return HMRM_OK;
 }
 
 int hmrm_get_stats(hmrm_ctx *c, hmrm_stats *out) {

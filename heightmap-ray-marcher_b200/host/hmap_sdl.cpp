@@ -13,7 +13,8 @@
 //   movement: W/S/D/A/Space/Q scaled by delta * move (:928-950), only without modifiers and with the console closed
 //   render:   cycle = (cycle + 1) % cycle_period (:976), then the frame body — here one hmrm_render call
 //   present:  FPS / console overlays (:1060-1125), SDL_UpdateTexture + RenderCopy + RenderPresent (:1082-1127)
-//   record:   screenshots/hmap_<id>_<n>.png after each frame, "Done recording." (:1131-1144)
+//   record:   screenshots/hmap_<id>_<n>.png after each frame, "Done recording." (:1131-1144); screenshots and recorded
+//             frames are PNG-encoded on the device (hmrm_encode_png)
 #ifdef HMAP_WITH_SDL
 
 #include <SDL2/SDL.h>
@@ -52,6 +53,9 @@ struct Shell {
 	TTF_Font *font;
 	SDL_Surface *fps_surface, *console_surface;
 	std::vector<uint8_t> framebuf;
+	uint8_t *png_file;       // pinned PNG file of the last screenshot, png_cap bytes
+	size_t png_cap;
+	uint64_t *png_bytes;     // pinned: its size
 
 	bool quit, show_fps, console_active, recording, fullscreen;
 	std::string console_buf;
@@ -61,7 +65,7 @@ struct Shell {
 
 	Shell(Config &c, hmrm_ctx *x, int prec, int trav)
 		: cfg(c), ctx(x), precision(prec), traversal(trav), window(NULL), renderer(NULL), texture(NULL), font(NULL),
-		  fps_surface(NULL), console_surface(NULL), quit(false), show_fps(false), console_active(false), recording(false),
+		  fps_surface(NULL), console_surface(NULL), png_file(NULL), png_cap(0), png_bytes(NULL), quit(false), show_fps(false), console_active(false), recording(false),
 		  fullscreen(false), console_buf(" "), recording_id(0), recording_frame_num(0), text_timer_ms(201) {}
 
 	void fatal(const std::string &msg) {
@@ -108,10 +112,28 @@ struct Shell {
 		framebuf.assign((size_t)cfg.screen_width * (size_t)cfg.screen_height * 4, 0);
 	}
 
+	// SavePNG (main/hmap.cpp:157-168): framebuf encoded on the device
 	void save_png(const std::string &path) {
-		std::string why;
-		if (!write_png(path, cfg.screen_width, cfg.screen_height, 4, framebuf.data(), &why))
-			std::cerr << "Failed to write screenshot to " << path << "\n";
+		const size_t cap = hmrm_png_bound(cfg.screen_width, cfg.screen_height, 4);
+		if (png_cap < cap) {
+			// pinned: the device writes the file straight into it
+			hmrm_host_free(png_file);
+			png_file = NULL;
+			png_cap = 0;
+			void *p = NULL;
+			if (hmrm_host_alloc(&p, cap) != HMRM_OK) fatal(std::string("hmrm_host_alloc: ") + hmrm_last_error(NULL));
+			png_file = (uint8_t *)p;
+			png_cap = cap;
+		}
+		if (!png_bytes) {
+			void *p = NULL;
+			if (hmrm_host_alloc(&p, sizeof(uint64_t)) != HMRM_OK) fatal(std::string("hmrm_host_alloc: ") + hmrm_last_error(NULL));
+			png_bytes = (uint64_t *)p;
+		}
+		if (hmrm_encode_png(ctx, framebuf.data(), cfg.screen_width, cfg.screen_height, 4, png_file, png_cap, png_bytes) !=
+		    HMRM_OK)
+			fatal(std::string("hmrm_encode_png: ") + hmrm_last_error(ctx));
+		if (!write_bytes(path, png_file, (size_t)*png_bytes)) std::cerr << "Failed to write screenshot to " << path << "\n";
 		else std::cout << "Saved screenshot at " << path << "\n";
 	}
 
@@ -343,6 +365,8 @@ struct Shell {
 		TTF_CloseFont(font);
 		TTF_Quit();
 		SDL_Quit();
+		hmrm_host_free(png_file);
+		hmrm_host_free(png_bytes);
 		return 0;
 	}
 };

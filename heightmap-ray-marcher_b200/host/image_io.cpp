@@ -1,4 +1,4 @@
-// See image_io.hpp.  PNG / PNM / TGA decode to the pixel values stb_image v2.27 would return, PNG encode.
+// See image_io.hpp.  PNG / PNM / TGA decode to the pixel values stb_image v2.27 would return.
 #include "image_internal.hpp"
 
 #include <zlib.h>
@@ -288,40 +288,11 @@ bool load_image_memory(const std::vector<uint8_t> &file, int want_channels, Imag
 	return true;
 }
 
-bool write_png(const std::string &path, int width, int height, int channels, const uint8_t *pixels, std::string *error) {
-	if (width <= 0 || height <= 0 || (channels != 3 && channels != 4)) { *error = "bad image"; return false; }
-	const size_t stride = (size_t)width * (size_t)channels;
-	std::vector<uint8_t> raw((stride + 1) * (size_t)height);
-	for (int y = 0; y < height; ++y) {
-		raw[(size_t)y * (stride + 1)] = 0;   // filter: none
-		std::memcpy(&raw[(size_t)y * (stride + 1) + 1], pixels + (size_t)y * stride, stride);
-	}
-	uLongf bound = compressBound((uLong)raw.size());
-	std::vector<uint8_t> z(bound);
-	if (compress2(z.data(), &bound, raw.data(), (uLong)raw.size(), 1) != Z_OK) { *error = "zlib compress failed"; return false; }
+bool write_bytes(const std::string &path, const uint8_t *data, size_t n) {
 	FILE *f = std::fopen(path.c_str(), "wb");
-	if (!f) { *error = "cannot open for writing"; return false; }
-	auto chunk = [&](const char *type, const uint8_t *data, size_t len) {
-		uint8_t hdr[8] = {(uint8_t)(len >> 24), (uint8_t)(len >> 16), (uint8_t)(len >> 8), (uint8_t)len,
-		                  (uint8_t)type[0], (uint8_t)type[1], (uint8_t)type[2], (uint8_t)type[3]};
-		std::fwrite(hdr, 1, 8, f);
-		if (len) std::fwrite(data, 1, len, f);
-		uLong crc = crc32(0L, hdr + 4, 4);
-		if (len) crc = crc32(crc, data, (uInt)len);
-		const uint8_t c[4] = {(uint8_t)(crc >> 24), (uint8_t)(crc >> 16), (uint8_t)(crc >> 8), (uint8_t)crc};
-		std::fwrite(c, 1, 4, f);
-	};
-	static const uint8_t sig[8] = {137, 80, 78, 71, 13, 10, 26, 10};
-	std::fwrite(sig, 1, 8, f);
-	uint8_t ihdr[13] = {(uint8_t)(width >> 24), (uint8_t)(width >> 16), (uint8_t)(width >> 8), (uint8_t)width,
-	                    (uint8_t)(height >> 24), (uint8_t)(height >> 16), (uint8_t)(height >> 8), (uint8_t)height,
-	                    8, (uint8_t)(channels == 4 ? 6 : 2), 0, 0, 0};
-	chunk("IHDR", ihdr, 13);
-	chunk("IDAT", z.data(), (size_t)bound);
-	chunk("IEND", NULL, 0);
-	const bool ok = std::fclose(f) == 0;
-	if (!ok) *error = "write failed";
-	return ok;
+	if (!f) return false;
+	const bool wrote = n == 0 || std::fwrite(data, 1, n, f) == n;
+	return std::fclose(f) == 0 && wrote;
 }
 
 } // namespace hmrm_host

@@ -152,6 +152,24 @@ int hmrm_wait(hmrm_ctx *ctx);
  * in its host buffer (so n + 1 host buffers are rotated); hmrm_wait_pending(ctx, 0) == hmrm_wait. */
 int hmrm_wait_pending(hmrm_ctx *ctx, int max_pending);
 
+/* ---- PNG frames, deflated on the device (kernel K3, csrc/k3_png.cuh) ----
+ * The file is 8-bit, not interlaced, colour type 6 for 4 channels and 2 for 3; the decoded pixels are the frame's, byte
+ * for byte.  Each row gets the PNG filter with the smallest sum of |residual|; the filtered stream is deflated in
+ * independent 4096-byte segments (fixed-Huffman LZ77, or stored when that is smaller), one IDAT chunk each. */
+/* worst-case file size for width x height x channels (3 | 4), 0 for other shapes; host arithmetic, no device work:
+ * with N = height * (width * channels + 1) and S = ceil(N / 4096) segments, N + 17 S + 65 */
+size_t hmrm_png_bound(int32_t width, int32_t height, int32_t channels);
+/* hmrm_render_async, but the frame leaves the device as a complete PNG file (colour type 6 for HMRM_PIXEL_RGBA8,
+ * 2 for HMRM_PIXEL_RGB8).  Whole frames only (cycle_period 1, band_count <= 1, no STEP_INDEX / RAY_DUMP).  png_out:
+ * pinned / registered host memory or device memory of ctx's device, capacity >= hmrm_png_bound; *png_bytes (same
+ * kinds of memory, 8-byte aligned) receives the file size.  Both are valid once hmrm_wait / hmrm_wait_pending covers
+ * the frame; up to four PNG frames may be in flight, as with hmrm_render_async. */
+int hmrm_render_png_async(hmrm_ctx *ctx, const hmrm_frame *f, uint8_t *png_out, size_t capacity, uint64_t *png_bytes);
+/* encode caller pixels (host memory, [height][width][channels], copied to the device); synchronous.  Sizes from 1 to
+ * 65536 per axis; png_out / png_bytes as for hmrm_render_png_async. */
+int hmrm_encode_png(hmrm_ctx *ctx, const uint8_t *pixels, int32_t width, int32_t height, int32_t channels,
+                    uint8_t *png_out, size_t capacity, uint64_t *png_bytes);
+
 int hmrm_get_stats(hmrm_ctx *ctx, hmrm_stats *out);            /* of the last render */
 /* traversal diagnostics of the last HMRM_FLAG_STATS render with a skip traversal: [0] jumps, [1] samples covered
  * by jumps, [2] single steps above a mip block, [3] level descents, [4] cell tests above the cell, [5] cell tests
