@@ -30,6 +30,8 @@ from .binding import (  # noqa: F401
     TRAVERSAL_PACK,
     TRAVERSAL_SKIP,
     TRAVERSAL_SKIP_FP64,
+    YUV_BT601,
+    YUV_BT709,
     Frame,
     HmrmError,
     Renderer,
@@ -41,11 +43,12 @@ from .binding import (  # noqa: F401
     load_library,
     pinned_empty,
     png_bound,
+    yuv420_bytes,
 )
 
 __all__ = [
     "Renderer", "Frame", "Stats", "HmrmError", "load_library", "library_path", "deg2rad", "camera_basis",
-    "get_ray", "png_bound", "pinned_empty", "PERSPECTIVE", "SPHERICAL", "ORTHOGRAPHIC", "FP64_EXACT", "FP32_FAST", "TRAVERSAL_AUTO",
+    "get_ray", "png_bound", "yuv420_bytes", "pinned_empty", "PERSPECTIVE", "SPHERICAL", "ORTHOGRAPHIC", "FP64_EXACT", "FP32_FAST", "TRAVERSAL_AUTO",
     "TRAVERSAL_BRUTE", "TRAVERSAL_SKIP", "TRAVERSAL_PACK", "FLAG_STATS", "FLAG_STEP_INDEX", "FLAG_RAY_DUMP", "PIXEL_RGBA8", "PIXEL_RGB8",
-    "LAYOUT_ROWMAJOR", "LAYOUT_TILE4", "LAYOUT_ZORDER",
+    "LAYOUT_ROWMAJOR", "LAYOUT_TILE4", "LAYOUT_ZORDER", "YUV_BT601", "YUV_BT709",
 ]

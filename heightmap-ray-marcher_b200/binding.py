@@ -21,6 +21,7 @@ TRAVERSAL_AUTO, TRAVERSAL_BRUTE, TRAVERSAL_SKIP, TRAVERSAL_SKIP_FP64, TRAVERSAL_
 FLAG_STATS, FLAG_STEP_INDEX, FLAG_RAY_DUMP = 1, 2, 4
 PIXEL_RGBA8, PIXEL_RGB8 = 0, 1
 LAYOUT_ROWMAJOR, LAYOUT_TILE4, LAYOUT_ZORDER = 0, 1, 2
+YUV_BT601, YUV_BT709 = 0, 1
 
 
 class HmrmError(RuntimeError):
@@ -98,6 +99,10 @@ PROTOTYPES = {
     "hmrm_render_png_async": (C.c_int, [C.c_void_p, C.POINTER(Frame), C.c_void_p, C.c_size_t, C.c_void_p]),
     "hmrm_encode_png": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_size_t,
                                   C.c_void_p]),
+    "hmrm_yuv420_bytes": (C.c_size_t, [C.c_int32, C.c_int32]),
+    "hmrm_render_yuv420_async": (C.c_int, [C.c_void_p, C.POINTER(Frame), C.c_int32, C.c_void_p, C.c_size_t]),
+    "hmrm_convert_yuv420": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_void_p,
+                                      C.c_size_t]),
     "hmrm_get_stats": (C.c_int, [C.c_void_p, C.POINTER(Stats)]),
     "hmrm_get_step_index": (C.c_int, [C.c_void_p, C.c_void_p]),
     "hmrm_get_ray_dump": (C.c_int, [C.c_void_p, C.c_void_p]),
@@ -179,6 +184,20 @@ def get_ray(frame: Frame, w: float, h: float):
 def png_bound(width: int, height: int, channels: int) -> int:
     """Worst-case PNG file size of a width x height x channels (3 | 4) frame (hmrm_png_bound); 0 for other shapes."""
     return int(load_library().hmrm_png_bound(int(width), int(height), int(channels)))
+
+
+def yuv420_bytes(width: int, height: int) -> int:
+    """Bytes of the I420 planes of a width x height frame (hmrm_yuv420_bytes); 0 outside [1, 65536] per axis."""
+    return int(load_library().hmrm_yuv420_bytes(int(width), int(height)))
+
+
+def yuv420_planes(buf: np.ndarray, width: int, height: int):
+    """(Y [H, W], Cb [ceil(H/2), ceil(W/2)], Cr) views of I420 bytes."""
+    cw, ch = (width + 1) // 2, (height + 1) // 2
+    y = buf[:width * height].reshape(height, width)
+    cb = buf[width * height:width * height + cw * ch].reshape(ch, cw)
+    cr = buf[width * height + cw * ch:width * height + 2 * cw * ch].reshape(ch, cw)
+    return y, cb, cr
 
 
 def _nbytes(a):
@@ -341,7 +360,8 @@ class Renderer:
         self._check(self._lib.hmrm_wait(self._h))
 
     def wait_pending(self, max_pending: int) -> None:
-        """Streaming: return once at most `max_pending` (0..3) frames of render_async / render_png_async are still in flight."""
+        """Streaming: return once at most `max_pending` (0..3) frames of render_async / render_png_async /
+        render_yuv420_async are still in flight."""
         self._check(self._lib.hmrm_wait_pending(self._h, max_pending))
 
     # -- PNG frames, deflated on the device -------------------------------------------------------
@@ -389,6 +409,49 @@ class Renderer:
             cached = (pinned_empty((bound,)), pinned_empty((1,), dtype=np.uint64))
             self._png_cache = cached
         return cached
+
+    # -- 4:2:0 video planes, converted on the device ----------------------------------------------
+    def render_yuv420_async(self, frame: Frame, out, matrix: int = YUV_BT709, capacity: int | None = None) -> None:
+        """hmrm_render_yuv420_async: `out` (pinned host or device memory of yuv420_bytes or more) receives the I420 planes
+        once wait / wait_pending covers the frame.  numpy arrays and torch tensors report their own sizes; a raw address
+        needs `capacity`."""
+        if capacity is None:
+            capacity = _nbytes(out)
+            if capacity is None:
+                raise ValueError("render_yuv420_async: pass capacity= with a raw output address")
+        self._check(self._lib.hmrm_render_yuv420_async(self._h, C.byref(frame), int(matrix), _ptr(out), int(capacity)))
+
+    def render_yuv420(self, frame: Frame | None = None, matrix: int = YUV_BT709, **overrides):
+        """One frame as (Y, Cb, Cr) uint8 planes.  They are views of one pinned buffer that the next render_yuv420 or
+        convert_yuv420 call overwrites: copy them to keep them."""
+        f = frame if frame is not None else self.frame(**overrides)
+        out = self._yuv_buffer(f.screen_width, f.screen_height)
+        self.render_yuv420_async(f, out, matrix)
+        self.wait()
+        return yuv420_planes(out, f.screen_width, f.screen_height)
+
+    def convert_yuv420(self, pixels: np.ndarray, matrix: int = YUV_BT709):
+        """[H, W, 3 | 4] uint8 pixels -> (Y, Cb, Cr) planes, converted on this context's device; the same buffer as
+        render_yuv420's."""
+        px = np.ascontiguousarray(pixels, dtype=np.uint8)
+        if px.ndim != 3 or px.shape[2] not in (3, 4):
+            raise ValueError("pixels must be [H, W, 3] or [H, W, 4] uint8")
+        h, w, ch = px.shape
+        out = self._yuv_buffer(w, h)
+        self._check(self._lib.hmrm_convert_yuv420(self._h, px.ctypes.data, w, h, ch, int(matrix), out.ctypes.data,
+                                                  out.nbytes))
+        return yuv420_planes(out, w, h)
+
+    def _yuv_buffer(self, width: int, height: int) -> np.ndarray:
+        """Pinned planes buffer of exactly the frame's size, kept while the shape repeats (as _png_buffers)."""
+        n = yuv420_bytes(width, height)
+        if n == 0:
+            raise ValueError(f"no YUV frame of {width}x{height}")
+        cached = getattr(self, "_yuv_cache", None)
+        if cached is None or cached.nbytes < n:
+            cached = pinned_empty((n,))
+            self._yuv_cache = cached
+        return cached[:n]
 
     def render_device(self, frame: Frame, d_out, stream=None) -> None:
         self._check(self._lib.hmrm_render_device(self._h, C.byref(frame), _ptr(d_out), _ptr(stream)))

@@ -26,6 +26,7 @@
 #include "k2_render_lin.cuh"
 #include "k2_render_pack.cuh"
 #include "k3_png.cuh"
+#include "k4_yuv.cuh"
 #include "peer_sync.cuh"
 #include "render_params.h"
 #include "synth_fbm.h"
@@ -131,8 +132,12 @@ struct hmrm_ctx {
 	int slot;                    // buffer of the most recent hmrm_render_async
 	// PNG encoding: scratch per ring slot, allocated by the first PNG frame that uses the slot
 	PngScratch png[kFrameRing];
-	uint8_t *d_png_in;           // hmrm_encode_png's device copy of the caller's pixels
+	uint8_t *d_png_in;           // hmrm_encode_png's / hmrm_convert_yuv420's device copy of the caller's pixels
 	size_t png_in_cap;
+	// YUV frames: the I420 planes K4 writes, per ring slot, allocated by the first YUV frame that uses the slot; the copy
+	// engine moves them to the caller's buffer
+	uint8_t *d_yuv[kFrameRing];
+	size_t yuv_cap[kFrameRing];
 
 	// per-launch resources, used round-robin so that up to kLaunchSlots kernels of this context may be in flight
 	LaunchSlot slots[kLaunchSlots];
@@ -789,7 +794,7 @@ int ensure_png_scratch(hmrm_ctx *c, int slot, const PngShape &s) {
 
 // The address the device writes `p` through: device memory of the context's device as it is, pinned / registered host
 // memory through its mapping.  Pageable memory is refused with a status (the device cannot write it).
-int png_device_view(hmrm_ctx *c, void *p, const char *what, void **dev) {
+int device_view(hmrm_ctx *c, void *p, const char *what, void **dev) {
 	cudaPointerAttributes a;
 	const cudaError_t e = cudaPointerGetAttributes(&a, p);
 	if (e != cudaSuccess) {
@@ -821,8 +826,8 @@ int png_outputs(hmrm_ctx *c, const PngShape &s, uint8_t *png_out, size_t capacit
 		return fail(c, HMRM_ERR_INVALID, "capacity %zu is below hmrm_png_bound = %llu", capacity, bound);
 	HMRM_CUDA(c, cudaSetDevice(c->device));
 	void *o = NULL, *z = NULL;
-	if (int rc = png_device_view(c, png_out, "png_out", &o)) return rc;
-	if (int rc = png_device_view(c, png_bytes, "png_bytes", &z)) return rc;
+	if (int rc = device_view(c, png_out, "png_out", &o)) return rc;
+	if (int rc = device_view(c, png_bytes, "png_bytes", &z)) return rc;
 	*d_out = (uint8_t *)o;
 	*d_size = (unsigned long long *)z;
 	return HMRM_OK;
@@ -845,6 +850,58 @@ int enqueue_png(hmrm_ctx *c, int slot, const uint8_t *d_img, int W, int H, int C
 	const int blocks = (int)std::min((words + 255) / 256, (unsigned long long)c->num_sms * 16ull);
 	k3_png_gather<<<blocks, 256, 0, st>>>(p.offsets, s.nseg + 2, p.meta, p.stage, d_dst, d_size);
 	HMRM_CUDA(c, cudaGetLastError());
+	return HMRM_OK;
+}
+
+// The caller's pixels in the context's staging buffer (hmrm_encode_png, hmrm_convert_yuv420), copied on c->stream.
+// The context must be drained: the buffer may be replaced.
+int stage_pixels(hmrm_ctx *c, const uint8_t *pixels, size_t bytes) {
+	if (bytes > c->png_in_cap) {
+		cudaFree(c->d_png_in);
+		c->d_png_in = NULL;
+		c->png_in_cap = 0;
+		HMRM_CUDA(c, cudaMalloc(&c->d_png_in, bytes));
+		c->png_in_cap = bytes;
+	}
+	HMRM_CUDA(c, cudaMemcpyAsync(c->d_png_in, pixels, bytes, cudaMemcpyDefault, c->stream));
+	return HMRM_OK;
+}
+
+// ---- YUV frames (K4, csrc/k4_yuv.cuh) ------------------------------------------------------------------------------
+int ensure_yuv_scratch(hmrm_ctx *c, int slot, size_t bytes) {
+	if (c->d_yuv[slot] && c->yuv_cap[slot] >= bytes) return HMRM_OK;
+	// the slot's previous YUV frame may still be converting into, or copying out of, the buffer about to be replaced
+	if (c->copy_pending[slot]) HMRM_CUDA(c, cudaEventSynchronize(c->ev_copied[slot]));
+	cudaFree(c->d_yuv[slot]);
+	c->d_yuv[slot] = NULL;
+	c->yuv_cap[slot] = 0;
+	HMRM_CUDA(c, cudaMalloc(&c->d_yuv[slot], bytes));
+	c->yuv_cap[slot] = bytes;
+	return HMRM_OK;
+}
+
+// validates matrix / out / capacity for a W x H frame
+int yuv_output(hmrm_ctx *c, int W, int H, int32_t matrix, uint8_t *out, size_t capacity) {
+	if (matrix != HMRM_YUV_BT601 && matrix != HMRM_YUV_BT709) return fail(c, HMRM_ERR_INVALID, "unknown YUV matrix %d", matrix);
+	if (!out) return fail(c, HMRM_ERR_INVALID, "out is NULL");
+	const unsigned long long need = yuv420_bytes(W, H);
+	if ((unsigned long long)capacity < need)
+		return fail(c, HMRM_ERR_INVALID, "capacity %zu is below hmrm_yuv420_bytes = %llu", capacity, need);
+	HMRM_CUDA(c, cudaSetDevice(c->device));
+	void *unused = NULL;
+	return device_view(c, out, "out", &unused);
+}
+
+// Enqueue K4 on `st`: d_img [H][W][C] -> the slot's planes, then one copy of them to `out` (host or device memory).
+int enqueue_yuv(hmrm_ctx *c, int slot, const uint8_t *d_img, int W, int H, int C, int32_t matrix, uint8_t *out,
+                cudaStream_t st) {
+	const size_t bytes = (size_t)yuv420_bytes(W, H);
+	if (int rc = ensure_yuv_scratch(c, slot, bytes)) return rc;
+	const dim3 grid((unsigned)(((W + 7) / 8 + kYuvThreads - 1) / kYuvThreads), (unsigned)((H + 1) / 2));
+	if (C == 4) k4_yuv420<4><<<grid, kYuvThreads, 0, st>>>(d_img, W, H, kYuvCoef[matrix], c->d_yuv[slot]);
+	else k4_yuv420<3><<<grid, kYuvThreads, 0, st>>>(d_img, W, H, kYuvCoef[matrix], c->d_yuv[slot]);
+	HMRM_CUDA(c, cudaGetLastError());
+	HMRM_CUDA(c, cudaMemcpyAsync(out, c->d_yuv[slot], bytes, cudaMemcpyDefault, st));
 	return HMRM_OK;
 }
 
@@ -954,6 +1011,8 @@ int hmrm_create(int device, hmrm_ctx **out) {
 	std::memset(c->png, 0, sizeof c->png);
 	c->d_png_in = NULL;
 	c->png_in_cap = 0;
+	std::memset(c->d_yuv, 0, sizeof c->d_yuv);
+	std::memset(c->yuv_cap, 0, sizeof c->yuv_cap);
 
 	c->launch_next = c->launch_last = 0;
 	c->last_had_stats = c->last_had_step_index = c->last_had_ray_dump = c->timing_valid = false;
@@ -1002,6 +1061,7 @@ void hmrm_destroy(hmrm_ctx *c) {
 	cudaFree(c->d_png_in);
 	for (int i = 0; i < kFrameRing; ++i) {
 		free_png_scratch(c->png[i]);
+		cudaFree(c->d_yuv[i]);
 		cudaFree(c->d_fb[i]);
 		if (c->ev_rendered[i]) cudaEventDestroy(c->ev_rendered[i]);
 		if (c->ev_copied[i]) cudaEventDestroy(c->ev_copied[i]);
@@ -1371,16 +1431,60 @@ int hmrm_encode_png(hmrm_ctx *c, const uint8_t *pixels, int32_t width, int32_t h
 	if (rc) return rc;
 	// synchronous: whatever the context has in flight finishes first, then ring slot 0's scratch is free
 	if ((rc = drain(c)) != HMRM_OK) return rc;
-	const size_t bytes = (size_t)width * (size_t)height * (size_t)channels;
-	if (bytes > c->png_in_cap) {
-		cudaFree(c->d_png_in);
-		c->d_png_in = NULL;
-		c->png_in_cap = 0;
-		HMRM_CUDA(c, cudaMalloc(&c->d_png_in, bytes));
-		c->png_in_cap = bytes;
-	}
-	HMRM_CUDA(c, cudaMemcpyAsync(c->d_png_in, pixels, bytes, cudaMemcpyDefault, c->stream));
+	if ((rc = stage_pixels(c, pixels, (size_t)width * (size_t)height * (size_t)channels)) != HMRM_OK) return rc;
 	if ((rc = enqueue_png(c, 0, c->d_png_in, width, height, channels, d_out, d_size, c->stream)) != HMRM_OK) return rc;
+	HMRM_CUDA(c, cudaStreamSynchronize(c->stream));
+	return HMRM_OK;
+}
+
+size_t hmrm_yuv420_bytes(int32_t width, int32_t height) { return (size_t)yuv420_bytes(width, height); }
+
+int hmrm_render_yuv420_async(hmrm_ctx *c, const hmrm_frame *f, int32_t matrix, uint8_t *out, size_t capacity) {
+	if (!c) return HMRM_ERR_INVALID;
+	if (!f) return fail(c, HMRM_ERR_INVALID, "frame is NULL");
+	if (f->cycle_period != 1 || f->cycle != 0) return fail(c, HMRM_ERR_INVALID, "YUV frames are whole frames: cycle_period 1");
+	if (f->band_count > 1) return fail(c, HMRM_ERR_INVALID, "YUV frames are whole frames: band_count <= 1");
+	if (f->flags & (HMRM_FLAG_STEP_INDEX | HMRM_FLAG_RAY_DUMP))
+		return fail(c, HMRM_ERR_INVALID, "YUV frames do not record step indices or ray dumps");
+	if (f->row_begin != 0 || (f->row_end != 0 && f->row_end != f->screen_height))
+		return fail(c, HMRM_ERR_INVALID, "YUV frames are whole frames: row_begin 0, row_end 0 or screen_height");
+	if (f->pixel_format != HMRM_PIXEL_RGBA8 && f->pixel_format != HMRM_PIXEL_RGB8)
+		return fail(c, HMRM_ERR_INVALID, "unknown pixel_format %d", (int)f->pixel_format);
+	if (f->screen_width < 2 || f->screen_height < 2 || f->screen_width > 65536 || f->screen_height > 65536)
+		return fail(c, HMRM_ERR_INVALID, "resolution %dx%d outside [2,65536]", f->screen_width, f->screen_height);
+	const int W = f->screen_width, H = f->screen_height, C = f->pixel_format == HMRM_PIXEL_RGB8 ? 3 : 4;
+	int rc = yuv_output(c, W, H, matrix, out, capacity);
+	if (rc) return rc;
+	if ((rc = ensure_framebuffer(c, W, H, f->pixel_format)) != HMRM_OK) return rc;
+	// the ring exactly as hmrm_render_async uses it for whole frames; conversion + copy take the place of the copy-out
+	const int slot = (c->slot + 1) % kFrameRing;
+	if ((rc = ensure_yuv_scratch(c, slot, (size_t)yuv420_bytes(W, H))) != HMRM_OK) return rc;
+	uint32_t *fb = c->d_fb[slot];
+	cudaStream_t cs = c->ring_stream[slot];
+	if (c->copy_pending[slot]) HMRM_CUDA(c, cudaStreamWaitEvent(cs, c->ev_copied[slot], 0));
+	if ((rc = enqueue_render(c, f, fb, cs, true)) != HMRM_OK) return rc;
+	HMRM_CUDA(c, cudaEventRecord(c->ev_rendered[slot], cs));
+	HMRM_CUDA(c, cudaStreamWaitEvent(c->copy_stream, c->ev_rendered[slot], 0));
+	if ((rc = enqueue_yuv(c, slot, (const uint8_t *)fb, W, H, C, matrix, out, c->copy_stream)) != HMRM_OK) return rc;
+	HMRM_CUDA(c, cudaEventRecord(c->ev_copied[slot], c->copy_stream));
+	c->copy_pending[slot] = true;
+	c->slot = slot;
+	return HMRM_OK;
+}
+
+int hmrm_convert_yuv420(hmrm_ctx *c, const uint8_t *pixels, int32_t width, int32_t height, int32_t channels,
+                        int32_t matrix, uint8_t *out, size_t capacity) {
+	if (!c) return HMRM_ERR_INVALID;
+	if (!pixels) return fail(c, HMRM_ERR_INVALID, "pixels is NULL");
+	if (yuv420_bytes(width, height) == 0 || (channels != 3 && channels != 4))
+		return fail(c, HMRM_ERR_INVALID, "image %dx%dx%d: need 1 <= width, height <= 65536 and 3 or 4 channels", width,
+		            height, channels);
+	int rc = yuv_output(c, width, height, matrix, out, capacity);
+	if (rc) return rc;
+	// synchronous: whatever the context has in flight finishes first, then ring slot 0's scratch is free
+	if ((rc = drain(c)) != HMRM_OK) return rc;
+	if ((rc = stage_pixels(c, pixels, (size_t)width * (size_t)height * (size_t)channels)) != HMRM_OK) return rc;
+	if ((rc = enqueue_yuv(c, 0, c->d_png_in, width, height, channels, matrix, out, c->stream)) != HMRM_OK) return rc;
 	HMRM_CUDA(c, cudaStreamSynchronize(c->stream));
 	return HMRM_OK;
 }

@@ -7,6 +7,7 @@
 //   hmap config.txt --headless out.png [--projection 1|2|3] [--precision fp64|fp32]
 //                   [--traversal auto|brute|skip] [--gpus N] [--stats-json file]
 //   hmap config.txt --script frames.txt [--frames N] [--out-prefix P | --record] [--gpus N] ...
+//   hmap config.txt --script frames.txt --video FILE|- [--fps N] [--video-matrix bt601|bt709] ...
 //   hmap config.txt --parse-only                    (grammar check: echo + validation, no GPU)
 //   hmap --decode-image in.png 3|4 out.raw          (image ingest check, no GPU)
 //
@@ -15,6 +16,9 @@
 // (:916-926).  Frame n goes to GPU n mod N, which renders and encodes it into one of four pinned PNG buffers it
 // rotates; the oldest frame of a device is written to its file when that device needs the buffer again.  --record
 // names files as the reference's recorder does (screenshots/hmap_<id>_<n>.png, :1132-1136) and prints its messages.
+// --video writes the frames, in script order, as one YUV4MPEG2 stream of limited-range 4:2:0 planes converted on the
+// device (kernel K4, hmrm_render_yuv420_async): the raw input every video encoder reads.  "-" is stdout, for a pipe
+// into an encoder; the config echo and the messages then go to stderr.
 // --headless with --gpus N > 1 assembles the frame's bands in one pinned host frame and device 0 encodes it.
 // Projection is not part of the grammar (keys 1/2/3 only, :851-868), hence --projection.
 // Headless frames are complete images: cycle_period is forced to 1 (the reference's own advice, :913).
@@ -22,6 +26,7 @@
 #include <cstdlib>
 #include <cstring>
 #include <ctime>
+#include <deque>
 #include <fstream>
 #include <iostream>
 #include <sstream>
@@ -43,25 +48,26 @@ int run_interactive(Config &cfg, hmrm_ctx *ctx, int precision, int traversal);  
 namespace {
 
 struct Options {
-	std::string config_path, headless_out, script_path, out_prefix, stats_json;
-	int projection, precision, traversal, gpus, frames;
+	std::string config_path, headless_out, script_path, out_prefix, stats_json, video_path;
+	int projection, precision, traversal, gpus, frames, fps, video_matrix;
 	bool record, parse_only;
-	Options() : projection(0), precision(HMRM_FP64_EXACT), traversal(HMRM_TRAVERSAL_AUTO), gpus(1), frames(-1),
-	            record(false), parse_only(false) {}
+	Options() : projection(0), precision(HMRM_FP64_EXACT), traversal(HMRM_TRAVERSAL_AUTO), gpus(1), frames(-1), fps(30),
+	            video_matrix(HMRM_YUV_BT709), record(false), parse_only(false) {}
 };
 
 void usage_and_exit() {
 	std::cerr << "USAGE: hmap.exe path/to/config.txt\n";     // main/hmap.cpp:528
 	std::cerr << "       hmap path/to/config.txt --headless out.png [--projection 1|2|3] [--precision fp64|fp32]\n"
 	             "            [--traversal auto|brute|skip] [--gpus N] [--script frames.txt [--frames N]\n"
-	             "            [--out-prefix P | --record]] [--stats-json file] [--parse-only]\n";
+	             "            [--out-prefix P | --record | --video FILE|- [--fps N] [--video-matrix bt601|bt709]]]\n"
+	             "            [--stats-json file] [--parse-only]\n";
 	std::exit(1);
 }
 
-const int kPngInFlight = 4;   // PNG frames one device may have in flight (the library's frame ring)
+const int kPngInFlight = 4;   // PNG or YUV frames one device may have in flight (the library's frame ring)
 
 struct PngBuffer {
-	uint8_t *file;            // pinned, hmrm_png_bound bytes
+	uint8_t *file;            // pinned, hmrm_png_bound bytes (--video: the frame's hmrm_yuv420_bytes of planes)
 	size_t cap;
 	uint64_t *bytes;          // pinned: the file size the device writes
 	int frame_index;
@@ -161,10 +167,11 @@ size_t png_bound_of(const hmrm_frame &f) {
 }
 
 struct Totals {
-	long long frames, rays, box_hits, surf_hits, steps, fetches, png_bytes;
+	long long frames, rays, box_hits, surf_hits, steps, fetches, png_bytes, video_bytes;
 	double kernel_ms;
 	int status;
-	Totals() : frames(0), rays(0), box_hits(0), surf_hits(0), steps(0), fetches(0), png_bytes(0), kernel_ms(0.0), status(0) {}
+	Totals() : frames(0), rays(0), box_hits(0), surf_hits(0), steps(0), fetches(0), png_bytes(0), video_bytes(0),
+	           kernel_ms(0.0), status(0) {}
 };
 
 // SavePNG, main/hmap.cpp:157-168: the file's bytes come from the device encoder
@@ -233,9 +240,22 @@ int main(int argc, char **argv) {
 		else if (a == "--record") opt.record = true;
 		else if (a == "--stats-json" && has_val) opt.stats_json = argv[++i];
 		else if (a == "--parse-only") opt.parse_only = true;
+		else if (a == "--video" && has_val) opt.video_path = argv[++i];
+		else if (a == "--fps" && has_val) opt.fps = std::atoi(argv[++i]);
+		else if (a == "--video-matrix" && has_val) {
+			const std::string v = argv[++i];
+			if (v == "bt601") opt.video_matrix = HMRM_YUV_BT601;
+			else if (v == "bt709") opt.video_matrix = HMRM_YUV_BT709;
+			else usage_and_exit();
+		}
 		else usage_and_exit();
 	}
-	if (opt.projection < 0 || opt.projection > 3 || opt.gpus < 1) usage_and_exit();
+	if (opt.projection < 0 || opt.projection > 3 || opt.gpus < 1 || opt.fps < 1) usage_and_exit();
+	const bool video = !opt.video_path.empty();
+	if (video && (opt.script_path.empty() || !opt.headless_out.empty() || opt.record || !opt.out_prefix.empty()))
+		usage_and_exit();
+	// a video on stdout leaves stdout to the stream
+	std::ostream &msg = opt.video_path == "-" ? std::cerr : std::cout;
 
 	// main/hmap.cpp:534-544
 	std::ifstream input(opt.config_path.c_str());
@@ -244,7 +264,7 @@ int main(int argc, char **argv) {
 		return 1;
 	}
 	Config cfg;
-	if (consume_config_stream(input, cfg, std::cout, std::cerr) != PARSE_OK) return 1;
+	if (consume_config_stream(input, cfg, msg, std::cerr) != PARSE_OK) return 1;
 	input.close();
 	if (opt.parse_only) return 0;
 
@@ -371,41 +391,112 @@ int main(int argc, char **argv) {
 			collect(d, totals);
 			d.stats_pending = false;
 		};
+		// --video: one Y4M stream; frames leave the devices in script order, through one FIFO of the devices of the
+		// frames in flight (each device's own frames are in order in its ring)
+		FILE *vf = NULL;
+		int video_w = 0, video_h = 0;
+		long long video_frames = 0;
+		std::deque<int> video_order;
+		if (video) {
+			vf = opt.video_path == "-" ? stdout : std::fopen(opt.video_path.c_str(), "wb");
+			if (!vf) {
+				std::cerr << "hmap: cannot open " << opt.video_path << " for writing\n";
+				return 1;
+			}
+		}
+		auto video_write = [&](const void *p, size_t n) {
+			if (std::fwrite(p, 1, n, vf) != n) {
+				std::cerr << "hmap: writing the video to " << opt.video_path << " failed\n";
+				std::exit(1);
+			}
+			totals.video_bytes += (long long)n;
+		};
+		auto video_header = [&](int w, int h) {
+			// C420jpeg: the 2x2 box puts chroma at the centre of the block
+			char head[160];
+			const int n = std::snprintf(head, sizeof head, "YUV4MPEG2 W%d H%d F%d:1 Ip A1:1 C420jpeg XCOLORRANGE=LIMITED\n",
+			                            w, h, opt.fps);
+			video_write(head, (size_t)n);
+			video_w = w;
+			video_h = h;
+		};
 		// the oldest frame of the device is complete once at most png_count - 1 newer ones are pending
 		auto retire_oldest = [&](Device &d) {
 			if (hmrm_wait_pending(d.ctx, d.png_count - 1) != HMRM_OK) die_hmrm(d.ctx, "hmrm_wait_pending");
 			const PngBuffer &b = d.png[d.png_head];
-			save_png(b.file, *b.bytes, frame_path(b.frame_index), totals);
+			if (video) {
+				video_write("FRAME\n", 6);
+				video_write(b.file, hmrm_yuv420_bytes(video_w, video_h));
+				video_frames += 1;
+			}
+			else save_png(b.file, *b.bytes, frame_path(b.frame_index), totals);
 			d.png_head = (d.png_head + 1) % kPngInFlight;
 			d.png_count -= 1;
 		};
-		auto drain = [&](Device &d) {
-			collect_pending(d);
-			while (d.png_count > 0) retire_oldest(d);
+		auto retire_first_video_frame = [&]() {
+			const int g = video_order.front();
+			video_order.pop_front();
+			retire_oldest(devs[(size_t)g]);
+		};
+		auto drain_all = [&]() {
+			for (size_t i = 0; i < devs.size(); ++i) collect_pending(devs[i]);
+			if (video) while (!video_order.empty()) retire_first_video_frame();
+			for (size_t i = 0; i < devs.size(); ++i)
+				while (devs[i].png_count > 0) retire_oldest(devs[i]);
 		};
 
 		for (int n = 0; n < n_frames; ++n) {
 			if (n < (int)lines.size()) {
 				std::istringstream iss(lines[(size_t)n]);
-				if (consume_config_stream(iss, cfg, std::cout, std::cerr) != PARSE_OK) return 1;
+				if (consume_config_stream(iss, cfg, msg, std::cerr) != PARSE_OK) return 1;
+			}
+			if (video && n > 0 && (cfg.screen_width != video_w || cfg.screen_height != video_h)) {
+				// the frames before this one stay a valid stream
+				drain_all();
+				std::fflush(vf);
+				if (vf != stdout) std::fclose(vf);
+				std::cerr << "hmap: frame " << n << " changes the resolution from " << video_w << "x" << video_h << " to "
+				          << cfg.screen_width << "x" << cfg.screen_height << "; a Y4M stream has one frame size\n";
+				return 1;
 			}
 			Device &d = devs[(size_t)(n % opt.gpus)];
-			if (d.png_count == kPngInFlight) retire_oldest(d);
+			if (video) {
+				while (d.png_count == kPngInFlight) retire_first_video_frame();
+			}
+			else if (d.png_count == kPngInFlight) retire_oldest(d);
 			if (cfg.maps_changed || cfg.should_update_heightmap) {
-				for (size_t i = 0; i < devs.size(); ++i) drain(devs[i]);
+				drain_all();
 				push_maps(devs, cfg);
 			}
 			collect_pending(d);
 			const hmrm_frame f = make_frame(cfg, opt);
 			PngBuffer &b = d.png[(d.png_head + d.png_count) % kPngInFlight];
-			ensure_png_buffer(b, png_bound_of(f));
-			if (hmrm_render_png_async(d.ctx, &f, b.file, b.cap, b.bytes) != HMRM_OK) die_hmrm(d.ctx, "hmrm_render_png_async");
+			if (video) {
+				if (n == 0) video_header(f.screen_width, f.screen_height);
+				ensure_png_buffer(b, hmrm_yuv420_bytes(f.screen_width, f.screen_height));
+				if (hmrm_render_yuv420_async(d.ctx, &f, opt.video_matrix, b.file, b.cap) != HMRM_OK)
+					die_hmrm(d.ctx, "hmrm_render_yuv420_async");
+				video_order.push_back(n % opt.gpus);
+			}
+			else {
+				ensure_png_buffer(b, png_bound_of(f));
+				if (hmrm_render_png_async(d.ctx, &f, b.file, b.cap, b.bytes) != HMRM_OK)
+					die_hmrm(d.ctx, "hmrm_render_png_async");
+			}
 			b.frame_index = n;
 			d.png_count += 1;
 			d.stats_pending = true;
 		}
-		for (size_t i = 0; i < devs.size(); ++i) drain(devs[i]);
-		std::cout << "Done recording.\n";      // :1142
+		drain_all();
+		if (video) {
+			if (n_frames <= 0) video_header(cfg.screen_width, cfg.screen_height);
+			if (std::fflush(vf) != 0 || (vf != stdout && std::fclose(vf) != 0)) {
+				std::cerr << "hmap: writing the video to " << opt.video_path << " failed\n";
+				return 1;
+			}
+			msg << "Saved video at " << opt.video_path << " (" << video_frames << " frames)\n";
+		}
+		else std::cout << "Done recording.\n";      // :1142
 	}
 
 	if (totals.status & HMRM_ERR_NONTERMINATING)
@@ -417,7 +508,9 @@ int main(int argc, char **argv) {
 		   << ", \"surf_hits\": " << totals.surf_hits << ", \"steps\": " << totals.steps << ", \"fetches\": "
 		   << totals.fetches << ", \"kernel_ms\": " << totals.kernel_ms << ", \"status\": " << totals.status
 		   << ", \"gpus\": " << opt.gpus << ", \"cpu_seconds\": " << (double)(std::clock() - t_start) / CLOCKS_PER_SEC
-		   << ", \"png_bytes\": " << totals.png_bytes << "}\n";
+		   << ", \"png_bytes\": " << totals.png_bytes;
+		if (video) js << ", \"video_bytes\": " << totals.video_bytes;
+		js << "}\n";
 	}
 
 	for (size_t i = 0; i < devs.size(); ++i) {

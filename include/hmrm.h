@@ -170,6 +170,36 @@ int hmrm_render_png_async(hmrm_ctx *ctx, const hmrm_frame *f, uint8_t *png_out, 
 int hmrm_encode_png(hmrm_ctx *ctx, const uint8_t *pixels, int32_t width, int32_t height, int32_t channels,
                     uint8_t *png_out, size_t capacity, uint64_t *png_bytes);
 
+/* ---- 4:2:0 video planes (kernel K4, csrc/k4_yuv.cuh): what every video encoder takes as input ----
+ * Limited-range ("TV range") 8-bit YCbCr.  Coefficients are 2^-14 fixed point: round(k * 2^14 * 219/255) for Y and
+ * round(k * 2^14 * 224/255) for Cb and Cr, with k the matrix's float coefficients:
+ *              Y (R, G, B)           Cb (R, G, B)            Cr (R, G, B)
+ *   BT.601     4207, 8260, 1604      -2428, -4768, 7196      7196, -6026, -1170
+ *   BT.709     2991, 10064, 1016     -1649, -5547, 7196      7196, -6536, -660
+ * Both chroma rows sum to 0: a grey pixel block gives exactly Cb = Cr = 128.
+ *   luma, per pixel:          Y = ((yr R + yg G + yb B + 2^13) >> 14) + 16
+ *   chroma, per 2x2 block:    sample (i, j) covers rows 2i, 2i+1 and columns 2j, 2j+1, indices clamped to H-1 and W-1
+ *                             (odd sizes replicate the last row / column); with SR, SG, SB the sums over those four
+ *                             pixels, Cb = ((cr SR + cg SG + cb SB + 2^15) >> 16) + 128, Cr the same with its own row.
+ *                             >> is an arithmetic shift (floor).
+ * Every output lies in [16, 240], within 0.51 of the float BT.601 / BT.709 value (of the block mean for chroma).
+ * Layout: planar I420 without row padding: Y [H][W], then Cb [ceil(H/2)][ceil(W/2)], then Cr of the same shape.
+ * The 2x2 box puts chroma at the centre of the block (Y4M's C420jpeg siting). */
+#define HMRM_YUV_BT601 0
+#define HMRM_YUV_BT709 1
+/* W*H + 2*ceil(W/2)*ceil(H/2) bytes; 0 outside [1, 65536] per axis.  Host arithmetic, no device work. */
+size_t hmrm_yuv420_bytes(int32_t width, int32_t height);
+/* hmrm_render_async, but the frame leaves the device as I420 planes (HMRM_YUV_* matrix) of the RGBA8 or RGB8 frame.
+ * Whole frames only (cycle_period 1, band_count <= 1, no row band, no STEP_INDEX / RAY_DUMP).  out: pinned / registered
+ * host memory or device memory of ctx's device, capacity >= hmrm_yuv420_bytes; valid once hmrm_wait / hmrm_wait_pending
+ * covers the frame.  Shares the ring with hmrm_render_async and hmrm_render_png_async: up to four frames of any of the
+ * three kinds may be in flight. */
+int hmrm_render_yuv420_async(hmrm_ctx *ctx, const hmrm_frame *f, int32_t matrix, uint8_t *out, size_t capacity);
+/* convert caller pixels ([height][width][channels], channels 3 | 4, host or device memory, copied to the device);
+ * synchronous.  Sizes from 1 to 65536 per axis; out as for hmrm_render_yuv420_async. */
+int hmrm_convert_yuv420(hmrm_ctx *ctx, const uint8_t *pixels, int32_t width, int32_t height, int32_t channels,
+                        int32_t matrix, uint8_t *out, size_t capacity);
+
 int hmrm_get_stats(hmrm_ctx *ctx, hmrm_stats *out);            /* of the last render */
 /* traversal diagnostics of the last HMRM_FLAG_STATS render with a skip traversal: [0] jumps, [1] samples covered
  * by jumps, [2] single steps above a mip block, [3] level descents, [4] cell tests above the cell, [5] cell tests
