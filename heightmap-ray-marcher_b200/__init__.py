@@ -17,6 +17,8 @@ from .binding import (  # noqa: F401
     FLAG_RAY_DUMP,
     FLAG_STATS,
     FLAG_STEP_INDEX,
+    FLAG_SUPERSAMPLE_MASK,
+    FLAG_SUPERSAMPLE_SHIFT,
     LAYOUT_ROWMAJOR,
     LAYOUT_TILE4,
     LAYOUT_ZORDER,
@@ -43,6 +45,7 @@ from .binding import (  # noqa: F401
     load_library,
     pinned_empty,
     png_bound,
+    supersample_flag,
     yuv420_bytes,
 )
 
@@ -51,4 +54,5 @@ __all__ = [
     "get_ray", "png_bound", "yuv420_bytes", "pinned_empty", "PERSPECTIVE", "SPHERICAL", "ORTHOGRAPHIC", "FP64_EXACT", "FP32_FAST", "TRAVERSAL_AUTO",
     "TRAVERSAL_BRUTE", "TRAVERSAL_SKIP", "TRAVERSAL_PACK", "FLAG_STATS", "FLAG_STEP_INDEX", "FLAG_RAY_DUMP", "PIXEL_RGBA8", "PIXEL_RGB8",
     "LAYOUT_ROWMAJOR", "LAYOUT_TILE4", "LAYOUT_ZORDER", "YUV_BT601", "YUV_BT709",
+    "FLAG_SUPERSAMPLE_SHIFT", "FLAG_SUPERSAMPLE_MASK", "supersample_flag",
 ]

@@ -19,6 +19,8 @@ PERSPECTIVE, SPHERICAL, ORTHOGRAPHIC = 1, 2, 3          # main/hmap.cpp:104-106
 FP64_EXACT, FP32_FAST = 0, 1
 TRAVERSAL_AUTO, TRAVERSAL_BRUTE, TRAVERSAL_SKIP, TRAVERSAL_SKIP_FP64, TRAVERSAL_PACK = 0, 1, 2, 3, 4
 FLAG_STATS, FLAG_STEP_INDEX, FLAG_RAY_DUMP = 1, 2, 4
+FLAG_SUPERSAMPLE_SHIFT = 8                               # flags bits 8-11 hold s - 1 (include/hmrm.h)
+FLAG_SUPERSAMPLE_MASK = 15 << FLAG_SUPERSAMPLE_SHIFT
 PIXEL_RGBA8, PIXEL_RGB8 = 0, 1
 LAYOUT_ROWMAJOR, LAYOUT_TILE4, LAYOUT_ZORDER = 0, 1, 2
 YUV_BT601, YUV_BT709 = 0, 1
@@ -181,6 +183,14 @@ def get_ray(frame: Frame, w: float, h: float):
     return tuple(pos), tuple(d)
 
 
+def supersample_flag(s: int) -> int:
+    """The flags bits of supersampling factor s (1..4): HMRM_FLAG_SUPERSAMPLE(s).  The frame stays W x H; each pixel is
+    the box filter of the s x s pixels of the same camera's sW x sH frame."""
+    if not isinstance(s, (int, np.integer)) or isinstance(s, bool) or not 1 <= int(s) <= 4:
+        raise ValueError(f"supersample factor {s!r} is not one of 1, 2, 3, 4")
+    return (int(s) - 1) << FLAG_SUPERSAMPLE_SHIFT
+
+
 def png_bound(width: int, height: int, channels: int) -> int:
     """Worst-case PNG file size of a width x height x channels (3 | 4) frame (hmrm_png_bound); 0 for other shapes."""
     return int(load_library().hmrm_png_bound(int(width), int(height), int(channels)))
@@ -325,7 +335,9 @@ class Renderer:
         return out
 
     # -- render ---------------------------------------------------------------------------
-    def frame(self, **overrides) -> Frame:
+    def frame(self, supersample: int | None = None, **overrides) -> Frame:
+        """The hmrm_frame of the current attributes; `overrides` set Frame fields, `supersample` (1..4) the
+        supersampling bits of its flags (the output size stays screen_width x screen_height)."""
         f = Frame()
         f.projection = self.image_plane
         f.screen_width, f.screen_height = self.screen_width, self.screen_height
@@ -341,6 +353,8 @@ class Renderer:
                 getattr(f, k)[:] = list(v)
             else:
                 setattr(f, k, v)
+        if supersample is not None:
+            f.flags = (f.flags & ~FLAG_SUPERSAMPLE_MASK) | supersample_flag(supersample)
         return f
 
     def render(self, frame: Frame | None = None, out: np.ndarray | None = None, **overrides) -> np.ndarray:

@@ -27,6 +27,7 @@
 #include "k2_render_pack.cuh"
 #include "k3_png.cuh"
 #include "k4_yuv.cuh"
+#include "k5_downsample.cuh"
 #include "peer_sync.cuh"
 #include "render_params.h"
 #include "synth_fbm.h"
@@ -39,6 +40,7 @@ std::string g_create_error;
 
 const int kLaunchSlots = 8;
 const int kFrameRing = 4;      // device frame buffers (and compute streams) whole frames rotate through
+const int kSubFrames = 4;      // supersampled sub-frame scratches, used round-robin
 
 // Everything one launch writes before / while its kernel runs.  A slot is reused only after the kernel that used
 // it last has finished (ev_end), so up to kLaunchSlots frames of one context may be in flight on any streams.
@@ -69,6 +71,15 @@ struct PngScratch {
 	unsigned long long *offsets;
 	unsigned long long filt_cap;  // bytes of filtered stream
 	int seg_cap;                  // segments
+};
+
+// The sW x sH RGBA8 render of a supersampled frame, read by K5.  It is reused only after the filter that read it last has
+// run (ev_read), so up to kSubFrames supersampled frames of one context may be in flight on any streams.
+struct SubFrame {
+	uint32_t *d;
+	size_t cap;                   // bytes
+	cudaEvent_t ev_read;
+	bool used;
 };
 
 } // namespace
@@ -138,6 +149,9 @@ struct hmrm_ctx {
 	// engine moves them to the caller's buffer
 	uint8_t *d_yuv[kFrameRing];
 	size_t yuv_cap[kFrameRing];
+	// supersampled frames (K5): sub-frame scratches, allocated by the first supersampled frame that uses them
+	SubFrame sub[kSubFrames];
+	int sub_next;
 
 	// per-launch resources, used round-robin so that up to kLaunchSlots kernels of this context may be in flight
 	LaunchSlot slots[kLaunchSlots];
@@ -206,6 +220,10 @@ int drain(hmrm_ctx *c) {
 	// kernels launched on the caller's streams (hmrm_render_device) are tracked by their slot's end event
 	for (int i = 0; i < kLaunchSlots; ++i) {
 		if (c->slots[i].used) HMRM_CUDA(c, cudaEventSynchronize(c->slots[i].ev_end));
+	}
+	// and so are the box filters that follow them
+	for (int i = 0; i < kSubFrames; ++i) {
+		if (c->sub[i].used) HMRM_CUDA(c, cudaEventSynchronize(c->sub[i].ev_read));
 	}
 	return HMRM_OK;
 }
@@ -664,6 +682,77 @@ int enqueue_render(hmrm_ctx *c, const hmrm_frame *f, uint32_t *d_out, cudaStream
 	return HMRM_OK;
 }
 
+// ---- supersampled frames (K5, csrc/k5_downsample.cuh) --------------------------------------------------------------
+int supersample_of(const hmrm_frame *f) {
+	return (int)((f->flags & HMRM_FLAG_SUPERSAMPLE_MASK) >> HMRM_FLAG_SUPERSAMPLE_SHIFT) + 1;
+}
+
+// The supersample field of a frame for the entry points that accept it: s = 1..4, and s > 1 for whole frames only.
+int check_supersample(hmrm_ctx *c, const hmrm_frame *f) {
+	const int s = supersample_of(f);
+	if (s > 4) return fail(c, HMRM_ERR_INVALID, "supersample factor %d: the field (flags bits 8-11) holds s - 1 <= 3", s);
+	if (s == 1) return HMRM_OK;
+	if ((long long)s * f->screen_width > 65536 || (long long)s * f->screen_height > 65536)
+		return fail(c, HMRM_ERR_INVALID, "supersample %d of %dx%d: the sub-frame is larger than 65536 per axis", s,
+		            f->screen_width, f->screen_height);
+	if (f->cycle_period != 1 || f->cycle != 0)
+		return fail(c, HMRM_ERR_INVALID, "supersampled frames are whole frames: cycle_period 1");
+	if (f->band_count > 1) return fail(c, HMRM_ERR_INVALID, "supersampled frames are whole frames: band_count <= 1");
+	if (f->row_begin != 0 || (f->row_end != 0 && f->row_end != f->screen_height))
+		return fail(c, HMRM_ERR_INVALID, "supersampled frames are whole frames: row_begin 0, row_end 0 or screen_height");
+	if (f->flags & (HMRM_FLAG_STEP_INDEX | HMRM_FLAG_RAY_DUMP))
+		return fail(c, HMRM_ERR_INVALID, "supersampled frames do not record step indices or ray dumps");
+	return HMRM_OK;
+}
+
+// Enqueue one whole frame on `stream` into d_out in the frame's pixel format: enqueue_render for s = 1; for s > 1 the
+// sW x sH RGBA8 sub-frame is rendered into a sub-frame scratch and K5 box-filters it into d_out on the same stream.
+int enqueue_frame(hmrm_ctx *c, const hmrm_frame *f, uint32_t *d_out, cudaStream_t stream) {
+	if (int rc = check_supersample(c, f)) return rc;
+	const int s = supersample_of(f);
+	if (s == 1) return enqueue_render(c, f, d_out, stream, true);
+	const int W = f->screen_width, H = f->screen_height;
+	hmrm_frame sf = *f;
+	sf.screen_width = s * W;
+	sf.screen_height = s * H;
+	sf.pixel_format = HMRM_PIXEL_RGBA8;
+	sf.flags &= ~HMRM_FLAG_SUPERSAMPLE_MASK;
+	sf.row_begin = sf.row_end = 0;
+	int row_begin = 0, row_end = 0;
+	if (int rc = validate_frame(c, &sf, &row_begin, &row_end)) return rc;
+	HMRM_CUDA(c, cudaSetDevice(c->device));
+
+	// take a scratch; wait (host side) for the filter that read it kSubFrames supersampled frames ago
+	SubFrame &b = c->sub[c->sub_next];
+	c->sub_next = (c->sub_next + 1) % kSubFrames;
+	if (b.used) HMRM_CUDA(c, cudaEventSynchronize(b.ev_read));
+	const size_t need = (size_t)sf.screen_width * (size_t)sf.screen_height * 4;
+	if (need > b.cap) {
+		cudaFree(b.d);
+		b.d = NULL;
+		b.cap = 0;
+		HMRM_CUDA(c, cudaMalloc(&b.d, need));
+		b.cap = need;
+	}
+	if (int rc = enqueue_render(c, &sf, b.d, stream, true)) return rc;
+	const dim3 grid((unsigned)(((W + kDownStrip - 1) / kDownStrip + kDownThreads - 1) / kDownThreads), (unsigned)H);
+	uint8_t *out = (uint8_t *)d_out;
+	const bool rgb8 = f->pixel_format == HMRM_PIXEL_RGB8;
+#define HMRM_LAUNCH_K5(S)                                                                                  \
+	do {                                                                                                   \
+		if (rgb8) k5_downsample<S, 3><<<grid, kDownThreads, 0, stream>>>(b.d, W, H, out);                  \
+		else k5_downsample<S, 4><<<grid, kDownThreads, 0, stream>>>(b.d, W, H, out);                      \
+	} while (0)
+	if (s == 2) HMRM_LAUNCH_K5(2);
+	else if (s == 3) HMRM_LAUNCH_K5(3);
+	else HMRM_LAUNCH_K5(4);
+#undef HMRM_LAUNCH_K5
+	HMRM_CUDA(c, cudaGetLastError());
+	HMRM_CUDA(c, cudaEventRecord(b.ev_read, stream));
+	b.used = true;
+	return HMRM_OK;
+}
+
 // D2H of what one launch rendered: rows [rb, re), or with band_count > 1 only the tile rows of that band (several
 // ranks may fill one shared, registered host frame, each over its own PCIe link): one strided copy + the ragged last
 // tile row.  Enqueued on the copy stream.
@@ -1013,6 +1102,8 @@ int hmrm_create(int device, hmrm_ctx **out) {
 	c->png_in_cap = 0;
 	std::memset(c->d_yuv, 0, sizeof c->d_yuv);
 	std::memset(c->yuv_cap, 0, sizeof c->yuv_cap);
+	std::memset(c->sub, 0, sizeof c->sub);
+	c->sub_next = 0;
 
 	c->launch_next = c->launch_last = 0;
 	c->last_had_stats = c->last_had_step_index = c->last_had_ray_dump = c->timing_valid = false;
@@ -1033,6 +1124,8 @@ int hmrm_create(int device, hmrm_ctx **out) {
 		if (err == cudaSuccess) err = cudaMalloc(&c->slots[i].d_stats, sizeof(DeviceStats));
 		if (err == cudaSuccess) err = cudaMalloc(&c->slots[i].d_tile_counter, 256);
 	}
+	for (int i = 0; i < kSubFrames && err == cudaSuccess; ++i)
+		err = cudaEventCreateWithFlags(&c->sub[i].ev_read, cudaEventDisableTiming);
 	if (err == cudaSuccess) err = cudaMalloc(&c->d_max_bits, 32);
 	if (err == cudaSuccess) err = cudaMalloc(&c->d_k1_counter, 256);
 	if (err == cudaSuccess) err = cudaMemset(c->d_k1_counter, 0, 256);
@@ -1067,6 +1160,12 @@ void hmrm_destroy(hmrm_ctx *c) {
 		if (c->ev_copied[i]) cudaEventDestroy(c->ev_copied[i]);
 	}
 	if (c->copy_stream) cudaStreamDestroy(c->copy_stream);
+	for (int i = 0; i < kSubFrames; ++i) {
+		SubFrame &b = c->sub[i];
+		if (b.used) cudaEventSynchronize(b.ev_read);      // a filter on a caller's stream may still read it
+		cudaFree(b.d);
+		if (b.ev_read) cudaEventDestroy(b.ev_read);
+	}
 	for (int i = 0; i < kLaunchSlots; ++i) {
 		LaunchSlot &sl = c->slots[i];
 		cudaFree(sl.d_step_index);
@@ -1293,13 +1392,15 @@ void hmrm_frame_defaults(hmrm_frame *f) {
 int hmrm_render_device(hmrm_ctx *c, const hmrm_frame *f, void *d_rgba_out, void *stream) {
 	if (!c) return HMRM_ERR_INVALID;
 	if (!d_rgba_out) return fail(c, HMRM_ERR_INVALID, "d_rgba_out is NULL");
-	return enqueue_render(c, f, (uint32_t *)d_rgba_out, stream ? (cudaStream_t)stream : c->stream, true);
+	if (!f) return fail(c, HMRM_ERR_INVALID, "frame is NULL");
+	return enqueue_frame(c, f, (uint32_t *)d_rgba_out, stream ? (cudaStream_t)stream : c->stream);
 }
 
 int hmrm_render_async(hmrm_ctx *c, const hmrm_frame *f, uint8_t *rgba_out) {
 	if (!c) return HMRM_ERR_INVALID;
 	if (!f) return fail(c, HMRM_ERR_INVALID, "frame is NULL");
 	if (!rgba_out) return fail(c, HMRM_ERR_INVALID, "rgba_out is NULL");
+	if (int rc = check_supersample(c, f)) return rc;
 	if (f->screen_width < 2 || f->screen_height < 2 || f->screen_width > 65536 || f->screen_height > 65536)
 		return fail(c, HMRM_ERR_INVALID, "resolution %dx%d outside [2,65536]", f->screen_width, f->screen_height);
 	HMRM_CUDA(c, cudaSetDevice(c->device));
@@ -1333,7 +1434,7 @@ int hmrm_render_async(hmrm_ctx *c, const hmrm_frame *f, uint8_t *rgba_out) {
 	// (Rendering a frame that finds the pipeline idle as four interleaved bands, each copied out as soon as its kernel
 	// is done, was measured: four launches mean four tails, the stream turns kernel-bound and stays "idle", 0.59 ->
 	// 0.63 ms per frame.  Frames stay whole.)
-	rc = enqueue_render(c, f, fb, cs, true);
+	rc = enqueue_frame(c, f, fb, cs);
 	if (rc) return rc;
 	HMRM_CUDA(c, cudaEventRecord(c->ev_rendered[slot], cs));
 	HMRM_CUDA(c, cudaStreamWaitEvent(c->copy_stream, c->ev_rendered[slot], 0));
@@ -1382,6 +1483,7 @@ size_t hmrm_png_bound(int32_t width, int32_t height, int32_t channels) {
 int hmrm_render_png_async(hmrm_ctx *c, const hmrm_frame *f, uint8_t *png_out, size_t capacity, uint64_t *png_bytes) {
 	if (!c) return HMRM_ERR_INVALID;
 	if (!f) return fail(c, HMRM_ERR_INVALID, "frame is NULL");
+	if (int rc = check_supersample(c, f)) return rc;
 	if (f->cycle_period != 1 || f->cycle != 0) return fail(c, HMRM_ERR_INVALID, "PNG frames are whole frames: cycle_period 1");
 	if (f->band_count > 1) return fail(c, HMRM_ERR_INVALID, "PNG frames are whole frames: band_count <= 1");
 	if (f->flags & (HMRM_FLAG_STEP_INDEX | HMRM_FLAG_RAY_DUMP))
@@ -1406,7 +1508,7 @@ int hmrm_render_png_async(hmrm_ctx *c, const hmrm_frame *f, uint8_t *png_out, si
 	uint32_t *fb = c->d_fb[slot];
 	cudaStream_t cs = c->ring_stream[slot];
 	if (c->copy_pending[slot]) HMRM_CUDA(c, cudaStreamWaitEvent(cs, c->ev_copied[slot], 0));
-	if ((rc = enqueue_render(c, f, fb, cs, true)) != HMRM_OK) return rc;
+	if ((rc = enqueue_frame(c, f, fb, cs)) != HMRM_OK) return rc;
 	HMRM_CUDA(c, cudaEventRecord(c->ev_rendered[slot], cs));
 	HMRM_CUDA(c, cudaStreamWaitEvent(c->copy_stream, c->ev_rendered[slot], 0));
 	rc = enqueue_png(c, slot, (const uint8_t *)fb, f->screen_width, f->screen_height, C, d_out, d_size, c->copy_stream);
@@ -1442,6 +1544,7 @@ size_t hmrm_yuv420_bytes(int32_t width, int32_t height) { return (size_t)yuv420_
 int hmrm_render_yuv420_async(hmrm_ctx *c, const hmrm_frame *f, int32_t matrix, uint8_t *out, size_t capacity) {
 	if (!c) return HMRM_ERR_INVALID;
 	if (!f) return fail(c, HMRM_ERR_INVALID, "frame is NULL");
+	if (int rc = check_supersample(c, f)) return rc;
 	if (f->cycle_period != 1 || f->cycle != 0) return fail(c, HMRM_ERR_INVALID, "YUV frames are whole frames: cycle_period 1");
 	if (f->band_count > 1) return fail(c, HMRM_ERR_INVALID, "YUV frames are whole frames: band_count <= 1");
 	if (f->flags & (HMRM_FLAG_STEP_INDEX | HMRM_FLAG_RAY_DUMP))
@@ -1462,7 +1565,7 @@ int hmrm_render_yuv420_async(hmrm_ctx *c, const hmrm_frame *f, int32_t matrix, u
 	uint32_t *fb = c->d_fb[slot];
 	cudaStream_t cs = c->ring_stream[slot];
 	if (c->copy_pending[slot]) HMRM_CUDA(c, cudaStreamWaitEvent(cs, c->ev_copied[slot], 0));
-	if ((rc = enqueue_render(c, f, fb, cs, true)) != HMRM_OK) return rc;
+	if ((rc = enqueue_frame(c, f, fb, cs)) != HMRM_OK) return rc;
 	HMRM_CUDA(c, cudaEventRecord(c->ev_rendered[slot], cs));
 	HMRM_CUDA(c, cudaStreamWaitEvent(c->copy_stream, c->ev_rendered[slot], 0));
 	if ((rc = enqueue_yuv(c, slot, (const uint8_t *)fb, W, H, C, matrix, out, c->copy_stream)) != HMRM_OK) return rc;
@@ -1675,6 +1778,7 @@ int hmrm_ipc_open(hmrm_ctx *c, const uint8_t handle[HMRM_IPC_HANDLE_BYTES], void
 int hmrm_render_peer(hmrm_ctx *c, const hmrm_frame *f, void *d_frame, void *d_ctrl, uint32_t use, void *stream) {
 	if (!c) return HMRM_ERR_INVALID;
 	if (!d_frame || !d_ctrl || use == 0u) return fail(c, HMRM_ERR_INVALID, "hmrm_render_peer: bad arguments");
+	if (f && supersample_of(f) != 1) return fail(c, HMRM_ERR_INVALID, "peer frames are band-split: no supersampling");
 	HMRM_CUDA(c, cudaSetDevice(c->device));
 	cudaStream_t s = stream ? (cudaStream_t)stream : c->stream;
 	PeerCtrl *ctrl = (PeerCtrl *)d_ctrl;
@@ -1690,6 +1794,7 @@ int hmrm_render_peer_staged(hmrm_ctx *c, const hmrm_frame *f, void *d_stage, voi
                             void *stream) {
 	if (!c) return HMRM_ERR_INVALID;
 	if (!d_stage || !d_frame || !d_ctrl || use == 0u) return fail(c, HMRM_ERR_INVALID, "hmrm_render_peer_staged: bad arguments");
+	if (f && supersample_of(f) != 1) return fail(c, HMRM_ERR_INVALID, "peer frames are band-split: no supersampling");
 	HMRM_CUDA(c, cudaSetDevice(c->device));
 	cudaStream_t s = stream ? (cudaStream_t)stream : c->stream;
 	PeerCtrl *ctrl = (PeerCtrl *)d_ctrl;

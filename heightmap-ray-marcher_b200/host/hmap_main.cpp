@@ -8,6 +8,7 @@
 //                   [--traversal auto|brute|skip] [--gpus N] [--stats-json file]
 //   hmap config.txt --script frames.txt [--frames N] [--out-prefix P | --record] [--gpus N] ...
 //   hmap config.txt --script frames.txt --video FILE|- [--fps N] [--video-matrix bt601|bt709] ...
+//   ... [--supersample 1|2|3|4]                    (anti-aliasing: the box filter of an N x N-times larger frame)
 //   hmap config.txt --parse-only                    (grammar check: echo + validation, no GPU)
 //   hmap --decode-image in.png 3|4 out.raw          (image ingest check, no GPU)
 //
@@ -21,6 +22,9 @@
 // into an encoder; the config echo and the messages then go to stderr.
 // --headless with --gpus N > 1 assembles the frame's bands in one pinned host frame and device 0 encodes it.
 // Projection is not part of the grammar (keys 1/2/3 only, :851-868), hence --projection.
+// --supersample N renders every headless, recorded or video frame at N x N rays per pixel and box-filters it on the
+// device (HMRM_FLAG_SUPERSAMPLE, kernel K5); the files keep the configured resolution.  Supersampled frames are whole
+// frames, so --headless over several devices (tile-row bands) refuses N > 1; --script still deals whole frames to them.
 // Headless frames are complete images: cycle_period is forced to 1 (the reference's own advice, :913).
 #include <cstdio>
 #include <cstdlib>
@@ -49,10 +53,10 @@ namespace {
 
 struct Options {
 	std::string config_path, headless_out, script_path, out_prefix, stats_json, video_path;
-	int projection, precision, traversal, gpus, frames, fps, video_matrix;
-	bool record, parse_only;
+	int projection, precision, traversal, gpus, frames, fps, video_matrix, supersample;
+	bool record, parse_only, supersample_given;
 	Options() : projection(0), precision(HMRM_FP64_EXACT), traversal(HMRM_TRAVERSAL_AUTO), gpus(1), frames(-1), fps(30),
-	            video_matrix(HMRM_YUV_BT709), record(false), parse_only(false) {}
+	            video_matrix(HMRM_YUV_BT709), supersample(1), record(false), parse_only(false), supersample_given(false) {}
 };
 
 void usage_and_exit() {
@@ -60,7 +64,7 @@ void usage_and_exit() {
 	std::cerr << "       hmap path/to/config.txt --headless out.png [--projection 1|2|3] [--precision fp64|fp32]\n"
 	             "            [--traversal auto|brute|skip] [--gpus N] [--script frames.txt [--frames N]\n"
 	             "            [--out-prefix P | --record | --video FILE|- [--fps N] [--video-matrix bt601|bt709]]]\n"
-	             "            [--stats-json file] [--parse-only]\n";
+	             "            [--supersample 1|2|3|4] [--stats-json file] [--parse-only]\n";
 	std::exit(1);
 }
 
@@ -130,6 +134,7 @@ hmrm_frame make_frame(const Config &cfg, const Options &opt) {
 	f.traversal = opt.traversal;
 	// counting costs per-warp atomics: only when the caller asked for the numbers (the cut-off status is always reported)
 	f.flags = opt.stats_json.empty() ? 0u : HMRM_FLAG_STATS;
+	f.flags |= HMRM_FLAG_SUPERSAMPLE(opt.supersample);
 	return f;
 }
 
@@ -242,6 +247,10 @@ int main(int argc, char **argv) {
 		else if (a == "--parse-only") opt.parse_only = true;
 		else if (a == "--video" && has_val) opt.video_path = argv[++i];
 		else if (a == "--fps" && has_val) opt.fps = std::atoi(argv[++i]);
+		else if (a == "--supersample" && has_val) {
+			opt.supersample = std::atoi(argv[++i]);
+			opt.supersample_given = true;
+		}
 		else if (a == "--video-matrix" && has_val) {
 			const std::string v = argv[++i];
 			if (v == "bt601") opt.video_matrix = HMRM_YUV_BT601;
@@ -251,6 +260,9 @@ int main(int argc, char **argv) {
 		else usage_and_exit();
 	}
 	if (opt.projection < 0 || opt.projection > 3 || opt.gpus < 1 || opt.fps < 1) usage_and_exit();
+	if (opt.supersample < 1 || opt.supersample > 4) usage_and_exit();
+	// one frame over several devices is dealt in tile-row bands, which supersampled frames are not
+	if (opt.supersample > 1 && !opt.headless_out.empty() && opt.script_path.empty() && opt.gpus > 1) usage_and_exit();
 	const bool video = !opt.video_path.empty();
 	if (video && (opt.script_path.empty() || !opt.headless_out.empty() || opt.record || !opt.out_prefix.empty()))
 		usage_and_exit();
@@ -510,6 +522,7 @@ int main(int argc, char **argv) {
 		   << ", \"gpus\": " << opt.gpus << ", \"cpu_seconds\": " << (double)(std::clock() - t_start) / CLOCKS_PER_SEC
 		   << ", \"png_bytes\": " << totals.png_bytes;
 		if (video) js << ", \"video_bytes\": " << totals.video_bytes;
+		if (opt.supersample_given) js << ", \"supersample\": " << opt.supersample;
 		js << "}\n";
 	}
 

@@ -49,6 +49,22 @@ extern "C" {
 #define HMRM_FLAG_STATS      1u  /* count rays / steps / fetches (hmrm_get_stats) */
 #define HMRM_FLAG_STEP_INDEX 2u  /* record the per-pixel first-hit step index (hmrm_get_step_index) */
 #define HMRM_FLAG_RAY_DUMP   4u  /* record the device's ray / slab distance / entry point per pixel (hmrm_get_ray_dump) */
+/* Supersampling (kernel K5, csrc/k5_downsample.cuh): bits 8-11 hold s - 1, s = 1..4 (0 = one ray per pixel, the
+ * reference's frame).  screen_width x screen_height (W x H) stays the OUTPUT size: every buffer, bound and shape is the
+ * one of the 1x frame.  A frame with factor s is the box filter of the reference's frame of the same camera at sW x sH:
+ *   subsample (s px + i, s py + j), 0 <= i, j < s, is pixel (s px + i, s py + j) of that sW x sH frame (bit-exact to the
+ *   reference, as every render here is);
+ *   each of R, G, B = (sum + s*s/2) / (s*s) in integers (floor division; s*s/2 = 0, 2, 4, 8 for s = 1..4), with the sum
+ *   of that channel over the s*s subsamples;  A = 255.
+ * The subsample rays come from the sW x sH image plane (w = x / (sW - 1)), not jittered around the 1x pixel centres.
+ * Accepted by hmrm_render, hmrm_render_async, hmrm_render_device, hmrm_render_png_async and hmrm_render_yuv420_async,
+ * for whole frames only: s > 1 with cycle_period != 1, band_count > 1, a partial row band, HMRM_FLAG_STEP_INDEX or
+ * HMRM_FLAG_RAY_DUMP, sW or sH above 65536, a field value above 3, or any s > 1 passed to hmrm_render_peer /
+ * hmrm_render_peer_staged is HMRM_ERR_INVALID.  With HMRM_FLAG_STATS, hmrm_get_stats describes the sW x sH render
+ * (rays = s*s*W*H; kernel_ms of the render kernel alone). */
+#define HMRM_FLAG_SUPERSAMPLE_SHIFT 8
+#define HMRM_FLAG_SUPERSAMPLE_MASK  (15u << HMRM_FLAG_SUPERSAMPLE_SHIFT)
+#define HMRM_FLAG_SUPERSAMPLE(s)    ((uint32_t)((s) - 1) << HMRM_FLAG_SUPERSAMPLE_SHIFT)   /* s = 1..4 */
 
 /* hmrm_frame.pixel_format: layout of the frame the render calls write */
 #define HMRM_PIXEL_RGBA8 0       /* the reference's framebuf: [H][W][4], A = 255 (main/hmap.cpp:139-154) */
