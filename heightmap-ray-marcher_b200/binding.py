@@ -87,6 +87,9 @@ PROTOTYPES = {
     "hmrm_set_maps_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32]),
     "hmrm_synth_maps": (C.c_int, [C.c_void_p, C.c_uint32, C.c_uint32]),
     "hmrm_get_maps": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p]),
+    "hmrm_set_maps16": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32]),
+    "hmrm_set_maps16_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32]),
+    "hmrm_synth_maps16": (C.c_int, [C.c_void_p, C.c_uint32, C.c_uint32]),
     "hmrm_set_layout": (C.c_int, [C.c_void_p, C.c_int]),
     "hmrm_get_layout": (C.c_int, [C.c_void_p]),
     "hmrm_update_heightmap": (C.c_int, [C.c_void_p, C.POINTER(C.c_double), C.c_double, C.c_double]),
@@ -306,6 +309,30 @@ class Renderer:
     def synth_maps(self, log2n: int, seed: int = 1234) -> None:
         """Synthetic fBm maps of size 2^log2n generated on the device (csrc/synth_fbm.h)."""
         self._check(self._lib.hmrm_synth_maps(self._h, log2n, seed))
+        self.map_height = self.map_width = 1 << log2n
+        self.update_heightmap()
+
+    def set_maps16(self, height_u16: np.ndarray, color_rgba8: np.ndarray) -> None:
+        """16-bit height samples [H,W] (used as R = G = B on the 0..65535 scale, include/hmrm.h) and the colormap."""
+        hm = np.ascontiguousarray(height_u16, dtype=np.uint16)
+        cm = np.ascontiguousarray(color_rgba8, dtype=np.uint8)
+        if hm.ndim != 2 or cm.ndim != 3 or cm.shape[2] != 4:
+            raise ValueError("height map must be [H,W] uint16 and colormap [H,W,4] uint8")
+        if hm.shape != cm.shape[:2]:
+            raise ValueError(f"heightmap dimensions ({hm.shape[1]}x{hm.shape[0]}) must match colormap "
+                             f"dimensions ({cm.shape[1]}x{cm.shape[0]})")
+        self._check(self._lib.hmrm_set_maps16(self._h, hm.ctypes.data, cm.ctypes.data, hm.shape[1], hm.shape[0]))
+        self.map_height, self.map_width = hm.shape
+        self.update_heightmap()
+
+    def set_maps16_device(self, d_height_u16, d_color_rgba8, width: int, height: int) -> None:
+        self._check(self._lib.hmrm_set_maps16_device(self._h, _ptr(d_height_u16), _ptr(d_color_rgba8), width, height))
+        self.map_height, self.map_width = height, width
+        self.update_heightmap()
+
+    def synth_maps16(self, log2n: int, seed: int = 1234) -> None:
+        """Synthetic 16-bit fBm height (hmrm_synth_height16) with synth_maps' colormap, generated on the device."""
+        self._check(self._lib.hmrm_synth_maps16(self._h, log2n, seed))
         self.map_height = self.map_width = 1 << log2n
         self.update_heightmap()
 

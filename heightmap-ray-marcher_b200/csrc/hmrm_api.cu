@@ -106,7 +106,8 @@ struct hmrm_ctx {
 
 	// maps
 	int map_w, map_h;
-	uint8_t *d_rgb;              // RGB8 [map_h][map_w][3]
+	uint8_t *d_rgb;              // RGB8 [map_h][map_w][3], or with height_bits 16 the u16 plane [map_h][map_w] (2n <= 3n bytes)
+	int height_bits;             // 8 (hmrm_set_maps, hmrm_synth_maps) or 16 (hmrm_set_maps16, hmrm_synth_maps16)
 	uint32_t *d_color;           // RGBA8
 	double *d_surf;              // fl(height + min_height)
 	unsigned long long *d_max_bits;  // [0] max, [1] min of surf (order-preserving bits); [2] quantiser error flag
@@ -195,6 +196,19 @@ __global__ void __launch_bounds__(256) k_synth_maps(uint32_t log2n, uint32_t see
 		rgb[3ULL * p + 1] = (uint8_t)v;
 		rgb[3ULL * p + 2] = (uint8_t)v;
 		rgba[p] = hmrm_synth_color(v, x, y, n);
+	}
+}
+
+// 16-bit height plane and the colormap of hmrm_synth_maps (the same seed gives the same colours)
+__global__ void __launch_bounds__(256) k_synth_maps16(uint32_t log2n, uint32_t seed, uint16_t *__restrict__ h16,
+                                                      uint32_t *__restrict__ rgba) {
+	const uint32_t n = 1u << log2n;
+	const unsigned long long total = (unsigned long long)n * n;
+	const unsigned long long stride = (unsigned long long)gridDim.x * blockDim.x;
+	for (unsigned long long p = (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x; p < total; p += stride) {
+		const uint32_t x = (uint32_t)(p & (n - 1u)), y = (uint32_t)(p >> log2n);
+		h16[p] = (uint16_t)hmrm_synth_height16(x, y, log2n, seed);
+		rgba[p] = hmrm_synth_color(hmrm_synth_height(x, y, log2n, seed), x, y, n);
 	}
 }
 
@@ -1069,6 +1083,7 @@ int hmrm_create(int device, hmrm_ctx **out) {
 	c->last_stream = NULL;
 	c->map_w = c->map_h = 0;
 	c->d_rgb = NULL;
+	c->height_bits = 8;
 	c->d_color = NULL;
 	c->d_surf = NULL;
 	c->d_max_bits = NULL;
@@ -1184,30 +1199,43 @@ void hmrm_destroy(hmrm_ctx *c) {
 	delete c;
 }
 
-int hmrm_set_maps(hmrm_ctx *c, const uint8_t *height_rgb8, const uint8_t *color_rgba8, int32_t w, int32_t h) {
-	if (!c) return HMRM_ERR_INVALID;
-	if (!height_rgb8 || !color_rgba8) return fail(c, HMRM_ERR_INVALID, "map pointers must not be NULL");
+namespace {
+
+// hmrm_set_maps* : height (RGB8, or u16 with bits 16) and colormap from host or device memory
+int upload_maps(hmrm_ctx *c, const void *height, const void *color_rgba8, int32_t w, int32_t h, int bits,
+                cudaMemcpyKind kind) {
+	if (!height || !color_rgba8) return fail(c, HMRM_ERR_INVALID, "map pointers must not be NULL");
 	int rc = alloc_maps(c, w, h);
 	if (rc) return rc;
 	const size_t n = (size_t)w * (size_t)h;
-	HMRM_CUDA(c, cudaMemcpyAsync(c->d_rgb, height_rgb8, n * 3, cudaMemcpyHostToDevice, c->stream));
-	HMRM_CUDA(c, cudaMemcpyAsync(c->d_color, color_rgba8, n * 4, cudaMemcpyHostToDevice, c->stream));
+	HMRM_CUDA(c, cudaMemcpyAsync(c->d_rgb, height, n * (bits == 16 ? 2 : 3), kind, c->stream));
+	HMRM_CUDA(c, cudaMemcpyAsync(c->d_color, color_rgba8, n * 4, kind, c->stream));
 	HMRM_CUDA(c, cudaStreamSynchronize(c->stream));
+	c->height_bits = bits;
 	c->maps_set = true;
 	return HMRM_OK;
 }
 
+} // namespace
+
+int hmrm_set_maps(hmrm_ctx *c, const uint8_t *height_rgb8, const uint8_t *color_rgba8, int32_t w, int32_t h) {
+	if (!c) return HMRM_ERR_INVALID;
+	return upload_maps(c, height_rgb8, color_rgba8, w, h, 8, cudaMemcpyHostToDevice);
+}
+
 int hmrm_set_maps_device(hmrm_ctx *c, const void *d_rgb8, const void *d_rgba8, int32_t w, int32_t h) {
 	if (!c) return HMRM_ERR_INVALID;
-	if (!d_rgb8 || !d_rgba8) return fail(c, HMRM_ERR_INVALID, "map pointers must not be NULL");
-	int rc = alloc_maps(c, w, h);
-	if (rc) return rc;
-	const size_t n = (size_t)w * (size_t)h;
-	HMRM_CUDA(c, cudaMemcpyAsync(c->d_rgb, d_rgb8, n * 3, cudaMemcpyDeviceToDevice, c->stream));
-	HMRM_CUDA(c, cudaMemcpyAsync(c->d_color, d_rgba8, n * 4, cudaMemcpyDeviceToDevice, c->stream));
-	HMRM_CUDA(c, cudaStreamSynchronize(c->stream));
-	c->maps_set = true;
-	return HMRM_OK;
+	return upload_maps(c, d_rgb8, d_rgba8, w, h, 8, cudaMemcpyDeviceToDevice);
+}
+
+int hmrm_set_maps16(hmrm_ctx *c, const uint16_t *height, const uint8_t *color_rgba8, int32_t w, int32_t h) {
+	if (!c) return HMRM_ERR_INVALID;
+	return upload_maps(c, height, color_rgba8, w, h, 16, cudaMemcpyHostToDevice);
+}
+
+int hmrm_set_maps16_device(hmrm_ctx *c, const void *d_height, const void *d_rgba8, int32_t w, int32_t h) {
+	if (!c) return HMRM_ERR_INVALID;
+	return upload_maps(c, d_height, d_rgba8, w, h, 16, cudaMemcpyDeviceToDevice);
 }
 
 int hmrm_synth_maps(hmrm_ctx *c, uint32_t log2n, uint32_t seed) {
@@ -1219,6 +1247,21 @@ int hmrm_synth_maps(hmrm_ctx *c, uint32_t log2n, uint32_t seed) {
 	k_synth_maps<<<c->num_sms * 8, 256, 0, c->stream>>>(log2n, seed, c->d_rgb, c->d_color);
 	HMRM_CUDA(c, cudaGetLastError());
 	HMRM_CUDA(c, cudaStreamSynchronize(c->stream));
+	c->height_bits = 8;
+	c->maps_set = true;
+	return HMRM_OK;
+}
+
+int hmrm_synth_maps16(hmrm_ctx *c, uint32_t log2n, uint32_t seed) {
+	if (!c) return HMRM_ERR_INVALID;
+	if (log2n < 4 || log2n > 15) return fail(c, HMRM_ERR_INVALID, "log2n %u outside [4,15]", log2n);
+	const int32_t n = (int32_t)(1u << log2n);
+	int rc = alloc_maps(c, n, n);
+	if (rc) return rc;
+	k_synth_maps16<<<c->num_sms * 8, 256, 0, c->stream>>>(log2n, seed, (uint16_t *)c->d_rgb, c->d_color);
+	HMRM_CUDA(c, cudaGetLastError());
+	HMRM_CUDA(c, cudaStreamSynchronize(c->stream));
+	c->height_bits = 16;
 	c->maps_set = true;
 	return HMRM_OK;
 }
@@ -1226,6 +1269,8 @@ int hmrm_synth_maps(hmrm_ctx *c, uint32_t log2n, uint32_t seed) {
 int hmrm_get_maps(hmrm_ctx *c, uint8_t *height_rgb8, uint8_t *color_rgba8) {
 	if (!c) return HMRM_ERR_INVALID;
 	if (!c->maps_set) return fail(c, HMRM_ERR_STATE, "maps not set");
+	if (height_rgb8 && c->height_bits == 16)
+		return fail(c, HMRM_ERR_STATE, "the height map is 16-bit (hmrm_set_maps16): it has no RGB8 plane; pass NULL");
 	HMRM_CUDA(c, cudaSetDevice(c->device));
 	const size_t n = (size_t)c->map_w * (size_t)c->map_h;
 	if (height_rgb8) HMRM_CUDA(c, cudaMemcpyAsync(height_rgb8, c->d_rgb, n * 3, cudaMemcpyDeviceToHost, c->stream));
@@ -1253,8 +1298,15 @@ int hmrm_update_heightmap(hmrm_ctx *c, const double lum[3], double min_height, d
 	HMRM_CUDA(c, cudaMemcpyAsync(c->d_max_bits, init_bits, sizeof init_bits, cudaMemcpyHostToDevice, c->stream));
 	int row_stride = (int)((n + (1LL << 20) - 1) / (1LL << 20));
 	if (row_stride < 1) row_stride = 1;
-	k1_range<<<c->num_sms * 8, 256, 0, c->stream>>>(c->d_rgb, c->map_w, c->map_h, row_stride, q, c->d_max_bits,
-	                                                 c->d_max_bits + 1);
+	// the same rows for either input, so equivalent 8- and 16-bit maps get the same quantiser
+	const bool grey16 = c->height_bits == 16;
+	const uint16_t *h16 = (const uint16_t *)c->d_rgb;
+	if (grey16)
+		k1_range<<<c->num_sms * 8, 256, 0, c->stream>>>(Grey16Cells{h16}, c->map_w, c->map_h, row_stride, q,
+		                                                 c->d_max_bits, c->d_max_bits + 1);
+	else
+		k1_range<<<c->num_sms * 8, 256, 0, c->stream>>>(Rgb8Cells{c->d_rgb}, c->map_w, c->map_h, row_stride, q,
+		                                                 c->d_max_bits, c->d_max_bits + 1);
 	HMRM_CUDA(c, cudaGetLastError());
 	unsigned long long bits[3] = {0ULL, 0ULL, 0ULL};
 	HMRM_CUDA(c, cudaMemcpyAsync(bits, c->d_max_bits, 16, cudaMemcpyDeviceToHost, c->stream));
@@ -1282,7 +1334,13 @@ int hmrm_update_heightmap(hmrm_ctx *c, const double lum[3], double min_height, d
 	{
 		uint16_t *plain1 = c->mip_levels > 1 ? c->d_dil : NULL;
 		uint16_t *plain2 = c->mip_levels > 2 ? c->d_dil + c->plain_offset[2] : NULL;
-		if (plain1) {
+		if (plain1 && grey16) {
+			k1_build16<<<c->num_sms * 8, 256, 0, c->stream>>>(h16, c->map_w, c->map_h, q, c->zq_scale, c->zq_offset,
+			                                                   c->d_surf, c->d_mip, c->layout,
+			                                                   pyr_level_pitch(c->layout, c->map_w), plain1, c->mip_w[1],
+			                                                   plain2, c->mip_levels > 2 ? c->mip_w[2] : 0);
+		}
+		else if (plain1) {
 			k1_build<<<c->num_sms * 8, 256, 0, c->stream>>>(c->d_rgb, c->map_w, c->map_h, q, c->zq_scale, c->zq_offset,
 			                                                 c->d_surf, c->d_mip, c->layout,
 			                                                 pyr_level_pitch(c->layout, c->map_w), plain1, c->mip_w[1], plain2,
@@ -1290,7 +1348,8 @@ int hmrm_update_heightmap(hmrm_ctx *c, const double lum[3], double min_height, d
 		}
 		else {
 			// 1x1 map: no pyramid
-			k1_prepass<<<1, 32, 0, c->stream>>>(c->d_rgb, n, q, c->d_surf, NULL, NULL, NULL);
+			if (grey16) k1_prepass<<<1, 32, 0, c->stream>>>(Grey16Cells{h16}, n, q, c->d_surf, NULL, NULL, NULL);
+			else k1_prepass<<<1, 32, 0, c->stream>>>(Rgb8Cells{c->d_rgb}, n, q, c->d_surf, NULL, NULL, NULL);
 			k1_quantise<<<1, 32, 0, c->stream>>>(c->d_surf, n, c->zq_scale, c->zq_offset, c->d_mip,
 			                                     (unsigned int *)(c->d_max_bits + 2));
 		}
@@ -1359,7 +1418,10 @@ int hmrm_get_heights(hmrm_ctx *c, double *heights) {
 	q.lum_b = c->lum[2];
 	q.min_height = c->min_height;
 	q.span = c->max_height - c->min_height;
-	k1_prepass<<<c->num_sms * 8, 256, 0, c->stream>>>(c->d_rgb, n, q, NULL, d_tmp, NULL, NULL);
+	if (c->height_bits == 16)
+		k1_prepass<<<c->num_sms * 8, 256, 0, c->stream>>>(Grey16Cells{(const uint16_t *)c->d_rgb}, n, q, NULL, d_tmp, NULL, NULL);
+	else
+		k1_prepass<<<c->num_sms * 8, 256, 0, c->stream>>>(Rgb8Cells{c->d_rgb}, n, q, NULL, d_tmp, NULL, NULL);
 	cudaError_t e = cudaGetLastError();
 	if (e == cudaSuccess) e = cudaMemcpyAsync(heights, d_tmp, (size_t)n * 8, cudaMemcpyDeviceToHost, c->stream);
 	if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);

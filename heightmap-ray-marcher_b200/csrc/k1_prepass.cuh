@@ -7,6 +7,12 @@
 // The reference keeps `height` and adds min_height again at every march step;
 // K1 stores `surf` (same two roundings, done once per cell) plus the global
 // maximum of surf, which bounds every terrain sample from above.
+//
+// 16-bit maps (hmrm_set_maps16) have one sample x per cell, used as R = G = B, and 65535 in place of 255:
+//   v      = clamp((lum_r*x + lum_g*x) + lum_b*x, 0, 65535)
+//   height = (v / 65535) * (max_height - min_height) + min_height
+// k1_range / k1_prepass take either input through a cell reader (Rgb8Cells, Grey16Cells); k1_build16 shares k1_build's
+// block body.
 #ifndef HMRM_K1_PREPASS_CUH
 #define HMRM_K1_PREPASS_CUH
 
@@ -21,7 +27,7 @@ struct PrepassParams {
 	double span;          // fl(max_height - min_height)
 };
 
-// exact u8 -> double without the quarter-rate I2F: (2^52 + n) - 2^52
+// exact u8 / u16 -> double without the quarter-rate I2F: (2^52 + n) - 2^52
 __device__ __forceinline__ double byte_to_double(uint32_t n) {
 	return fsub(__hiloint2double(0x43300000, (int)n), 4503599627370496.0);
 }
@@ -33,6 +39,28 @@ __device__ __forceinline__ double height_of(const PrepassParams &q, uint32_t r, 
 	else if (v > 255.0) v = 255.0;
 	return fadd(fmul(fdiv(v, 255.0), q.span), q.min_height);
 }
+
+// the same for one 16-bit sample x (R = G = B = x) on the 0..65535 scale
+__device__ __forceinline__ double height16_of(const PrepassParams &q, uint32_t x) {
+	const double d = byte_to_double(x);
+	double v = fadd(fadd(fmul(q.lum_r, d), fmul(q.lum_g, d)), fmul(q.lum_b, d));
+	if (v < 0.0) v = 0.0;
+	else if (v > 65535.0) v = 65535.0;
+	return fadd(fmul(fdiv(v, 65535.0), q.span), q.min_height);
+}
+
+// cell readers: the height of cell p of the map ([h][w] row-major)
+struct Rgb8Cells {
+	const uint8_t *__restrict__ rgb8;          // [n][3]
+	__device__ __forceinline__ double height(const PrepassParams &q, long long p) const {
+		const uint8_t *px = rgb8 + 3 * p;
+		return height_of(q, px[0], px[1], px[2]);
+	}
+};
+struct Grey16Cells {
+	const uint16_t *__restrict__ h16;          // [n]
+	__device__ __forceinline__ double height(const PrepassParams &q, long long p) const { return height16_of(q, h16[p]); }
+};
 
 // order-preserving map double -> uint64 so that atomicMax works on FP64 values
 __device__ __forceinline__ unsigned long long ordered_bits(double v) {
@@ -50,16 +78,16 @@ __host__ __device__ inline double from_ordered_bits(unsigned long long o) {
 	return v;
 }
 
-// rgb8: [n][3]; surf: [n] (may be NULL); heights: [n] (may be NULL, parity checks only)
-__global__ void __launch_bounds__(256) k1_prepass(const uint8_t *__restrict__ rgb8, long long n, PrepassParams q,
+// cells: Rgb8Cells | Grey16Cells over [n] cells; surf: [n] (may be NULL); heights: [n] (may be NULL, parity checks only)
+template <class Cells>
+__global__ void __launch_bounds__(256) k1_prepass(Cells cells, long long n, PrepassParams q,
                                                   double *__restrict__ surf, double *__restrict__ heights,
                                                   unsigned long long *__restrict__ max_surf_bits,
                                                   unsigned long long *__restrict__ min_surf_bits) {
 	unsigned long long local_max = 0ULL, local_min = ~0ULL;
 	const long long stride = (long long)gridDim.x * blockDim.x;
 	for (long long p = (long long)blockIdx.x * blockDim.x + threadIdx.x; p < n; p += stride) {
-		const uint8_t *px = rgb8 + 3 * p;
-		const double h = height_of(q, px[0], px[1], px[2]);
+		const double h = cells.height(q, p);
 		if (heights) heights[p] = h;
 		const double s = fadd(h, q.min_height);
 		if (surf) surf[p] = s;
@@ -115,7 +143,8 @@ __device__ __forceinline__ int zq16(double z, double zq_scale, double zq_offset)
 }
 
 // min / max of surf over every `row_stride`-th row (order-preserving bit patterns, atomics)
-__global__ void __launch_bounds__(256) k1_range(const uint8_t *__restrict__ rgb8, int w, int h, int row_stride,
+template <class Cells>
+__global__ void __launch_bounds__(256) k1_range(Cells cells, int w, int h, int row_stride,
                                                 PrepassParams q, unsigned long long *__restrict__ max_bits,
                                                 unsigned long long *__restrict__ min_bits) {
 	unsigned long long local_max = 0ULL, local_min = ~0ULL;
@@ -125,8 +154,7 @@ __global__ void __launch_bounds__(256) k1_range(const uint8_t *__restrict__ rgb8
 	for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
 		const int x = (int)(i % w);
 		const long long y = (i / w) * row_stride;
-		const uint8_t *px = rgb8 + 3 * (y * w + x);
-		const unsigned long long ob = ordered_bits(fadd(height_of(q, px[0], px[1], px[2]), q.min_height));
+		const unsigned long long ob = ordered_bits(fadd(cells.height(q, y * w + x), q.min_height));
 		if (ob > local_max) local_max = ob;
 		if (ob < local_min) local_min = ob;
 	}
@@ -142,28 +170,18 @@ __global__ void __launch_bounds__(256) k1_range(const uint8_t *__restrict__ rgb8
 	}
 }
 
-// Fused build: one thread owns a 4x4 block of cells.  Reads RGB8 once, writes surf (FP64), level 0 (Zq16 per cell)
-// and the plain max-mip levels 1 and 2 of that block.  HBM-bound: 3 B in, 8 + 2 + 0.5 + 0.125 B out per cell.
-__global__ void __launch_bounds__(256) k1_build(const uint8_t *__restrict__ rgb8, int w, int h, PrepassParams q,
-                                                double zq_scale, double zq_offset, double *__restrict__ surf,
+// Fused build: one thread owns a 4x4 block of cells.  Reads the map once, writes surf (FP64), level 0 (Zq16 per cell)
+// and the plain max-mip levels 1 and 2 of that block.  HBM-bound: 3 B (RGB8) or 2 B (16-bit) in, 8 + 2 + 0.5 + 0.125 B
+// out per cell.  `Rows` turns four cells of one row into their surf and Zq16 values (Rgb8Rows, Grey16Rows).
+template <class Rows>
+__device__ __forceinline__ void k1_build_blocks(const Rows &rows, int w, int h, double *__restrict__ surf,
                                                 uint16_t *__restrict__ lv0, int layout, unsigned pitch0,
-                                                uint16_t *__restrict__ plain1, int w1,
-                                                uint16_t *__restrict__ plain2, int w2) {
+                                                uint16_t *__restrict__ plain1, int w1, uint16_t *__restrict__ plain2,
+                                                int w2) {
 	const int tiles_x = (w + 3) / 4, tiles_y = (h + 3) / 4;
 	const long long n_tiles = (long long)tiles_x * tiles_y;
 	const long long stride = (long long)gridDim.x * blockDim.x;
-	const bool vec = (w & 3) == 0;     // rows are 4-byte aligned in rgb8, 8-byte in lv0, 32-byte in surf
-	// Grey cells (R == G == B: every greyscale image after stb's channel replication, vendor/stb_image.h:1758) take
-	// their height from a 256-entry table built by the same expressions: bit-identical, and it removes the IEEE divide
-	// and ~60 other instructions per cell, which is what bounds this kernel (ncu: issue-active 66 %, DRAM 62 %).
-	__shared__ double s_grey[256];
-	__shared__ unsigned short z_grey[256];
-	for (int v = threadIdx.x; v < 256; v += blockDim.x) {
-		const double sv = fadd(height_of(q, (uint32_t)v, (uint32_t)v, (uint32_t)v), q.min_height);
-		s_grey[v] = sv;
-		z_grey[v] = (unsigned short)zq16(sv, zq_scale, zq_offset);
-	}
-	__syncthreads();
+	const bool vec = (w & 3) == 0;     // rows are 4-byte aligned in rgb8, 8-byte in the 16-bit plane and lv0, 32-byte in surf
 	for (long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x; t < n_tiles; t += stride) {
 		const int bx = (int)(t % tiles_x), by = (int)(t / tiles_x);
 		const int x0 = bx * 4, y0 = by * 4;
@@ -176,41 +194,10 @@ __global__ void __launch_bounds__(256) k1_build(const uint8_t *__restrict__ rgb8
 			const int y = y0 + j;
 			if (y >= h) break;
 			const size_t row = (size_t)y * (size_t)w + (size_t)x0;
-			uint32_t r[4], g[4], b[4];
 			int valid = min(4, w - x0);
-			if (vec) {
-				const uint32_t *p = (const uint32_t *)(rgb8 + 3 * row);
-				const uint32_t a0 = __ldg(p), a1 = __ldg(p + 1), a2 = __ldg(p + 2);
-				r[0] = a0 & 255u; g[0] = (a0 >> 8) & 255u; b[0] = (a0 >> 16) & 255u;
-				r[1] = a0 >> 24; g[1] = a1 & 255u; b[1] = (a1 >> 8) & 255u;
-				r[2] = (a1 >> 16) & 255u; g[2] = a1 >> 24; b[2] = a2 & 255u;
-				r[3] = (a2 >> 8) & 255u; g[3] = (a2 >> 16) & 255u; b[3] = a2 >> 24;
-			}
-			else {
-				for (int i = 0; i < 4; ++i) {
-					const bool in = i < valid;
-					const uint8_t *p = rgb8 + 3 * (row + (in ? i : 0));
-					r[i] = p[0]; g[i] = p[1]; b[i] = p[2];
-				}
-			}
 			double s[4];
 			int zq[4];
-			const bool grey = r[0] == g[0] && g[0] == b[0] && r[1] == g[1] && g[1] == b[1] &&
-			                  r[2] == g[2] && g[2] == b[2] && r[3] == g[3] && g[3] == b[3];
-			if (grey) {
-#pragma unroll
-				for (int i = 0; i < 4; ++i) {
-					s[i] = s_grey[r[i]];
-					zq[i] = (int)z_grey[r[i]];
-				}
-			}
-			else {
-#pragma unroll
-				for (int i = 0; i < 4; ++i) {
-					s[i] = fadd(height_of(q, r[i], g[i], b[i]), q.min_height);
-					zq[i] = zq16(s[i], zq_scale, zq_offset);
-				}
-			}
+			rows.load(row, valid, vec, s, zq);
 #pragma unroll
 			for (int i = 0; i < 4; ++i) {
 				if (i < valid) m1[j >> 1][i >> 1] = max(m1[j >> 1][i >> 1], zq[i]);
@@ -247,6 +234,107 @@ __global__ void __launch_bounds__(256) k1_build(const uint8_t *__restrict__ rgb8
 		}
 		if (plain2) plain2[(size_t)by * w2 + bx] = (uint16_t)m2;
 	}
+}
+
+// RGB8 rows: three 4-byte words per row when w % 4 == 0, else single cells (clamped to the last valid one)
+struct Rgb8Rows {
+	const uint8_t *__restrict__ rgb8;
+	PrepassParams q;
+	double zq_scale, zq_offset;
+	const double *s_grey;
+	const unsigned short *z_grey;
+	__device__ __forceinline__ void load(size_t row, int valid, bool vec, double s[4], int zq[4]) const {
+		uint32_t r[4], g[4], b[4];
+		if (vec) {
+			const uint32_t *p = (const uint32_t *)(rgb8 + 3 * row);
+			const uint32_t a0 = __ldg(p), a1 = __ldg(p + 1), a2 = __ldg(p + 2);
+			r[0] = a0 & 255u; g[0] = (a0 >> 8) & 255u; b[0] = (a0 >> 16) & 255u;
+			r[1] = a0 >> 24; g[1] = a1 & 255u; b[1] = (a1 >> 8) & 255u;
+			r[2] = (a1 >> 16) & 255u; g[2] = a1 >> 24; b[2] = a2 & 255u;
+			r[3] = (a2 >> 8) & 255u; g[3] = (a2 >> 16) & 255u; b[3] = a2 >> 24;
+		}
+		else {
+			for (int i = 0; i < 4; ++i) {
+				const bool in = i < valid;
+				const uint8_t *p = rgb8 + 3 * (row + (in ? i : 0));
+				r[i] = p[0]; g[i] = p[1]; b[i] = p[2];
+			}
+		}
+		const bool grey = r[0] == g[0] && g[0] == b[0] && r[1] == g[1] && g[1] == b[1] &&
+		                  r[2] == g[2] && g[2] == b[2] && r[3] == g[3] && g[3] == b[3];
+		if (grey) {
+#pragma unroll
+			for (int i = 0; i < 4; ++i) {
+				s[i] = s_grey[r[i]];
+				zq[i] = (int)z_grey[r[i]];
+			}
+		}
+		else {
+#pragma unroll
+			for (int i = 0; i < 4; ++i) {
+				s[i] = fadd(height_of(q, r[i], g[i], b[i]), q.min_height);
+				zq[i] = zq16(s[i], zq_scale, zq_offset);
+			}
+		}
+	}
+};
+
+__global__ void __launch_bounds__(256) k1_build(const uint8_t *__restrict__ rgb8, int w, int h, PrepassParams q,
+                                                double zq_scale, double zq_offset, double *__restrict__ surf,
+                                                uint16_t *__restrict__ lv0, int layout, unsigned pitch0,
+                                                uint16_t *__restrict__ plain1, int w1,
+                                                uint16_t *__restrict__ plain2, int w2) {
+	// Grey cells (R == G == B: every greyscale image after stb's channel replication, vendor/stb_image.h:1758) take
+	// their height from a 256-entry table built by the same expressions: bit-identical, and it removes the IEEE divide
+	// and ~60 other instructions per cell, which is what bounds this kernel (ncu: issue-active 66 %, DRAM 62 %).
+	__shared__ double s_grey[256];
+	__shared__ unsigned short z_grey[256];
+	for (int v = threadIdx.x; v < 256; v += blockDim.x) {
+		const double sv = fadd(height_of(q, (uint32_t)v, (uint32_t)v, (uint32_t)v), q.min_height);
+		s_grey[v] = sv;
+		z_grey[v] = (unsigned short)zq16(sv, zq_scale, zq_offset);
+	}
+	__syncthreads();
+	const Rgb8Rows rows = {rgb8, q, zq_scale, zq_offset, s_grey, z_grey};
+	k1_build_blocks(rows, w, h, surf, lv0, layout, pitch0, plain1, w1, plain2, w2);
+}
+
+// ---- 16-bit maps ------------------------------------------------------------------------------------------
+//
+// Every 16-bit cell is grey, so the height is a function of the sample alone; but a 65536-entry table of surf and Zq16
+// does not fit shared memory, and gathering from it in L2 measured slower than the arithmetic: 1.10 ms (two tables,
+// 8 + 2 B) and 1.12 ms (one 16 B table) against 0.78 ms for the divide per cell, at 16384^2
+// (profiles/r06_k1_16_table_variants.txt).
+// 16-bit rows: one 8-byte word per row when w % 4 == 0, else single samples (clamped to the last valid one)
+struct Grey16Rows {
+	const uint16_t *__restrict__ h16;
+	PrepassParams q;
+	double zq_scale, zq_offset;
+	__device__ __forceinline__ void load(size_t row, int valid, bool vec, double s[4], int zq[4]) const {
+		uint32_t x[4];
+		if (vec) {
+			const uint2 a = __ldg((const uint2 *)(h16 + row));
+			x[0] = a.x & 0xFFFFu; x[1] = a.x >> 16; x[2] = a.y & 0xFFFFu; x[3] = a.y >> 16;
+		}
+		else {
+#pragma unroll
+			for (int i = 0; i < 4; ++i) x[i] = __ldg(h16 + row + (i < valid ? i : 0));
+		}
+#pragma unroll
+		for (int i = 0; i < 4; ++i) {
+			s[i] = fadd(height16_of(q, x[i]), q.min_height);
+			zq[i] = zq16(s[i], zq_scale, zq_offset);
+		}
+	}
+};
+
+__global__ void __launch_bounds__(256) k1_build16(const uint16_t *__restrict__ h16, int w, int h, PrepassParams q,
+                                                  double zq_scale, double zq_offset, double *__restrict__ surf,
+                                                  uint16_t *__restrict__ lv0, int layout, unsigned pitch0,
+                                                  uint16_t *__restrict__ plain1, int w1,
+                                                  uint16_t *__restrict__ plain2, int w2) {
+	const Grey16Rows rows = {h16, q, zq_scale, zq_offset};
+	k1_build_blocks(rows, w, h, surf, lv0, layout, pitch0, plain1, w1, plain2, w2);
 }
 
 // q0[p] = Zq(surf[p]); flags an error if a value does not fit 16 bits (cannot happen with the host's scale)

@@ -46,8 +46,8 @@ HMRM_SYNTH_FN uint32_t hmrm_synth_smooth(uint32_t t16) {
 	return (uint32_t)((t2 * (uint64_t)(196608u - 2u * t16)) >> 16);
 }
 
-/* Height sample in [0,255] at pixel (x,y) of a 2^log2n square map. */
-HMRM_SYNTH_FN uint32_t hmrm_synth_height(uint32_t x, uint32_t y, uint32_t log2n, uint32_t seed) {
+/* fBm sum at pixel (x,y) of a 2^log2n square map, and the same sum for the all-ones lattice in *top. */
+HMRM_SYNTH_FN uint32_t hmrm_synth_acc(uint32_t x, uint32_t y, uint32_t log2n, uint32_t seed, uint32_t *top_out) {
 	const uint32_t octaves = log2n - 2u;
 	uint32_t acc = 0u;   /* sum of (16-bit value << 8) >> octave */
 	uint32_t top = 0u;   /* the same sum for the all-ones lattice */
@@ -67,12 +67,31 @@ HMRM_SYNTH_FN uint32_t hmrm_synth_height(uint32_t x, uint32_t y, uint32_t log2n,
 		acc += (v << 8) >> o;
 		top += (65535u << 8) >> o;
 	}
+	*top_out = top;
+	return acc;
+}
+
+/* Height sample in [0,255] at pixel (x,y) of a 2^log2n square map. */
+HMRM_SYNTH_FN uint32_t hmrm_synth_height(uint32_t x, uint32_t y, uint32_t log2n, uint32_t seed) {
+	uint32_t top;
+	const uint32_t acc = hmrm_synth_acc(x, y, log2n, seed, &top);
 	/* contrast stretch [15 %, 85 %] of the range -> [0,255], clamped */
 	const uint64_t lo = ((uint64_t)top * 15u) / 100u;
 	const uint64_t hi = ((uint64_t)top * 85u) / 100u;
 	if ((uint64_t)acc <= lo) return 0u;
 	if ((uint64_t)acc >= hi) return 255u;
 	return (uint32_t)((((uint64_t)acc - lo) * 255u) / (hi - lo));
+}
+
+/* The same field on the 16-bit scale, [0,65535]: the same stretch with 65535 for 255 (hmrm_synth_maps16). */
+HMRM_SYNTH_FN uint32_t hmrm_synth_height16(uint32_t x, uint32_t y, uint32_t log2n, uint32_t seed) {
+	uint32_t top;
+	const uint32_t acc = hmrm_synth_acc(x, y, log2n, seed, &top);
+	const uint64_t lo = ((uint64_t)top * 15u) / 100u;
+	const uint64_t hi = ((uint64_t)top * 85u) / 100u;
+	if ((uint64_t)acc <= lo) return 0u;
+	if ((uint64_t)acc >= hi) return 65535u;
+	return (uint32_t)((((uint64_t)acc - lo) * 65535u) / (hi - lo));
 }
 
 /* Colormap texel for height sample v at pixel (x,y) of an n*n map: RGBA. */

@@ -17,7 +17,7 @@ Config::Config()
 	  lum_g(0.587), lum_b(0.114), grid_width(0.05), step_dist(5.0 * 0.05), cycle_period(47), cycle(0),
 	  hang(-M_PI / 4.0), vang(M_PI / 2.0), mouse_sens(1.0), scroll_sens(1.0), move_speed(0.05),
 	  ortho_width(2.0 * 0.05), recording_frame_count(200), image_plane(1), bg_r(0), bg_g(0), bg_b(0),
-	  maps_changed(false), should_update_heightmap(false) {
+	  height_bits(8), maps_changed(false), should_update_heightmap(false) {
 	cam_pos[0] = -5.0;
 	cam_pos[1] = 5.0;
 	cam_pos[2] = 0.0;
@@ -122,7 +122,17 @@ ParseStatus consume_config_stream(std::istream &input, Config &c, std::ostream &
 
 		if (id == "heightmap") {
 			input >> c.heightmap_path;
-			if (!load_map(c.heightmap_path, 3, &c.heightmap, "heightmap", err)) return PARSE_FATAL;
+			if (c.height_bits == 16) {
+				std::string why;
+				Image16 img;
+				if (!load_heightmap16(c.heightmap_path, &img, &why)) {
+					err << "Failed to load image for heightmap from " << c.heightmap_path << "\n";
+					err << "  (" << why << ")\n";
+					return PARSE_FATAL;
+				}
+				c.heightmap16 = img;
+			}
+			else if (!load_map(c.heightmap_path, 3, &c.heightmap, "heightmap", err)) return PARSE_FATAL;
 			c.should_update_heightmap = true;
 			c.maps_changed = true;
 			echo(c, id, out);
@@ -189,7 +199,9 @@ ParseStatus consume_config_stream(std::istream &input, Config &c, std::ostream &
 	}
 
 	// validation, main/hmap.cpp:491-515
-	if (c.heightmap.pixels.empty()) {
+	const bool h16 = c.height_bits == 16;
+	const int hw = h16 ? c.heightmap16.width : c.heightmap.width, hh = h16 ? c.heightmap16.height : c.heightmap.height;
+	if (h16 ? c.heightmap16.samples.empty() : c.heightmap.pixels.empty()) {
 		err << "Must specify heightmap in config\n";
 		return PARSE_FATAL;
 	}
@@ -197,8 +209,8 @@ ParseStatus consume_config_stream(std::istream &input, Config &c, std::ostream &
 		err << "Must specify colormap in config\n";
 		return PARSE_FATAL;
 	}
-	if (c.heightmap.width != c.colormap.width || c.heightmap.height != c.colormap.height) {
-		err << "heightmap dimensions (" << c.heightmap.width << "x" << c.heightmap.height
+	if (hw != c.colormap.width || hh != c.colormap.height) {
+		err << "heightmap dimensions (" << hw << "x" << hh
 		    << ") must match colormap dimensions (" << c.colormap.width << "x" << c.colormap.height << ")\n";
 		return PARSE_FATAL;
 	}

@@ -29,7 +29,9 @@ struct Config {
 	int image_plane;                          // :107 (selected by keys 1/2/3 in the reference; --projection here)
 	unsigned char bg_r, bg_g, bg_b;           // :110-112
 
-	Image heightmap;                          // RGB8  (stbi_load(...,3), :320-321)
+	Image heightmap;                          // RGB8  (stbi_load(...,3), :320-321), with height_bits 8
+	Image16 heightmap16;                      // one 16-bit sample per pixel (load_heightmap16), with height_bits 16
+	int height_bits;                          // 8 | 16 (hmap --height-bits): the depth the `heightmap` key loads at
 	Image colormap;                           // RGBA8 (stbi_load(...,4), :341-342)
 
 	// change tracking for the caller (what must be pushed to the device)

@@ -9,8 +9,9 @@
 //   hmap config.txt --script frames.txt [--frames N] [--out-prefix P | --record] [--gpus N] ...
 //   hmap config.txt --script frames.txt --video FILE|- [--fps N] [--video-matrix bt601|bt709] ...
 //   ... [--supersample 1|2|3|4]                    (anti-aliasing: the box filter of an N x N-times larger frame)
+//   ... [--height-bits 8|16]                       (16: heightmaps load at full precision, hmrm_set_maps16)
 //   hmap config.txt --parse-only                    (grammar check: echo + validation, no GPU)
-//   hmap --decode-image in.png 3|4 out.raw          (image ingest check, no GPU)
+//   hmap --decode-image in.png 3|4|h16 out.raw      (image ingest check, no GPU; h16: little-endian u16 samples)
 //
 // --script: one line of config grammar per frame (what the reference's console accepts, :760-804),
 // applied before the frame is rendered — the programmatic animation the reference leaves as a stub
@@ -25,6 +26,9 @@
 // --supersample N renders every headless, recorded or video frame at N x N rays per pixel and box-filters it on the
 // device (HMRM_FLAG_SUPERSAMPLE, kernel K5); the files keep the configured resolution.  Supersampled frames are whole
 // frames, so --headless over several devices (tile-row bands) refuses N > 1; --script still deals whole frames to them.
+// --height-bits 16 loads every `heightmap` of the config, the script and the console with load_heightmap16 (16-bit PNG
+// and PNM samples as stored, grey 8-bit files widened x257) and passes it to hmrm_set_maps16; the default, 8, is the
+// reference's RGB8 ingest.
 // Headless frames are complete images: cycle_period is forced to 1 (the reference's own advice, :913).
 #include <cstdio>
 #include <cstdlib>
@@ -53,10 +57,10 @@ namespace {
 
 struct Options {
 	std::string config_path, headless_out, script_path, out_prefix, stats_json, video_path;
-	int projection, precision, traversal, gpus, frames, fps, video_matrix, supersample;
+	int projection, precision, traversal, gpus, frames, fps, video_matrix, supersample, height_bits;
 	bool record, parse_only, supersample_given;
 	Options() : projection(0), precision(HMRM_FP64_EXACT), traversal(HMRM_TRAVERSAL_AUTO), gpus(1), frames(-1), fps(30),
-	            video_matrix(HMRM_YUV_BT709), supersample(1), record(false), parse_only(false), supersample_given(false) {}
+	            video_matrix(HMRM_YUV_BT709), supersample(1), height_bits(8), record(false), parse_only(false), supersample_given(false) {}
 };
 
 void usage_and_exit() {
@@ -64,7 +68,8 @@ void usage_and_exit() {
 	std::cerr << "       hmap path/to/config.txt --headless out.png [--projection 1|2|3] [--precision fp64|fp32]\n"
 	             "            [--traversal auto|brute|skip] [--gpus N] [--script frames.txt [--frames N]\n"
 	             "            [--out-prefix P | --record | --video FILE|- [--fps N] [--video-matrix bt601|bt709]]]\n"
-	             "            [--supersample 1|2|3|4] [--stats-json file] [--parse-only]\n";
+	             "            [--supersample 1|2|3|4] [--height-bits 8|16] [--stats-json file] [--parse-only]\n"
+	             "       hmap --decode-image in 3|4|h16 out.raw\n";
 	std::exit(1);
 }
 
@@ -96,7 +101,11 @@ void die_hmrm(hmrm_ctx *ctx, const char *what) {
 
 void push_maps(std::vector<Device> &devs, Config &cfg) {
 	for (size_t i = 0; i < devs.size(); ++i) {
-		if (cfg.maps_changed &&
+		if (cfg.maps_changed && cfg.height_bits == 16 &&
+		    hmrm_set_maps16(devs[i].ctx, cfg.heightmap16.samples.data(), cfg.colormap.pixels.data(),
+		                    cfg.heightmap16.width, cfg.heightmap16.height) != HMRM_OK)
+			die_hmrm(devs[i].ctx, "hmrm_set_maps16");
+		if (cfg.maps_changed && cfg.height_bits == 8 &&
 		    hmrm_set_maps(devs[i].ctx, cfg.heightmap.pixels.data(), cfg.colormap.pixels.data(), cfg.heightmap.width,
 		                  cfg.heightmap.height) != HMRM_OK)
 			die_hmrm(devs[i].ctx, "hmrm_set_maps");
@@ -203,8 +212,24 @@ void collect(Device &d, Totals &t) {
 
 int decode_image_mode(int argc, char **argv) {
 	if (argc != 5) usage_and_exit();
-	Image img;
 	std::string why;
+	if (std::strcmp(argv[3], "h16") == 0) {
+		Image16 img;
+		if (!load_heightmap16(argv[2], &img, &why)) {
+			std::cerr << "Failed to load image from " << argv[2] << " (" << why << ")\n";
+			return 1;
+		}
+		std::vector<uint8_t> le(img.samples.size() * 2);
+		for (size_t i = 0; i < img.samples.size(); ++i) {
+			le[2 * i] = (uint8_t)(img.samples[i] & 255u);
+			le[2 * i + 1] = (uint8_t)(img.samples[i] >> 8);
+		}
+		std::ofstream out(argv[4], std::ios::binary);
+		out.write((const char *)le.data(), (std::streamsize)le.size());
+		std::cout << img.width << " " << img.height << " 1\n";
+		return out ? 0 : 1;
+	}
+	Image img;
 	if (!load_image(argv[2], std::atoi(argv[3]), &img, &why)) {
 		std::cerr << "Failed to load image from " << argv[2] << " (" << why << ")\n";
 		return 1;
@@ -247,6 +272,12 @@ int main(int argc, char **argv) {
 		else if (a == "--parse-only") opt.parse_only = true;
 		else if (a == "--video" && has_val) opt.video_path = argv[++i];
 		else if (a == "--fps" && has_val) opt.fps = std::atoi(argv[++i]);
+		else if (a == "--height-bits" && has_val) {
+			const std::string v = argv[++i];
+			if (v == "8") opt.height_bits = 8;
+			else if (v == "16") opt.height_bits = 16;
+			else usage_and_exit();
+		}
 		else if (a == "--supersample" && has_val) {
 			opt.supersample = std::atoi(argv[++i]);
 			opt.supersample_given = true;
@@ -276,6 +307,7 @@ int main(int argc, char **argv) {
 		return 1;
 	}
 	Config cfg;
+	cfg.height_bits = opt.height_bits;
 	if (consume_config_stream(input, cfg, msg, std::cerr) != PARSE_OK) return 1;
 	input.close();
 	if (opt.parse_only) return 0;

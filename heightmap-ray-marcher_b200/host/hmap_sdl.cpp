@@ -74,7 +74,11 @@ struct Shell {
 	}
 
 	void push_maps_if_needed() {
-		if (cfg.maps_changed &&
+		if (cfg.maps_changed && cfg.height_bits == 16 &&
+		    hmrm_set_maps16(ctx, cfg.heightmap16.samples.data(), cfg.colormap.pixels.data(), cfg.heightmap16.width,
+		                    cfg.heightmap16.height) != HMRM_OK)
+			fatal(std::string("hmrm_set_maps16: ") + hmrm_last_error(ctx));
+		if (cfg.maps_changed && cfg.height_bits == 8 &&
 		    hmrm_set_maps(ctx, cfg.heightmap.pixels.data(), cfg.colormap.pixels.data(), cfg.heightmap.width,
 		                  cfg.heightmap.height) != HMRM_OK)
 			fatal(std::string("hmrm_set_maps: ") + hmrm_last_error(ctx));

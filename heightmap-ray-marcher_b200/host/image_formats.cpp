@@ -669,6 +669,13 @@ bool decode_pnm(const std::vector<uint8_t> &file, int want_channels, Decoded *ou
 	// >> 8, i.e. it keeps the SECOND byte of every sample; and when the channel count has to change it runs its 8-bit
 	// converter over the 16-bit buffer and then reads past its end (vendor/stb_image.h:7449-7453, :1202-1206) —
 	// undefined pixels that cannot be reproduced.  Only the well-defined case is accepted.
+	if (out->keep16) {
+		out->channels16 = comp;
+		out->px16.resize((size_t)w * (size_t)h * (size_t)comp);
+		for (size_t i = 0; i < out->px16.size(); ++i)
+			out->px16[i] = (uint16_t)((file[s.pos + 2 * i] << 8) | file[s.pos + 2 * i + 1]);
+		return true;
+	}
 	if (want_channels != comp) return fail(error, "16-bit PNM whose channel count must change: stb_image 2.27 reads out of bounds here (undefined pixels)");
 	out->px.resize((size_t)w * (size_t)h * (size_t)comp);
 	for (size_t i = 0; i < out->px.size(); ++i) out->px[i] = file[s.pos + 2 * i + 1];

@@ -10,7 +10,12 @@ namespace hmrm_host {
 struct Decoded {
 	int w, h, channels;
 	std::vector<uint8_t> px;
-	Decoded() : w(0), h(0), channels(0) {}
+	// set by the caller: also keep the samples of a 16-bit PNG (not palette) or 16-bit PNM in px16 at full precision
+	// (load_heightmap16), channels16 per pixel: the file's own channels, without the alpha a tRNS colour key adds to px
+	bool keep16;
+	int channels16;
+	std::vector<uint16_t> px16;
+	Decoded() : w(0), h(0), channels(0), keep16(false), channels16(0) {}
 };
 
 // stbi__convert_format for 8-bit data (vendor/stb_image.h:1735-1781): grey -> R=G=B, missing alpha -> 255, alpha dropped

@@ -5,6 +5,7 @@
 
 #include <cstdio>
 #include <cstring>
+#include <string>
 
 namespace hmrm_host {
 namespace {
@@ -213,6 +214,10 @@ bool decode_png(const std::vector<uint8_t> &file, Decoded *out, std::string *err
 	const size_t npx = (size_t)w * h;
 	out->w = (int)w;
 	out->h = (int)h;
+	if (out->keep16 && depth == 16) {
+		out->px16 = smp;
+		out->channels16 = src_n;
+	}
 	if (color == 3) {
 		// palette expansion (stbi__expand_png_palette): RGB, or RGBA when a tRNS chunk exists
 		const bool alpha = !trns.empty();
@@ -285,6 +290,56 @@ bool load_image_memory(const std::vector<uint8_t> &file, int want_channels, Imag
 	else { ok = false; err = "unknown image type"; }
 	if (!ok) { *error = err; return false; }
 	convert_channels(d, want_channels, out);
+	return true;
+}
+
+bool load_heightmap16(const std::string &path, Image16 *out, std::string *error) {
+	std::vector<uint8_t> file;
+	if (!read_file(path, &file)) { *error = path + ": cannot read file"; return false; }
+	const size_t n = file.size();
+	Decoded d;
+	d.keep16 = true;
+	std::string err;
+	bool ok = true;
+	bool decoded = false;
+	if (n >= 8 && file[0] == 137 && file[1] == 'P' && file[2] == 'N' && file[3] == 'G') ok = decoded = decode_png(file, &d, &err);
+	else if (n >= 2 && file[0] == 'P' && (file[1] == '5' || file[1] == '6')) ok = decoded = decode_pnm(file, 1, &d, &err);
+	if (!ok) { *error = path + ": " + err; return false; }
+	const size_t npx = (size_t)d.w * (size_t)d.h;
+	out->samples.resize(npx);
+	if (!d.px16.empty()) {
+		// 16-bit samples as the file stores them: grey (+ alpha, dropped), or RGB(A) whose three channels agree
+		const int cn = d.channels16;
+		for (size_t i = 0; i < npx; ++i) {
+			const uint16_t *t = &d.px16[i * (size_t)cn];
+			if (cn >= 3 && (t[0] != t[1] || t[1] != t[2])) {
+				*error = path + ": 16-bit heightmap is not grey (R, G and B differ at pixel " + std::to_string(i % (size_t)d.w) +
+				         ", " + std::to_string(i / (size_t)d.w) + ")";
+				return false;
+			}
+			out->samples[i] = t[0];
+		}
+		out->width = d.w;
+		out->height = d.h;
+		return true;
+	}
+	// everything else through the 8-bit decoder: it must be grey, and each sample v becomes 257 v (= v / 255 of 65535)
+	Image img;
+	if (decoded) convert_channels(d, 3, &img);
+	else if (!load_image_memory(file, 3, &img, &err)) { *error = path + ": " + err; return false; }
+	const size_t npx8 = (size_t)img.width * (size_t)img.height;
+	out->samples.resize(npx8);
+	for (size_t i = 0; i < npx8; ++i) {
+		const uint8_t *t = &img.pixels[3 * i];
+		if (t[0] != t[1] || t[1] != t[2]) {
+			*error = path + ": heightmap is not grey (R, G and B differ at pixel " + std::to_string(i % (size_t)img.width) +
+			         ", " + std::to_string(i / (size_t)img.width) + ")";
+			return false;
+		}
+		out->samples[i] = (uint16_t)(t[0] * 257u);
+	}
+	out->width = img.width;
+	out->height = img.height;
 	return true;
 }
 

@@ -45,6 +45,21 @@ bool load_image(const std::string &path, int want_channels, Image *out, std::str
 // The same on a file already in memory (stbi_load_from_memory's role).
 bool load_image_memory(const std::vector<uint8_t> &file, int want_channels, Image *out, std::string *error);
 
+// One 16-bit sample per pixel: a heightmap loaded at full precision (hmrm_set_maps16).
+struct Image16 {
+	int width, height;
+	std::vector<uint16_t> samples;    // row-major, top row first
+	Image16() : width(0), height(0) {}
+};
+
+// Load a heightmap at 16 bits (hmap --height-bits 16):
+//   16-bit PNG, grey or grey + alpha: the samples, alpha dropped;
+//   16-bit PNG, RGB or RGBA: accepted only if R = G = B at every pixel (alpha dropped);
+//   binary PGM / PPM (P5 / P6) with maxval > 255: the big-endian samples as stored (a PPM only if it is grey);
+//   any other file: decoded by load_image to 8-bit RGB, which must be grey (R = G = B everywhere), and widened x257.
+// Anything else is refused: false, and a message naming the file in `error`.
+bool load_heightmap16(const std::string &path, Image16 *out, std::string *error);
+
 // Write n bytes to `path` (a PNG file the device encoded: hmrm_render_png_async / hmrm_encode_png).  Returns false on
 // failure.
 bool write_bytes(const std::string &path, const uint8_t *data, size_t n);

@@ -140,6 +140,25 @@ int hmrm_set_maps_device(hmrm_ctx *ctx, const void *d_height_rgb8, const void *d
 int hmrm_synth_maps(hmrm_ctx *ctx, uint32_t log2n, uint32_t seed);
 int hmrm_get_maps(hmrm_ctx *ctx, uint8_t *height_rgb8, uint8_t *color_rgba8);   /* download (either may be NULL) */
 
+/* ---- 16-bit height maps: UpdateHeightmap (main/hmap.cpp:171-191) with 65535 in place of 255 ----
+ * A 16-bit map has one channel, height [map_height][map_width] (uint16_t).  Its sample x is used as R = G = B, as stb
+ * replicates a grey image, so lum keeps its meaning.  Each line is rounded separately, in this order, without FMA:
+ *   v      = (lum_r*x + lum_g*x) + lum_b*x,  clamped to [0, 65535]
+ *   height = (v / 65535) * (max_height - min_height) + min_height
+ *   surf   = height + min_height          (what the march compares against)
+ * For x = 257 * v8 and a unit lum vector, v / 65535 and v8 / 255 are the same correctly rounded number, so the heights
+ * are bit-identical to those of the grey 8-bit map v8.  After any of these calls hmrm_update_heightmap builds the
+ * pyramid as for 8-bit maps, and hmrm_get_heights returns the heights above.  hmrm_set_maps / hmrm_set_maps_device /
+ * hmrm_synth_maps switch the context back to 8 bits.  hmrm_get_maps on a 16-bit map returns the colormap; a non-NULL
+ * height_rgb8 is HMRM_ERR_STATE.  NULL pointers and sizes outside [1, 32768] are HMRM_ERR_INVALID. */
+int hmrm_set_maps16(hmrm_ctx *ctx, const uint16_t *height, const uint8_t *color_rgba8,
+                    int32_t map_width, int32_t map_height);
+/* same, from device memory of ctx's device (copied) */
+int hmrm_set_maps16_device(hmrm_ctx *ctx, const void *d_height, const void *d_color_rgba8,
+                           int32_t map_width, int32_t map_height);
+/* synthetic 16-bit map: hmrm_synth_height16 (csrc/synth_fbm.h) and exactly hmrm_synth_maps' colormap */
+int hmrm_synth_maps16(hmrm_ctx *ctx, uint32_t log2n, uint32_t seed);
+
 /* layout of the height pyramid (HMRM_LAYOUT_*; also the HMRM_LAYOUT environment variable at hmrm_create:
  * rowmajor | tile4 | zorder).  Takes effect at the next hmrm_update_heightmap, which must follow. */
 int hmrm_set_layout(hmrm_ctx *ctx, int layout);
