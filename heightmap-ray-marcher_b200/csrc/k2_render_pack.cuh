@@ -461,7 +461,14 @@ __device__ __noinline__ void pack_refill(const RenderParams &P, PackQueue Q, con
 					// (re)build the integer model for the window that contains nr.n, anchored on its exact first sample
 					bool model = pack_slopes(P, ax, ay, az, nr);
 					if (model) {
-						advance_exact(ax, ay, az, anchor, nr.n & ~(HMRM_LIN_PERIOD - 1u));
+						// an exact decision (advance_exact to sample at_n) may have moved the anchor past the window's first
+						// sample, which advance_exact cannot go back to: restart from sample 0
+						const unsigned wbase = nr.n & ~(HMRM_LIN_PERIOD - 1u);
+						if (anchor > wbase) {
+							pack_exact_start(P, gr, ex, ey, ez, ax, ay, az);
+							anchor = 0u;
+						}
+						advance_exact(ax, ay, az, anchor, wbase);
 						model = pack_rebase(P, ax, ay, az, nr);
 					}
 					nr.miss_rgba = rgba;

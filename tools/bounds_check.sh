@@ -3,5 +3,5 @@
 # the production build.
 set -e
 HMRM_NVCC_EXTRA="-DHMRM_BOUNDS_CHECK" python heightmap-ray-marcher_b200/build.py --force > /dev/null 2>&1
-python -m pytest tests/test_gpu_parity.py tests/test_gpu_fuzz.py -m gpu -q 2>&1 | tail -4
+python -m pytest tests/test_gpu_parity.py tests/test_gpu_fuzz.py tests/test_gpu_pyramid_fuzz.py -m gpu -q 2>&1 | tail -4
 python heightmap-ray-marcher_b200/build.py --force > /dev/null 2>&1
