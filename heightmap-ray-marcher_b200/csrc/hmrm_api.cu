@@ -385,7 +385,7 @@ __global__ void k_reset_slot(unsigned int *tile_counter, unsigned int *stats_wor
 	for (unsigned i = threadIdx.x; i < sizeof(DeviceStats) / 4; i += 32) stats_words[i] = 0u;
 }
 
-// Enqueue one frame on `stream`, writing RGBA8 into d_out.
+// Enqueue one frame on `stream`, writing the frame's pixel format into d_out (any alignment).
 int enqueue_render(hmrm_ctx *c, const hmrm_frame *f, uint32_t *d_out, cudaStream_t stream, bool timed) {
 	int row_begin = 0, row_end = 0;
 	int rc = validate_frame(c, f, &row_begin, &row_end);
@@ -534,7 +534,9 @@ int enqueue_render(hmrm_ctx *c, const hmrm_frame *f, uint32_t *d_out, cudaStream
 	P.color = c->d_color;
 	P.fb = d_out;
 	P.pixel_format = f->pixel_format;
-	P.rgb_words = (W % 4) == 0 ? 1 : 0;
+	// hmrm_render_device and the peer calls take any caller pointer: word stores only where they are aligned
+	P.fb_unaligned = ((uintptr_t)d_out & 3u) != 0u ? 1 : 0;
+	P.rgb_words = (W % 4) == 0 && !P.fb_unaligned ? 1 : 0;
 	P.bg[0] = f->bg[0];
 	P.bg[1] = f->bg[1];
 	P.bg[2] = f->bg[2];

@@ -343,7 +343,7 @@ __device__ __forceinline__ void pack_flush_counters(const RenderParams &P, unsig
 // one finished pixel (any lane, any time): main/hmap.cpp:139-154
 __device__ __forceinline__ void pack_store(const RenderParams &P, unsigned pixel, uint32_t rgba, int first_hit) {
 	const size_t at = (size_t)(pixel >> 16) * (size_t)P.W + (size_t)(pixel & 0xFFFFu);
-	if (P.pixel_format == 0) P.fb[HMRM_CHECKED(P, at, (size_t)P.W * (size_t)P.H)] = rgba;
+	if (P.pixel_format == 0) store_rgba8(P, HMRM_CHECKED(P, at, (size_t)P.W * (size_t)P.H), rgba);
 	else {
 		uint8_t *o = (uint8_t *)P.fb + HMRM_CHECKED(P, at * 3, (size_t)P.W * (size_t)P.H * 3);
 		o[0] = (uint8_t)rgba;

@@ -149,6 +149,20 @@ __device__ __noinline__ void dump_ray(const RenderParams &P, int px, int py, con
 	o[9] = entered ? ez : 0.0;
 }
 
+// RGBA8 pixel `at` (index into [H][W]): one 32-bit store, or four byte stores into a destination that is not 4-byte
+// aligned (hmrm_render_device and the peer calls accept any device pointer).
+__device__ __forceinline__ void store_rgba8(const RenderParams &P, size_t at, uint32_t rgba) {
+	if (!P.fb_unaligned) {
+		P.fb[at] = rgba;
+		return;
+	}
+	uint8_t *o = (uint8_t *)P.fb + at * 4;
+	o[0] = (uint8_t)rgba;
+	o[1] = (uint8_t)(rgba >> 8);
+	o[2] = (uint8_t)(rgba >> 16);
+	o[3] = (uint8_t)(rgba >> 24);
+}
+
 // SetPixel (main/hmap.cpp:139-154).  Called by the whole warp (8x4-pixel tile, lane = 8 * row + column); `active`
 // lanes own a pixel of this frame.  RGBA8: one 32-bit store per pixel, A = 255.  RGB8 (HMRM_PIXEL_RGB8: the alpha
 // byte is always 255 in the reference, so it is dead weight on PCIe / NVLink): a tile row is 24 contiguous bytes;
@@ -156,7 +170,7 @@ __device__ __noinline__ void dump_ray(const RenderParams &P, int px, int py, con
 // 32-bit words from their neighbours' colours (two shuffles), otherwise every lane stores its 3 bytes.
 __device__ __forceinline__ void store_pixel(const RenderParams &P, int px, int py, bool active, uint32_t rgba) {
 	if (P.pixel_format == 0) {
-		if (active) P.fb[HMRM_CHECKED(P, (size_t)py * (size_t)P.W + (size_t)px, (size_t)P.W * (size_t)P.H)] = rgba;
+		if (active) store_rgba8(P, HMRM_CHECKED(P, (size_t)py * (size_t)P.W + (size_t)px, (size_t)P.W * (size_t)P.H), rgba);
 		return;
 	}
 	const int lane = threadIdx.x & 31, i = lane & 7;
@@ -170,7 +184,7 @@ __device__ __forceinline__ void store_pixel(const RenderParams &P, int px, int p
 		if (i < 6) {
 			const int sh = 8 * ((i * 4) % 3);
 			const uint32_t word = (A >> sh) | (B << (24 - sh));
-			const size_t at = ((size_t)py * (size_t)P.W + (size_t)(px & ~7)) * 3;   // multiple of 4 (W % 4 == 0)
+			const size_t at = ((size_t)py * (size_t)P.W + (size_t)(px & ~7)) * 3;   // multiple of 4 (W % 4 == 0, fb aligned)
 			*(uint32_t *)(fb8 + HMRM_CHECKED(P, at + (size_t)i * 4, (size_t)P.W * (size_t)P.H * 3)) = word;
 		}
 	}

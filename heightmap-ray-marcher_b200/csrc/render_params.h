@@ -56,9 +56,9 @@ struct RenderParams {
 	const double *surf;            // fl(height + min_height), row-major [map_h][map_w]
 	const uint32_t *color;         // RGBA8 little-endian, row-major
 	// outputs
-	uint32_t *fb;                  // RGBA8 [H][W], or packed RGB8 [H][W][3] (pixel_format 1)
+	uint32_t *fb;                  // RGBA8 [H][W], or packed RGB8 [H][W][3] (pixel_format 1); any alignment (fb_unaligned)
 	int pixel_format;              // HMRM_PIXEL_RGBA8 (0) / HMRM_PIXEL_RGB8 (1)
-	int rgb_words;                 // RGB8: rows are 4-byte aligned (W % 4 == 0) -> tile rows go out as 32-bit words
+	int rgb_words;                 // RGB8: rows are 4-byte aligned (W % 4 == 0, fb aligned) -> tile rows go out as 32-bit words
 	int32_t *step_index;           // optional [H][W]
 	double *ray_dump;              // optional [H][W][10] (HMRM_FLAG_RAY_DUMP, ray_setup.cuh:dump_ray)
 	DeviceStats *stats;            // optional
@@ -76,7 +76,7 @@ struct RenderParams {
 	uint2 lv_desc[16];             // per level: (element offset into lv, layout's pitch term)
 	uint32_t bg_rgba;              // bg colour with alpha 255
 	uint8_t bg[3];
-	uint8_t pad;
+	uint8_t fb_unaligned;          // fb is not 4-byte aligned (a caller's device pointer): RGBA8 pixels go out as 4 bytes
 };
 
 } // namespace hmrm

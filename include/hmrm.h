@@ -175,7 +175,9 @@ void hmrm_frame_defaults(hmrm_frame *f);            /* the reference's defaults,
  * pixel_format = HMRM_PIXEL_RGB8, [screen_height][screen_width][3], stride W*3.
  * Only the pixels selected by cycle/cycle_period and the row band are written. Synchronous. */
 int hmrm_render(hmrm_ctx *ctx, const hmrm_frame *f, uint8_t *rgba_out);
-/* device output (same layout) on `stream` (a cudaStream_t, NULL = ctx's own stream); asynchronous */
+/* device output (same layout) on `stream` (a cudaStream_t, NULL = ctx's own stream); asynchronous.  d_rgba_out may
+ * have any alignment (so may d_frame and d_stage of hmrm_render_peer / hmrm_render_peer_staged): an address that is
+ * not a multiple of 4 is written byte by byte, as K3's and K5's device outputs already may be. */
 int hmrm_render_device(hmrm_ctx *ctx, const hmrm_frame *f, void *d_rgba_out, void *stream);
 /* render into the context's device framebuffer(s) and copy rows [row_begin,row_end) to (pinned or registered) host
  * memory asynchronously; hmrm_wait() joins.  rgba_out always addresses the WHOLE frame; with band_count > 1 only the
