@@ -636,7 +636,7 @@ int enqueue_render(hmrm_ctx *c, const hmrm_frame *f, uint32_t *d_out, cudaStream
 
 	const int n_tiles = P.tiles_x * P.tiles_y;
 	const int warps_per_block = 8;
-	int blocks = c->num_sms * 4;   // persistent CTAs: 4 x 256 threads per SM at <= 64 registers
+	int blocks = c->num_sms * 4;   // brute and FP64 skip kernels: persistent CTAs, 4 x 256 threads per SM (lin, pack: below)
 	const int max_useful = (n_tiles + warps_per_block - 1) / warps_per_block;
 	if (blocks > max_useful) blocks = max_useful;
 	if (blocks < 1) blocks = 1;
@@ -646,23 +646,30 @@ int enqueue_render(hmrm_ctx *c, const hmrm_frame *f, uint32_t *d_out, cudaStream
 	if (traversal == HMRM_TRAVERSAL_SKIP) {
 		const bool stats_kernel = want_stats || want_steps || want_dump;
 		const int lin_warps = HMRM_LIN_THREADS / 32;
-		int lin_blocks = c->num_sms * HMRM_LIN_CTAS;
+		const bool large = n_tiles >= HMRM_LIN_LARGE_TILES;
+		int lin_blocks = c->num_sms * (large ? HMRM_LIN_CTAS_LARGE : HMRM_LIN_CTAS);
 		if (lin_blocks > (n_tiles + lin_warps - 1) / lin_warps) lin_blocks = (n_tiles + lin_warps - 1) / lin_warps;
 		if (lin_blocks < 1) lin_blocks = 1;
-#define HMRM_LAUNCH_LIN(LAYOUT)                                                                              \
-		do {                                                                                                 \
-			if (stats_kernel) k2_render_lin<true, LAYOUT><<<lin_blocks, HMRM_LIN_THREADS, 0, stream>>>(P);   \
-			else k2_render_lin<false, LAYOUT><<<lin_blocks, HMRM_LIN_THREADS, 0, stream>>>(P);               \
+#define HMRM_LAUNCH_LIN_SHAPE(LAYOUT, CTAS)                                                                        \
+		do {                                                                                                       \
+			if (stats_kernel) k2_render_lin<true, LAYOUT, CTAS><<<lin_blocks, HMRM_LIN_THREADS, 0, stream>>>(P);   \
+			else k2_render_lin<false, LAYOUT, CTAS><<<lin_blocks, HMRM_LIN_THREADS, 0, stream>>>(P);               \
+		} while (0)
+#define HMRM_LAUNCH_LIN(LAYOUT)                                                                                    \
+		do {                                                                                                       \
+			if (large) HMRM_LAUNCH_LIN_SHAPE(LAYOUT, HMRM_LIN_CTAS_LARGE);                                         \
+			else HMRM_LAUNCH_LIN_SHAPE(LAYOUT, HMRM_LIN_CTAS);                                                     \
 		} while (0)
 		if (c->layout == HMRM_LAYOUT_TILE4) HMRM_LAUNCH_LIN(kLayoutTile4);
 		else if (c->layout == HMRM_LAYOUT_ZORDER) HMRM_LAUNCH_LIN(kLayoutZOrder);
 		else HMRM_LAUNCH_LIN(kLayoutRowMajor);
 #undef HMRM_LAUNCH_LIN
+#undef HMRM_LAUNCH_LIN_SHAPE
 	}
 	else if (traversal == HMRM_TRAVERSAL_PACK) {
 		const bool stats_kernel = want_stats || want_steps || want_dump;
 		const int lin_warps = HMRM_LIN_THREADS / 32;
-		int lin_blocks = c->num_sms * HMRM_LIN_CTAS;
+		int lin_blocks = c->num_sms * HMRM_PACK_CTAS;
 		if (lin_blocks > (n_tiles + lin_warps - 1) / lin_warps) lin_blocks = (n_tiles + lin_warps - 1) / lin_warps;
 		if (lin_blocks < 1) lin_blocks = 1;
 #define HMRM_LAUNCH_PACK(LAYOUT)                                                                              \

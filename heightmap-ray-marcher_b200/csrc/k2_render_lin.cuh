@@ -46,12 +46,21 @@
 
 namespace hmrm {
 
-// launch shape: persistent CTAs of HMRM_LIN_THREADS threads, HMRM_LIN_CTAS of them per SM
+// Launch shape: persistent CTAs of HMRM_LIN_THREADS threads.  A launch of at least HMRM_LIN_LARGE_TILES tiles runs
+// HMRM_LIN_CTAS_LARGE of them per SM (40 registers: more warps to cover the latency of the dependent mip fetches, at
+// the price of some spills), a smaller one HMRM_LIN_CTAS (64 registers).  Measured on a B200 at 1000 W
+// (profiles/r09_lin32_ab.txt): 6 CTAs are 6-10 % faster than 4 on the 4K and 8K frames, 8-11 % slower on 1280x720.
 #ifndef HMRM_LIN_THREADS
 #define HMRM_LIN_THREADS 256
 #endif
 #ifndef HMRM_LIN_CTAS
 #define HMRM_LIN_CTAS 4
+#endif
+#ifndef HMRM_LIN_CTAS_LARGE
+#define HMRM_LIN_CTAS_LARGE 6
+#endif
+#ifndef HMRM_LIN_LARGE_TILES
+#define HMRM_LIN_LARGE_TILES 100000     // 3.2 M pixels: a 4K frame is 259200 tiles, one 8-way band of an 8K frame 129600
 #endif
 
 #define HMRM_LIN_FRAC 16
@@ -97,22 +106,44 @@ __device__ __noinline__ void advance_exact(AxisState &ax, AxisState &ay, AxisSta
 	}
 }
 
-struct LinAxis {
-	long long d;     // per-step motion in units * 2^16
-	long long a0;    // V_0 * 2^16 + 2^15: position of the base sample, pre-shifted, with the rounding half added
-};
-
-// 2^16 V_j + (fraction): V_j = V_0 + round(j D / 2^16) is the arithmetic shift of this by 16.  One IMAD.WIDE (the
-// 64-bit addend is free) and one IMAD; |a0| < 2^47 + 2^15 and j |D| < 2^17 * 2^42, so it cannot wrap.
-__device__ __forceinline__ long long lin_acc(const LinAxis &l, unsigned j) {
-	return l.a0 + (long long)((unsigned long long)j * (unsigned long long)l.d);
-}
-
 // slope of one axis of the integer model; false if it does not fit (|motion| >= 2^26 units per step, NaN)
 __device__ __forceinline__ bool lin_slope(double s_units, long long &d) {
 	if (!(fabs(s_units) < 67108864.0)) return false;
 	d = __double2ll_rn(s_units * 65536.0);
 	return true;
+}
+
+// One axis of the integer model in 32 bits.  The slope D (units * 2^16, |D| < 2^42) is split once per ray into
+// Di = D >> 16 (arithmetic) and Df = D & 0xFFFF, so that D = 2^16 Di + Df and
+//     V_j = floor((2^16 V_0 + 2^15 + j D) / 2^16) = V_0 + j Di + floor((j Df + 2^15) / 2^16)
+// (j Di 2^16 is a multiple of 2^16 and leaves the floor).  The loop evaluates j < HMRM_LIN_PERIOD = 2^16 only, so
+// j Df + 2^15 < 2^16 (2^16 - 1) + 2^15 < 2^32: the last term is exact in unsigned 32 bits, and the sum, taken modulo
+// 2^32, is V_j itself whenever V_j fits an int.  Why it does, see march_lin.
+struct LinAxis32 {
+	int v0;          // V_0: position of the base sample (units)
+	int di;          // D >> 16: whole units per step, |di| < 2^26; its sign is the direction of motion
+	unsigned df;     // D & 0xFFFF: the fraction of a unit per step, * 2^16
+};
+
+__device__ __forceinline__ LinAxis32 lin_split(long long d) {
+	return LinAxis32{0, (int)(d >> HMRM_LIN_FRAC), (unsigned)d & 0xFFFFu};
+}
+
+__device__ __forceinline__ int lin_at(const LinAxis32 &l, unsigned j) {
+	return (int)((unsigned)l.v0 + j * (unsigned)l.di + ((j * l.df + (1u << (HMRM_LIN_FRAC - 1))) >> HMRM_LIN_FRAC));
+}
+
+// The first j at which V_j of an axis leaves [-2^31, 2^31), or 0xFFFFFFFF if it does not for any j <= HMRM_LIN_PERIOD.
+// V_j is monotone in j, so it stays out from there on.  One 64-bit divide, and only for an axis that could get there
+// at all: |V_j - V_0| <= j ((|D| >> 16) + 1) + 1.
+__device__ __forceinline__ unsigned lin_exit_j(const LinAxis32 &l) {
+	const long long d = ((long long)l.di << HMRM_LIN_FRAC) + (long long)l.df;
+	const long long di_abs = (d < 0 ? -d : d) >> HMRM_LIN_FRAC;
+	if (d == 0 || llabs((long long)l.v0) + (di_abs + 1) * (long long)HMRM_LIN_PERIOD + 1 <= 2147483647LL) return 0xFFFFFFFFu;
+	// a0 = 2^16 V_0 + 2^15 is in (-2^47, 2^47); V_j >= 2^31 iff a0 + j d >= 2^47, V_j < -2^31 iff a0 + j d < -2^47
+	const long long a0 = ((long long)l.v0 << HMRM_LIN_FRAC) + (1LL << (HMRM_LIN_FRAC - 1));
+	const long long j = d > 0 ? ((1LL << 47) - a0 + d - 1) / d : (a0 + (1LL << 47)) / -d + 1;
+	return j > (long long)HMRM_LIN_PERIOD ? 0xFFFFFFFFu : (unsigned)j;
 }
 
 template <bool kStats, int kLayout>
@@ -140,19 +171,24 @@ __device__ __forceinline__ void march_lin(const RenderParams &P, const Ray &ray,
 	// same magic-number form.
 	const double zc = P.zq_offset - HMRM_MAGIC;
 	const double zs16 = P.zq_scale * 16.0, zo16 = __fma_rn(16.0, zc, HMRM_MAGIC);
-	LinAxis lx, ly, lz;
-	bool model = lin_slope(ax.s * P.fx_scale, lx.d) && lin_slope(-ay.s * P.fx_scale, ly.d) && lin_slope(az.s * zs16, lz.d);
+	long long dx = 0, dy = 0, dz = 0;
+	bool model = lin_slope(ax.s * P.fx_scale, dx) && lin_slope(-ay.s * P.fx_scale, dy) && lin_slope(az.s * zs16, dz);
 	model = model && fabs(zc) < 1.0e12;
 	// no lateral motion and not coming down: such a ray can only end by the reference's hang; the per-step loop cuts it
-	model = model && (lx.d != 0 || ly.d != 0 || lz.d < 0);
+	model = model && (dx != 0 || dy != 0 || dz < 0);
+	LinAxis32 lx = lin_split(dx), ly = lin_split(dy), lz = lin_split(dz);
+	// Every V the loop below evaluates fits an int, so lin_at gives it exactly, in x and y because the loop only moves
+	// on from samples that are inside the grid or within the margin of it (otherwise it has decided the ray): a rebase
+	// gives |V_0| < 2^31 (magic_decode), a single step adds < 2^26 + 1 units to |V| <= 2^30 + 2^20 + 4 (grid <= 2^30
+	// units, k <= 20), and a jump ends inside a cleared neighbourhood clipped to the grid.  Nothing bounds z that way
+	// (an ascending ray is never limited by est_z): from the first j at which V_z leaves [-2^31, 2^31), jz_out, the
+	// loop uses +-2^30 instead, which is far above or below everything the 16-bit pyramid holds.
+	unsigned jz_out = 0xFFFFFFFFu;
 	auto rebase = [&]() -> bool {                     // V_0 of the model := the exact anchor
-		int vx, vy, vz;
-		const bool okx = magic_decode(__fma_rn(ax.p, P.fx_scale, HMRM_MAGIC), vx);
-		const bool oky = magic_decode(__fma_rn(ay.p, -P.fx_scale, HMRM_MAGIC), vy);
-		const bool okz = magic_decode(__fma_rn(az.p, zs16, zo16), vz);
-		lx.a0 = ((long long)vx << HMRM_LIN_FRAC) + (1LL << (HMRM_LIN_FRAC - 1));
-		ly.a0 = ((long long)vy << HMRM_LIN_FRAC) + (1LL << (HMRM_LIN_FRAC - 1));
-		lz.a0 = ((long long)vz << HMRM_LIN_FRAC) + (1LL << (HMRM_LIN_FRAC - 1));
+		const bool okx = magic_decode(__fma_rn(ax.p, P.fx_scale, HMRM_MAGIC), lx.v0);
+		const bool oky = magic_decode(__fma_rn(ay.p, -P.fx_scale, HMRM_MAGIC), ly.v0);
+		const bool okz = magic_decode(__fma_rn(az.p, zs16, zo16), lz.v0);
+		jz_out = lin_exit_j(lz);
 		return okx && oky && okz;
 	};
 	unsigned base = 0u;       // sample index of V_0
@@ -160,9 +196,9 @@ __device__ __forceinline__ void march_lin(const RenderParams &P, const Ray &ray,
 
 	bool finished = false;     // the integer-model loop reached a verdict
 	if (model) {
-	const float inv_adx = fast_rcp(fabsf((float)lx.d) * (1.0f / 65536.0f));
-	const float inv_ady = fast_rcp(fabsf((float)ly.d) * (1.0f / 65536.0f));
-	const float adz = fabsf((float)lz.d) * (1.0f / 65536.0f);
+	const float inv_adx = fast_rcp(fabsf((float)dx) * (1.0f / 65536.0f));
+	const float inv_ady = fast_rcp(fabsf((float)dy) * (1.0f / 65536.0f));
+	const float adz = fabsf((float)dz) * (1.0f / 65536.0f);
 	const float inv_adz = fast_rcp(adz);
 	const int cell_exit = (int)fminf(P.cell_exit_scale * adz + 512.0f, 1.0e9f);
 	const int cell_mask = (1 << k) - 1;
@@ -176,7 +212,6 @@ __device__ __forceinline__ void march_lin(const RenderParams &P, const Ray &ray,
 	// `above q` / `below q` with the model's error (< 1.6/16 Zq) and Zq16's rounding (ties at q +- 1/2) covered
 	auto above = [&](int vz, int q) -> bool { return vz > (q << 4) + HMRM_LIN_ZMARGIN && q < 65535; };
 
-	long long wx = lin_acc(lx, 0u), wy = lin_acc(ly, 0u), wz = lin_acc(lz, 0u);   // model position of sample n, * 2^16
 	for (;;) {
 		// keep the error bound: re-anchor the model on an exact position every HMRM_LIN_PERIOD samples
 		if (n - base >= HMRM_LIN_PERIOD) {
@@ -193,7 +228,6 @@ __device__ __forceinline__ void march_lin(const RenderParams &P, const Ray &ray,
 				model = false;
 				break;
 			}
-			wx = lin_acc(lx, 0u); wy = lin_acc(ly, 0u); wz = lin_acc(lz, 0u);
 		}
 		const unsigned j = n - base;
 		if (kStats) {                        // [6]: warp-level iterations (lane utilisation = lane iterations / 32 / this)
@@ -206,28 +240,22 @@ __device__ __forceinline__ void march_lin(const RenderParams &P, const Ray &ray,
 		}
 		// does this sample need the exact treatment?  (within the margin of the grid edge; at level 0 also of a cell edge)
 		bool exact = false;
-		// V = w >> 16.  It is a non-negative 32-bit number iff the high word of w is in [0, 2^16); the grid extents are
-		// <= 2^30 units, so "inside by the margin" is then a 32-bit statement.
-		const int vx = (int)(wx >> HMRM_LIN_FRAC), vy = (int)(wy >> HMRM_LIN_FRAC);      // low 32 bits: one funnel shift
-		const bool inside = ((unsigned)((unsigned long long)wx >> 32) | (unsigned)((unsigned long long)wy >> 32)) < 65536u &&
-		                    (unsigned)vx - (unsigned)HMRM_LIN_MARGIN < P.lin_span_x && (unsigned)vy - (unsigned)HMRM_LIN_MARGIN < P.lin_span_y;
+		// (j < HMRM_LIN_PERIOD here, as lin_at requires)
+		const int vx = lin_at(lx, j), vy = lin_at(ly, j);
+		const bool inside = (unsigned)vx - (unsigned)HMRM_LIN_MARGIN < P.lin_span_x && (unsigned)vy - (unsigned)HMRM_LIN_MARGIN < P.lin_span_y;
 		if (!inside) {
 			// Certainly outside the grid (main/hmap.cpp:1006-1011)?  The reference truncates toward zero (:1001-1004), so
 			// coordinates in (-1, 0) cells still map to cell 0: the low edge of the grid is at -1 cell, not at 0.
-			const long long fx = wx >> HMRM_LIN_FRAC, fy = wy >> HMRM_LIN_FRAC;
-			const long long low_edge = -(1LL << k) - HMRM_LIN_MARGIN;
-			if (fx < low_edge || fy < low_edge || fx >= (long long)P.lin_grid_x + HMRM_LIN_MARGIN ||
-			    fy >= (long long)P.lin_grid_y + HMRM_LIN_MARGIN) {
+			const int low_edge = -(1 << k) - HMRM_LIN_MARGIN;
+			if (vx < low_edge || vy < low_edge || vx >= (int)P.lin_grid_x + HMRM_LIN_MARGIN || vy >= (int)P.lin_grid_y + HMRM_LIN_MARGIN) {
 				finished = true;
 				break;
 			}
 			exact = true;         // (the whole (-1, 0] strip of the truncation quirk goes the exact way too)
 		}
-		// height: the shifted value fits 32 bits iff the high word is in [-2^15, 2^15); otherwise it is far above or far
-		// below everything the 16-bit pyramid can hold
-		const int wz_hi = (int)(wz >> 32);
-		int vz = (int)(wz >> HMRM_LIN_FRAC);
-		if ((unsigned)(wz_hi + 32768) >= 65536u) vz = wz_hi < 0 ? -1073741824 : 1073741824;
+		// height: from jz_out on, far above or far below everything the 16-bit pyramid can hold
+		int vz = lin_at(lz, j);
+		if (j >= jz_out) vz = lz.di < 0 ? -1073741824 : 1073741824;
 
 		int q = 0;
 		if (!exact) {
@@ -254,11 +282,11 @@ __device__ __forceinline__ void march_lin(const RenderParams &P, const Ray &ray,
 					// room (units) along the direction of motion inside the 3x3 neighbourhood of blocks, clipped to the grid
 					const unsigned w = 1u << (k + level), mask = w - 1u;
 					const unsigned ux = (unsigned)vx, uy = (unsigned)vy;
-					const int room_x = (int)(lx.d >= 0 ? min((ux | mask) + 1u + w, P.lin_grid_x) - ux : min((ux & mask) + w, ux));
-					const int room_y = (int)(ly.d >= 0 ? min((uy | mask) + 1u + w, P.lin_grid_y) - uy : min((uy & mask) + w, uy));
+					const int room_x = (int)(lx.di >= 0 ? min((ux | mask) + 1u + w, P.lin_grid_x) - ux : min((ux & mask) + w, ux));
+					const int room_y = (int)(ly.di >= 0 ? min((uy | mask) + 1u + w, P.lin_grid_y) - uy : min((uy & mask) + w, uy));
 					est_xy = fminf(__int2float_rz(room_x - (HMRM_LIN_MARGIN + 1)) * inv_adx,
 					               __int2float_rz(room_y - (HMRM_LIN_MARGIN + 1)) * inv_ady);
-					est_z = lz.d < 0 ? __int2float_rz(vz - (q << 4) - (HMRM_LIN_ZMARGIN + 2)) * inv_adz : 3.0e38f;
+					est_z = lz.di < 0 ? __int2float_rz(vz - (q << 4) - (HMRM_LIN_ZMARGIN + 2)) * inv_adz : 3.0e38f;
 					// climb while z leaves room for (much) wider blocks and the wider neighbourhood is cleared too
 					if (!(est_z >= P.climb_ratio * est_xy) || level + P.lstride > P.ltop) break;
 					const int q2 = probe(level + P.lstride, vx, vy);
@@ -364,10 +392,6 @@ __device__ __forceinline__ void march_lin(const RenderParams &P, const Ray &ray,
 		}
 next_sample:
 		n += m;
-		{
-			const unsigned jn = n - base;
-			wx = lin_acc(lx, jn); wy = lin_acc(ly, jn); wz = lin_acc(lz, jn);
-		}
 	}
 	}   // if (model)
 
@@ -403,8 +427,8 @@ next_sample:
 	tally.fetches = fetches;
 }
 
-template <bool kStats, int kLayout>
-__global__ void __launch_bounds__(HMRM_LIN_THREADS, HMRM_LIN_CTAS) k2_render_lin(const __grid_constant__ RenderParams P) {
+template <bool kStats, int kLayout, int kCtas>
+__global__ void __launch_bounds__(HMRM_LIN_THREADS, kCtas) k2_render_lin(const __grid_constant__ RenderParams P) {
 	const int lane = threadIdx.x & 31;
 	const unsigned n_tiles = (unsigned)(P.tiles_x * P.tiles_y);
 

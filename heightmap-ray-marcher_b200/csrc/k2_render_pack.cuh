@@ -32,6 +32,24 @@
 
 namespace hmrm {
 
+// launch shape: persistent CTAs of HMRM_LIN_THREADS threads, HMRM_PACK_CTAS of them per SM
+#ifndef HMRM_PACK_CTAS
+#define HMRM_PACK_CTAS 4
+#endif
+
+// This kernel keeps the 64-bit form of the integer model (k2_render_lin.cuh, fact 4): a ray's record holds D and
+// 2^16 V_0 + 2^15 per axis, and V_j = lin_acc(l, j) >> 16.
+struct LinAxis {
+	long long d;     // per-step motion in units * 2^16
+	long long a0;    // V_0 * 2^16 + 2^15: position of the base sample, pre-shifted, with the rounding half added
+};
+
+// 2^16 V_j + (fraction).  One IMAD.WIDE (the 64-bit addend is free) and one IMAD; |a0| < 2^47 + 2^15 and
+// j |D| < 2^17 * 2^42, so it cannot wrap.
+__device__ __forceinline__ long long lin_acc(const LinAxis &l, unsigned j) {
+	return l.a0 + (long long)((unsigned long long)j * (unsigned long long)l.d);
+}
+
 #ifndef HMRM_PACK_THRESH
 #define HMRM_PACK_THRESH 16
 #endif
@@ -511,10 +529,6 @@ __device__ __noinline__ void pack_refill(const RenderParams &P, PackQueue Q, con
 	io[3] = tiles_left ? 1u : 0u;
 	io[4] = 0u;
 }
-
-#ifndef HMRM_PACK_CTAS
-#define HMRM_PACK_CTAS HMRM_LIN_CTAS
-#endif
 
 template <bool kStats, int kLayout>
 __global__ void __launch_bounds__(HMRM_LIN_THREADS, HMRM_PACK_CTAS) k2_render_pack(const __grid_constant__ RenderParams P) {
