@@ -19,6 +19,8 @@ from .binding import (  # noqa: F401
     FLAG_STEP_INDEX,
     FLAG_SUPERSAMPLE_MASK,
     FLAG_SUPERSAMPLE_SHIFT,
+    JPEG_420,
+    JPEG_444,
     LAYOUT_ROWMAJOR,
     LAYOUT_TILE4,
     LAYOUT_ZORDER,
@@ -41,6 +43,7 @@ from .binding import (  # noqa: F401
     camera_basis,
     deg2rad,
     get_ray,
+    jpeg_bound,
     library_path,
     load_library,
     pinned_empty,
@@ -54,5 +57,5 @@ __all__ = [
     "get_ray", "png_bound", "yuv420_bytes", "pinned_empty", "PERSPECTIVE", "SPHERICAL", "ORTHOGRAPHIC", "FP64_EXACT", "FP32_FAST", "TRAVERSAL_AUTO",
     "TRAVERSAL_BRUTE", "TRAVERSAL_SKIP", "TRAVERSAL_PACK", "FLAG_STATS", "FLAG_STEP_INDEX", "FLAG_RAY_DUMP", "PIXEL_RGBA8", "PIXEL_RGB8",
     "LAYOUT_ROWMAJOR", "LAYOUT_TILE4", "LAYOUT_ZORDER", "YUV_BT601", "YUV_BT709",
-    "FLAG_SUPERSAMPLE_SHIFT", "FLAG_SUPERSAMPLE_MASK", "supersample_flag",
+    "FLAG_SUPERSAMPLE_SHIFT", "FLAG_SUPERSAMPLE_MASK", "supersample_flag", "jpeg_bound", "JPEG_420", "JPEG_444",
 ]

@@ -24,6 +24,7 @@ FLAG_SUPERSAMPLE_MASK = 15 << FLAG_SUPERSAMPLE_SHIFT
 PIXEL_RGBA8, PIXEL_RGB8 = 0, 1
 LAYOUT_ROWMAJOR, LAYOUT_TILE4, LAYOUT_ZORDER = 0, 1, 2
 YUV_BT601, YUV_BT709 = 0, 1
+JPEG_420, JPEG_444 = 0, 1
 
 
 class HmrmError(RuntimeError):
@@ -104,6 +105,11 @@ PROTOTYPES = {
     "hmrm_render_png_async": (C.c_int, [C.c_void_p, C.POINTER(Frame), C.c_void_p, C.c_size_t, C.c_void_p]),
     "hmrm_encode_png": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_size_t,
                                   C.c_void_p]),
+    "hmrm_jpeg_bound": (C.c_size_t, [C.c_int32, C.c_int32, C.c_int32]),
+    "hmrm_render_jpeg_async": (C.c_int, [C.c_void_p, C.POINTER(Frame), C.c_int32, C.c_int32, C.c_void_p, C.c_size_t,
+                                         C.c_void_p]),
+    "hmrm_encode_jpeg": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32,
+                                   C.c_void_p, C.c_size_t, C.c_void_p]),
     "hmrm_yuv420_bytes": (C.c_size_t, [C.c_int32, C.c_int32]),
     "hmrm_render_yuv420_async": (C.c_int, [C.c_void_p, C.POINTER(Frame), C.c_int32, C.c_void_p, C.c_size_t]),
     "hmrm_convert_yuv420": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_void_p,
@@ -197,6 +203,12 @@ def supersample_flag(s: int) -> int:
 def png_bound(width: int, height: int, channels: int) -> int:
     """Worst-case PNG file size of a width x height x channels (3 | 4) frame (hmrm_png_bound); 0 for other shapes."""
     return int(load_library().hmrm_png_bound(int(width), int(height), int(channels)))
+
+
+def jpeg_bound(width: int, height: int, chroma: int = JPEG_420) -> int:
+    """Worst-case JPEG file size of a width x height frame in chroma mode JPEG_420 | JPEG_444 (hmrm_jpeg_bound);
+    0 outside [1, 65535] per axis or for another chroma value."""
+    return int(load_library().hmrm_jpeg_bound(int(width), int(height), int(chroma)))
 
 
 def yuv420_bytes(width: int, height: int) -> int:
@@ -402,7 +414,7 @@ class Renderer:
 
     def wait_pending(self, max_pending: int) -> None:
         """Streaming: return once at most `max_pending` (0..3) frames of render_async / render_png_async /
-        render_yuv420_async are still in flight."""
+        render_yuv420_async / render_jpeg_async are still in flight."""
         self._check(self._lib.hmrm_wait_pending(self._h, max_pending))
 
     # -- PNG frames, deflated on the device -------------------------------------------------------
@@ -410,14 +422,7 @@ class Renderer:
         """hmrm_render_png_async: `out` (pinned host or device memory of png_bound bytes or more) receives the PNG file,
         `size_out` (one uint64 in the same kinds of memory) its size, once wait / wait_pending covers the frame.
         numpy arrays and torch tensors report their own sizes; a raw address needs `capacity`."""
-        if capacity is None:
-            capacity = _nbytes(out)
-            if capacity is None:
-                raise ValueError("render_png_async: pass capacity= with a raw output address")
-        size_bytes = _nbytes(size_out)
-        if size_bytes is not None and (size_bytes < 8 or str(getattr(size_out, "dtype", "")).split(".")[-1]
-                                       not in ("uint64", "int64")):
-            raise ValueError("render_png_async: size_out must hold one 64-bit integer")
+        capacity = self._file_capacity("render_png_async", out, size_out, capacity)
         self._check(self._lib.hmrm_render_png_async(self._h, C.byref(frame), _ptr(out), int(capacity), _ptr(size_out)))
 
     def render_png(self, frame: Frame | None = None, **overrides) -> bytes:
@@ -450,6 +455,68 @@ class Renderer:
             cached = (pinned_empty((bound,)), pinned_empty((1,), dtype=np.uint64))
             self._png_cache = cached
         return cached
+
+    # -- JPEG frames, encoded on the device ---------------------------------------------------------
+    def render_jpeg_async(self, frame: Frame, out, size_out, quality: int = 90, chroma: int = JPEG_420,
+                          capacity: int | None = None) -> None:
+        """hmrm_render_jpeg_async: `out` (pinned host or device memory of jpeg_bound bytes or more) receives the JPEG
+        file, `size_out` (one uint64 in the same kinds of memory) its size, once wait / wait_pending covers the frame.
+        numpy arrays and torch tensors report their own sizes; a raw address needs `capacity`."""
+        capacity = self._file_capacity("render_jpeg_async", out, size_out, capacity)
+        self._check(self._lib.hmrm_render_jpeg_async(self._h, C.byref(frame), int(quality), int(chroma), _ptr(out),
+                                                     int(capacity), _ptr(size_out)))
+
+    def render_jpeg(self, frame: Frame | None = None, quality: int = 90, chroma: int = JPEG_420, **overrides) -> bytes:
+        """One frame as a complete JPEG file (include/hmrm.h defines it to the byte)."""
+        f = frame if frame is not None else self.frame(**overrides)
+        out, size = self._jpeg_buffers(f.screen_width, f.screen_height, chroma)
+        self.render_jpeg_async(f, out, size, quality, chroma)
+        self.wait()
+        return out[:int(size[0])].tobytes()
+
+    def encode_jpeg(self, pixels, quality: int = 90, chroma: int = JPEG_420) -> bytes:
+        """[H, W, 3 | 4] uint8 pixels (a numpy array, or a contiguous uint8 CUDA tensor of this device) -> JPEG file,
+        encoded on this context's device."""
+        if hasattr(pixels, "data_ptr") and getattr(pixels, "is_cuda", False):
+            if pixels.dim() != 3 or pixels.shape[2] not in (3, 4) or not pixels.is_contiguous() or \
+                    str(pixels.dtype) != "torch.uint8":
+                raise ValueError("pixels must be a contiguous [H, W, 3] or [H, W, 4] uint8 tensor")
+            h, w, ch = (int(v) for v in pixels.shape)
+            ptr = int(pixels.data_ptr())
+        else:
+            px = np.ascontiguousarray(pixels, dtype=np.uint8)
+            if px.ndim != 3 or px.shape[2] not in (3, 4):
+                raise ValueError("pixels must be [H, W, 3] or [H, W, 4] uint8")
+            h, w, ch = px.shape
+            ptr = px.ctypes.data
+        out, size = self._jpeg_buffers(w, h, chroma)
+        self._check(self._lib.hmrm_encode_jpeg(self._h, ptr, w, h, ch, int(quality), int(chroma), out.ctypes.data,
+                                               out.nbytes, size.ctypes.data))
+        return out[:int(size[0])].tobytes()
+
+    def _jpeg_buffers(self, width: int, height: int, chroma: int):
+        """Pinned file + size buffers, kept while they are large enough (as _png_buffers)."""
+        bound = jpeg_bound(width, height, chroma)
+        if bound == 0:
+            raise ValueError(f"no JPEG of {width}x{height} in chroma mode {chroma}")
+        cached = getattr(self, "_jpeg_cache", None)
+        if cached is None or cached[0].nbytes < bound:
+            cached = (pinned_empty((bound,)), pinned_empty((1,), dtype=np.uint64))
+            self._jpeg_cache = cached
+        return cached[0][:bound], cached[1]
+
+    @staticmethod
+    def _file_capacity(name: str, out, size_out, capacity):
+        """The capacity of a file destination (its own size unless given), after checking the size word."""
+        if capacity is None:
+            capacity = _nbytes(out)
+            if capacity is None:
+                raise ValueError(f"{name}: pass capacity= with a raw output address")
+        size_bytes = _nbytes(size_out)
+        if size_bytes is not None and (size_bytes < 8 or str(getattr(size_out, "dtype", "")).split(".")[-1]
+                                       not in ("uint64", "int64")):
+            raise ValueError(f"{name}: size_out must hold one 64-bit integer")
+        return capacity
 
     # -- 4:2:0 video planes, converted on the device ----------------------------------------------
     def render_yuv420_async(self, frame: Frame, out, matrix: int = YUV_BT709, capacity: int | None = None) -> None:

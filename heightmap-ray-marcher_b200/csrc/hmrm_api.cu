@@ -28,6 +28,7 @@
 #include "k3_png.cuh"
 #include "k4_yuv.cuh"
 #include "k5_downsample.cuh"
+#include "k6_jpeg.cuh"
 #include "peer_sync.cuh"
 #include "render_params.h"
 #include "synth_fbm.h"
@@ -71,6 +72,18 @@ struct PngScratch {
 	unsigned long long *offsets;
 	unsigned long long filt_cap;  // bytes of filtered stream
 	int seg_cap;                  // segments
+};
+
+// K6 scratch of one ring slot: quantised coefficients, AC bit counts and bit offsets per block, the rows' bit buffers
+// and stuffed pieces, row sizes, piece offsets, header / EOI.  Each slot has its own, as with PngScratch.
+struct JpegScratch {
+	int16_t *coef;
+	uint16_t *acbits;
+	uint32_t *boff, *rowbits;
+	uint8_t *stage, *meta;
+	unsigned long long *rowsize, *offsets;
+	unsigned long long blocks_cap, words_cap, stage_cap;   // blocks, row-buffer words, staged bytes
+	int rows_cap;
 };
 
 // The sW x sH RGBA8 render of a supersampled frame, read by K5.  It is reused only after the filter that read it last has
@@ -144,7 +157,9 @@ struct hmrm_ctx {
 	int slot;                    // buffer of the most recent hmrm_render_async
 	// PNG encoding: scratch per ring slot, allocated by the first PNG frame that uses the slot
 	PngScratch png[kFrameRing];
-	uint8_t *d_png_in;           // hmrm_encode_png's / hmrm_convert_yuv420's device copy of the caller's pixels
+	// JPEG encoding: scratch per ring slot, allocated by the first JPEG frame that uses the slot
+	JpegScratch jpeg[kFrameRing];
+	uint8_t *d_png_in;           // hmrm_encode_png's / _jpeg's / hmrm_convert_yuv420's device copy of the caller's pixels
 	size_t png_in_cap;
 	// YUV frames: the I420 planes K4 writes, per ring slot, allocated by the first YUV frame that uses the slot; the copy
 	// engine moves them to the caller's buffer
@@ -928,18 +943,21 @@ int device_view(hmrm_ctx *c, void *p, const char *what, void **dev) {
 	            c->device);
 }
 
-// validates png_out / capacity / png_bytes for a W x H x C file and resolves their device addresses
-int png_outputs(hmrm_ctx *c, const PngShape &s, uint8_t *png_out, size_t capacity, uint64_t *png_bytes, uint8_t **d_out,
-                unsigned long long **d_size) {
-	if (!png_out || !png_bytes) return fail(c, HMRM_ERR_INVALID, "png_out and png_bytes must not be NULL");
-	if ((uintptr_t)png_bytes % 8 != 0) return fail(c, HMRM_ERR_INVALID, "png_bytes must be 8-byte aligned");
-	const unsigned long long bound = png_bound(s);
+// validates the file destination `out` / capacity / size word `bytes` of an encoded file (fmt "png" | "jpeg") whose
+// worst-case size is `bound`, and resolves their device addresses
+int file_outputs(hmrm_ctx *c, const char *fmt, unsigned long long bound, uint8_t *out, size_t capacity, uint64_t *bytes,
+                 uint8_t **d_out, unsigned long long **d_size) {
+	if (!out || !bytes) return fail(c, HMRM_ERR_INVALID, "%s_out and %s_bytes must not be NULL", fmt, fmt);
+	if ((uintptr_t)bytes % 8 != 0) return fail(c, HMRM_ERR_INVALID, "%s_bytes must be 8-byte aligned", fmt);
 	if ((unsigned long long)capacity < bound)
-		return fail(c, HMRM_ERR_INVALID, "capacity %zu is below hmrm_png_bound = %llu", capacity, bound);
+		return fail(c, HMRM_ERR_INVALID, "capacity %zu is below hmrm_%s_bound = %llu", capacity, fmt, bound);
 	HMRM_CUDA(c, cudaSetDevice(c->device));
 	void *o = NULL, *z = NULL;
-	if (int rc = device_view(c, png_out, "png_out", &o)) return rc;
-	if (int rc = device_view(c, png_bytes, "png_bytes", &z)) return rc;
+	char what[32];
+	std::snprintf(what, sizeof what, "%s_out", fmt);
+	if (int rc = device_view(c, out, what, &o)) return rc;
+	std::snprintf(what, sizeof what, "%s_bytes", fmt);
+	if (int rc = device_view(c, bytes, what, &z)) return rc;
 	*d_out = (uint8_t *)o;
 	*d_size = (unsigned long long *)z;
 	return HMRM_OK;
@@ -960,7 +978,8 @@ int enqueue_png(hmrm_ctx *c, int slot, const uint8_t *d_img, int W, int H, int C
 	k3_png_finish<<<1, 1024, 0, st>>>(p.info, s.nseg, s.total, W, H, C, p.offsets, p.meta);
 	const unsigned long long words = png_bound(s) / 16 + 2;
 	const int blocks = (int)std::min((words + 255) / 256, (unsigned long long)c->num_sms * 16ull);
-	k3_png_gather<<<blocks, 256, 0, st>>>(p.offsets, s.nseg + 2, p.meta, p.stage, d_dst, d_size);
+	k3_png_gather<<<blocks, 256, 0, st>>>(p.offsets, s.nseg + 2, p.meta, p.meta + kPngMetaTail, p.stage, kPngStageStride,
+	                                      d_dst, d_size);
 	HMRM_CUDA(c, cudaGetLastError());
 	return HMRM_OK;
 }
@@ -1014,6 +1033,92 @@ int enqueue_yuv(hmrm_ctx *c, int slot, const uint8_t *d_img, int W, int H, int C
 	else k4_yuv420<3><<<grid, kYuvThreads, 0, st>>>(d_img, W, H, kYuvCoef[matrix], c->d_yuv[slot]);
 	HMRM_CUDA(c, cudaGetLastError());
 	HMRM_CUDA(c, cudaMemcpyAsync(out, c->d_yuv[slot], bytes, cudaMemcpyDefault, st));
+	return HMRM_OK;
+}
+
+// The refusals every whole-frame encoder shares (hmrm_render_png_async, _yuv420_async, _jpeg_async); kind names the
+// frames in the messages.
+int check_whole_frame(hmrm_ctx *c, const hmrm_frame *f, const char *kind) {
+	if (!f) return fail(c, HMRM_ERR_INVALID, "frame is NULL");
+	if (int rc = check_supersample(c, f)) return rc;
+	if (f->cycle_period != 1 || f->cycle != 0) return fail(c, HMRM_ERR_INVALID, "%s frames are whole frames: cycle_period 1", kind);
+	if (f->band_count > 1) return fail(c, HMRM_ERR_INVALID, "%s frames are whole frames: band_count <= 1", kind);
+	if (f->flags & (HMRM_FLAG_STEP_INDEX | HMRM_FLAG_RAY_DUMP))
+		return fail(c, HMRM_ERR_INVALID, "%s frames do not record step indices or ray dumps", kind);
+	if (f->row_begin != 0 || (f->row_end != 0 && f->row_end != f->screen_height))
+		return fail(c, HMRM_ERR_INVALID, "%s frames are whole frames: row_begin 0, row_end 0 or screen_height", kind);
+	if (f->pixel_format != HMRM_PIXEL_RGBA8 && f->pixel_format != HMRM_PIXEL_RGB8)
+		return fail(c, HMRM_ERR_INVALID, "unknown pixel_format %d", (int)f->pixel_format);
+	if (f->screen_width < 2 || f->screen_height < 2 || f->screen_width > 65536 || f->screen_height > 65536)
+		return fail(c, HMRM_ERR_INVALID, "resolution %dx%d outside [2,65536]", f->screen_width, f->screen_height);
+	return HMRM_OK;
+}
+
+// ---- JPEG frames (K6, csrc/k6_jpeg.cuh) ----------------------------------------------------------------------------
+void free_jpeg_scratch(JpegScratch &p) {
+	cudaFree(p.coef);
+	cudaFree(p.acbits);
+	cudaFree(p.boff);
+	cudaFree(p.rowbits);
+	cudaFree(p.stage);
+	cudaFree(p.meta);
+	cudaFree(p.rowsize);
+	cudaFree(p.offsets);
+	std::memset(&p, 0, sizeof p);
+}
+
+int ensure_jpeg_scratch(hmrm_ctx *c, int slot, const JpegShape &s) {
+	JpegScratch &p = c->jpeg[slot];
+	const unsigned long long words = s.row_words * (unsigned long long)s.mcuy;
+	const unsigned long long staged = s.row_stride * (unsigned long long)s.mcuy;
+	if (p.coef && p.blocks_cap >= s.blocks && p.words_cap >= words && p.stage_cap >= staged && p.rows_cap >= s.mcuy)
+		return HMRM_OK;
+	// the slot's previous JPEG frame may still be encoding from the buffers about to be replaced
+	if (c->copy_pending[slot]) HMRM_CUDA(c, cudaEventSynchronize(c->ev_copied[slot]));
+	free_jpeg_scratch(p);
+	HMRM_CUDA(c, cudaMalloc(&p.coef, (size_t)s.blocks * 64 * sizeof(int16_t)));
+	HMRM_CUDA(c, cudaMalloc(&p.acbits, (size_t)s.blocks * sizeof(uint16_t)));
+	HMRM_CUDA(c, cudaMalloc(&p.boff, (size_t)s.blocks * sizeof(uint32_t)));
+	HMRM_CUDA(c, cudaMalloc(&p.rowbits, (size_t)words * sizeof(uint32_t)));
+	HMRM_CUDA(c, cudaMalloc(&p.stage, (size_t)staged));
+	HMRM_CUDA(c, cudaMalloc(&p.meta, kJpegMetaBytes));
+	HMRM_CUDA(c, cudaMalloc(&p.rowsize, (size_t)s.mcuy * sizeof(unsigned long long)));
+	HMRM_CUDA(c, cudaMalloc(&p.offsets, ((size_t)s.mcuy + 3) * sizeof(unsigned long long)));
+	p.blocks_cap = s.blocks;
+	p.words_cap = words;
+	p.stage_cap = staged;
+	p.rows_cap = s.mcuy;
+	return HMRM_OK;
+}
+
+int jpeg_params(hmrm_ctx *c, int32_t quality, int32_t chroma) {
+	if (quality < 1 || quality > 100) return fail(c, HMRM_ERR_INVALID, "JPEG quality %d outside [1,100]", quality);
+	if (chroma != HMRM_JPEG_420 && chroma != HMRM_JPEG_444) return fail(c, HMRM_ERR_INVALID, "unknown JPEG chroma %d", chroma);
+	return HMRM_OK;
+}
+
+// Enqueue the K6 launches and K3's gather on `st`: d_img [H][W][C] -> JPEG file at d_dst, its size at d_size.
+int enqueue_jpeg(hmrm_ctx *c, int slot, const uint8_t *d_img, int W, int H, int C, int quality, int chroma,
+                 uint8_t *d_dst, unsigned long long *d_size, cudaStream_t st) {
+	JpegShape s;
+	jpeg_shape(W, H, chroma == HMRM_JPEG_420, &s);
+	if (int rc = ensure_jpeg_scratch(c, slot, s)) return rc;
+	const JpegScratch &p = c->jpeg[slot];
+	const int tile_mcus = kJpegTileBlocks / s.bpm;
+	const dim3 grid((unsigned)((s.mcux + tile_mcus - 1) / tile_mcus), (unsigned)s.mcuy);
+	const JpegQuant q = jpeg_quant(quality);
+	if (C == 4 && s.s420) k6_jpeg_blocks<4, true><<<grid, kJpegBlockThreads, 0, st>>>(d_img, W, H, s.mcux, q, p.coef, p.acbits);
+	else if (C == 4) k6_jpeg_blocks<4, false><<<grid, kJpegBlockThreads, 0, st>>>(d_img, W, H, s.mcux, q, p.coef, p.acbits);
+	else if (s.s420) k6_jpeg_blocks<3, true><<<grid, kJpegBlockThreads, 0, st>>>(d_img, W, H, s.mcux, q, p.coef, p.acbits);
+	else k6_jpeg_blocks<3, false><<<grid, kJpegBlockThreads, 0, st>>>(d_img, W, H, s.mcux, q, p.coef, p.acbits);
+	k6_jpeg_rows<<<s.mcuy, kJpegRowThreads, 0, st>>>(p.coef, p.acbits, s.mcux, s.bpm, s.mcuy, p.boff, p.rowbits,
+	                                                 s.row_words, p.stage, s.row_stride, p.rowsize);
+	k6_jpeg_finish<<<1, 1024, 0, st>>>(p.rowsize, s.mcuy, jpeg_header(s, quality), p.offsets, p.meta);
+	const unsigned long long words = jpeg_bound(s) / 16 + 2;
+	const int blocks = (int)std::min((words + 255) / 256, (unsigned long long)c->num_sms * 16ull);
+	k3_png_gather<<<blocks, 256, 0, st>>>(p.offsets, s.mcuy + 2, p.meta, p.meta + kJpegMetaTail, p.stage, s.row_stride,
+	                                      d_dst, d_size);
+	HMRM_CUDA(c, cudaGetLastError());
 	return HMRM_OK;
 }
 
@@ -1122,6 +1227,7 @@ int hmrm_create(int device, hmrm_ctx **out) {
 	c->slot = 0;
 	c->fb_format = HMRM_PIXEL_RGBA8;
 	std::memset(c->png, 0, sizeof c->png);
+	std::memset(c->jpeg, 0, sizeof c->jpeg);
 	c->d_png_in = NULL;
 	c->png_in_cap = 0;
 	std::memset(c->d_yuv, 0, sizeof c->d_yuv);
@@ -1178,6 +1284,7 @@ void hmrm_destroy(hmrm_ctx *c) {
 	cudaFree(c->d_png_in);
 	for (int i = 0; i < kFrameRing; ++i) {
 		free_png_scratch(c->png[i]);
+		free_jpeg_scratch(c->jpeg[i]);
 		cudaFree(c->d_yuv[i]);
 		cudaFree(c->d_fb[i]);
 		if (c->ev_rendered[i]) cudaEventDestroy(c->ev_rendered[i]);
@@ -1553,24 +1660,13 @@ size_t hmrm_png_bound(int32_t width, int32_t height, int32_t channels) {
 
 int hmrm_render_png_async(hmrm_ctx *c, const hmrm_frame *f, uint8_t *png_out, size_t capacity, uint64_t *png_bytes) {
 	if (!c) return HMRM_ERR_INVALID;
-	if (!f) return fail(c, HMRM_ERR_INVALID, "frame is NULL");
-	if (int rc = check_supersample(c, f)) return rc;
-	if (f->cycle_period != 1 || f->cycle != 0) return fail(c, HMRM_ERR_INVALID, "PNG frames are whole frames: cycle_period 1");
-	if (f->band_count > 1) return fail(c, HMRM_ERR_INVALID, "PNG frames are whole frames: band_count <= 1");
-	if (f->flags & (HMRM_FLAG_STEP_INDEX | HMRM_FLAG_RAY_DUMP))
-		return fail(c, HMRM_ERR_INVALID, "PNG frames do not record step indices or ray dumps");
-	if (f->row_begin != 0 || (f->row_end != 0 && f->row_end != f->screen_height))
-		return fail(c, HMRM_ERR_INVALID, "PNG frames are whole frames: row_begin 0, row_end 0 or screen_height");
-	if (f->pixel_format != HMRM_PIXEL_RGBA8 && f->pixel_format != HMRM_PIXEL_RGB8)
-		return fail(c, HMRM_ERR_INVALID, "unknown pixel_format %d", (int)f->pixel_format);
-	if (f->screen_width < 2 || f->screen_height < 2 || f->screen_width > 65536 || f->screen_height > 65536)
-		return fail(c, HMRM_ERR_INVALID, "resolution %dx%d outside [2,65536]", f->screen_width, f->screen_height);
+	if (int rc = check_whole_frame(c, f, "PNG")) return rc;
 	const int C = f->pixel_format == HMRM_PIXEL_RGB8 ? 3 : 4;
-	PngShape s;
+	PngShape s{};
 	png_shape(f->screen_width, f->screen_height, C, &s);
 	uint8_t *d_out = NULL;
 	unsigned long long *d_size = NULL;
-	int rc = png_outputs(c, s, png_out, capacity, png_bytes, &d_out, &d_size);
+	int rc = file_outputs(c, "png", png_bound(s), png_out, capacity, png_bytes, &d_out, &d_size);
 	if (rc) return rc;
 	if ((rc = ensure_framebuffer(c, f->screen_width, f->screen_height, f->pixel_format)) != HMRM_OK) return rc;
 	// the ring exactly as hmrm_render_async uses it for whole frames; the encoder takes the place of the copy-out
@@ -1600,7 +1696,7 @@ int hmrm_encode_png(hmrm_ctx *c, const uint8_t *pixels, int32_t width, int32_t h
 		            height, channels);
 	uint8_t *d_out = NULL;
 	unsigned long long *d_size = NULL;
-	int rc = png_outputs(c, s, png_out, capacity, png_bytes, &d_out, &d_size);
+	int rc = file_outputs(c, "png", png_bound(s), png_out, capacity, png_bytes, &d_out, &d_size);
 	if (rc) return rc;
 	// synchronous: whatever the context has in flight finishes first, then ring slot 0's scratch is free
 	if ((rc = drain(c)) != HMRM_OK) return rc;
@@ -1610,22 +1706,73 @@ int hmrm_encode_png(hmrm_ctx *c, const uint8_t *pixels, int32_t width, int32_t h
 	return HMRM_OK;
 }
 
+size_t hmrm_jpeg_bound(int32_t width, int32_t height, int32_t chroma) {
+	JpegShape s;
+	if ((chroma != HMRM_JPEG_420 && chroma != HMRM_JPEG_444) || !jpeg_shape(width, height, chroma == HMRM_JPEG_420, &s))
+		return 0;
+	return (size_t)jpeg_bound(s);
+}
+
+int hmrm_render_jpeg_async(hmrm_ctx *c, const hmrm_frame *f, int32_t quality, int32_t chroma, uint8_t *jpeg_out,
+                           size_t capacity, uint64_t *jpeg_bytes) {
+	if (!c) return HMRM_ERR_INVALID;
+	if (int rc = check_whole_frame(c, f, "JPEG")) return rc;
+	if (int rc = jpeg_params(c, quality, chroma)) return rc;
+	JpegShape s;
+	if (!jpeg_shape(f->screen_width, f->screen_height, chroma == HMRM_JPEG_420, &s))
+		return fail(c, HMRM_ERR_INVALID, "resolution %dx%d: a JPEG frame is at most 65535 pixels per axis",
+		            f->screen_width, f->screen_height);
+	const int C = f->pixel_format == HMRM_PIXEL_RGB8 ? 3 : 4;
+	uint8_t *d_out = NULL;
+	unsigned long long *d_size = NULL;
+	int rc = file_outputs(c, "jpeg", jpeg_bound(s), jpeg_out, capacity, jpeg_bytes, &d_out, &d_size);
+	if (rc) return rc;
+	if ((rc = ensure_framebuffer(c, f->screen_width, f->screen_height, f->pixel_format)) != HMRM_OK) return rc;
+	// the ring exactly as hmrm_render_async uses it for whole frames; the encoder takes the place of the copy-out
+	const int slot = (c->slot + 1) % kFrameRing;
+	if ((rc = ensure_jpeg_scratch(c, slot, s)) != HMRM_OK) return rc;
+	uint32_t *fb = c->d_fb[slot];
+	cudaStream_t cs = c->ring_stream[slot];
+	if (c->copy_pending[slot]) HMRM_CUDA(c, cudaStreamWaitEvent(cs, c->ev_copied[slot], 0));
+	if ((rc = enqueue_frame(c, f, fb, cs)) != HMRM_OK) return rc;
+	HMRM_CUDA(c, cudaEventRecord(c->ev_rendered[slot], cs));
+	HMRM_CUDA(c, cudaStreamWaitEvent(c->copy_stream, c->ev_rendered[slot], 0));
+	rc = enqueue_jpeg(c, slot, (const uint8_t *)fb, f->screen_width, f->screen_height, C, quality, chroma, d_out, d_size,
+	                  c->copy_stream);
+	if (rc) return rc;
+	HMRM_CUDA(c, cudaEventRecord(c->ev_copied[slot], c->copy_stream));
+	c->copy_pending[slot] = true;
+	c->slot = slot;
+	return HMRM_OK;
+}
+
+int hmrm_encode_jpeg(hmrm_ctx *c, const uint8_t *pixels, int32_t width, int32_t height, int32_t channels,
+                     int32_t quality, int32_t chroma, uint8_t *jpeg_out, size_t capacity, uint64_t *jpeg_bytes) {
+	if (!c) return HMRM_ERR_INVALID;
+	if (!pixels) return fail(c, HMRM_ERR_INVALID, "pixels is NULL");
+	if (int rc = jpeg_params(c, quality, chroma)) return rc;
+	JpegShape s;
+	if (!jpeg_shape(width, height, chroma == HMRM_JPEG_420, &s) || (channels != 3 && channels != 4))
+		return fail(c, HMRM_ERR_INVALID, "image %dx%dx%d: need 1 <= width, height <= 65535 and 3 or 4 channels", width,
+		            height, channels);
+	uint8_t *d_out = NULL;
+	unsigned long long *d_size = NULL;
+	int rc = file_outputs(c, "jpeg", jpeg_bound(s), jpeg_out, capacity, jpeg_bytes, &d_out, &d_size);
+	if (rc) return rc;
+	// synchronous: whatever the context has in flight finishes first, then ring slot 0's scratch is free
+	if ((rc = drain(c)) != HMRM_OK) return rc;
+	if ((rc = stage_pixels(c, pixels, (size_t)width * (size_t)height * (size_t)channels)) != HMRM_OK) return rc;
+	rc = enqueue_jpeg(c, 0, c->d_png_in, width, height, channels, quality, chroma, d_out, d_size, c->stream);
+	if (rc) return rc;
+	HMRM_CUDA(c, cudaStreamSynchronize(c->stream));
+	return HMRM_OK;
+}
+
 size_t hmrm_yuv420_bytes(int32_t width, int32_t height) { return (size_t)yuv420_bytes(width, height); }
 
 int hmrm_render_yuv420_async(hmrm_ctx *c, const hmrm_frame *f, int32_t matrix, uint8_t *out, size_t capacity) {
 	if (!c) return HMRM_ERR_INVALID;
-	if (!f) return fail(c, HMRM_ERR_INVALID, "frame is NULL");
-	if (int rc = check_supersample(c, f)) return rc;
-	if (f->cycle_period != 1 || f->cycle != 0) return fail(c, HMRM_ERR_INVALID, "YUV frames are whole frames: cycle_period 1");
-	if (f->band_count > 1) return fail(c, HMRM_ERR_INVALID, "YUV frames are whole frames: band_count <= 1");
-	if (f->flags & (HMRM_FLAG_STEP_INDEX | HMRM_FLAG_RAY_DUMP))
-		return fail(c, HMRM_ERR_INVALID, "YUV frames do not record step indices or ray dumps");
-	if (f->row_begin != 0 || (f->row_end != 0 && f->row_end != f->screen_height))
-		return fail(c, HMRM_ERR_INVALID, "YUV frames are whole frames: row_begin 0, row_end 0 or screen_height");
-	if (f->pixel_format != HMRM_PIXEL_RGBA8 && f->pixel_format != HMRM_PIXEL_RGB8)
-		return fail(c, HMRM_ERR_INVALID, "unknown pixel_format %d", (int)f->pixel_format);
-	if (f->screen_width < 2 || f->screen_height < 2 || f->screen_width > 65536 || f->screen_height > 65536)
-		return fail(c, HMRM_ERR_INVALID, "resolution %dx%d outside [2,65536]", f->screen_width, f->screen_height);
+	if (int rc = check_whole_frame(c, f, "YUV")) return rc;
 	const int W = f->screen_width, H = f->screen_height, C = f->pixel_format == HMRM_PIXEL_RGB8 ? 3 : 4;
 	int rc = yuv_output(c, W, H, matrix, out, capacity);
 	if (rc) return rc;

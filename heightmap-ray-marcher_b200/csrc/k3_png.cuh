@@ -15,7 +15,8 @@
 //                   constant signature / IHDR and the last IDAT (final empty fixed block 03 00 + Adler-32) + IEND;
 //   k3_png_gather   output-driven: each thread assembles one aligned 16-byte word of the file (binary search of the
 //                   piece offsets) and stores it, so the stores stay aligned and coalesced even when the destination is
-//                   pinned host memory written over PCIe; it also stores the file size.
+//                   pinned host memory written over PCIe; it also stores the file size.  K6 (JPEG) writes its files
+//                   with it too: any file made of a head piece, pieces at a fixed stride and a tail piece.
 // A segment may match back across its start (never before byte 0 of the stream) but never past its end, and a match is
 // at most 258 bytes: the block decodes with any inflate.
 #pragma once
@@ -31,7 +32,6 @@ constexpr int kPngMaskWords = kPngSeg / 32 + 4;   // + zero words read past the 
 constexpr int kPngHeadBytes = 33;                  // signature + IHDR chunk
 constexpr int kPngTailBytes = 30;                  // last IDAT chunk (6 data bytes) + IEND chunk
 constexpr int kPngMetaTail = 64;                   // offset of the tail piece inside the meta buffer
-constexpr int kPngMetaTotal = 128;                 // offset of the file size (uint64) inside the meta buffer
 constexpr int kPngMetaBytes = 256;
 
 struct PngSegInfo {
@@ -423,7 +423,6 @@ __global__ void __launch_bounds__(1024) k3_png_finish(const PngSegInfo *__restri
 		offsets[0] = 0;
 		offsets[nseg + 1] = off;
 		offsets[nseg + 2] = off + kPngTailBytes;
-		*(unsigned long long *)(meta + kPngMetaTotal) = off + kPngTailBytes;
 	}
 	if (t == 0) {
 		static const uint8_t sig[8] = {137, 80, 78, 71, 13, 10, 26, 10};
@@ -450,18 +449,21 @@ __global__ void __launch_bounds__(1024) k3_png_finish(const PngSegInfo *__restri
 	}
 }
 
-__device__ __forceinline__ const uint8_t *png_piece(int i, int npieces, const uint8_t *meta, const uint8_t *stage) {
-	if (i == 0) return meta;
-	if (i == npieces - 1) return meta + kPngMetaTail;
-	return stage + (size_t)(i - 1) * kPngStageStride;
+// piece 0 is `first`, piece npieces - 1 is `last`, piece i between them starts at stage + (i - 1) * stride
+__device__ __forceinline__ const uint8_t *png_piece(int i, int npieces, const uint8_t *first, const uint8_t *last,
+                                                    const uint8_t *stage, unsigned long long stride) {
+	if (i == 0) return first;
+	if (i == npieces - 1) return last;
+	return stage + (unsigned long long)(i - 1) * stride;
 }
 
 // Each thread writes the bytes of one 16-byte-aligned word of the destination (word -1: the bytes before the first
-// aligned address).  Grid-stride; the file size is read from the meta buffer.
+// aligned address).  Grid-stride; offsets[0..npieces]: where each piece starts in the file, then the file size.
 __global__ void __launch_bounds__(256) k3_png_gather(const unsigned long long *__restrict__ offsets, int npieces,
-                                                     const uint8_t *__restrict__ meta, const uint8_t *__restrict__ stage,
+                                                     const uint8_t *__restrict__ first, const uint8_t *__restrict__ final_piece,
+                                                     const uint8_t *__restrict__ stage, unsigned long long piece_stride,
                                                      uint8_t *dst, unsigned long long *size_out) {
-	const unsigned long long total = *(const unsigned long long *)(meta + kPngMetaTotal);
+	const unsigned long long total = offsets[npieces];
 	const unsigned long long head = (16u - ((uintptr_t)dst & 15u)) & 15u;
 	const long long last = total > head ? (long long)((total - head + 15) / 16) - 1 : -1;
 	const long long stride = (long long)gridDim.x * blockDim.x;
@@ -482,13 +484,13 @@ __global__ void __launch_bounds__(256) k3_png_gather(const unsigned long long *_
 		}
 		int i = a;
 		unsigned long long end = offsets[i + 1];
-		const uint8_t *src = png_piece(i, npieces, meta, stage) - offsets[i];
+		const uint8_t *src = png_piece(i, npieces, first, final_piece, stage, piece_stride) - offsets[i];
 		const bool whole = hi - lo == 16 && lo_s >= 0;
 		unsigned long long w0 = 0, w1 = 0;
 		for (unsigned long long k = lo; k < hi; ++k) {
 			while (k >= end) {
 				i += 1;
-				src = png_piece(i, npieces, meta, stage) - offsets[i];
+				src = png_piece(i, npieces, first, final_piece, stage, piece_stride) - offsets[i];
 				end = offsets[i + 1];
 			}
 			const unsigned long long v = src[k];

@@ -237,6 +237,50 @@ int hmrm_render_yuv420_async(hmrm_ctx *ctx, const hmrm_frame *f, int32_t matrix,
 int hmrm_convert_yuv420(hmrm_ctx *ctx, const uint8_t *pixels, int32_t width, int32_t height, int32_t channels,
                         int32_t matrix, uint8_t *out, size_t capacity);
 
+/* ---- JPEG frames, encoded on the device (kernel K6, csrc/k6_jpeg.cuh) ----
+ * A JPEG frame is exactly the file libjpeg-turbo writes for the frame's R, G, B (alpha ignored) with baseline coding,
+ * the standard tables, IJG quality scaling and one restart interval per MCU row; in Pillow's words
+ *   Image.fromarray(rgb).save(f, "JPEG", quality=q, subsampling=2 (4:2:0) or 0 (4:4:4), restart_marker_rows=1).
+ * All integer; >> is an arithmetic shift:
+ * 1. Colour, JFIF full-range BT.601 in 2^-16 fixed point (not K4's limited-range matrix):
+ *      Y  = (19595 R + 38470 G + 7471 B + 32768) >> 16
+ *      Cb = (-11059 R - 21709 G + 32768 B + 8421375) >> 16
+ *      Cr = (32768 R - 27439 G - 5329 B + 8421375) >> 16
+ * 2. Planes.  Y, and all three planes in 4:4:4: columns replicated to a multiple of 8, rows to whole MCU rows (16 rows
+ *    for 4:2:0 luma, 8 otherwise).  4:2:0 chroma: source columns replicated to 16 ceil(ceil(W/2)/8), an odd last source
+ *    row duplicated, each sample (a + b + c + d + bias) >> 2 over its 2x2 source block with bias 1, 2, 1, 2, ... by
+ *    output column, then chroma rows replicated down to a multiple of 8 (libjpeg's order; not "pad, then downsample").
+ * 3. Blocks: libjpeg's jfdctint ("islow") forward DCT on sample - 128; the Annex K.1 tables scaled by quality,
+ *    s = q < 50 ? 5000 / q : 200 - 2q, entry = clamp((base s + 50) / 100, 1, 255); a coefficient c against entry t
+ *    becomes (|c| + 4t) / (8t), truncated, with c's sign.  In 4:2:0 a luma block of an MCU outside
+ *    ceil(W/8) x ceil(H/8) is a dummy block: AC 0, DC copied from the block to its left, or, in a bottom dummy row, from
+ *    the last block of the MCU's row above.
+ * 4. Entropy coding: the Annex K.3 Huffman tables; a DC predictor per component, reset at every restart; the restart
+ *    interval is one MCU row (DRI = MCUs per row, RST0 .. RST7 cyclically); padding before a marker and at the end is
+ *    1-bits; 0xFF in the data is stuffed as FF 00.
+ * 5. Markers: SOI; APP0 JFIF 1.01 (density units 0, 1x1, no thumbnail); DQT 0 (luma), DQT 1 (chroma), zig-zag order;
+ *    SOF0 (8 bit; components 1, 2, 3, sampling 0x22 / 0x11 / 0x11 or 0x11 x 3, tables 0 / 1 / 1); DHT DC0, AC0, DC1,
+ *    AC1; DRI; SOS (03 01 00 02 11 03 11 00 3f 00); the data; EOI.  The header is 629 bytes, EOI adds 2.
+ * Sizes run from 1 to 65535 per axis (SOF0's fields are 16 bits), quality from 1 to 100. */
+#define HMRM_JPEG_420 0
+#define HMRM_JPEG_444 1
+/* Worst-case file size, 0 outside the limits; host arithmetic.  With B the blocks including 4:2:0's dummies (MCUs x 6
+ * or x 3) and R the MCU rows: 631 + 415 B + 4 R.  Proof: a block codes at most 11 + 11 DC bits (code, then |diff| <=
+ * 2047) and, per AC position, at most 16 + 10 bits (a ZRL covers 16 positions with 11 bits, EOB replaces a zero
+ * position with at most 16), so 1660 bits; a row of b blocks is at most ceil(1660 b / 8) <= 207.5 b + 1 bytes with its
+ * padding, at most 415 b + 2 after stuffing, + 2 for its RST marker; + 629 + 2 for the header and EOI. */
+size_t hmrm_jpeg_bound(int32_t width, int32_t height, int32_t chroma);
+/* hmrm_render_png_async, but the frame leaves the device as a JPEG file of quality 1..100 and chroma HMRM_JPEG_420 |
+ * HMRM_JPEG_444: the same refusals (whole frames only), destinations (pinned / registered host or device memory, any
+ * alignment; jpeg_bytes 8-byte aligned) and four-frame ring, shared with raw, PNG and YUV frames; HMRM_FLAG_SUPERSAMPLE
+ * is accepted.  A frame above 65535 pixels per axis is HMRM_ERR_INVALID. */
+int hmrm_render_jpeg_async(hmrm_ctx *ctx, const hmrm_frame *f, int32_t quality, int32_t chroma, uint8_t *jpeg_out,
+                           size_t capacity, uint64_t *jpeg_bytes);
+/* encode caller pixels ([height][width][channels], channels 3 | 4, host or device memory, copied to the device);
+ * synchronous.  jpeg_out / jpeg_bytes as for hmrm_render_jpeg_async. */
+int hmrm_encode_jpeg(hmrm_ctx *ctx, const uint8_t *pixels, int32_t width, int32_t height, int32_t channels,
+                     int32_t quality, int32_t chroma, uint8_t *jpeg_out, size_t capacity, uint64_t *jpeg_bytes);
+
 int hmrm_get_stats(hmrm_ctx *ctx, hmrm_stats *out);            /* of the last render */
 /* traversal diagnostics of the last HMRM_FLAG_STATS render with a skip traversal: [0] jumps, [1] samples covered
  * by jumps, [2] single steps above a mip block, [3] level descents, [4] cell tests above the cell, [5] cell tests
