@@ -36,6 +36,7 @@ from .binding import (  # noqa: F401
     TRAVERSAL_SKIP_FP64,
     YUV_BT601,
     YUV_BT709,
+    Camera,
     Frame,
     HmrmError,
     Renderer,
@@ -53,7 +54,7 @@ from .binding import (  # noqa: F401
 )
 
 __all__ = [
-    "Renderer", "Frame", "Stats", "HmrmError", "load_library", "library_path", "deg2rad", "camera_basis",
+    "Renderer", "Frame", "Camera", "Stats", "HmrmError", "load_library", "library_path", "deg2rad", "camera_basis",
     "get_ray", "png_bound", "yuv420_bytes", "pinned_empty", "PERSPECTIVE", "SPHERICAL", "ORTHOGRAPHIC", "FP64_EXACT", "FP32_FAST", "TRAVERSAL_AUTO",
     "TRAVERSAL_BRUTE", "TRAVERSAL_SKIP", "TRAVERSAL_PACK", "FLAG_STATS", "FLAG_STEP_INDEX", "FLAG_RAY_DUMP", "PIXEL_RGBA8", "PIXEL_RGB8",
     "LAYOUT_ROWMAJOR", "LAYOUT_TILE4", "LAYOUT_ZORDER", "YUV_BT601", "YUV_BT709",

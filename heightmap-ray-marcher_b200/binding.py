@@ -61,6 +61,16 @@ class Frame(C.Structure):
     ]
 
 
+class Camera(C.Structure):
+    """`hmrm_camera`: one motion-blur sub-frame's camera (angles in radians, as in Frame)."""
+
+    _fields_ = [
+        ("cam_pos", C.c_double * 3),
+        ("hang", C.c_double),
+        ("vang", C.c_double),
+    ]
+
+
 class Stats(C.Structure):
     """`hmrm_stats`."""
 
@@ -93,6 +103,7 @@ PROTOTYPES = {
     "hmrm_synth_maps16": (C.c_int, [C.c_void_p, C.c_uint32, C.c_uint32]),
     "hmrm_set_layout": (C.c_int, [C.c_void_p, C.c_int]),
     "hmrm_get_layout": (C.c_int, [C.c_void_p]),
+    "hmrm_set_motion_blur": (C.c_int, [C.c_void_p, C.POINTER(Camera), C.c_int32]),
     "hmrm_update_heightmap": (C.c_int, [C.c_void_p, C.POINTER(C.c_double), C.c_double, C.c_double]),
     "hmrm_get_heights": (C.c_int, [C.c_void_p, C.c_void_p]),
     "hmrm_frame_defaults": (None, [C.POINTER(Frame)]),
@@ -367,6 +378,27 @@ class Renderer:
 
     def get_layout(self) -> int:
         return int(self._lib.hmrm_get_layout(self._h))
+
+    def set_motion_blur(self, cams) -> None:
+        """Motion blur of every following whole-frame render (include/hmrm.h, hmrm_set_motion_blur): `cams` is a
+        sequence of (pos, hang, vang) with pos three numbers and angles in radians, or an [n, 5] float64 array of rows
+        (x, y, z, hang, vang); n = 1..16.  `[]` turns blur off."""
+        rows = np.asarray(cams, dtype=np.float64) if isinstance(cams, np.ndarray) else None
+        if rows is None:
+            flat = []
+            for pos, hang, vang in cams:
+                pos = [float(v) for v in pos]
+                if len(pos) != 3:
+                    raise ValueError(f"a motion-blur camera's pos has three components, not {len(pos)}")
+                flat.append([*pos, float(hang), float(vang)])
+            rows = np.array(flat, dtype=np.float64).reshape(-1, 5)
+        if rows.ndim != 2 or rows.shape[1] != 5:
+            raise ValueError(f"motion-blur cameras must be [n, 5], not {rows.shape}")
+        arr = (Camera * max(len(rows), 1))()
+        for i, r in enumerate(rows):
+            arr[i].cam_pos[:] = [float(v) for v in r[:3]]
+            arr[i].hang, arr[i].vang = float(r[3]), float(r[4])
+        self._check(self._lib.hmrm_set_motion_blur(self._h, arr, len(rows)))
 
     def heights(self) -> np.ndarray:
         out = np.empty((self.map_height, self.map_width), dtype=np.float64)

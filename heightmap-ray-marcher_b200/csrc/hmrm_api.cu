@@ -41,7 +41,8 @@ std::string g_create_error;
 
 const int kLaunchSlots = 8;
 const int kFrameRing = 4;      // device frame buffers (and compute streams) whole frames rotate through
-const int kSubFrames = 4;      // supersampled sub-frame scratches, used round-robin
+const int kSubFrames = 4;      // sub-frame scratches of supersampled / motion-blurred frames, used round-robin
+const int kBlurMax = 16;       // most motion-blur sub-frames (hmrm_set_motion_blur)
 
 // Everything one launch writes before / while its kernel runs.  A slot is reused only after the kernel that used
 // it last has finished (ev_end), so up to kLaunchSlots frames of one context may be in flight on any streams.
@@ -86,11 +87,15 @@ struct JpegScratch {
 	int rows_cap;
 };
 
-// The sW x sH RGBA8 render of a supersampled frame, read by K5.  It is reused only after the filter that read it last has
-// run (ev_read), so up to kSubFrames supersampled frames of one context may be in flight on any streams.
+// The sW x sH RGBA8 renders of one supersampled or motion-blurred frame, read by K5: up to kDownMaxPlanes planes, and
+// K5's accumulator when a blurred frame has more sub-frames than planes.  Inside the frame the planes are reused in
+// stream order; across frames the scratch is reused only after the filter that read it last has run (ev_read), so up to
+// kSubFrames such frames of one context may be in flight on any streams.
 struct SubFrame {
 	uint32_t *d;
 	size_t cap;                   // bytes
+	uint2 *acc;                   // [H][W] sums (K5's kK5First .. kK5Last)
+	size_t acc_cap;               // bytes
 	cudaEvent_t ev_read;
 	bool used;
 };
@@ -168,6 +173,9 @@ struct hmrm_ctx {
 	// supersampled frames (K5): sub-frame scratches, allocated by the first supersampled frame that uses them
 	SubFrame sub[kSubFrames];
 	int sub_next;
+	// motion blur (hmrm_set_motion_blur): blur_n sub-frame cameras, 0 = off; read when a frame is enqueued
+	int blur_n;
+	hmrm_camera blur_cams[kBlurMax];
 
 	// per-launch resources, used round-robin so that up to kLaunchSlots kernels of this context may be in flight
 	LaunchSlot slots[kLaunchSlots];
@@ -400,8 +408,12 @@ __global__ void k_reset_slot(unsigned int *tile_counter, unsigned int *stats_wor
 	for (unsigned i = threadIdx.x; i < sizeof(DeviceStats) / 4; i += 32) stats_words[i] = 0u;
 }
 
-// Enqueue one frame on `stream`, writing the frame's pixel format into d_out (any alignment).
-int enqueue_render(hmrm_ctx *c, const hmrm_frame *f, uint32_t *d_out, cudaStream_t stream, bool timed) {
+// Enqueue one frame on `stream`, writing the frame's pixel format into d_out (any alignment).  acc_slot >= 0: a later
+// sub-frame of a motion-blurred frame whose first sub-frame used launch slot acc_slot (on the same stream).  Its
+// statistics add into that slot's block (no reset), the slot's ev_end moves past this kernel, and hmrm_get_stats then
+// reports that slot: the sums over the sub-frames, timed from the first one's start to the last one's end.
+int enqueue_render(hmrm_ctx *c, const hmrm_frame *f, uint32_t *d_out, cudaStream_t stream, bool timed,
+                   int acc_slot = -1) {
 	int row_begin = 0, row_end = 0;
 	int rc = validate_frame(c, f, &row_begin, &row_end);
 	if (rc) return rc;
@@ -409,7 +421,9 @@ int enqueue_render(hmrm_ctx *c, const hmrm_frame *f, uint32_t *d_out, cudaStream
 	const int W = f->screen_width, H = f->screen_height;
 	if ((rc = ensure_tables(c, W, H)) != HMRM_OK) return rc;
 
-	// take a launch slot; wait (host side) for the kernel that used it kLaunchSlots launches ago
+	// take a launch slot; wait (host side) for the kernel that used it kLaunchSlots launches ago.  A blurred frame's
+	// later sub-frames skip the slot that accumulates its statistics: its ev_end is their own latest kernel.
+	if (c->launch_next == acc_slot) c->launch_next = (acc_slot + 1) % kLaunchSlots;
 	const int ls = c->launch_next;
 	c->launch_next = (ls + 1) % kLaunchSlots;
 	LaunchSlot &slot = c->slots[ls];
@@ -586,10 +600,11 @@ int enqueue_render(hmrm_ctx *c, const hmrm_frame *f, uint32_t *d_out, cudaStream
 		HMRM_CUDA(c, cudaMemsetAsync(slot.d_ray_dump, 0xFF, need * 80, stream));    // NaN = not rendered
 		P.ray_dump = slot.d_ray_dump;
 	}
-	P.stats = slot.d_stats;
+	P.stats = acc_slot >= 0 ? c->slots[acc_slot].d_stats : slot.d_stats;
 	P.tile_counter = slot.d_tile_counter;
 
-	if (!c->knobs.reset_kernel) {
+	if (acc_slot >= 0) HMRM_CUDA(c, cudaMemsetAsync(slot.d_tile_counter, 0, sizeof(unsigned int), stream));
+	else if (!c->knobs.reset_kernel) {
 		HMRM_CUDA(c, cudaMemsetAsync(slot.d_tile_counter, 0, sizeof(unsigned int), stream));
 		HMRM_CUDA(c, cudaMemsetAsync(slot.d_stats, 0, sizeof(DeviceStats), stream));
 	}
@@ -709,6 +724,10 @@ int enqueue_render(hmrm_ctx *c, const hmrm_frame *f, uint32_t *d_out, cudaStream
 	HMRM_CUDA(c, cudaEventRecord(slot.ev_end, stream));
 	slot.used = true;
 	c->launch_last = ls;
+	if (acc_slot >= 0) {
+		HMRM_CUDA(c, cudaEventRecord(c->slots[acc_slot].ev_end, stream));
+		c->launch_last = acc_slot;
+	}
 
 	c->last_stream = stream;
 	c->last_had_stats = want_stats;
@@ -720,51 +739,94 @@ int enqueue_render(hmrm_ctx *c, const hmrm_frame *f, uint32_t *d_out, cudaStream
 	return HMRM_OK;
 }
 
-// ---- supersampled frames (K5, csrc/k5_downsample.cuh) --------------------------------------------------------------
+// ---- supersampled and motion-blurred frames (K5, csrc/k5_downsample.cuh) -------------------------------------------
 int supersample_of(const hmrm_frame *f) {
 	return (int)((f->flags & HMRM_FLAG_SUPERSAMPLE_MASK) >> HMRM_FLAG_SUPERSAMPLE_SHIFT) + 1;
 }
 
-// The supersample field of a frame for the entry points that accept it: s = 1..4, and s > 1 for whole frames only.
+// The supersample field of a frame for the entry points that accept it, s = 1..4, and the context's motion blur: frames
+// with s > 1 or blur are whole frames only.
 int check_supersample(hmrm_ctx *c, const hmrm_frame *f) {
 	const int s = supersample_of(f);
 	if (s > 4) return fail(c, HMRM_ERR_INVALID, "supersample factor %d: the field (flags bits 8-11) holds s - 1 <= 3", s);
-	if (s == 1) return HMRM_OK;
-	if ((long long)s * f->screen_width > 65536 || (long long)s * f->screen_height > 65536)
+	if (s == 1 && c->blur_n == 0) return HMRM_OK;
+	const char *kind = c->blur_n ? "motion-blurred" : "supersampled";
+	if (s > 1 && ((long long)s * f->screen_width > 65536 || (long long)s * f->screen_height > 65536))
 		return fail(c, HMRM_ERR_INVALID, "supersample %d of %dx%d: the sub-frame is larger than 65536 per axis", s,
 		            f->screen_width, f->screen_height);
 	if (f->cycle_period != 1 || f->cycle != 0)
-		return fail(c, HMRM_ERR_INVALID, "supersampled frames are whole frames: cycle_period 1");
-	if (f->band_count > 1) return fail(c, HMRM_ERR_INVALID, "supersampled frames are whole frames: band_count <= 1");
+		return fail(c, HMRM_ERR_INVALID, "%s frames are whole frames: cycle_period 1", kind);
+	if (f->band_count > 1) return fail(c, HMRM_ERR_INVALID, "%s frames are whole frames: band_count <= 1", kind);
 	if (f->row_begin != 0 || (f->row_end != 0 && f->row_end != f->screen_height))
-		return fail(c, HMRM_ERR_INVALID, "supersampled frames are whole frames: row_begin 0, row_end 0 or screen_height");
+		return fail(c, HMRM_ERR_INVALID, "%s frames are whole frames: row_begin 0, row_end 0 or screen_height", kind);
 	if (f->flags & (HMRM_FLAG_STEP_INDEX | HMRM_FLAG_RAY_DUMP))
-		return fail(c, HMRM_ERR_INVALID, "supersampled frames do not record step indices or ray dumps");
+		return fail(c, HMRM_ERR_INVALID, "%s frames do not record step indices or ray dumps", kind);
 	return HMRM_OK;
 }
 
-// Enqueue one whole frame on `stream` into d_out in the frame's pixel format: enqueue_render for s = 1; for s > 1 the
-// sW x sH RGBA8 sub-frame is rendered into a sub-frame scratch and K5 box-filters it into d_out on the same stream.
+void set_camera(hmrm_frame *f, const hmrm_camera &cam) {
+	f->cam_pos[0] = cam.cam_pos[0];
+	f->cam_pos[1] = cam.cam_pos[1];
+	f->cam_pos[2] = cam.cam_pos[2];
+	f->hang = cam.hang;
+	f->vang = cam.vang;
+}
+
+// K5 over `planes` sub-frame planes in phase `phase` (kK5First and kK5Middle always reduce kDownMaxPlanes planes)
+template <int S, int G>
+void launch_k5_planes(int phase, bool rgb8, dim3 grid, cudaStream_t st, const uint32_t *sub, size_t plane, int W, int H,
+                      uint8_t *out, uint2 *acc, uint32_t n) {
+	if (phase == kK5Only && rgb8) k5_downsample<S, 3, G, kK5Only><<<grid, kDownThreads, 0, st>>>(sub, W, H, out, plane);
+	else if (phase == kK5Only) k5_downsample<S, 4, G, kK5Only><<<grid, kDownThreads, 0, st>>>(sub, W, H, out, plane);
+	else if (phase == kK5First)
+		k5_downsample<S, 4, kDownMaxPlanes, kK5First><<<grid, kDownThreads, 0, st>>>(sub, W, H, out, plane, acc);
+	else if (phase == kK5Middle)
+		k5_downsample<S, 4, kDownMaxPlanes, kK5Middle><<<grid, kDownThreads, 0, st>>>(sub, W, H, out, plane, acc);
+	else if (rgb8) k5_downsample<S, 3, G, kK5Last><<<grid, kDownThreads, 0, st>>>(sub, W, H, out, plane, acc, n);
+	else k5_downsample<S, 4, G, kK5Last><<<grid, kDownThreads, 0, st>>>(sub, W, H, out, plane, acc, n);
+}
+
+template <int S>
+void launch_k5(int planes, int phase, bool rgb8, dim3 grid, cudaStream_t st, const uint32_t *sub, size_t plane, int W,
+               int H, uint8_t *out, uint2 *acc, uint32_t n) {
+	if (planes == 1) launch_k5_planes<S, 1>(phase, rgb8, grid, st, sub, plane, W, H, out, acc, n);
+	else if (planes == 2) launch_k5_planes<S, 2>(phase, rgb8, grid, st, sub, plane, W, H, out, acc, n);
+	else if (planes == 3) launch_k5_planes<S, 3>(phase, rgb8, grid, st, sub, plane, W, H, out, acc, n);
+	else launch_k5_planes<S, 4>(phase, rgb8, grid, st, sub, plane, W, H, out, acc, n);
+}
+
+// Enqueue one whole frame on `stream` into d_out in the frame's pixel format.  Without supersampling or blur this is
+// enqueue_render.  Otherwise its n sub-frames (n = 1 without blur: the frame's own camera) are rendered at sW x sH into
+// the planes of one sub-frame scratch, kDownMaxPlanes at a time, and K5 reduces each group into d_out, or through the
+// scratch's accumulator when n > kDownMaxPlanes, all on the same stream.
 int enqueue_frame(hmrm_ctx *c, const hmrm_frame *f, uint32_t *d_out, cudaStream_t stream) {
 	if (int rc = check_supersample(c, f)) return rc;
 	const int s = supersample_of(f);
-	if (s == 1) return enqueue_render(c, f, d_out, stream, true);
-	const int W = f->screen_width, H = f->screen_height;
+	const int n = c->blur_n > 0 ? c->blur_n : 1;
 	hmrm_frame sf = *f;
+	if (c->blur_n == 1) set_camera(&sf, c->blur_cams[0]);
+	if (s == 1 && n == 1) return enqueue_render(c, &sf, d_out, stream, true);
+	const int W = f->screen_width, H = f->screen_height;
 	sf.screen_width = s * W;
 	sf.screen_height = s * H;
 	sf.pixel_format = HMRM_PIXEL_RGBA8;
 	sf.flags &= ~HMRM_FLAG_SUPERSAMPLE_MASK;
 	sf.row_begin = sf.row_end = 0;
-	int row_begin = 0, row_end = 0;
-	if (int rc = validate_frame(c, &sf, &row_begin, &row_end)) return rc;
+	// every sub-frame is checked before any of them is enqueued
+	for (int j = 0; j < n; ++j) {
+		if (c->blur_n > 1) set_camera(&sf, c->blur_cams[j]);
+		int row_begin = 0, row_end = 0;
+		if (int rc = validate_frame(c, &sf, &row_begin, &row_end)) return rc;
+	}
 	HMRM_CUDA(c, cudaSetDevice(c->device));
 
-	// take a scratch; wait (host side) for the filter that read it kSubFrames supersampled frames ago
+	// take a scratch; wait (host side) for the filter that read it kSubFrames such frames ago
 	SubFrame &b = c->sub[c->sub_next];
 	c->sub_next = (c->sub_next + 1) % kSubFrames;
 	if (b.used) HMRM_CUDA(c, cudaEventSynchronize(b.ev_read));
-	const size_t need = (size_t)sf.screen_width * (size_t)sf.screen_height * 4;
+	const int G = std::min(n, kDownMaxPlanes);
+	const size_t plane = (size_t)sf.screen_width * (size_t)sf.screen_height;     // words
+	const size_t need = plane * 4 * (size_t)G;
 	if (need > b.cap) {
 		cudaFree(b.d);
 		b.d = NULL;
@@ -772,20 +834,33 @@ int enqueue_frame(hmrm_ctx *c, const hmrm_frame *f, uint32_t *d_out, cudaStream_
 		HMRM_CUDA(c, cudaMalloc(&b.d, need));
 		b.cap = need;
 	}
-	if (int rc = enqueue_render(c, &sf, b.d, stream, true)) return rc;
+	const size_t acc_need = n > G ? (size_t)W * (size_t)H * sizeof(uint2) : 0;
+	if (acc_need > b.acc_cap) {
+		cudaFree(b.acc);
+		b.acc = NULL;
+		b.acc_cap = 0;
+		HMRM_CUDA(c, cudaMalloc(&b.acc, acc_need));
+		b.acc_cap = acc_need;
+	}
 	const dim3 grid((unsigned)(((W + kDownStrip - 1) / kDownStrip + kDownThreads - 1) / kDownThreads), (unsigned)H);
 	uint8_t *out = (uint8_t *)d_out;
 	const bool rgb8 = f->pixel_format == HMRM_PIXEL_RGB8;
-#define HMRM_LAUNCH_K5(S)                                                                                  \
-	do {                                                                                                   \
-		if (rgb8) k5_downsample<S, 3><<<grid, kDownThreads, 0, stream>>>(b.d, W, H, out);                  \
-		else k5_downsample<S, 4><<<grid, kDownThreads, 0, stream>>>(b.d, W, H, out);                      \
-	} while (0)
-	if (s == 2) HMRM_LAUNCH_K5(2);
-	else if (s == 3) HMRM_LAUNCH_K5(3);
-	else HMRM_LAUNCH_K5(4);
-#undef HMRM_LAUNCH_K5
-	HMRM_CUDA(c, cudaGetLastError());
+	const uint32_t divisor = (uint32_t)(n * s * s);
+	int acc_slot = -1;
+	for (int j = 0; j < n; ++j) {
+		// a plane is rendered again only after the K5 launch that read it, which precedes it on this stream
+		if (c->blur_n > 1) set_camera(&sf, c->blur_cams[j]);
+		if (int rc = enqueue_render(c, &sf, b.d + (size_t)(j % G) * plane, stream, true, acc_slot)) return rc;
+		if (j == 0) acc_slot = c->launch_last;
+		if (j % G != G - 1 && j != n - 1) continue;
+		const int planes = j % G + 1;
+		const int phase = n == G ? kK5Only : j < G ? kK5First : j == n - 1 ? kK5Last : kK5Middle;
+		if (s == 1) launch_k5<1>(planes, phase, rgb8, grid, stream, b.d, plane, W, H, out, b.acc, divisor);
+		else if (s == 2) launch_k5<2>(planes, phase, rgb8, grid, stream, b.d, plane, W, H, out, b.acc, divisor);
+		else if (s == 3) launch_k5<3>(planes, phase, rgb8, grid, stream, b.d, plane, W, H, out, b.acc, divisor);
+		else launch_k5<4>(planes, phase, rgb8, grid, stream, b.d, plane, W, H, out, b.acc, divisor);
+		HMRM_CUDA(c, cudaGetLastError());
+	}
 	HMRM_CUDA(c, cudaEventRecord(b.ev_read, stream));
 	b.used = true;
 	return HMRM_OK;
@@ -1234,6 +1309,7 @@ int hmrm_create(int device, hmrm_ctx **out) {
 	std::memset(c->yuv_cap, 0, sizeof c->yuv_cap);
 	std::memset(c->sub, 0, sizeof c->sub);
 	c->sub_next = 0;
+	c->blur_n = 0;
 
 	c->launch_next = c->launch_last = 0;
 	c->last_had_stats = c->last_had_step_index = c->last_had_ray_dump = c->timing_valid = false;
@@ -1295,6 +1371,7 @@ void hmrm_destroy(hmrm_ctx *c) {
 		SubFrame &b = c->sub[i];
 		if (b.used) cudaEventSynchronize(b.ev_read);      // a filter on a caller's stream may still read it
 		cudaFree(b.d);
+		cudaFree(b.acc);
 		if (b.ev_read) cudaEventDestroy(b.ev_read);
 	}
 	for (int i = 0; i < kLaunchSlots; ++i) {
@@ -1880,6 +1957,16 @@ int hmrm_set_layout(hmrm_ctx *c, int layout) {
 
 int hmrm_get_layout(hmrm_ctx *c) { return c ? c->layout_wanted : -1; }
 
+int hmrm_set_motion_blur(hmrm_ctx *c, const hmrm_camera *cams, int32_t n) {
+	if (!c) return HMRM_ERR_INVALID;
+	if (n < 0 || n > kBlurMax) return fail(c, HMRM_ERR_INVALID, "motion blur of %d sub-frames outside [0,%d]", n, kBlurMax);
+	if (n > 0 && !cams) return fail(c, HMRM_ERR_INVALID, "cams is NULL");
+	// frames already enqueued keep the cameras they were enqueued with: they are copied into each frame's launches
+	if (n > 0) std::memcpy(c->blur_cams, cams, (size_t)n * sizeof(hmrm_camera));
+	c->blur_n = n;
+	return HMRM_OK;
+}
+
 int hmrm_debug_aabb(hmrm_ctx *c, int32_t n, const double *rays, const double *boxes, double *out) {
 	if (!c) return HMRM_ERR_INVALID;
 	if (n < 1 || !rays || !boxes || !out) return fail(c, HMRM_ERR_INVALID, "hmrm_debug_aabb: bad arguments");
@@ -1996,7 +2083,8 @@ int hmrm_ipc_open(hmrm_ctx *c, const uint8_t handle[HMRM_IPC_HANDLE_BYTES], void
 int hmrm_render_peer(hmrm_ctx *c, const hmrm_frame *f, void *d_frame, void *d_ctrl, uint32_t use, void *stream) {
 	if (!c) return HMRM_ERR_INVALID;
 	if (!d_frame || !d_ctrl || use == 0u) return fail(c, HMRM_ERR_INVALID, "hmrm_render_peer: bad arguments");
-	if (f && supersample_of(f) != 1) return fail(c, HMRM_ERR_INVALID, "peer frames are band-split: no supersampling");
+	if (f && (supersample_of(f) != 1 || c->blur_n > 0))
+		return fail(c, HMRM_ERR_INVALID, "peer frames are band-split: no supersampling or motion blur");
 	HMRM_CUDA(c, cudaSetDevice(c->device));
 	cudaStream_t s = stream ? (cudaStream_t)stream : c->stream;
 	PeerCtrl *ctrl = (PeerCtrl *)d_ctrl;
@@ -2012,7 +2100,8 @@ int hmrm_render_peer_staged(hmrm_ctx *c, const hmrm_frame *f, void *d_stage, voi
                             void *stream) {
 	if (!c) return HMRM_ERR_INVALID;
 	if (!d_stage || !d_frame || !d_ctrl || use == 0u) return fail(c, HMRM_ERR_INVALID, "hmrm_render_peer_staged: bad arguments");
-	if (f && supersample_of(f) != 1) return fail(c, HMRM_ERR_INVALID, "peer frames are band-split: no supersampling");
+	if (f && (supersample_of(f) != 1 || c->blur_n > 0))
+		return fail(c, HMRM_ERR_INVALID, "peer frames are band-split: no supersampling or motion blur");
 	HMRM_CUDA(c, cudaSetDevice(c->device));
 	cudaStream_t s = stream ? (cudaStream_t)stream : c->stream;
 	PeerCtrl *ctrl = (PeerCtrl *)d_ctrl;

@@ -11,6 +11,7 @@
 //   ... [--supersample 1|2|3|4]                    (anti-aliasing: the box filter of an N x N-times larger frame)
 //   ... [--height-bits 8|16]                       (16: heightmaps load at full precision, hmrm_set_maps16)
 //   ... [--jpeg Q [--jpeg-chroma 420|444]]         (JPEG files / Motion-JPEG video of quality Q instead of PNG / Y4M)
+//   ... [--motion-blur K [--shutter F]]            (--script only: each frame averages K cameras towards the next one)
 //   hmap config.txt --parse-only                    (grammar check: echo + validation, no GPU)
 //   hmap --decode-image in.png 3|4|h16 out.raw      (image ingest check, no GPU; h16: little-endian u16 samples)
 //
@@ -35,6 +36,14 @@
 // With --video it writes Motion-JPEG instead of Y4M: the frames' JPEG files back to back in script order, the stream
 // `ffmpeg -f mjpeg -framerate N -i` reads.  Such a stream carries no frame rate or matrix, so --fps and
 // --video-matrix are refused with --jpeg.
+// --motion-blur K (1-16, --script only) blurs every recorded or video frame over the camera's motion to the next frame
+// (hmrm_set_motion_blur, kernel K5).  With c_n the camera after script line n and c_{n+1} the camera of the next rendered
+// frame, sub-frame j of frame n uses t = (F * j) / K and c = c_n + t * (c_{n+1} - c_n), per component of cam_pos, hang
+// and vang, in doubles and in that order; F is --shutter (0 < F <= 1, default 0.5), the fraction of the frame interval
+// the shutter stays open.  Angles are not wrapped: a turn from 350 to 370 degrees blurs over 20 degrees, one from 350
+// to 10 over 340.  Line n+1 is applied once frame n's maps are on the devices and its frame is built, so frame n renders
+// with exactly its own maps and fields.  The last rendered frame has no successor and is rendered without blur.
+// --motion-blur 1 renders exactly the frames without the option.
 // Headless frames are complete images: cycle_period is forced to 1 (the reference's own advice, :913).
 #include <cstdio>
 #include <cstdlib>
@@ -65,11 +74,13 @@ struct Options {
 	std::string config_path, headless_out, script_path, out_prefix, stats_json, video_path;
 	int projection, precision, traversal, gpus, frames, fps, video_matrix, supersample, height_bits;
 	int jpeg_quality, jpeg_chroma;   // jpeg_quality 0: PNG stills and Y4M video
-	bool record, parse_only, supersample_given, y4m_option_given, jpeg_chroma_given;
+	int motion_blur;                 // 0: not given
+	double shutter;
+	bool record, parse_only, supersample_given, y4m_option_given, jpeg_chroma_given, shutter_given;
 	Options() : projection(0), precision(HMRM_FP64_EXACT), traversal(HMRM_TRAVERSAL_AUTO), gpus(1), frames(-1), fps(30),
 	            video_matrix(HMRM_YUV_BT709), supersample(1), height_bits(8), jpeg_quality(0), jpeg_chroma(HMRM_JPEG_420),
-	            record(false), parse_only(false), supersample_given(false), y4m_option_given(false),
-	            jpeg_chroma_given(false) {}
+	            motion_blur(0), shutter(0.5), record(false), parse_only(false), supersample_given(false),
+	            y4m_option_given(false), jpeg_chroma_given(false), shutter_given(false) {}
 };
 
 void usage_and_exit() {
@@ -78,7 +89,7 @@ void usage_and_exit() {
 	             "            [--traversal auto|brute|skip] [--gpus N] [--script frames.txt [--frames N]\n"
 	             "            [--out-prefix P | --record | --video FILE|- [--fps N] [--video-matrix bt601|bt709]]]\n"
 	             "            [--supersample 1|2|3|4] [--height-bits 8|16] [--jpeg Q [--jpeg-chroma 420|444]]\n"
-	             "            [--stats-json file] [--parse-only]\n"
+	             "            [--motion-blur 1..16 [--shutter F]] [--stats-json file] [--parse-only]\n"
 	             "       hmap --decode-image in 3|4|h16 out.raw\n";
 	std::exit(1);
 }
@@ -127,6 +138,26 @@ void push_maps(std::vector<Device> &devs, Config &cfg) {
 	}
 	cfg.maps_changed = false;
 	cfg.should_update_heightmap = false;
+}
+
+hmrm_camera camera_of(const Config &cfg) {
+	hmrm_camera c;
+	c.cam_pos[0] = cfg.cam_pos[0];
+	c.cam_pos[1] = cfg.cam_pos[1];
+	c.cam_pos[2] = cfg.cam_pos[2];
+	c.hang = cfg.hang;
+	c.vang = cfg.vang;
+	return c;
+}
+
+// --motion-blur: sub-frame j of k between cameras a and b (see the header comment)
+hmrm_camera blur_camera(const hmrm_camera &a, const hmrm_camera &b, double shutter, int j, int k) {
+	const double t = (shutter * j) / k;
+	hmrm_camera c;
+	for (int i = 0; i < 3; ++i) c.cam_pos[i] = a.cam_pos[i] + t * (b.cam_pos[i] - a.cam_pos[i]);
+	c.hang = a.hang + t * (b.hang - a.hang);
+	c.vang = a.vang + t * (b.vang - a.vang);
+	return c;
 }
 
 hmrm_frame make_frame(const Config &cfg, const Options &opt) {
@@ -318,6 +349,17 @@ int main(int argc, char **argv) {
 			opt.jpeg_quality = std::atoi(argv[++i]);
 			if (opt.jpeg_quality < 1 || opt.jpeg_quality > 100) usage_and_exit();
 		}
+		else if (a == "--motion-blur" && has_val) {
+			opt.motion_blur = std::atoi(argv[++i]);
+			if (opt.motion_blur < 1 || opt.motion_blur > 16) usage_and_exit();
+		}
+		else if (a == "--shutter" && has_val) {
+			const char *v = argv[++i];
+			char *end = NULL;
+			opt.shutter = std::strtod(v, &end);
+			if (end == v || *end != '\0' || !(opt.shutter > 0.0 && opt.shutter <= 1.0)) usage_and_exit();
+			opt.shutter_given = true;
+		}
 		else if (a == "--jpeg-chroma" && has_val) {
 			const std::string v = argv[++i];
 			if (v == "420") opt.jpeg_chroma = HMRM_JPEG_420;
@@ -331,6 +373,10 @@ int main(int argc, char **argv) {
 	if (opt.supersample < 1 || opt.supersample > 4) usage_and_exit();
 	// one frame over several devices is dealt in tile-row bands, which supersampled frames are not
 	if (opt.supersample > 1 && !opt.headless_out.empty() && opt.script_path.empty() && opt.gpus > 1) usage_and_exit();
+	// motion blur needs the next frame's camera: recordings only
+	if (opt.motion_blur && (opt.script_path.empty() || !opt.headless_out.empty())) usage_and_exit();
+	if (opt.shutter_given && !opt.motion_blur) usage_and_exit();
+	const bool blur = opt.motion_blur > 1;
 	const bool video = !opt.video_path.empty();
 	if (video && (opt.script_path.empty() || !opt.headless_out.empty() || opt.record || !opt.out_prefix.empty()))
 		usage_and_exit();
@@ -545,11 +591,15 @@ int main(int argc, char **argv) {
 				while (devs[i].png_count > 0) retire_oldest(devs[i]);
 		};
 
+		auto apply_line = [&](int n) {
+			if (n >= (int)lines.size()) return true;
+			std::istringstream iss(lines[(size_t)n]);
+			return consume_config_stream(iss, cfg, msg, std::cerr) == PARSE_OK;
+		};
+		bool line_applied = false;      // --motion-blur: line n was applied while frame n - 1 was set up
 		for (int n = 0; n < n_frames; ++n) {
-			if (n < (int)lines.size()) {
-				std::istringstream iss(lines[(size_t)n]);
-				if (consume_config_stream(iss, cfg, msg, std::cerr) != PARSE_OK) return 1;
-			}
+			if (!line_applied && !apply_line(n)) return 1;
+			line_applied = false;
 			if (video && !opt.jpeg_quality && n > 0 && (cfg.screen_width != video_w || cfg.screen_height != video_h)) {
 				// the frames before this one stay a valid stream
 				drain_all();
@@ -570,6 +620,19 @@ int main(int argc, char **argv) {
 			}
 			collect_pending(d);
 			const hmrm_frame f = make_frame(cfg, opt);
+			if (blur) {
+				// the cameras from this frame's towards the next rendered frame's; the last frame is plain
+				hmrm_camera cams[16];
+				int k = 0;
+				if (n + 1 < n_frames) {
+					const hmrm_camera from = camera_of(cfg);
+					if (!apply_line(n + 1)) return 1;
+					line_applied = true;
+					const hmrm_camera to = camera_of(cfg);
+					for (k = 0; k < opt.motion_blur; ++k) cams[k] = blur_camera(from, to, opt.shutter, k, opt.motion_blur);
+				}
+				if (hmrm_set_motion_blur(d.ctx, cams, k) != HMRM_OK) die_hmrm(d.ctx, "hmrm_set_motion_blur");
+			}
 			PngBuffer &b = d.png[(d.png_head + d.png_count) % kPngInFlight];
 			if (video && !opt.jpeg_quality) {
 				if (n == 0) video_header(f.screen_width, f.screen_height);
@@ -611,6 +674,7 @@ int main(int argc, char **argv) {
 		if (opt.jpeg_quality) js << ", \"jpeg_bytes\": " << totals.jpeg_bytes;
 		if (video) js << ", \"video_bytes\": " << totals.video_bytes;
 		if (opt.supersample_given) js << ", \"supersample\": " << opt.supersample;
+		if (opt.motion_blur) js << ", \"motion_blur\": " << opt.motion_blur << ", \"shutter\": " << opt.shutter;
 		js << "}\n";
 	}
 

@@ -164,6 +164,32 @@ int hmrm_synth_maps16(hmrm_ctx *ctx, uint32_t log2n, uint32_t seed);
 int hmrm_set_layout(hmrm_ctx *ctx, int layout);
 int hmrm_get_layout(hmrm_ctx *ctx);
 
+/* ---- motion blur (kernel K5, csrc/k5_downsample.cuh): a frame averages the scene over several cameras ----
+ * The state belongs to the context, as the layout does.  It is copied, so the caller may free `cams`.  Each render call
+ * reads it when the frame is ENQUEUED: frames already in flight keep the cameras they were enqueued with.
+ * With n >= 1, sub-frame j (0 <= j < n) is the reference's frame of `f` with cam_pos, hang and vang replaced by cams[j],
+ * rendered at sW x sH when `f` has supersample factor s.  The fields of `f` that hold the camera are not used; every other
+ * field comes from `f`.  Output pixel: each of R, G, B = (sum + N/2) / N in integers (floor division), N = n*s*s, with
+ * the sum of that channel over the s x s subsamples of all n sub-frames (at most 16*16*255 = 65280);  A = 255.  There is
+ * one rounding, not HMRM_FLAG_SUPERSAMPLE's box filter followed by an average.  Consequences:
+ *   n = 1 is the supersampled frame of cams[0] (HMRM_FLAG_SUPERSAMPLE's definition);
+ *   cams[0] equal to f's camera with n = 1 gives exactly the frame without blur;
+ *   n identical cameras give the frame of that camera without blur, for every s <= 4 and n <= 16 (for every possible
+ *   sum, the rounded mean of n copies of a rounded mean is that rounded mean).
+ * Accepted by hmrm_render, hmrm_render_async, hmrm_render_device, hmrm_render_png_async, hmrm_render_yuv420_async and
+ * hmrm_render_jpeg_async; while n >= 1 they refuse what HMRM_FLAG_SUPERSAMPLE refuses (cycle_period != 1,
+ * band_count > 1, a partial row band, HMRM_FLAG_STEP_INDEX or HMRM_FLAG_RAY_DUMP) with HMRM_ERR_INVALID and nothing
+ * written, and so do hmrm_render_peer and hmrm_render_peer_staged.  With HMRM_FLAG_STATS, hmrm_get_stats gives sums over
+ * the n sub-frame renders (rays = n*s*s*W*H, steps and fetches summed, max_steps the maximum) and kernel_ms from the start
+ * of the first sub-frame render to the end of the last. */
+typedef struct hmrm_camera {
+	double cam_pos[3];   /* as hmrm_frame.cam_pos */
+	double hang, vang;   /* radians, as hmrm_frame */
+} hmrm_camera;
+/* n = 0 (the default): every render is as without this call.  n = 1..16: every whole-frame render on ctx averages n
+ * sub-frames.  n < 0, n > 16 or NULL cams with n > 0 is HMRM_ERR_INVALID and leaves the previous state in place. */
+int hmrm_set_motion_blur(hmrm_ctx *ctx, const hmrm_camera *cams, int32_t n);
+
 /* ---- prepass: replaces UpdateHeightmap, main/hmap.cpp:171-191 (kernel K1) ---- */
 int hmrm_update_heightmap(hmrm_ctx *ctx, const double lum[3], double min_height, double max_height);
 /* heights exactly as the reference's heightmap_buf (double[H][W], main/hmap.cpp:53), for parity checks */
