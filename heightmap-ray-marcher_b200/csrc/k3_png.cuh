@@ -7,8 +7,9 @@
 //                   stream (H * (W*C + 1) bytes);
 //   k3_png_deflate  one warp per kPngSeg-byte segment of the filtered stream: greedy LZ77 over three candidate distances
 //                   (1, C, and W*C + 1 = the same byte one row up, while that is <= 32768), coded as one fixed-Huffman
-//                   block closed by the sync-flush idiom (EOB, empty stored block), or as one stored block when that is
-//                   not larger.  Either way the segment ends byte-aligned, so segments concatenate as they are.  Each
+//                   block closed by the sync-flush idiom (EOB, empty stored block), or as one stored block only when
+//                   that is strictly smaller (3 + token bits + 10 > 8 (n + 1); a byte tie stays coded).  Either way
+//                   the segment ends byte-aligned, so segments concatenate as they are.  Each
 //                   segment is its own IDAT chunk, CRC-32 included, staged at a fixed stride; the first one carries the
 //                   zlib header 78 01.  The warp also sums the segment's Adler-32 partials;
 //   k3_png_finish   one CTA: exclusive scan of the chunk sizes, Adler-32 of the whole stream from the partials, the

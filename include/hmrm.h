@@ -217,8 +217,22 @@ int hmrm_wait_pending(hmrm_ctx *ctx, int max_pending);
 
 /* ---- PNG frames, deflated on the device (kernel K3, csrc/k3_png.cuh) ----
  * The file is 8-bit, not interlaced, colour type 6 for 4 channels and 2 for 3; the decoded pixels are the frame's, byte
- * for byte.  Each row gets the PNG filter with the smallest sum of |residual|; the filtered stream is deflated in
- * independent 4096-byte segments (fixed-Huffman LZ77, or stored when that is smaller), one IDAT chunk each. */
+ * for byte.  The file is exactly this function of the pixels (C channels, W x H):
+ * 1. Filter, per row: for each type t = 0 None, 1 Sub, 2 Up, 3 Average, 4 Paeth, the sum over the row's W C bytes of
+ *    min(r, 256 - r), r = residual & 255; the row above row 0 is zero, a and c are zero for the first C bytes.  The
+ *    smallest sum wins, the lowest type on a tie.  The filtered stream is H rows of 1 + W C bytes (type, residuals).
+ * 2. Segments: the stream is cut into 4096-byte segments, the last one shorter; each is deflated on its own.
+ * 3. Greedy parse of a segment: at position o each candidate distance, in the order 1, C, W C + 1 (the last only while
+ *    W C + 1 <= 32768), has a run: the number of bytes from o on that equal the byte that many positions back.  A run
+ *    may reach back before the segment's start, never before byte 0 of the stream, and stops at the segment's end; it
+ *    is capped at 258.  The longest run, if it is at least 3, is a match (the earlier distance on a tie), else the byte
+ *    is one literal.
+ * 4. Coding: the segment is one fixed-Huffman block (RFC 1951: BFINAL 0, BTYPE 01, the tokens, EOB) followed by an
+ *    empty stored block (3 header bits, alignment to a byte, 00 00 FF FF).  With n the segment's bytes and `bits` the
+ *    tokens' bits, it stays so when 3 + bits + 10 <= 8 (n + 1), that is when its bytes do not exceed the n + 5 of a
+ *    stored block (a tie stays coded); otherwise it is one stored block: 00, LEN, NLEN, the n bytes.
+ * 5. Framing: signature; IHDR; one IDAT chunk per segment, the first one led by the zlib header 78 01; an IDAT of
+ *    03 00 (a final empty fixed block) and the big-endian Adler-32 of the filtered stream; IEND. */
 /* worst-case file size for width x height x channels (3 | 4), 0 for other shapes; host arithmetic, no device work:
  * with N = height * (width * channels + 1) and S = ceil(N / 4096) segments, N + 17 S + 65 */
 size_t hmrm_png_bound(int32_t width, int32_t height, int32_t channels);

@@ -9,6 +9,7 @@ from PIL import Image
 
 import helpers as H
 import scenes as S
+from test_gpu_png import assert_equals_model
 
 pytestmark = pytest.mark.gpu
 
@@ -40,6 +41,7 @@ def test_headless_png_matches_reference_frame(hmrm, oracle, name, tmp_path):
     assert f"Saved screenshot at {out}" in res.stdout            # main/hmap.cpp:166
     got = np.asarray(Image.open(out).convert("RGBA"))
     assert np.array_equal(got, H.golden_frames()[name])
+    assert_equals_model(out.read_bytes(), H.golden_frames()[name], name)
     meta = H.golden_meta()[name]
     st = json.loads(stats.read_text())
     assert (st["rays"], st["box_hits"], st["surf_hits"], st["steps"]) == (
@@ -63,6 +65,7 @@ def test_script_recording_matches_oracle_per_frame(hmrm, oracle, tmp_path):
         want, _, _ = H.oracle_render_scene(oracle, dict(scene, **s), maps)
         got = np.asarray(Image.open(tmp_path / f"f_{i}.png").convert("RGBA"))
         assert np.array_equal(got, want), f"frame {i}"
+        assert_equals_model((tmp_path / f"f_{i}.png").read_bytes(), want, f"frame {i}")
 
 
 def test_brute_and_fp64_flags(hmrm, oracle, tmp_path):
@@ -73,6 +76,7 @@ def test_brute_and_fp64_flags(hmrm, oracle, tmp_path):
                           "--precision", "fp64"], capture_output=True, text=True, cwd=str(tmp_path))
     assert res.returncode == 0, res.stderr
     assert np.array_equal(np.asarray(Image.open(out).convert("RGBA")), H.golden_frames()["spher_basic"])
+    assert_equals_model(out.read_bytes(), H.golden_frames()["spher_basic"], "brute fp64")
 
 
 @pytest.mark.parametrize("name,gpus", [("persp_basic", 2), ("spher_wide", 3), ("ortho_fine", 5)])
@@ -91,6 +95,7 @@ def test_one_frame_over_several_devices_equals_the_reference_frame(hmrm, oracle,
                          cwd=str(tmp_path), env=env)
     assert res.returncode == 0, res.stderr
     assert np.array_equal(np.asarray(Image.open(out).convert("RGBA")), H.golden_frames()[name])
+    assert_equals_model(out.read_bytes(), H.golden_frames()[name], f"{name} over {gpus} devices")
     meta = H.golden_meta()[name]
     st = json.loads(stats.read_text())
     assert (st["rays"], st["box_hits"], st["surf_hits"], st["steps"]) == (
@@ -113,3 +118,4 @@ def test_recording_over_several_devices(hmrm, oracle, tmp_path):
         want, _, _ = H.oracle_render_scene(oracle, dict(scene, **s), maps)
         got = np.asarray(Image.open(tmp_path / f"f_{i}.png").convert("RGBA"))
         assert np.array_equal(got, want), f"frame {i}"
+        assert_equals_model((tmp_path / f"f_{i}.png").read_bytes(), want, f"frame {i}")

@@ -17,6 +17,7 @@ import pytest
 import destinations_model as M
 import helpers as H
 import scenes as S
+from test_gpu_png import assert_sampled_segments_equal_model
 from test_png_encode import check_png
 from test_supersample import box_reduce
 from test_yuv420 import BT601, BT709, yuv420_model
@@ -381,6 +382,7 @@ def test_png_and_yuv_at_the_axis_limit(renderer, w, h):
         data = renderer.encode_png(px)
         assert np.array_equal(check_png(data)[0], px), (w, h, ch)
         assert np.array_equal(np.asarray(Image.open(io.BytesIO(data))), px), (w, h, ch)
+        assert_sampled_segments_equal_model(data, px, seed=w + ch)
         for matrix in (BT601, BT709):
             got = renderer.convert_yuv420(px, matrix)
             for plane, g, want in zip(("Y", "Cb", "Cr"), got, yuv420_model(px, matrix)):

@@ -17,7 +17,7 @@ import pytest
 import helpers as H
 import jpeg_model as J
 import scenes as S
-from test_gpu_png import _write_scene
+from test_gpu_png import _write_scene, assert_equals_model
 from test_motion_blur import blur_cameras, blur_reduce
 from test_png_encode import check_png
 from test_yuv420 import BT709, i420, read_y4m, yuv420_model
@@ -224,6 +224,7 @@ def test_encoded_outputs_are_of_the_blurred_frame(hmrm, renderer, oracle, name, 
         data = renderer.render_png(f)
         _assert_same(check_png(data)[0], want[:, :, :ch], f"{name} PNG channels={ch} (checker)")
         _assert_same(np.asarray(Image.open(io.BytesIO(data))), want[:, :, :ch], f"{name} PNG channels={ch} (PIL)")
+        assert_equals_model(data, want, f"{name} PNG channels={ch}")
         for matrix in (hmrm.YUV_BT601, hmrm.YUV_BT709):
             got = renderer.render_yuv420(f, matrix=matrix)
             for plane, g, w in zip("Y Cb Cr".split(), got, yuv420_model(want, matrix)):
@@ -285,7 +286,9 @@ def test_frames_in_flight_keep_their_own_state(hmrm, renderer, oracle):
         if k == "raw":
             _assert_same(raw[j % 4], want[j], what)
         elif k == "png":
-            _assert_same(check_png(files[j % 4][:int(sizes[j % 4][0])].tobytes())[0], want[j], what)
+            data = files[j % 4][:int(sizes[j % 4][0])].tobytes()
+            _assert_same(check_png(data)[0], want[j], what)
+            assert_equals_model(data, want[j], what)
         elif k == "yuv":
             assert i420(yuv420_model(want[j], BT709)) == yuv[j % 4].tobytes(), what
         else:
@@ -457,6 +460,7 @@ def test_hmap_motion_blur_png_y4m_mjpeg_jpeg(hmrm, oracle, gpus, tmp_path):
     # want[-1], the last frame, is the oracle's plain frame of the last camera: it has no successor to blur towards
     for i, w in enumerate(want):
         _assert_same(check_png((tmp_path / f"f_{i}.png").read_bytes())[0], w, f"PNG frame {i}")
+        assert_equals_model((tmp_path / f"f_{i}.png").read_bytes(), w, f"PNG frame {i}")
     st = json.loads((tmp_path / "stats.json").read_text())
     assert st["motion_blur"] == 4 and st["shutter"] == 0.5 and st["frames"] == len(states)
     assert st["rays"] == 160 * 90 * (4 * (len(states) - 1) + 1)

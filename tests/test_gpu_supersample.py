@@ -15,7 +15,7 @@ import pytest
 
 import helpers as H
 import scenes as S
-from test_gpu_png import _write_scene
+from test_gpu_png import _write_scene, assert_equals_model
 from test_png_encode import check_png
 from test_supersample import box_reduce
 from test_yuv420 import BT709, i420, read_y4m, yuv420_model
@@ -126,6 +126,7 @@ def test_render_png_s2_decodes_to_filtered_frame(hmrm, renderer, oracle, name):
         data = renderer.render_png(_frame(hmrm, renderer, scene, 2, pixel_format=fmt))
         _assert_same(check_png(data)[0], want[:, :, :ch], f"{name} channels={ch} (checker)")
         _assert_same(np.asarray(Image.open(io.BytesIO(data))), want[:, :, :ch], f"{name} channels={ch} (PIL)")
+        assert_equals_model(data, want, f"{name} channels={ch}")
 
 
 @pytest.mark.parametrize("name", ["persp_basic", "ortho_fine", "defaults_grid"])
@@ -192,7 +193,9 @@ def test_ring_mixes_factors_and_outputs(hmrm, renderer, oracle):
         if kinds[j] == "raw":
             _assert_same(raw[j % 4], want[j], what)
         elif kinds[j] == "png":
-            _assert_same(check_png(png[j % 4][:int(sizes[j % 4][0])].tobytes())[0], want[j], what)
+            data = png[j % 4][:int(sizes[j % 4][0])].tobytes()
+            _assert_same(check_png(data)[0], want[j], what)
+            assert_equals_model(data, want[j], what)
         else:
             assert i420(yuv420_model(want[j], BT709)) == yuv[j % 4].tobytes(), what
 
@@ -292,6 +295,7 @@ def test_hmap_headless_supersample(hmrm, oracle, tmp_path):
                          capture_output=True, text=True, cwd=str(tmp_path))
     assert res.returncode == 0, res.stderr
     _assert_same(check_png(out.read_bytes())[0], expected(oracle, scene, 2), "hmap --headless --supersample 2")
+    assert_equals_model(out.read_bytes(), expected(oracle, scene, 2), "hmap --headless --supersample 2")
     st = json.loads(stats.read_text())
     assert st["supersample"] == 2 and st["rays"] == 4 * scene["width"] * scene["height"]
     # without the option the statistics do not name it
@@ -300,6 +304,7 @@ def test_hmap_headless_supersample(hmrm, oracle, tmp_path):
     assert res.returncode == 0, res.stderr
     assert "supersample" not in json.loads(stats.read_text())
     _assert_same(check_png(out.read_bytes())[0], H.golden_frames()["persp_basic"], "hmap --headless")
+    assert_equals_model(out.read_bytes(), H.golden_frames()["persp_basic"], "hmap --headless")
 
 
 # ---- 10. hmap --script --video - --supersample 2 over several contexts ----
