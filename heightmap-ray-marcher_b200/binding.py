@@ -245,6 +245,14 @@ def _nbytes(a):
     return None
 
 
+def _pixels(pixels):
+    """`pixels` as a contiguous [H, W, 3 | 4] uint8 numpy array, and its shape."""
+    px = np.ascontiguousarray(pixels, dtype=np.uint8)
+    if px.ndim != 3 or px.shape[2] not in (3, 4):
+        raise ValueError("pixels must be [H, W, 3] or [H, W, 4] uint8")
+    return px, px.shape
+
+
 def _ptr(a) -> int:
     if a is None:
         return 0
@@ -286,6 +294,7 @@ class Renderer:
         self.precision = FP64_EXACT
         self.traversal = TRAVERSAL_AUTO
         self.map_width = self.map_height = 0
+        self._pinned_cache = {}
 
     # -- lifetime -------------------------------------------------------------------------
     def close(self) -> None:
@@ -467,26 +476,17 @@ class Renderer:
 
     def encode_png(self, pixels: np.ndarray) -> bytes:
         """[H, W, 3 | 4] uint8 pixels -> PNG file, encoded on this context's device."""
-        px = np.ascontiguousarray(pixels, dtype=np.uint8)
-        if px.ndim != 3 or px.shape[2] not in (3, 4):
-            raise ValueError("pixels must be [H, W, 3] or [H, W, 4] uint8")
-        h, w, ch = px.shape
+        px, (h, w, ch) = _pixels(pixels)
         out, size = self._png_buffers(w, h, ch)
         self._check(self._lib.hmrm_encode_png(self._h, px.ctypes.data, w, h, ch, out.ctypes.data, out.nbytes,
                                               size.ctypes.data))
         return out[:int(size[0])].tobytes()
 
     def _png_buffers(self, width: int, height: int, channels: int):
-        """Pinned file + size buffers, kept for the last shape: pinning ~33 MB per 4K call would cost more than the
-        encode."""
         bound = png_bound(width, height, channels)
         if bound == 0:
             raise ValueError(f"no PNG of {width}x{height}x{channels}")
-        cached = getattr(self, "_png_cache", None)
-        if cached is None or cached[0].nbytes < bound:
-            cached = (pinned_empty((bound,)), pinned_empty((1,), dtype=np.uint64))
-            self._png_cache = cached
-        return cached
+        return self._pinned("png", bound)
 
     # -- JPEG frames, encoded on the device ---------------------------------------------------------
     def render_jpeg_async(self, frame: Frame, out, size_out, quality: int = 90, chroma: int = JPEG_420,
@@ -516,10 +516,7 @@ class Renderer:
             h, w, ch = (int(v) for v in pixels.shape)
             ptr = int(pixels.data_ptr())
         else:
-            px = np.ascontiguousarray(pixels, dtype=np.uint8)
-            if px.ndim != 3 or px.shape[2] not in (3, 4):
-                raise ValueError("pixels must be [H, W, 3] or [H, W, 4] uint8")
-            h, w, ch = px.shape
+            px, (h, w, ch) = _pixels(pixels)
             ptr = px.ctypes.data
         out, size = self._jpeg_buffers(w, h, chroma)
         self._check(self._lib.hmrm_encode_jpeg(self._h, ptr, w, h, ch, int(quality), int(chroma), out.ctypes.data,
@@ -527,19 +524,23 @@ class Renderer:
         return out[:int(size[0])].tobytes()
 
     def _jpeg_buffers(self, width: int, height: int, chroma: int):
-        """Pinned file + size buffers, kept while they are large enough (as _png_buffers)."""
         bound = jpeg_bound(width, height, chroma)
         if bound == 0:
             raise ValueError(f"no JPEG of {width}x{height} in chroma mode {chroma}")
-        cached = getattr(self, "_jpeg_cache", None)
-        if cached is None or cached[0].nbytes < bound:
-            cached = (pinned_empty((bound,)), pinned_empty((1,), dtype=np.uint64))
-            self._jpeg_cache = cached
-        return cached[0][:bound], cached[1]
+        return self._pinned("jpeg", bound)
+
+    def _pinned(self, key: str, nbytes: int):
+        """A pinned buffer of `nbytes` and a pinned uint64 size word, kept per output `key` while large enough: pinning
+        ~33 MB per 4K call would cost more than the encode.  Only the next call of the same output overwrites them."""
+        cached = self._pinned_cache.get(key)
+        if cached is None or cached[0].nbytes < nbytes:
+            cached = (pinned_empty((nbytes,)), pinned_empty((1,), dtype=np.uint64))
+            self._pinned_cache[key] = cached
+        return cached[0][:nbytes], cached[1]
 
     @staticmethod
     def _file_capacity(name: str, out, size_out, capacity):
-        """The capacity of a file destination (its own size unless given), after checking the size word."""
+        """The capacity of a destination (its own size unless given), after checking the size word if there is one."""
         if capacity is None:
             capacity = _nbytes(out)
             if capacity is None:
@@ -555,10 +556,7 @@ class Renderer:
         """hmrm_render_yuv420_async: `out` (pinned host or device memory of yuv420_bytes or more) receives the I420 planes
         once wait / wait_pending covers the frame.  numpy arrays and torch tensors report their own sizes; a raw address
         needs `capacity`."""
-        if capacity is None:
-            capacity = _nbytes(out)
-            if capacity is None:
-                raise ValueError("render_yuv420_async: pass capacity= with a raw output address")
+        capacity = self._file_capacity("render_yuv420_async", out, None, capacity)
         self._check(self._lib.hmrm_render_yuv420_async(self._h, C.byref(frame), int(matrix), _ptr(out), int(capacity)))
 
     def render_yuv420(self, frame: Frame | None = None, matrix: int = YUV_BT709, **overrides):
@@ -573,25 +571,17 @@ class Renderer:
     def convert_yuv420(self, pixels: np.ndarray, matrix: int = YUV_BT709):
         """[H, W, 3 | 4] uint8 pixels -> (Y, Cb, Cr) planes, converted on this context's device; the same buffer as
         render_yuv420's."""
-        px = np.ascontiguousarray(pixels, dtype=np.uint8)
-        if px.ndim != 3 or px.shape[2] not in (3, 4):
-            raise ValueError("pixels must be [H, W, 3] or [H, W, 4] uint8")
-        h, w, ch = px.shape
+        px, (h, w, ch) = _pixels(pixels)
         out = self._yuv_buffer(w, h)
         self._check(self._lib.hmrm_convert_yuv420(self._h, px.ctypes.data, w, h, ch, int(matrix), out.ctypes.data,
                                                   out.nbytes))
         return yuv420_planes(out, w, h)
 
     def _yuv_buffer(self, width: int, height: int) -> np.ndarray:
-        """Pinned planes buffer of exactly the frame's size, kept while the shape repeats (as _png_buffers)."""
         n = yuv420_bytes(width, height)
         if n == 0:
             raise ValueError(f"no YUV frame of {width}x{height}")
-        cached = getattr(self, "_yuv_cache", None)
-        if cached is None or cached.nbytes < n:
-            cached = pinned_empty((n,))
-            self._yuv_cache = cached
-        return cached[:n]
+        return self._pinned("yuv", n)[0]
 
     def render_device(self, frame: Frame, d_out, stream=None) -> None:
         self._check(self._lib.hmrm_render_device(self._h, C.byref(frame), _ptr(d_out), _ptr(stream)))

@@ -65,28 +65,6 @@ struct LaunchSlot {
 	size_t dump_cap;             // pixels
 };
 
-// K3 scratch of one ring slot: filtered stream, staged chunks, per-segment sizes / Adler-32 partials, piece offsets,
-// signature / IHDR / tail chunks.  Each slot has its own, so two frames in flight never share it.
-struct PngScratch {
-	uint8_t *filt, *stage, *meta;
-	PngSegInfo *info;
-	unsigned long long *offsets;
-	unsigned long long filt_cap;  // bytes of filtered stream
-	int seg_cap;                  // segments
-};
-
-// K6 scratch of one ring slot: quantised coefficients, AC bit counts and bit offsets per block, the rows' bit buffers
-// and stuffed pieces, row sizes, piece offsets, header / EOI.  Each slot has its own, as with PngScratch.
-struct JpegScratch {
-	int16_t *coef;
-	uint16_t *acbits;
-	uint32_t *boff, *rowbits;
-	uint8_t *stage, *meta;
-	unsigned long long *rowsize, *offsets;
-	unsigned long long blocks_cap, words_cap, stage_cap;   // blocks, row-buffer words, staged bytes
-	int rows_cap;
-};
-
 // The sW x sH RGBA8 renders of one supersampled or motion-blurred frame, read by K5: up to kDownMaxPlanes planes, and
 // K5's accumulator when a blurred frame has more sub-frames than planes.  Inside the frame the planes are reused in
 // stream order; across frames the scratch is reused only after the filter that read it last has run (ev_read), so up to
@@ -160,16 +138,12 @@ struct hmrm_ctx {
 	bool copy_pending[kFrameRing];
 	int fb_format;               // pixel format of what the ring holds (a change re-zeroes it, like a new resolution)
 	int slot;                    // buffer of the most recent hmrm_render_async
-	// PNG encoding: scratch per ring slot, allocated by the first PNG frame that uses the slot
-	PngScratch png[kFrameRing];
-	// JPEG encoding: scratch per ring slot, allocated by the first JPEG frame that uses the slot
-	JpegScratch jpeg[kFrameRing];
-	uint8_t *d_png_in;           // hmrm_encode_png's / _jpeg's / hmrm_convert_yuv420's device copy of the caller's pixels
-	size_t png_in_cap;
-	// YUV frames: the I420 planes K4 writes, per ring slot, allocated by the first YUV frame that uses the slot; the copy
-	// engine moves them to the caller's buffer
-	uint8_t *d_yuv[kFrameRing];
-	size_t yuv_cap[kFrameRing];
+	// encoder scratch per ring slot, grown by the first frame that needs more: K3 (PNG), K4 (YUV) and K6 (JPEG) carve
+	// their pieces from it (png_pieces, jpeg_pieces; K4's I420 planes are the whole of it)
+	uint8_t *d_scratch[kFrameRing];
+	size_t scratch_cap[kFrameRing];
+	uint8_t *d_pixels;           // hmrm_encode_png's / _jpeg's / hmrm_convert_yuv420's device copy of the caller's pixels
+	size_t pixels_cap;
 	// supersampled frames (K5): sub-frame scratches, allocated by the first supersampled frame that uses them
 	SubFrame sub[kSubFrames];
 	int sub_next;
@@ -206,6 +180,19 @@ int fail(hmrm_ctx *ctx, int code, const char *fmt, ...) {
 	} while (0)
 
 bool finite3(const double *v) { return std::isfinite(v[0]) && std::isfinite(v[1]) && std::isfinite(v[2]); }
+
+// Grows the device buffer *p of *cap bytes to at least `need` bytes.  Its contents are not kept; the caller makes sure
+// no work in flight still uses it.
+template <class T>
+int grow(hmrm_ctx *c, T **p, size_t *cap, size_t need) {
+	if (need <= *cap) return HMRM_OK;
+	cudaFree(*p);
+	*p = NULL;
+	*cap = 0;
+	HMRM_CUDA(c, cudaMalloc(p, need));
+	*cap = need;
+	return HMRM_OK;
+}
 
 __global__ void __launch_bounds__(256) k_synth_maps(uint32_t log2n, uint32_t seed, uint8_t *__restrict__ rgb,
                                                     uint32_t *__restrict__ rgba) {
@@ -744,16 +731,9 @@ int supersample_of(const hmrm_frame *f) {
 	return (int)((f->flags & HMRM_FLAG_SUPERSAMPLE_MASK) >> HMRM_FLAG_SUPERSAMPLE_SHIFT) + 1;
 }
 
-// The supersample field of a frame for the entry points that accept it, s = 1..4, and the context's motion blur: frames
-// with s > 1 or blur are whole frames only.
-int check_supersample(hmrm_ctx *c, const hmrm_frame *f) {
-	const int s = supersample_of(f);
-	if (s > 4) return fail(c, HMRM_ERR_INVALID, "supersample factor %d: the field (flags bits 8-11) holds s - 1 <= 3", s);
-	if (s == 1 && c->blur_n == 0) return HMRM_OK;
-	const char *kind = c->blur_n ? "motion-blurred" : "supersampled";
-	if (s > 1 && ((long long)s * f->screen_width > 65536 || (long long)s * f->screen_height > 65536))
-		return fail(c, HMRM_ERR_INVALID, "supersample %d of %dx%d: the sub-frame is larger than 65536 per axis", s,
-		            f->screen_width, f->screen_height);
+// The refusals of frames that can only be whole frames: supersampled, motion-blurred and encoded ones; kind names the
+// frames in the messages.
+int check_whole_frame(hmrm_ctx *c, const hmrm_frame *f, const char *kind) {
 	if (f->cycle_period != 1 || f->cycle != 0)
 		return fail(c, HMRM_ERR_INVALID, "%s frames are whole frames: cycle_period 1", kind);
 	if (f->band_count > 1) return fail(c, HMRM_ERR_INVALID, "%s frames are whole frames: band_count <= 1", kind);
@@ -762,6 +742,18 @@ int check_supersample(hmrm_ctx *c, const hmrm_frame *f) {
 	if (f->flags & (HMRM_FLAG_STEP_INDEX | HMRM_FLAG_RAY_DUMP))
 		return fail(c, HMRM_ERR_INVALID, "%s frames do not record step indices or ray dumps", kind);
 	return HMRM_OK;
+}
+
+// The supersample field of a frame for the entry points that accept it, s = 1..4, and the context's motion blur: frames
+// with s > 1 or blur are whole frames only.
+int check_supersample(hmrm_ctx *c, const hmrm_frame *f) {
+	const int s = supersample_of(f);
+	if (s > 4) return fail(c, HMRM_ERR_INVALID, "supersample factor %d: the field (flags bits 8-11) holds s - 1 <= 3", s);
+	if (s == 1 && c->blur_n == 0) return HMRM_OK;
+	if (s > 1 && ((long long)s * f->screen_width > 65536 || (long long)s * f->screen_height > 65536))
+		return fail(c, HMRM_ERR_INVALID, "supersample %d of %dx%d: the sub-frame is larger than 65536 per axis", s,
+		            f->screen_width, f->screen_height);
+	return check_whole_frame(c, f, c->blur_n ? "motion-blurred" : "supersampled");
 }
 
 void set_camera(hmrm_frame *f, const hmrm_camera &cam) {
@@ -826,22 +818,8 @@ int enqueue_frame(hmrm_ctx *c, const hmrm_frame *f, uint32_t *d_out, cudaStream_
 	if (b.used) HMRM_CUDA(c, cudaEventSynchronize(b.ev_read));
 	const int G = std::min(n, kDownMaxPlanes);
 	const size_t plane = (size_t)sf.screen_width * (size_t)sf.screen_height;     // words
-	const size_t need = plane * 4 * (size_t)G;
-	if (need > b.cap) {
-		cudaFree(b.d);
-		b.d = NULL;
-		b.cap = 0;
-		HMRM_CUDA(c, cudaMalloc(&b.d, need));
-		b.cap = need;
-	}
-	const size_t acc_need = n > G ? (size_t)W * (size_t)H * sizeof(uint2) : 0;
-	if (acc_need > b.acc_cap) {
-		cudaFree(b.acc);
-		b.acc = NULL;
-		b.acc_cap = 0;
-		HMRM_CUDA(c, cudaMalloc(&b.acc, acc_need));
-		b.acc_cap = acc_need;
-	}
+	if (int rc = grow(c, &b.d, &b.cap, plane * 4 * (size_t)G)) return rc;
+	if (int rc = grow(c, &b.acc, &b.acc_cap, n > G ? (size_t)W * (size_t)H * sizeof(uint2) : 0)) return rc;
 	const dim3 grid((unsigned)(((W + kDownStrip - 1) / kDownStrip + kDownThreads - 1) / kDownThreads), (unsigned)H);
 	uint8_t *out = (uint8_t *)d_out;
 	const bool rgb8 = f->pixel_format == HMRM_PIXEL_RGB8;
@@ -866,12 +844,13 @@ int enqueue_frame(hmrm_ctx *c, const hmrm_frame *f, uint32_t *d_out, cudaStream_
 	return HMRM_OK;
 }
 
-// D2H of what one launch rendered: rows [rb, re), or with band_count > 1 only the tile rows of that band (several
-// ranks may fill one shared, registered host frame, each over its own PCIe link): one strided copy + the ragged last
-// tile row.  Enqueued on the copy stream.
-int enqueue_copy_out(hmrm_ctx *c, const hmrm_frame *f, const uint32_t *fb, uint8_t *rgba_out, int rb, int re,
-                     cudaMemcpyKind kind = cudaMemcpyDeviceToHost, cudaStream_t on = NULL) {
-	const cudaStream_t copy_stream = on ? on : c->copy_stream;
+// D2H of what one launch of `f` rendered: its row band [rb, re), or with band_count > 1 only the tile rows of that band
+// (several ranks may fill one shared, registered host frame, each over its own PCIe link): one strided copy + the
+// ragged last tile row.  Enqueued on copy_stream.
+int enqueue_copy_out(hmrm_ctx *c, const hmrm_frame *f, const uint32_t *fb, uint8_t *rgba_out, cudaMemcpyKind kind,
+                     cudaStream_t copy_stream) {
+	int rb = f->row_begin, re = f->row_end;
+	if (rb == 0 && re == 0) re = f->screen_height;
 	const size_t row_bytes = (size_t)f->screen_width * (f->pixel_format == HMRM_PIXEL_RGB8 ? 3 : 4);
 	if (f->band_count > 1) {
 		const int tile_rows = (re - rb + 3) / 4;
@@ -968,30 +947,50 @@ int peer_arrive(hmrm_ctx *c, PeerCtrl *ctrl, const hmrm_frame *f, unsigned int u
 	return HMRM_OK;
 }
 
-// ---- PNG frames (K3, csrc/k3_png.cuh) ------------------------------------------------------------------------------
-void free_png_scratch(PngScratch &p) {
-	cudaFree(p.filt);
-	cudaFree(p.stage);
-	cudaFree(p.meta);
-	cudaFree(p.info);
-	cudaFree(p.offsets);
-	std::memset(&p, 0, sizeof p);
+// ---- encoder scratch of the ring slots ------------------------------------------------------------------------------
+// One buffer per slot serves K3, K4 and K6 alike.  Two frames of one slot are ordered on one stream (the copy stream, or
+// c->stream after drain for the one-shot calls), and each encoder writes every scratch byte it reads within its frame,
+// so what an earlier frame of another format left there is never read.
+int ensure_slot_scratch(hmrm_ctx *c, int slot, size_t need) {
+	if (need <= c->scratch_cap[slot]) return HMRM_OK;
+	// the slot's previous frame may still be encoding from, or copying out of, the buffer about to be replaced
+	if (c->copy_pending[slot]) HMRM_CUDA(c, cudaEventSynchronize(c->ev_copied[slot]));
+	return grow(c, &c->d_scratch[slot], &c->scratch_cap[slot], need);
 }
 
-int ensure_png_scratch(hmrm_ctx *c, int slot, const PngShape &s) {
-	PngScratch &p = c->png[slot];
-	if (p.filt && p.filt_cap >= s.total && p.seg_cap >= s.nseg) return HMRM_OK;
-	// the slot's previous PNG frame may still be encoding from the buffers about to be replaced
-	if (c->copy_pending[slot]) HMRM_CUDA(c, cudaEventSynchronize(c->ev_copied[slot]));
-	free_png_scratch(p);
-	HMRM_CUDA(c, cudaMalloc(&p.filt, (size_t)s.total));
-	HMRM_CUDA(c, cudaMalloc(&p.stage, (size_t)s.nseg * kPngStageStride));
-	HMRM_CUDA(c, cudaMalloc(&p.meta, kPngMetaBytes));
-	HMRM_CUDA(c, cudaMalloc(&p.info, (size_t)s.nseg * sizeof(PngSegInfo)));
-	HMRM_CUDA(c, cudaMalloc(&p.offsets, ((size_t)s.nseg + 3) * sizeof(unsigned long long)));
-	p.filt_cap = s.total;
-	p.seg_cap = s.nseg;
-	return HMRM_OK;
+// Lays pieces out back to back from `base`, each on a 256-byte boundary (K3's gather reads uint4 words of the staged
+// pieces, K6 int16 / uint32 arrays); `bytes` is what they take.  From base 0 it only counts.
+struct Carve {
+	uintptr_t base;
+	size_t bytes;
+	template <class T>
+	T *take(unsigned long long n) {
+		T *p = (T *)(base + bytes);
+		bytes += ((size_t)n * sizeof(T) + 255) & ~(size_t)255;
+		return p;
+	}
+};
+
+// ---- PNG frames (K3, csrc/k3_png.cuh) ------------------------------------------------------------------------------
+// K3's pieces of a slot's scratch: filtered stream, staged chunks, signature / IHDR / tail chunks, per-segment sizes /
+// Adler-32 partials, piece offsets
+struct PngPieces {
+	uint8_t *filt, *stage, *meta;
+	PngSegInfo *info;
+	unsigned long long *offsets;
+	size_t bytes;
+};
+
+PngPieces png_pieces(const PngShape &s, uint8_t *scratch) {
+	Carve k = {(uintptr_t)scratch, 0};
+	PngPieces p;
+	p.filt = k.take<uint8_t>(s.total);
+	p.stage = k.take<uint8_t>((unsigned long long)s.nseg * kPngStageStride);
+	p.meta = k.take<uint8_t>(kPngMetaBytes);
+	p.info = k.take<PngSegInfo>((unsigned long long)s.nseg);
+	p.offsets = k.take<unsigned long long>((unsigned long long)s.nseg + 3);
+	p.bytes = k.bytes;
+	return p;
 }
 
 // The address the device writes `p` through: device memory of the context's device as it is, pinned / registered host
@@ -1039,12 +1038,11 @@ int file_outputs(hmrm_ctx *c, const char *fmt, unsigned long long bound, uint8_t
 }
 
 // Enqueue the four K3 launches on `st`: d_img [H][W][C] -> PNG file at d_dst, its size at d_size.
-int enqueue_png(hmrm_ctx *c, int slot, const uint8_t *d_img, int W, int H, int C, uint8_t *d_dst,
+int enqueue_png(hmrm_ctx *c, uint8_t *scratch, const uint8_t *d_img, int W, int H, int C, uint8_t *d_dst,
                 unsigned long long *d_size, cudaStream_t st) {
-	PngShape s;
+	PngShape s{};
 	png_shape(W, H, C, &s);
-	if (int rc = ensure_png_scratch(c, slot, s)) return rc;
-	const PngScratch &p = c->png[slot];
+	const PngPieces p = png_pieces(s, scratch);
 	k3_png_filter<<<H, 256, 0, st>>>(d_img, (int)s.row_bytes, C, p.filt);
 	// the byte one row up is a candidate distance while deflate can reach it
 	const int row_dist = s.row_bytes + 1 <= 32768ull ? (int)(s.row_bytes + 1) : 0;
@@ -1059,33 +1057,7 @@ int enqueue_png(hmrm_ctx *c, int slot, const uint8_t *d_img, int W, int H, int C
 	return HMRM_OK;
 }
 
-// The caller's pixels in the context's staging buffer (hmrm_encode_png, hmrm_convert_yuv420), copied on c->stream.
-// The context must be drained: the buffer may be replaced.
-int stage_pixels(hmrm_ctx *c, const uint8_t *pixels, size_t bytes) {
-	if (bytes > c->png_in_cap) {
-		cudaFree(c->d_png_in);
-		c->d_png_in = NULL;
-		c->png_in_cap = 0;
-		HMRM_CUDA(c, cudaMalloc(&c->d_png_in, bytes));
-		c->png_in_cap = bytes;
-	}
-	HMRM_CUDA(c, cudaMemcpyAsync(c->d_png_in, pixels, bytes, cudaMemcpyDefault, c->stream));
-	return HMRM_OK;
-}
-
 // ---- YUV frames (K4, csrc/k4_yuv.cuh) ------------------------------------------------------------------------------
-int ensure_yuv_scratch(hmrm_ctx *c, int slot, size_t bytes) {
-	if (c->d_yuv[slot] && c->yuv_cap[slot] >= bytes) return HMRM_OK;
-	// the slot's previous YUV frame may still be converting into, or copying out of, the buffer about to be replaced
-	if (c->copy_pending[slot]) HMRM_CUDA(c, cudaEventSynchronize(c->ev_copied[slot]));
-	cudaFree(c->d_yuv[slot]);
-	c->d_yuv[slot] = NULL;
-	c->yuv_cap[slot] = 0;
-	HMRM_CUDA(c, cudaMalloc(&c->d_yuv[slot], bytes));
-	c->yuv_cap[slot] = bytes;
-	return HMRM_OK;
-}
-
 // validates matrix / out / capacity for a W x H frame
 int yuv_output(hmrm_ctx *c, int W, int H, int32_t matrix, uint8_t *out, size_t capacity) {
 	if (matrix != HMRM_YUV_BT601 && matrix != HMRM_YUV_BT709) return fail(c, HMRM_ERR_INVALID, "unknown YUV matrix %d", matrix);
@@ -1098,30 +1070,25 @@ int yuv_output(hmrm_ctx *c, int W, int H, int32_t matrix, uint8_t *out, size_t c
 	return device_view(c, out, "out", &unused);
 }
 
-// Enqueue K4 on `st`: d_img [H][W][C] -> the slot's planes, then one copy of them to `out` (host or device memory).
-int enqueue_yuv(hmrm_ctx *c, int slot, const uint8_t *d_img, int W, int H, int C, int32_t matrix, uint8_t *out,
+// Enqueue K4 on `st`: d_img [H][W][C] -> I420 planes in the slot's scratch, then one copy of them to `out` (host or
+// device memory).
+int enqueue_yuv(hmrm_ctx *c, uint8_t *scratch, const uint8_t *d_img, int W, int H, int C, int32_t matrix, uint8_t *out,
                 cudaStream_t st) {
 	const size_t bytes = (size_t)yuv420_bytes(W, H);
-	if (int rc = ensure_yuv_scratch(c, slot, bytes)) return rc;
 	const dim3 grid((unsigned)(((W + 7) / 8 + kYuvThreads - 1) / kYuvThreads), (unsigned)((H + 1) / 2));
-	if (C == 4) k4_yuv420<4><<<grid, kYuvThreads, 0, st>>>(d_img, W, H, kYuvCoef[matrix], c->d_yuv[slot]);
-	else k4_yuv420<3><<<grid, kYuvThreads, 0, st>>>(d_img, W, H, kYuvCoef[matrix], c->d_yuv[slot]);
+	if (C == 4) k4_yuv420<4><<<grid, kYuvThreads, 0, st>>>(d_img, W, H, kYuvCoef[matrix], scratch);
+	else k4_yuv420<3><<<grid, kYuvThreads, 0, st>>>(d_img, W, H, kYuvCoef[matrix], scratch);
 	HMRM_CUDA(c, cudaGetLastError());
-	HMRM_CUDA(c, cudaMemcpyAsync(out, c->d_yuv[slot], bytes, cudaMemcpyDefault, st));
+	HMRM_CUDA(c, cudaMemcpyAsync(out, scratch, bytes, cudaMemcpyDefault, st));
 	return HMRM_OK;
 }
 
 // The refusals every whole-frame encoder shares (hmrm_render_png_async, _yuv420_async, _jpeg_async); kind names the
 // frames in the messages.
-int check_whole_frame(hmrm_ctx *c, const hmrm_frame *f, const char *kind) {
+int check_encoded_frame(hmrm_ctx *c, const hmrm_frame *f, const char *kind) {
 	if (!f) return fail(c, HMRM_ERR_INVALID, "frame is NULL");
 	if (int rc = check_supersample(c, f)) return rc;
-	if (f->cycle_period != 1 || f->cycle != 0) return fail(c, HMRM_ERR_INVALID, "%s frames are whole frames: cycle_period 1", kind);
-	if (f->band_count > 1) return fail(c, HMRM_ERR_INVALID, "%s frames are whole frames: band_count <= 1", kind);
-	if (f->flags & (HMRM_FLAG_STEP_INDEX | HMRM_FLAG_RAY_DUMP))
-		return fail(c, HMRM_ERR_INVALID, "%s frames do not record step indices or ray dumps", kind);
-	if (f->row_begin != 0 || (f->row_end != 0 && f->row_end != f->screen_height))
-		return fail(c, HMRM_ERR_INVALID, "%s frames are whole frames: row_begin 0, row_end 0 or screen_height", kind);
+	if (int rc = check_whole_frame(c, f, kind)) return rc;
 	if (f->pixel_format != HMRM_PIXEL_RGBA8 && f->pixel_format != HMRM_PIXEL_RGB8)
 		return fail(c, HMRM_ERR_INVALID, "unknown pixel_format %d", (int)f->pixel_format);
 	if (f->screen_width < 2 || f->screen_height < 2 || f->screen_width > 65536 || f->screen_height > 65536)
@@ -1130,40 +1097,30 @@ int check_whole_frame(hmrm_ctx *c, const hmrm_frame *f, const char *kind) {
 }
 
 // ---- JPEG frames (K6, csrc/k6_jpeg.cuh) ----------------------------------------------------------------------------
-void free_jpeg_scratch(JpegScratch &p) {
-	cudaFree(p.coef);
-	cudaFree(p.acbits);
-	cudaFree(p.boff);
-	cudaFree(p.rowbits);
-	cudaFree(p.stage);
-	cudaFree(p.meta);
-	cudaFree(p.rowsize);
-	cudaFree(p.offsets);
-	std::memset(&p, 0, sizeof p);
-}
+// K6's pieces of a slot's scratch: quantised coefficients, AC bit counts and bit offsets per block, the rows' bit buffers
+// and stuffed pieces, header / EOI, row sizes, piece offsets
+struct JpegPieces {
+	int16_t *coef;
+	uint16_t *acbits;
+	uint32_t *boff, *rowbits;
+	uint8_t *stage, *meta;
+	unsigned long long *rowsize, *offsets;
+	size_t bytes;
+};
 
-int ensure_jpeg_scratch(hmrm_ctx *c, int slot, const JpegShape &s) {
-	JpegScratch &p = c->jpeg[slot];
-	const unsigned long long words = s.row_words * (unsigned long long)s.mcuy;
-	const unsigned long long staged = s.row_stride * (unsigned long long)s.mcuy;
-	if (p.coef && p.blocks_cap >= s.blocks && p.words_cap >= words && p.stage_cap >= staged && p.rows_cap >= s.mcuy)
-		return HMRM_OK;
-	// the slot's previous JPEG frame may still be encoding from the buffers about to be replaced
-	if (c->copy_pending[slot]) HMRM_CUDA(c, cudaEventSynchronize(c->ev_copied[slot]));
-	free_jpeg_scratch(p);
-	HMRM_CUDA(c, cudaMalloc(&p.coef, (size_t)s.blocks * 64 * sizeof(int16_t)));
-	HMRM_CUDA(c, cudaMalloc(&p.acbits, (size_t)s.blocks * sizeof(uint16_t)));
-	HMRM_CUDA(c, cudaMalloc(&p.boff, (size_t)s.blocks * sizeof(uint32_t)));
-	HMRM_CUDA(c, cudaMalloc(&p.rowbits, (size_t)words * sizeof(uint32_t)));
-	HMRM_CUDA(c, cudaMalloc(&p.stage, (size_t)staged));
-	HMRM_CUDA(c, cudaMalloc(&p.meta, kJpegMetaBytes));
-	HMRM_CUDA(c, cudaMalloc(&p.rowsize, (size_t)s.mcuy * sizeof(unsigned long long)));
-	HMRM_CUDA(c, cudaMalloc(&p.offsets, ((size_t)s.mcuy + 3) * sizeof(unsigned long long)));
-	p.blocks_cap = s.blocks;
-	p.words_cap = words;
-	p.stage_cap = staged;
-	p.rows_cap = s.mcuy;
-	return HMRM_OK;
+JpegPieces jpeg_pieces(const JpegShape &s, uint8_t *scratch) {
+	Carve k = {(uintptr_t)scratch, 0};
+	JpegPieces p;
+	p.coef = k.take<int16_t>(s.blocks * 64);
+	p.acbits = k.take<uint16_t>(s.blocks);
+	p.boff = k.take<uint32_t>(s.blocks);
+	p.rowbits = k.take<uint32_t>(s.row_words * (unsigned long long)s.mcuy);
+	p.stage = k.take<uint8_t>(s.row_stride * (unsigned long long)s.mcuy);
+	p.meta = k.take<uint8_t>(kJpegMetaBytes);
+	p.rowsize = k.take<unsigned long long>((unsigned long long)s.mcuy);
+	p.offsets = k.take<unsigned long long>((unsigned long long)s.mcuy + 3);
+	p.bytes = k.bytes;
+	return p;
 }
 
 int jpeg_params(hmrm_ctx *c, int32_t quality, int32_t chroma) {
@@ -1173,12 +1130,11 @@ int jpeg_params(hmrm_ctx *c, int32_t quality, int32_t chroma) {
 }
 
 // Enqueue the K6 launches and K3's gather on `st`: d_img [H][W][C] -> JPEG file at d_dst, its size at d_size.
-int enqueue_jpeg(hmrm_ctx *c, int slot, const uint8_t *d_img, int W, int H, int C, int quality, int chroma,
+int enqueue_jpeg(hmrm_ctx *c, uint8_t *scratch, const uint8_t *d_img, int W, int H, int C, int quality, int chroma,
                  uint8_t *d_dst, unsigned long long *d_size, cudaStream_t st) {
-	JpegShape s;
+	JpegShape s{};
 	jpeg_shape(W, H, chroma == HMRM_JPEG_420, &s);
-	if (int rc = ensure_jpeg_scratch(c, slot, s)) return rc;
-	const JpegScratch &p = c->jpeg[slot];
+	const JpegPieces p = jpeg_pieces(s, scratch);
 	const int tile_mcus = kJpegTileBlocks / s.bpm;
 	const dim3 grid((unsigned)((s.mcux + tile_mcus - 1) / tile_mcus), (unsigned)s.mcuy);
 	const JpegQuant q = jpeg_quant(quality);
@@ -1194,6 +1150,93 @@ int enqueue_jpeg(hmrm_ctx *c, int slot, const uint8_t *d_img, int W, int H, int 
 	k3_png_gather<<<blocks, 256, 0, st>>>(p.offsets, s.mcuy + 2, p.meta, p.meta + kJpegMetaTail, p.stage, s.row_stride,
 	                                      d_dst, d_size);
 	HMRM_CUDA(c, cudaGetLastError());
+	return HMRM_OK;
+}
+
+// ---- the output stage, the frame ring and the one-shot encoders -----------------------------------------------------
+// Where a finished [H][W][C] image goes.  PNG, JPEG and YUV work in `scratch` bytes of a ring slot's scratch.
+struct Output {
+	enum Kind { RAW, PNG, JPEG, YUV } kind;
+	uint8_t *dst;                  // RAW, YUV: the caller's memory, written by the copy engine; PNG, JPEG: the device
+	                               // address of the file destination (file_outputs)
+	unsigned long long *size;      // PNG, JPEG: the device address of the file's size word
+	size_t scratch;
+	const hmrm_frame *frame;       // RAW: the frame whose row band, or band of band_count, is copied out
+	int quality, chroma;           // JPEG
+	int matrix;                    // YUV
+};
+
+// Enqueue the output stage of the image d_img on `st`, with ring slot `slot`'s scratch
+int enqueue_output(hmrm_ctx *c, const Output &o, int slot, const uint8_t *d_img, int W, int H, int C, cudaStream_t st) {
+	uint8_t *scratch = c->d_scratch[slot];
+	switch (o.kind) {
+	case Output::RAW: return enqueue_copy_out(c, o.frame, (const uint32_t *)d_img, o.dst, cudaMemcpyDeviceToHost, st);
+	case Output::PNG: return enqueue_png(c, scratch, d_img, W, H, C, o.dst, o.size, st);
+	case Output::JPEG: return enqueue_jpeg(c, scratch, d_img, W, H, C, o.quality, o.chroma, o.dst, o.size, st);
+	case Output::YUV: return enqueue_yuv(c, scratch, d_img, W, H, C, o.matrix, o.dst, st);
+	}
+	return fail(c, HMRM_ERR_INVALID, "unknown output kind %d", (int)o.kind);
+}
+
+// The frame ring, the one owner of its protocol: every frame of hmrm_render_async, _png_async, _jpeg_async and
+// _yuv420_async is rendered into a ring buffer on the buffer's compute stream, and its output stage runs on the copy
+// stream.  Whole frames (cycle_period 1) rotate through kFrameRing device buffers so that the output stage of frame n
+// overlaps the kernels of frames n+1 and n+2; the progressive interleave (cycle_period > 1) accumulates in the one
+// persistent buffer.  Each buffer has its own compute stream, so the kernel of the next frame starts filling SMs as the
+// CTAs of this one run out of tiles (a handful of grazing tiles take ~50x the mean: the tail of a frame leaves most SMs
+// idle).
+int enqueue_ring(hmrm_ctx *c, const hmrm_frame *f, const Output &o) {
+	int rc = ensure_framebuffer(c, f->screen_width, f->screen_height, f->pixel_format);
+	if (rc) return rc;
+	const bool whole = f->cycle_period == 1 && (f->flags & (HMRM_FLAG_STEP_INDEX | HMRM_FLAG_RAY_DUMP)) == 0;
+	const int slot = whole ? (c->slot + 1) % kFrameRing : 0;
+	if ((rc = ensure_slot_scratch(c, slot, o.scratch)) != HMRM_OK) return rc;
+	uint32_t *fb = c->d_fb[slot];
+	cudaStream_t cs = c->ring_stream[slot];
+	// nothing may be written into this buffer (by the kernel, or by the copy below) while an earlier frame's output
+	// stage still reads it
+	if (c->copy_pending[slot]) HMRM_CUDA(c, cudaStreamWaitEvent(cs, c->ev_copied[slot], 0));
+	if (!whole) {
+		// progressive frames and step-index captures are ordered after everything else
+		for (int i = 1; i < kFrameRing; ++i) HMRM_CUDA(c, cudaStreamSynchronize(c->ring_stream[i]));
+		if (f->cycle_period != 1 && c->slot != 0) {
+			// the newest picture lives in another buffer of the ring: a progressive frame must land on top of it
+			HMRM_CUDA(c, cudaMemcpyAsync(c->d_fb[0], c->d_fb[c->slot], (size_t)c->fb_w * (size_t)c->fb_h * 4,
+			                             cudaMemcpyDeviceToDevice, cs));
+		}
+	}
+	// (Rendering a frame that finds the pipeline idle as four interleaved bands, each copied out as soon as its kernel
+	// is done, was measured: four launches mean four tails, the stream turns kernel-bound and stays "idle", 0.59 ->
+	// 0.63 ms per frame.  Frames stay whole.)
+	if ((rc = enqueue_frame(c, f, fb, cs)) != HMRM_OK) return rc;
+	HMRM_CUDA(c, cudaEventRecord(c->ev_rendered[slot], cs));
+	HMRM_CUDA(c, cudaStreamWaitEvent(c->copy_stream, c->ev_rendered[slot], 0));
+	const int C = f->pixel_format == HMRM_PIXEL_RGB8 ? 3 : 4;
+	rc = enqueue_output(c, o, slot, (const uint8_t *)fb, f->screen_width, f->screen_height, C, c->copy_stream);
+	if (rc) return rc;
+	HMRM_CUDA(c, cudaEventRecord(c->ev_copied[slot], c->copy_stream));
+	c->copy_pending[slot] = true;
+	c->slot = slot;
+	return HMRM_OK;
+}
+
+// The caller's pixels in the context's staging buffer, copied on c->stream.  The context must be drained: the buffer
+// may be replaced.
+int stage_pixels(hmrm_ctx *c, const uint8_t *pixels, size_t bytes) {
+	if (int rc = grow(c, &c->d_pixels, &c->pixels_cap, bytes)) return rc;
+	HMRM_CUDA(c, cudaMemcpyAsync(c->d_pixels, pixels, bytes, cudaMemcpyDefault, c->stream));
+	return HMRM_OK;
+}
+
+// hmrm_encode_png, _jpeg and hmrm_convert_yuv420: synchronous.  Whatever the context has in flight finishes first, then
+// ring slot 0's scratch is free for the output stage of the caller's [H][W][C] pixels on c->stream.
+int encode_staged(hmrm_ctx *c, const Output &o, const uint8_t *pixels, int W, int H, int C) {
+	int rc = drain(c);
+	if (rc) return rc;
+	if ((rc = stage_pixels(c, pixels, (size_t)W * (size_t)H * (size_t)C)) != HMRM_OK) return rc;
+	if ((rc = ensure_slot_scratch(c, 0, o.scratch)) != HMRM_OK) return rc;
+	if ((rc = enqueue_output(c, o, 0, c->d_pixels, W, H, C, c->stream)) != HMRM_OK) return rc;
+	HMRM_CUDA(c, cudaStreamSynchronize(c->stream));
 	return HMRM_OK;
 }
 
@@ -1301,12 +1344,10 @@ int hmrm_create(int device, hmrm_ctx **out) {
 	c->copy_stream = NULL;
 	c->slot = 0;
 	c->fb_format = HMRM_PIXEL_RGBA8;
-	std::memset(c->png, 0, sizeof c->png);
-	std::memset(c->jpeg, 0, sizeof c->jpeg);
-	c->d_png_in = NULL;
-	c->png_in_cap = 0;
-	std::memset(c->d_yuv, 0, sizeof c->d_yuv);
-	std::memset(c->yuv_cap, 0, sizeof c->yuv_cap);
+	std::memset(c->d_scratch, 0, sizeof c->d_scratch);
+	std::memset(c->scratch_cap, 0, sizeof c->scratch_cap);
+	c->d_pixels = NULL;
+	c->pixels_cap = 0;
 	std::memset(c->sub, 0, sizeof c->sub);
 	c->sub_next = 0;
 	c->blur_n = 0;
@@ -1357,11 +1398,9 @@ void hmrm_destroy(hmrm_ctx *c) {
 	cudaFree(c->d_htab);
 
 	if (c->copy_stream) cudaStreamSynchronize(c->copy_stream);
-	cudaFree(c->d_png_in);
+	cudaFree(c->d_pixels);
 	for (int i = 0; i < kFrameRing; ++i) {
-		free_png_scratch(c->png[i]);
-		free_jpeg_scratch(c->jpeg[i]);
-		cudaFree(c->d_yuv[i]);
+		cudaFree(c->d_scratch[i]);
 		cudaFree(c->d_fb[i]);
 		if (c->ev_rendered[i]) cudaEventDestroy(c->ev_rendered[i]);
 		if (c->ev_copied[i]) cudaEventDestroy(c->ev_copied[i]);
@@ -1661,44 +1700,9 @@ int hmrm_render_async(hmrm_ctx *c, const hmrm_frame *f, uint8_t *rgba_out) {
 	HMRM_CUDA(c, cudaSetDevice(c->device));
 	if (f->pixel_format != HMRM_PIXEL_RGBA8 && f->pixel_format != HMRM_PIXEL_RGB8)
 		return fail(c, HMRM_ERR_INVALID, "unknown pixel_format %d", (int)f->pixel_format);
-	int rc = ensure_framebuffer(c, f->screen_width, f->screen_height, f->pixel_format);
-	if (rc) return rc;
-	// Whole frames (cycle_period 1) rotate through kFrameRing device buffers so that the copy-out of frame n overlaps
-	// the kernels of frames n+1 and n+2; the progressive interleave (cycle_period > 1) accumulates in the one
-	// persistent buffer.  Each buffer has its own compute stream, so the kernel of the next frame starts filling SMs as
-	// the CTAs of this one run out of tiles (a handful of grazing tiles take ~50x the mean: the tail of a frame
-	// leaves most SMs idle).
-	const bool whole = f->cycle_period == 1 && (f->flags & (HMRM_FLAG_STEP_INDEX | HMRM_FLAG_RAY_DUMP)) == 0;
-	const int slot = whole ? (c->slot + 1) % kFrameRing : 0;
-	uint32_t *fb = c->d_fb[slot];
-	cudaStream_t cs = c->ring_stream[slot];
-	// nothing may be written into this buffer (by the kernel, or by the copy below) while an earlier frame is still
-	// being copied out of it
-	if (c->copy_pending[slot]) HMRM_CUDA(c, cudaStreamWaitEvent(cs, c->ev_copied[slot], 0));
-	if (!whole) {
-		// progressive frames and step-index captures are ordered after everything else
-		for (int i = 1; i < kFrameRing; ++i) HMRM_CUDA(c, cudaStreamSynchronize(c->ring_stream[i]));
-		if (f->cycle_period != 1 && c->slot != 0) {
-			// the newest picture lives in another buffer of the ring: a progressive frame must land on top of it
-			HMRM_CUDA(c, cudaMemcpyAsync(c->d_fb[0], c->d_fb[c->slot], (size_t)c->fb_w * (size_t)c->fb_h * 4,
-			                             cudaMemcpyDeviceToDevice, cs));
-		}
-	}
-	int rb = f->row_begin, re = f->row_end;
-	if (rb == 0 && re == 0) re = f->screen_height;
-	// (Rendering a frame that finds the pipeline idle as four interleaved bands, each copied out as soon as its kernel
-	// is done, was measured: four launches mean four tails, the stream turns kernel-bound and stays "idle", 0.59 ->
-	// 0.63 ms per frame.  Frames stay whole.)
-	rc = enqueue_frame(c, f, fb, cs);
-	if (rc) return rc;
-	HMRM_CUDA(c, cudaEventRecord(c->ev_rendered[slot], cs));
-	HMRM_CUDA(c, cudaStreamWaitEvent(c->copy_stream, c->ev_rendered[slot], 0));
-	rc = enqueue_copy_out(c, f, fb, rgba_out, rb, re);
-	if (rc) return rc;
-	HMRM_CUDA(c, cudaEventRecord(c->ev_copied[slot], c->copy_stream));
-	c->copy_pending[slot] = true;
-	c->slot = slot;
-	return HMRM_OK;
+	Output o = {Output::RAW, rgba_out};
+	o.frame = f;
+	return enqueue_ring(c, f, o);
 }
 
 int hmrm_wait_pending(hmrm_ctx *c, int max_pending) {
@@ -1737,30 +1741,13 @@ size_t hmrm_png_bound(int32_t width, int32_t height, int32_t channels) {
 
 int hmrm_render_png_async(hmrm_ctx *c, const hmrm_frame *f, uint8_t *png_out, size_t capacity, uint64_t *png_bytes) {
 	if (!c) return HMRM_ERR_INVALID;
-	if (int rc = check_whole_frame(c, f, "PNG")) return rc;
-	const int C = f->pixel_format == HMRM_PIXEL_RGB8 ? 3 : 4;
+	if (int rc = check_encoded_frame(c, f, "PNG")) return rc;
 	PngShape s{};
-	png_shape(f->screen_width, f->screen_height, C, &s);
-	uint8_t *d_out = NULL;
-	unsigned long long *d_size = NULL;
-	int rc = file_outputs(c, "png", png_bound(s), png_out, capacity, png_bytes, &d_out, &d_size);
-	if (rc) return rc;
-	if ((rc = ensure_framebuffer(c, f->screen_width, f->screen_height, f->pixel_format)) != HMRM_OK) return rc;
-	// the ring exactly as hmrm_render_async uses it for whole frames; the encoder takes the place of the copy-out
-	const int slot = (c->slot + 1) % kFrameRing;
-	if ((rc = ensure_png_scratch(c, slot, s)) != HMRM_OK) return rc;
-	uint32_t *fb = c->d_fb[slot];
-	cudaStream_t cs = c->ring_stream[slot];
-	if (c->copy_pending[slot]) HMRM_CUDA(c, cudaStreamWaitEvent(cs, c->ev_copied[slot], 0));
-	if ((rc = enqueue_frame(c, f, fb, cs)) != HMRM_OK) return rc;
-	HMRM_CUDA(c, cudaEventRecord(c->ev_rendered[slot], cs));
-	HMRM_CUDA(c, cudaStreamWaitEvent(c->copy_stream, c->ev_rendered[slot], 0));
-	rc = enqueue_png(c, slot, (const uint8_t *)fb, f->screen_width, f->screen_height, C, d_out, d_size, c->copy_stream);
-	if (rc) return rc;
-	HMRM_CUDA(c, cudaEventRecord(c->ev_copied[slot], c->copy_stream));
-	c->copy_pending[slot] = true;
-	c->slot = slot;
-	return HMRM_OK;
+	png_shape(f->screen_width, f->screen_height, f->pixel_format == HMRM_PIXEL_RGB8 ? 3 : 4, &s);
+	Output o = {Output::PNG};
+	if (int rc = file_outputs(c, "png", png_bound(s), png_out, capacity, png_bytes, &o.dst, &o.size)) return rc;
+	o.scratch = png_pieces(s, NULL).bytes;
+	return enqueue_ring(c, f, o);
 }
 
 int hmrm_encode_png(hmrm_ctx *c, const uint8_t *pixels, int32_t width, int32_t height, int32_t channels,
@@ -1771,16 +1758,10 @@ int hmrm_encode_png(hmrm_ctx *c, const uint8_t *pixels, int32_t width, int32_t h
 	if (!png_shape(width, height, channels, &s))
 		return fail(c, HMRM_ERR_INVALID, "image %dx%dx%d: need 1 <= width, height <= 65536 and 3 or 4 channels", width,
 		            height, channels);
-	uint8_t *d_out = NULL;
-	unsigned long long *d_size = NULL;
-	int rc = file_outputs(c, "png", png_bound(s), png_out, capacity, png_bytes, &d_out, &d_size);
-	if (rc) return rc;
-	// synchronous: whatever the context has in flight finishes first, then ring slot 0's scratch is free
-	if ((rc = drain(c)) != HMRM_OK) return rc;
-	if ((rc = stage_pixels(c, pixels, (size_t)width * (size_t)height * (size_t)channels)) != HMRM_OK) return rc;
-	if ((rc = enqueue_png(c, 0, c->d_png_in, width, height, channels, d_out, d_size, c->stream)) != HMRM_OK) return rc;
-	HMRM_CUDA(c, cudaStreamSynchronize(c->stream));
-	return HMRM_OK;
+	Output o = {Output::PNG};
+	if (int rc = file_outputs(c, "png", png_bound(s), png_out, capacity, png_bytes, &o.dst, &o.size)) return rc;
+	o.scratch = png_pieces(s, NULL).bytes;
+	return encode_staged(c, o, pixels, width, height, channels);
 }
 
 size_t hmrm_jpeg_bound(int32_t width, int32_t height, int32_t chroma) {
@@ -1793,34 +1774,18 @@ size_t hmrm_jpeg_bound(int32_t width, int32_t height, int32_t chroma) {
 int hmrm_render_jpeg_async(hmrm_ctx *c, const hmrm_frame *f, int32_t quality, int32_t chroma, uint8_t *jpeg_out,
                            size_t capacity, uint64_t *jpeg_bytes) {
 	if (!c) return HMRM_ERR_INVALID;
-	if (int rc = check_whole_frame(c, f, "JPEG")) return rc;
+	if (int rc = check_encoded_frame(c, f, "JPEG")) return rc;
 	if (int rc = jpeg_params(c, quality, chroma)) return rc;
 	JpegShape s;
 	if (!jpeg_shape(f->screen_width, f->screen_height, chroma == HMRM_JPEG_420, &s))
 		return fail(c, HMRM_ERR_INVALID, "resolution %dx%d: a JPEG frame is at most 65535 pixels per axis",
 		            f->screen_width, f->screen_height);
-	const int C = f->pixel_format == HMRM_PIXEL_RGB8 ? 3 : 4;
-	uint8_t *d_out = NULL;
-	unsigned long long *d_size = NULL;
-	int rc = file_outputs(c, "jpeg", jpeg_bound(s), jpeg_out, capacity, jpeg_bytes, &d_out, &d_size);
-	if (rc) return rc;
-	if ((rc = ensure_framebuffer(c, f->screen_width, f->screen_height, f->pixel_format)) != HMRM_OK) return rc;
-	// the ring exactly as hmrm_render_async uses it for whole frames; the encoder takes the place of the copy-out
-	const int slot = (c->slot + 1) % kFrameRing;
-	if ((rc = ensure_jpeg_scratch(c, slot, s)) != HMRM_OK) return rc;
-	uint32_t *fb = c->d_fb[slot];
-	cudaStream_t cs = c->ring_stream[slot];
-	if (c->copy_pending[slot]) HMRM_CUDA(c, cudaStreamWaitEvent(cs, c->ev_copied[slot], 0));
-	if ((rc = enqueue_frame(c, f, fb, cs)) != HMRM_OK) return rc;
-	HMRM_CUDA(c, cudaEventRecord(c->ev_rendered[slot], cs));
-	HMRM_CUDA(c, cudaStreamWaitEvent(c->copy_stream, c->ev_rendered[slot], 0));
-	rc = enqueue_jpeg(c, slot, (const uint8_t *)fb, f->screen_width, f->screen_height, C, quality, chroma, d_out, d_size,
-	                  c->copy_stream);
-	if (rc) return rc;
-	HMRM_CUDA(c, cudaEventRecord(c->ev_copied[slot], c->copy_stream));
-	c->copy_pending[slot] = true;
-	c->slot = slot;
-	return HMRM_OK;
+	Output o = {Output::JPEG};
+	if (int rc = file_outputs(c, "jpeg", jpeg_bound(s), jpeg_out, capacity, jpeg_bytes, &o.dst, &o.size)) return rc;
+	o.scratch = jpeg_pieces(s, NULL).bytes;
+	o.quality = quality;
+	o.chroma = chroma;
+	return enqueue_ring(c, f, o);
 }
 
 int hmrm_encode_jpeg(hmrm_ctx *c, const uint8_t *pixels, int32_t width, int32_t height, int32_t channels,
@@ -1832,42 +1797,24 @@ int hmrm_encode_jpeg(hmrm_ctx *c, const uint8_t *pixels, int32_t width, int32_t 
 	if (!jpeg_shape(width, height, chroma == HMRM_JPEG_420, &s) || (channels != 3 && channels != 4))
 		return fail(c, HMRM_ERR_INVALID, "image %dx%dx%d: need 1 <= width, height <= 65535 and 3 or 4 channels", width,
 		            height, channels);
-	uint8_t *d_out = NULL;
-	unsigned long long *d_size = NULL;
-	int rc = file_outputs(c, "jpeg", jpeg_bound(s), jpeg_out, capacity, jpeg_bytes, &d_out, &d_size);
-	if (rc) return rc;
-	// synchronous: whatever the context has in flight finishes first, then ring slot 0's scratch is free
-	if ((rc = drain(c)) != HMRM_OK) return rc;
-	if ((rc = stage_pixels(c, pixels, (size_t)width * (size_t)height * (size_t)channels)) != HMRM_OK) return rc;
-	rc = enqueue_jpeg(c, 0, c->d_png_in, width, height, channels, quality, chroma, d_out, d_size, c->stream);
-	if (rc) return rc;
-	HMRM_CUDA(c, cudaStreamSynchronize(c->stream));
-	return HMRM_OK;
+	Output o = {Output::JPEG};
+	if (int rc = file_outputs(c, "jpeg", jpeg_bound(s), jpeg_out, capacity, jpeg_bytes, &o.dst, &o.size)) return rc;
+	o.scratch = jpeg_pieces(s, NULL).bytes;
+	o.quality = quality;
+	o.chroma = chroma;
+	return encode_staged(c, o, pixels, width, height, channels);
 }
 
 size_t hmrm_yuv420_bytes(int32_t width, int32_t height) { return (size_t)yuv420_bytes(width, height); }
 
 int hmrm_render_yuv420_async(hmrm_ctx *c, const hmrm_frame *f, int32_t matrix, uint8_t *out, size_t capacity) {
 	if (!c) return HMRM_ERR_INVALID;
-	if (int rc = check_whole_frame(c, f, "YUV")) return rc;
-	const int W = f->screen_width, H = f->screen_height, C = f->pixel_format == HMRM_PIXEL_RGB8 ? 3 : 4;
-	int rc = yuv_output(c, W, H, matrix, out, capacity);
-	if (rc) return rc;
-	if ((rc = ensure_framebuffer(c, W, H, f->pixel_format)) != HMRM_OK) return rc;
-	// the ring exactly as hmrm_render_async uses it for whole frames; conversion + copy take the place of the copy-out
-	const int slot = (c->slot + 1) % kFrameRing;
-	if ((rc = ensure_yuv_scratch(c, slot, (size_t)yuv420_bytes(W, H))) != HMRM_OK) return rc;
-	uint32_t *fb = c->d_fb[slot];
-	cudaStream_t cs = c->ring_stream[slot];
-	if (c->copy_pending[slot]) HMRM_CUDA(c, cudaStreamWaitEvent(cs, c->ev_copied[slot], 0));
-	if ((rc = enqueue_frame(c, f, fb, cs)) != HMRM_OK) return rc;
-	HMRM_CUDA(c, cudaEventRecord(c->ev_rendered[slot], cs));
-	HMRM_CUDA(c, cudaStreamWaitEvent(c->copy_stream, c->ev_rendered[slot], 0));
-	if ((rc = enqueue_yuv(c, slot, (const uint8_t *)fb, W, H, C, matrix, out, c->copy_stream)) != HMRM_OK) return rc;
-	HMRM_CUDA(c, cudaEventRecord(c->ev_copied[slot], c->copy_stream));
-	c->copy_pending[slot] = true;
-	c->slot = slot;
-	return HMRM_OK;
+	if (int rc = check_encoded_frame(c, f, "YUV")) return rc;
+	if (int rc = yuv_output(c, f->screen_width, f->screen_height, matrix, out, capacity)) return rc;
+	Output o = {Output::YUV, out};
+	o.scratch = (size_t)yuv420_bytes(f->screen_width, f->screen_height);
+	o.matrix = matrix;
+	return enqueue_ring(c, f, o);
 }
 
 int hmrm_convert_yuv420(hmrm_ctx *c, const uint8_t *pixels, int32_t width, int32_t height, int32_t channels,
@@ -1877,14 +1824,11 @@ int hmrm_convert_yuv420(hmrm_ctx *c, const uint8_t *pixels, int32_t width, int32
 	if (yuv420_bytes(width, height) == 0 || (channels != 3 && channels != 4))
 		return fail(c, HMRM_ERR_INVALID, "image %dx%dx%d: need 1 <= width, height <= 65536 and 3 or 4 channels", width,
 		            height, channels);
-	int rc = yuv_output(c, width, height, matrix, out, capacity);
-	if (rc) return rc;
-	// synchronous: whatever the context has in flight finishes first, then ring slot 0's scratch is free
-	if ((rc = drain(c)) != HMRM_OK) return rc;
-	if ((rc = stage_pixels(c, pixels, (size_t)width * (size_t)height * (size_t)channels)) != HMRM_OK) return rc;
-	if ((rc = enqueue_yuv(c, 0, c->d_png_in, width, height, channels, matrix, out, c->stream)) != HMRM_OK) return rc;
-	HMRM_CUDA(c, cudaStreamSynchronize(c->stream));
-	return HMRM_OK;
+	if (int rc = yuv_output(c, width, height, matrix, out, capacity)) return rc;
+	Output o = {Output::YUV, out};
+	o.scratch = (size_t)yuv420_bytes(width, height);
+	o.matrix = matrix;
+	return encode_staged(c, o, pixels, width, height, channels);
 }
 
 int hmrm_get_stats(hmrm_ctx *c, hmrm_stats *out) {
@@ -2112,9 +2056,7 @@ int hmrm_render_peer_staged(hmrm_ctx *c, const hmrm_frame *f, void *d_stage, voi
 	// with the copy engine: large transfers instead of the kernel's 24- or 32-byte row pieces
 	rc = peer_wait_word(c, &ctrl->released, use - 1u, &ctrl->error, s);
 	if (rc) return rc;
-	int rb = f->row_begin, re = f->row_end;
-	if (rb == 0 && re == 0) re = f->screen_height;
-	rc = enqueue_copy_out(c, f, (const uint32_t *)d_stage, (uint8_t *)d_frame, rb, re, cudaMemcpyDeviceToDevice, s);
+	rc = enqueue_copy_out(c, f, (const uint32_t *)d_stage, (uint8_t *)d_frame, cudaMemcpyDeviceToDevice, s);
 	if (rc) return rc;
 	return peer_arrive(c, ctrl, f, use, s);
 }

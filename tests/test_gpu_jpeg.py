@@ -120,7 +120,7 @@ def test_encode_jpeg_bit_offsets_past_2_32(hmrm, renderer):
     assert len(want) * 8 > 2 ** 32
     got = renderer.encode_jpeg(torch.from_numpy(px).to("cuda:0"), 100, hmrm.JPEG_444)
     assert len(got) == len(want) and got == want
-    renderer._jpeg_cache = None
+    renderer._pinned_cache.pop("jpeg", None)
 
 
 @pytest.mark.parametrize("name", GOLDEN_NAMES)
