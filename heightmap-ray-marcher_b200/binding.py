@@ -110,6 +110,9 @@ PROTOTYPES = {
     "hmrm_render": (C.c_int, [C.c_void_p, C.POINTER(Frame), C.c_void_p]),
     "hmrm_render_device": (C.c_int, [C.c_void_p, C.POINTER(Frame), C.c_void_p, C.c_void_p]),
     "hmrm_render_async": (C.c_int, [C.c_void_p, C.POINTER(Frame), C.c_void_p]),
+    "hmrm_render_views": (C.c_int, [C.c_void_p, C.POINTER(Frame), C.POINTER(Camera), C.c_int32, C.c_void_p]),
+    "hmrm_render_views_device": (C.c_int, [C.c_void_p, C.POINTER(Frame), C.POINTER(Camera), C.c_int32, C.c_void_p,
+                                           C.c_void_p]),
     "hmrm_wait": (C.c_int, [C.c_void_p]),
     "hmrm_wait_pending": (C.c_int, [C.c_void_p, C.c_int]),
     "hmrm_png_bound": (C.c_size_t, [C.c_int32, C.c_int32, C.c_int32]),
@@ -263,6 +266,31 @@ def _ptr(a) -> int:
     return int(a)
 
 
+def _cameras(cams, what: str):
+    """(hmrm_camera array, n) of a sequence of (pos, hang, vang) with pos three numbers and angles in radians, or of
+    rows (x, y, z, hang, vang): an [n, 5] array or a sequence of five-number rows.  `what` names the cameras in the
+    errors."""
+    if not isinstance(cams, np.ndarray):
+        cams = list(cams)
+        if cams and all(hasattr(c, "__len__") and len(c) == 5 for c in cams):
+            cams = np.asarray(cams, dtype=np.float64)
+    rows = np.asarray(cams, dtype=np.float64) if isinstance(cams, np.ndarray) else None
+    if rows is None:
+        flat = []
+        for pos, hang, vang in cams:
+            pos = [float(v) for v in pos]
+            if len(pos) != 3:
+                raise ValueError(f"a {what} camera's pos has three components, not {len(pos)}")
+            flat.append([*pos, float(hang), float(vang)])
+        rows = np.array(flat, dtype=np.float64).reshape(-1, 5)
+    if rows.ndim != 2 or rows.shape[1] != 5:
+        raise ValueError(f"{what} cameras must be [n, 5], not {rows.shape}")
+    arr = (Camera * max(len(rows), 1))()
+    if len(rows):
+        np.ctypeslib.as_array(C.cast(arr, C.POINTER(C.c_double)), shape=(len(rows), 5))[...] = rows
+    return arr, len(rows)
+
+
 class Renderer:
     """One rendering context on one CUDA device.
 
@@ -392,22 +420,8 @@ class Renderer:
         """Motion blur of every following whole-frame render (include/hmrm.h, hmrm_set_motion_blur): `cams` is a
         sequence of (pos, hang, vang) with pos three numbers and angles in radians, or an [n, 5] float64 array of rows
         (x, y, z, hang, vang); n = 1..16.  `[]` turns blur off."""
-        rows = np.asarray(cams, dtype=np.float64) if isinstance(cams, np.ndarray) else None
-        if rows is None:
-            flat = []
-            for pos, hang, vang in cams:
-                pos = [float(v) for v in pos]
-                if len(pos) != 3:
-                    raise ValueError(f"a motion-blur camera's pos has three components, not {len(pos)}")
-                flat.append([*pos, float(hang), float(vang)])
-            rows = np.array(flat, dtype=np.float64).reshape(-1, 5)
-        if rows.ndim != 2 or rows.shape[1] != 5:
-            raise ValueError(f"motion-blur cameras must be [n, 5], not {rows.shape}")
-        arr = (Camera * max(len(rows), 1))()
-        for i, r in enumerate(rows):
-            arr[i].cam_pos[:] = [float(v) for v in r[:3]]
-            arr[i].hang, arr[i].vang = float(r[3]), float(r[4])
-        self._check(self._lib.hmrm_set_motion_blur(self._h, arr, len(rows)))
+        arr, n = _cameras(cams, "motion-blur")
+        self._check(self._lib.hmrm_set_motion_blur(self._h, arr, n))
 
     def heights(self) -> np.ndarray:
         out = np.empty((self.map_height, self.map_width), dtype=np.float64)
@@ -585,6 +599,31 @@ class Renderer:
 
     def render_device(self, frame: Frame, d_out, stream=None) -> None:
         self._check(self._lib.hmrm_render_device(self._h, C.byref(frame), _ptr(d_out), _ptr(stream)))
+
+    # -- many cameras in one launch (hmrm_render_views) ----------------------------------------------
+    def render_views(self, cams, frame: Frame | None = None, out: np.ndarray | None = None, **overrides) -> np.ndarray:
+        """The views of `frame` (or of the current attributes and `overrides`) at the cameras `cams`, rendered in one
+        launch: [n, H, W, C] uint8, view j equal to render() with cam_pos, hang and vang of cams[j].  `cams` is a
+        sequence of (pos, hang, vang) or an [n, 5] float64 array of rows (x, y, z, hang, vang), angles in radians."""
+        arr, n = _cameras(cams, "view")
+        f = frame if frame is not None else self.frame(**overrides)
+        shape = (n, f.screen_height, f.screen_width, 3 if f.pixel_format == PIXEL_RGB8 else 4)
+        if out is None:
+            out = np.empty(shape, dtype=np.uint8)
+        if out.dtype != np.uint8 or not out.flags.c_contiguous or out.size != int(np.prod(shape)):
+            raise ValueError(f"out must be a contiguous uint8 array of {shape}")
+        self._check(self._lib.hmrm_render_views(self._h, C.byref(f), arr, n, out.ctypes.data))
+        return out.reshape(shape)
+
+    def render_views_device(self, frame: Frame, cams, d_out, stream=None) -> None:
+        """hmrm_render_views_device: the views into `d_out` (a CUDA uint8 tensor or a raw device address of at least
+        n * H * W * C bytes, any alignment), ordered on `stream` (NULL: the context's)."""
+        arr, n = _cameras(cams, "view")
+        need = n * frame.screen_height * frame.screen_width * (3 if frame.pixel_format == PIXEL_RGB8 else 4)
+        have = _nbytes(d_out)
+        if have is not None and have < need:
+            raise ValueError(f"d_out holds {have} bytes, the views need {need}")
+        self._check(self._lib.hmrm_render_views_device(self._h, C.byref(frame), arr, n, _ptr(d_out), _ptr(stream)))
 
     def stats(self) -> Stats:
         st = Stats()

@@ -63,6 +63,9 @@ struct LaunchSlot {
 	size_t step_cap;             // pixels
 	double *d_ray_dump;          // HMRM_FLAG_RAY_DUMP output, [pixels][10]
 	size_t dump_cap;             // pixels
+	uint8_t *view_host;          // hmrm_render_views: pinned staging of a batch's view records, schedule and spherical
+	uint8_t *d_view;             // tables, and their device copy (view_pieces)
+	size_t view_cap;             // bytes of each
 };
 
 // The sW x sH RGBA8 renders of one supersampled or motion-blurred frame, read by K5: up to kDownMaxPlanes planes, and
@@ -83,7 +86,7 @@ struct SubFrame {
 // Experiment knobs (environment, read ONCE in hmrm_create): they never change a result, only how the work is
 // scheduled / how many fetches are issued.
 struct Knobs {
-	bool no_row_order, no_batch, debug_sched, reset_kernel, peer_memops;
+	bool no_row_order, no_batch, debug_sched, reset_kernel, peer_memops, views_view_major;
 	int lmin_bias, lstride, lstart, sky_batch;
 	float cell_exit, climb;
 	bool zq_shrink_set;
@@ -144,6 +147,8 @@ struct hmrm_ctx {
 	size_t scratch_cap[kFrameRing];
 	uint8_t *d_pixels;           // hmrm_encode_png's / _jpeg's / hmrm_convert_yuv420's device copy of the caller's pixels
 	size_t pixels_cap;
+	uint8_t *d_views;            // hmrm_render_views' device copy of the views before they go to the caller's memory
+	size_t views_cap;
 	// supersampled frames (K5): sub-frame scratches, allocated by the first supersampled frame that uses them
 	SubFrame sub[kSubFrames];
 	int sub_next;
@@ -395,6 +400,183 @@ __global__ void k_reset_slot(unsigned int *tile_counter, unsigned int *stats_wor
 	for (unsigned i = threadIdx.x; i < sizeof(DeviceStats) / 4; i += 32) stats_words[i] = 0u;
 }
 
+// Takes a launch slot and waits (host side) for the kernel that used it kLaunchSlots launches ago.  A blurred frame's
+// later sub-frames skip the slot that accumulates its statistics (acc_slot): its ev_end is their own latest kernel.
+int take_slot(hmrm_ctx *c, int acc_slot, int *ls) {
+	if (c->launch_next == acc_slot) c->launch_next = (acc_slot + 1) % kLaunchSlots;
+	*ls = c->launch_next;
+	c->launch_next = (*ls + 1) % kLaunchSlots;
+	LaunchSlot &slot = c->slots[*ls];
+	if (slot.used) HMRM_CUDA(c, cudaEventSynchronize(slot.ev_end));
+	return HMRM_OK;
+}
+
+// The fields of P that one frame of `f` and every view of a batch of `f` share: screen, map, box, march constants,
+// tables, pixel format and background; plus the camera constants of pc.
+void frame_params(hmrm_ctx *c, const hmrm_frame *f, const PlaneConst &pc, RenderParams *P) {
+	std::memset(P, 0, sizeof *P);
+	P->projection = f->projection;
+	P->W = f->screen_width;
+	P->H = f->screen_height;
+	P->tiles_x = (P->W + 7) / 8;
+	P->inv_tiles_x = std::nextafterf(1.0f / (float)P->tiles_x, 0.0f) * (1.0f - 1.0e-6f);
+	P->map_w = c->map_w;
+	P->map_h = c->map_h;
+	const Vec3 *src[5] = {&pc.cam, &pc.ul, &pc.pr, &pc.pd, &pc.look};
+	double *dst[5] = {P->cam, P->ul, P->pr, P->pd, P->look};
+	for (int i = 0; i < 5; ++i) {
+		dst[i][0] = src[i]->x;
+		dst[i][1] = src[i]->y;
+		dst[i][2] = src[i]->z;
+	}
+	// main/hmap.cpp:967-974
+	P->c0[0] = 0.0;
+	P->c0[1] = 0.0;
+	P->c0[2] = c->min_height;
+	P->c1[0] = P->c0[0] + c->map_w * f->grid_width;
+	P->c1[1] = P->c0[1] - c->map_h * f->grid_width;
+	P->c1[2] = c->max_height;
+	for (int i = 0; i < 3; ++i) {
+		P->bmin[i] = std::fmin(P->c0[i], P->c1[i]);
+		P->bmax[i] = std::fmax(P->c0[i], P->c1[i]);
+	}
+	P->gw = f->grid_width;
+	P->nudge = f->grid_width * 0.01;
+	P->step_dist = f->step_dist;
+	P->max_surf = c->max_surf;
+	P->wtab = c->d_wtab;
+	P->htab = c->d_htab;
+	P->row_order = NULL;
+	P->batch_from_tile = 0xFFFFFFFFu;
+	P->sky_batch = (unsigned)c->knobs.sky_batch;
+	P->surf = c->d_surf;
+	P->color = c->d_color;
+	P->pixel_format = f->pixel_format;
+	P->bg[0] = f->bg[0];
+	P->bg[1] = f->bg[1];
+	P->bg[2] = f->bg[2];
+	P->bg_rgba = (uint32_t)f->bg[0] | ((uint32_t)f->bg[1] << 8) | ((uint32_t)f->bg[2] << 16) | 0xFF000000u;
+}
+
+// The skip traversals' constants of P (c->skip_ready).  The caller falls back to HMRM_TRAVERSAL_BRUTE when
+// P->fx_bits < 1 or P->fx_scale is not finite.
+void skip_params(hmrm_ctx *c, const hmrm_frame *f, RenderParams *P) {
+	int dim = c->map_w > c->map_h ? c->map_w : c->map_h, clog = 0;
+	while ((1 << clog) < dim) clog += 1;
+	P->fx_bits = 30 - clog < 20 ? 30 - clog : 20;
+	P->fx_scale = std::ldexp(1.0, P->fx_bits) / f->grid_width;
+	if (P->fx_bits >= 1) {
+		P->lin_grid_x = (unsigned)c->map_w << P->fx_bits;
+		P->lin_grid_y = (unsigned)c->map_h << P->fx_bits;
+		P->lin_span_x = P->lin_grid_x - 2u * HMRM_LIN_MARGIN;
+		P->lin_span_y = P->lin_grid_y - 2u * HMRM_LIN_MARGIN;
+	}
+	P->zq_scale = c->zq_scale;
+	P->zq_offset = c->zq_offset;
+	P->inv_gw_up = (1.0 / f->grid_width) * 1.000001;
+	P->ltop = c->mip_levels - 1;
+	// lowest useful block: about one step wide (measured: profiles/r01_knob_sweep.txt)
+	const double step_cells = f->step_dist / f->grid_width;
+	int lmin = 1;
+	while (lmin < P->ltop && (double)(1 << lmin) < step_cells) lmin += 1;
+	// tuning knobs for experiments (never affect results, only how many fetches are issued): read once, hmrm_create
+	lmin += c->knobs.lmin_bias;
+	if (lmin < 1) lmin = 1;
+	if (lmin > P->ltop) lmin = P->ltop;
+	P->lmin = lmin;
+	P->lstride = c->knobs.lstride < 1 ? 1 : c->knobs.lstride;
+	P->cell_exit_scale = c->knobs.cell_exit;
+	P->climb_ratio = c->knobs.climb;
+	const int lstart = lmin + c->knobs.lstart * P->lstride;
+	P->lstart = lstart > P->ltop ? P->ltop : (lstart < lmin ? lmin : lstart);
+	P->lv = c->d_mip;
+	P->lv_total = (unsigned long long)(c->mip_offset[c->mip_levels - 1] +
+	                                   pyr_level_elems(c->layout, c->mip_w[c->mip_levels - 1], c->mip_h[c->mip_levels - 1]));
+	P->layout = c->layout;
+	for (int l = 0; l < 16; ++l) {
+		P->lv_desc[l].x = (l < c->mip_levels) ? (unsigned)c->mip_offset[l] : 0u;
+		P->lv_desc[l].y = (l < c->mip_levels) ? pyr_level_pitch(c->layout, c->mip_w[l]) : 0u;
+	}
+}
+
+// Tile-row schedule: rows whose rays graze the terrain (direction just below the horizon) march for hundreds of
+// steps at low clearance and cost ~50x the mean tile; rows that look up cost nothing.  Start the expensive rows
+// first (cost proxy 1/|dir.z| of the centre ray for dir.z < 0).  Depends on the projection, W, H, hfov, vang and the
+// rows only, not on the camera position or heading, so a flythrough computes it once and views with one vang share it.
+// order[0 .. tiles_y) gets the tile rows t (frame tile row first + t * step) costliest first; `sky_first` the position
+// in it from which on every row's lowest pixel row still looks up (cheap sky; a hint only).  `cost_scratch` is working
+// space the caller may keep across calls.
+void row_schedule(const PlaneConst &pc, int H, int row_begin, int first, int step, int tiles_y, int *order,
+                  int *sky_first, std::vector<std::pair<double, int> > *cost_scratch) {
+	std::vector<std::pair<double, int> > &cost = *cost_scratch;
+	cost.resize((size_t)tiles_y);
+	for (int t = 0; t < tiles_y; ++t) {
+		int py = row_begin + (first + t * step) * 4 + 2;
+		if (py > H - 1) py = H - 1;
+		Vec3 pos, dir;
+		plane_ray(pc, 0.5, (double)py / (H - 1), &pos, &dir);
+		const double dz = dir.z;
+		cost[(size_t)t].first = (dz < 0.0) ? -1.0 / std::fmax(-dz, 1e-3) : 1.0 + dz;   // ascending sort key
+		cost[(size_t)t].second = t;
+	}
+	std::stable_sort(cost.begin(), cost.end());
+	for (int t = 0; t < tiles_y; ++t) order[t] = cost[(size_t)t].second;
+	*sky_first = tiles_y;
+	for (int t = tiles_y - 1; t >= 0; --t) {
+		int py = row_begin + (first + order[t] * step) * 4 + 3;
+		if (py > H - 1) py = H - 1;
+		Vec3 pos, dir;
+		plane_ray(pc, 0.5, (double)py / (H - 1), &pos, &dir);
+		if (!(dir.z >= 0.0) || !(cost[(size_t)t].first >= 1.0)) break;
+		*sky_first = t;
+	}
+}
+
+// The persistent lin kernel over P's tiles: HMRM_LIN_CTAS_LARGE CTAs per SM from HMRM_LIN_LARGE_TILES tiles on,
+// HMRM_LIN_CTAS below, and no more CTAs than it takes to give every warp one tile.
+template <bool kViews>
+int launch_lin(hmrm_ctx *c, const RenderParams &P, bool stats_kernel, cudaStream_t stream) {
+	const int n_tiles = P.tiles_x * P.tiles_y;
+	const int lin_warps = HMRM_LIN_THREADS / 32;
+	const bool large = n_tiles >= HMRM_LIN_LARGE_TILES;
+	int lin_blocks = c->num_sms * (large ? HMRM_LIN_CTAS_LARGE : HMRM_LIN_CTAS);
+	if (lin_blocks > (n_tiles + lin_warps - 1) / lin_warps) lin_blocks = (n_tiles + lin_warps - 1) / lin_warps;
+	if (lin_blocks < 1) lin_blocks = 1;
+#define HMRM_LAUNCH_LIN_SHAPE(LAYOUT, CTAS)                                                                              \
+	do {                                                                                                                 \
+		if (stats_kernel) k2_render_lin<true, LAYOUT, CTAS, kViews><<<lin_blocks, HMRM_LIN_THREADS, 0, stream>>>(P);     \
+		else k2_render_lin<false, LAYOUT, CTAS, kViews><<<lin_blocks, HMRM_LIN_THREADS, 0, stream>>>(P);                 \
+	} while (0)
+#define HMRM_LAUNCH_LIN(LAYOUT)                                                                                          \
+	do {                                                                                                                 \
+		if (large) HMRM_LAUNCH_LIN_SHAPE(LAYOUT, HMRM_LIN_CTAS_LARGE);                                                   \
+		else HMRM_LAUNCH_LIN_SHAPE(LAYOUT, HMRM_LIN_CTAS);                                                               \
+	} while (0)
+	if (c->layout == HMRM_LAYOUT_TILE4) HMRM_LAUNCH_LIN(kLayoutTile4);
+	else if (c->layout == HMRM_LAYOUT_ZORDER) HMRM_LAUNCH_LIN(kLayoutZOrder);
+	else HMRM_LAUNCH_LIN(kLayoutRowMajor);
+#undef HMRM_LAUNCH_LIN
+#undef HMRM_LAUNCH_LIN_SHAPE
+	return HMRM_OK;
+}
+
+// Zeroes slot ls's tile-queue counter and (unless acc_slot >= 0) statistics block on `stream`.
+int reset_slot(hmrm_ctx *c, LaunchSlot &slot, int acc_slot, cudaStream_t stream) {
+	if (acc_slot >= 0) HMRM_CUDA(c, cudaMemsetAsync(slot.d_tile_counter, 0, sizeof(unsigned int), stream));
+	else if (!c->knobs.reset_kernel) {
+		HMRM_CUDA(c, cudaMemsetAsync(slot.d_tile_counter, 0, sizeof(unsigned int), stream));
+		HMRM_CUDA(c, cudaMemsetAsync(slot.d_stats, 0, sizeof(DeviceStats), stream));
+	}
+	else {
+		// experiment (HMRM_RESET_KERNEL): one tiny kernel instead of the two memsets.  Measured: 0.4411 vs 0.4365 ms per
+		// flythrough4k frame, 0.2268 vs 0.2286 ms per 8K band frame at N = 8 — nothing in it; a kernel needs a CTA slot
+		// that the previous frame's persistent CTAs still hold, the memsets do not
+		k_reset_slot<<<1, 32, 0, stream>>>(slot.d_tile_counter, (unsigned int *)slot.d_stats);
+		HMRM_CUDA(c, cudaGetLastError());
+	}
+	return HMRM_OK;
+}
+
 // Enqueue one frame on `stream`, writing the frame's pixel format into d_out (any alignment).  acc_slot >= 0: a later
 // sub-frame of a motion-blurred frame whose first sub-frame used launch slot acc_slot (on the same stream).  Its
 // statistics add into that slot's block (no reset), the slot's ev_end moves past this kernel, and hmrm_get_stats then
@@ -408,27 +590,18 @@ int enqueue_render(hmrm_ctx *c, const hmrm_frame *f, uint32_t *d_out, cudaStream
 	const int W = f->screen_width, H = f->screen_height;
 	if ((rc = ensure_tables(c, W, H)) != HMRM_OK) return rc;
 
-	// take a launch slot; wait (host side) for the kernel that used it kLaunchSlots launches ago.  A blurred frame's
-	// later sub-frames skip the slot that accumulates its statistics: its ev_end is their own latest kernel.
-	if (c->launch_next == acc_slot) c->launch_next = (acc_slot + 1) % kLaunchSlots;
-	const int ls = c->launch_next;
-	c->launch_next = (ls + 1) % kLaunchSlots;
+	int ls = 0;
+	if ((rc = take_slot(c, acc_slot, &ls)) != HMRM_OK) return rc;
 	LaunchSlot &slot = c->slots[ls];
-	if (slot.used) HMRM_CUDA(c, cudaEventSynchronize(slot.ev_end));
 
 	const PlaneConst pc = build_plane(*f);
 
 	RenderParams P;
-	std::memset(&P, 0, sizeof P);
-	P.projection = f->projection;
-	P.W = W;
-	P.H = H;
+	frame_params(c, f, pc, &P);
 	P.row_begin = row_begin;
 	P.row_end = row_end;
 	P.cycle = f->cycle;
 	P.period = f->cycle_period;
-	P.tiles_x = (W + 7) / 8;
-	P.inv_tiles_x = std::nextafterf(1.0f / (float)P.tiles_x, 0.0f) * (1.0f - 1.0e-6f);
 	const int tile_rows = (row_end - row_begin + 3) / 4;
 	if (f->band_count > 1) {
 		// interleaved bands: sky rows are almost free and terrain rows are not, so contiguous bands balance badly
@@ -441,32 +614,6 @@ int enqueue_render(hmrm_ctx *c, const hmrm_frame *f, uint32_t *d_out, cudaStream
 		P.tile_y_step = 1;
 		P.tiles_y = tile_rows;
 	}
-	P.map_w = c->map_w;
-	P.map_h = c->map_h;
-	const Vec3 *src[5] = {&pc.cam, &pc.ul, &pc.pr, &pc.pd, &pc.look};
-	double *dst[5] = {P.cam, P.ul, P.pr, P.pd, P.look};
-	for (int i = 0; i < 5; ++i) {
-		dst[i][0] = src[i]->x;
-		dst[i][1] = src[i]->y;
-		dst[i][2] = src[i]->z;
-	}
-	// main/hmap.cpp:967-974
-	P.c0[0] = 0.0;
-	P.c0[1] = 0.0;
-	P.c0[2] = c->min_height;
-	P.c1[0] = P.c0[0] + c->map_w * f->grid_width;
-	P.c1[1] = P.c0[1] - c->map_h * f->grid_width;
-	P.c1[2] = c->max_height;
-	for (int i = 0; i < 3; ++i) {
-		P.bmin[i] = std::fmin(P.c0[i], P.c1[i]);
-		P.bmax[i] = std::fmax(P.c0[i], P.c1[i]);
-	}
-	P.gw = f->grid_width;
-	P.nudge = f->grid_width * 0.01;
-	P.step_dist = f->step_dist;
-	P.max_surf = c->max_surf;
-	P.wtab = c->d_wtab;
-	P.htab = c->d_htab;
 
 	if (f->projection == HMRM_SPHERICAL) {
 		const size_t need = (size_t)(2 * W + 2 * H);
@@ -489,40 +636,14 @@ int enqueue_render(hmrm_ctx *c, const hmrm_frame *f, uint32_t *d_out, cudaStream
 		P.cos_va = slot.d_sph + 2 * W + H;
 	}
 
-	// Tile-row schedule: rows whose rays graze the terrain (direction just below the horizon) march for hundreds of
-	// steps at low clearance and cost ~50x the mean tile; rows that look up cost nothing.  Start the expensive rows
-	// first (cost proxy 1/|dir.z| of the centre ray for dir.z < 0).  Depends on the view geometry only, not on the
-	// camera position or heading, so a flythrough computes it once.
-	P.row_order = NULL;
-	P.batch_from_tile = 0xFFFFFFFFu;
-	P.sky_batch = (unsigned)c->knobs.sky_batch;
+	// tile-row schedule (row_schedule), cached per launch slot
 	if (f->projection != HMRM_ORTHOGRAPHIC && P.tiles_y > 1 && !c->knobs.no_row_order) {
 		const double key[8] = {(double)f->projection, (double)W, (double)H, f->vang, f->hfov, (double)row_begin,
 		                       (double)(P.tile_y_first * 65536 + P.tile_y_step), (double)P.tiles_y};
 		if (!slot.row_key_valid || std::memcmp(key, slot.row_key, sizeof key) != 0) {
-			std::vector<std::pair<double, int> > cost((size_t)P.tiles_y);
-			for (int t = 0; t < P.tiles_y; ++t) {
-				int py = row_begin + (P.tile_y_first + t * P.tile_y_step) * 4 + 2;
-				if (py > H - 1) py = H - 1;
-				Vec3 pos, dir;
-				plane_ray(pc, 0.5, (double)py / (H - 1), &pos, &dir);
-				const double dz = dir.z;
-				cost[(size_t)t].first = (dz < 0.0) ? -1.0 / std::fmax(-dz, 1e-3) : 1.0 + dz;   // ascending sort key
-				cost[(size_t)t].second = t;
-			}
-			std::stable_sort(cost.begin(), cost.end());
 			std::vector<int> order((size_t)P.tiles_y);
-			for (int t = 0; t < P.tiles_y; ++t) order[(size_t)t] = cost[(size_t)t].second;
-			// the rows at the end of the schedule whose lowest pixel row still looks up: cheap sky (a hint only)
-			slot.row_sky_first = P.tiles_y;
-			for (int t = P.tiles_y - 1; t >= 0; --t) {
-				int py = row_begin + (P.tile_y_first + order[(size_t)t] * P.tile_y_step) * 4 + 3;
-				if (py > H - 1) py = H - 1;
-				Vec3 pos, dir;
-				plane_ray(pc, 0.5, (double)py / (H - 1), &pos, &dir);
-				if (!(dir.z >= 0.0) || !(cost[(size_t)t].first >= 1.0)) break;
-				slot.row_sky_first = t;
-			}
+			std::vector<std::pair<double, int> > cost;
+			row_schedule(pc, H, row_begin, P.tile_y_first, P.tile_y_step, P.tiles_y, order.data(), &slot.row_sky_first, &cost);
 			if (P.tiles_y > slot.row_cap) {
 				cudaFree(slot.d_row_order);
 				slot.d_row_order = NULL;
@@ -546,17 +667,10 @@ int enqueue_render(hmrm_ctx *c, const hmrm_frame *f, uint32_t *d_out, cudaStream
 			             P.batch_from_tile, P.tiles_x * P.tiles_y);
 	}
 
-	P.surf = c->d_surf;
-	P.color = c->d_color;
 	P.fb = d_out;
-	P.pixel_format = f->pixel_format;
 	// hmrm_render_device and the peer calls take any caller pointer: word stores only where they are aligned
 	P.fb_unaligned = ((uintptr_t)d_out & 3u) != 0u ? 1 : 0;
 	P.rgb_words = (W % 4) == 0 && !P.fb_unaligned ? 1 : 0;
-	P.bg[0] = f->bg[0];
-	P.bg[1] = f->bg[1];
-	P.bg[2] = f->bg[2];
-	P.bg_rgba = (uint32_t)f->bg[0] | ((uint32_t)f->bg[1] << 8) | ((uint32_t)f->bg[2] << 16) | 0xFF000000u;
 
 	const bool want_stats = (f->flags & HMRM_FLAG_STATS) != 0;
 	const bool want_steps = (f->flags & HMRM_FLAG_STEP_INDEX) != 0;
@@ -589,19 +703,7 @@ int enqueue_render(hmrm_ctx *c, const hmrm_frame *f, uint32_t *d_out, cudaStream
 	}
 	P.stats = acc_slot >= 0 ? c->slots[acc_slot].d_stats : slot.d_stats;
 	P.tile_counter = slot.d_tile_counter;
-
-	if (acc_slot >= 0) HMRM_CUDA(c, cudaMemsetAsync(slot.d_tile_counter, 0, sizeof(unsigned int), stream));
-	else if (!c->knobs.reset_kernel) {
-		HMRM_CUDA(c, cudaMemsetAsync(slot.d_tile_counter, 0, sizeof(unsigned int), stream));
-		HMRM_CUDA(c, cudaMemsetAsync(slot.d_stats, 0, sizeof(DeviceStats), stream));
-	}
-	else {
-		// experiment (HMRM_RESET_KERNEL): one tiny kernel instead of the two memsets.  Measured: 0.4411 vs 0.4365 ms per
-		// flythrough4k frame, 0.2268 vs 0.2286 ms per 8K band frame at N = 8 — nothing in it; a kernel needs a CTA slot
-		// that the previous frame's persistent CTAs still hold, the memsets do not
-		k_reset_slot<<<1, 32, 0, stream>>>(slot.d_tile_counter, (unsigned int *)slot.d_stats);
-		HMRM_CUDA(c, cudaGetLastError());
-	}
+	if ((rc = reset_slot(c, slot, acc_slot, stream)) != HMRM_OK) return rc;
 
 	int traversal = f->traversal;
 	if (traversal == HMRM_TRAVERSAL_AUTO) traversal = c->skip_ready ? HMRM_TRAVERSAL_SKIP : HMRM_TRAVERSAL_BRUTE;
@@ -611,44 +713,8 @@ int enqueue_render(hmrm_ctx *c, const hmrm_frame *f, uint32_t *d_out, cudaStream
 	if (traversal != HMRM_TRAVERSAL_BRUTE) {
 		if (!c->skip_ready)
 			return fail(c, HMRM_ERR_STATE, "the height range could not be quantised; use HMRM_TRAVERSAL_BRUTE");
-		int dim = c->map_w > c->map_h ? c->map_w : c->map_h, clog = 0;
-		while ((1 << clog) < dim) clog += 1;
-		P.fx_bits = 30 - clog < 20 ? 30 - clog : 20;
-		P.fx_scale = std::ldexp(1.0, P.fx_bits) / f->grid_width;
-		if (P.fx_bits >= 1) {
-			P.lin_grid_x = (unsigned)c->map_w << P.fx_bits;
-			P.lin_grid_y = (unsigned)c->map_h << P.fx_bits;
-			P.lin_span_x = P.lin_grid_x - 2u * HMRM_LIN_MARGIN;
-			P.lin_span_y = P.lin_grid_y - 2u * HMRM_LIN_MARGIN;
-		}
-		P.zq_scale = c->zq_scale;
-		P.zq_offset = c->zq_offset;
-		P.inv_gw_up = (1.0 / f->grid_width) * 1.000001;
-		P.ltop = c->mip_levels - 1;
-		// lowest useful block: about one step wide (measured: profiles/r01_knob_sweep.txt)
-		const double step_cells = f->step_dist / f->grid_width;
-		int lmin = 1;
-		while (lmin < P.ltop && (double)(1 << lmin) < step_cells) lmin += 1;
-		// tuning knobs for experiments (never affect results, only how many fetches are issued): read once, hmrm_create
-		lmin += c->knobs.lmin_bias;
-		if (lmin < 1) lmin = 1;
-		if (lmin > P.ltop) lmin = P.ltop;
-		P.lmin = lmin;
-		P.lstride = c->knobs.lstride < 1 ? 1 : c->knobs.lstride;
-		P.cell_exit_scale = c->knobs.cell_exit;
-		P.climb_ratio = c->knobs.climb;
-		const int lstart = lmin + c->knobs.lstart * P.lstride;
-		P.lstart = lstart > P.ltop ? P.ltop : (lstart < lmin ? lmin : lstart);
-		if (P.fx_bits < 1) traversal = HMRM_TRAVERSAL_BRUTE;
-		P.lv = c->d_mip;
-		P.lv_total = (unsigned long long)(c->mip_offset[c->mip_levels - 1] +
-		                                  pyr_level_elems(c->layout, c->mip_w[c->mip_levels - 1], c->mip_h[c->mip_levels - 1]));
-		P.layout = c->layout;
-		for (int l = 0; l < 16; ++l) {
-			P.lv_desc[l].x = (l < c->mip_levels) ? (unsigned)c->mip_offset[l] : 0u;
-			P.lv_desc[l].y = (l < c->mip_levels) ? pyr_level_pitch(c->layout, c->mip_w[l]) : 0u;
-		}
-		if (!std::isfinite(P.fx_scale)) traversal = HMRM_TRAVERSAL_BRUTE;
+		skip_params(c, f, &P);
+		if (P.fx_bits < 1 || !std::isfinite(P.fx_scale)) traversal = HMRM_TRAVERSAL_BRUTE;
 	}
 
 	const int n_tiles = P.tiles_x * P.tiles_y;
@@ -661,27 +727,7 @@ int enqueue_render(hmrm_ctx *c, const hmrm_frame *f, uint32_t *d_out, cudaStream
 	(void)timed;
 	HMRM_CUDA(c, cudaEventRecord(slot.ev_begin, stream));
 	if (traversal == HMRM_TRAVERSAL_SKIP) {
-		const bool stats_kernel = want_stats || want_steps || want_dump;
-		const int lin_warps = HMRM_LIN_THREADS / 32;
-		const bool large = n_tiles >= HMRM_LIN_LARGE_TILES;
-		int lin_blocks = c->num_sms * (large ? HMRM_LIN_CTAS_LARGE : HMRM_LIN_CTAS);
-		if (lin_blocks > (n_tiles + lin_warps - 1) / lin_warps) lin_blocks = (n_tiles + lin_warps - 1) / lin_warps;
-		if (lin_blocks < 1) lin_blocks = 1;
-#define HMRM_LAUNCH_LIN_SHAPE(LAYOUT, CTAS)                                                                        \
-		do {                                                                                                       \
-			if (stats_kernel) k2_render_lin<true, LAYOUT, CTAS><<<lin_blocks, HMRM_LIN_THREADS, 0, stream>>>(P);   \
-			else k2_render_lin<false, LAYOUT, CTAS><<<lin_blocks, HMRM_LIN_THREADS, 0, stream>>>(P);               \
-		} while (0)
-#define HMRM_LAUNCH_LIN(LAYOUT)                                                                                    \
-		do {                                                                                                       \
-			if (large) HMRM_LAUNCH_LIN_SHAPE(LAYOUT, HMRM_LIN_CTAS_LARGE);                                         \
-			else HMRM_LAUNCH_LIN_SHAPE(LAYOUT, HMRM_LIN_CTAS);                                                     \
-		} while (0)
-		if (c->layout == HMRM_LAYOUT_TILE4) HMRM_LAUNCH_LIN(kLayoutTile4);
-		else if (c->layout == HMRM_LAYOUT_ZORDER) HMRM_LAUNCH_LIN(kLayoutZOrder);
-		else HMRM_LAUNCH_LIN(kLayoutRowMajor);
-#undef HMRM_LAUNCH_LIN
-#undef HMRM_LAUNCH_LIN_SHAPE
+		if ((rc = launch_lin<false>(c, P, want_stats || want_steps || want_dump, stream)) != HMRM_OK) return rc;
 	}
 	else if (traversal == HMRM_TRAVERSAL_PACK) {
 		const bool stats_kernel = want_stats || want_steps || want_dump;
@@ -1240,6 +1286,204 @@ int encode_staged(hmrm_ctx *c, const Output &o, const uint8_t *pixels, int W, in
 	return HMRM_OK;
 }
 
+// ---- batches of views (hmrm_render_views, k2_render_lin<..., kViews = true>) ---------------------------------------
+const int kMaxViews = 65536;                 // a schedule entry holds the view in 16 bits
+const long long kMaxViewTiles = 1LL << 26;   // tile_row_col's float quotient is exact below 2^26 tiles
+
+// The refusals of hmrm_render_views and hmrm_render_views_device; nothing is enqueued before they pass.
+int check_views(hmrm_ctx *c, const hmrm_frame *f, const hmrm_camera *cams, int n, const void *out) {
+	if (!f) return fail(c, HMRM_ERR_INVALID, "frame is NULL");
+	if (!cams) return fail(c, HMRM_ERR_INVALID, "cams is NULL");
+	if (!out) return fail(c, HMRM_ERR_INVALID, "output is NULL");
+	if (n < 1 || n > kMaxViews) return fail(c, HMRM_ERR_INVALID, "%d views outside [1,%d]", n, kMaxViews);
+	if (c->blur_n > 0) return fail(c, HMRM_ERR_INVALID, "views are single frames: no motion blur");
+	if (supersample_of(f) != 1) return fail(c, HMRM_ERR_INVALID, "views are single frames: no supersampling");
+	if (int rc = check_whole_frame(c, f, "view")) return rc;
+	if (f->traversal != HMRM_TRAVERSAL_AUTO && f->traversal != HMRM_TRAVERSAL_SKIP)
+		return fail(c, HMRM_ERR_INVALID, "views take HMRM_TRAVERSAL_AUTO or HMRM_TRAVERSAL_SKIP, not %d", f->traversal);
+	for (int j = 0; j < n; ++j) {
+		if (!finite3(cams[j].cam_pos) || !std::isfinite(cams[j].hang) || !std::isfinite(cams[j].vang))
+			return fail(c, HMRM_ERR_INVALID, "camera %d of the views is not finite", j);
+	}
+	hmrm_frame sf = *f;
+	set_camera(&sf, cams[0]);
+	int row_begin = 0, row_end = 0;
+	if (int rc = validate_frame(c, &sf, &row_begin, &row_end)) return rc;
+	const long long tiles = (long long)n * ((f->screen_width + 7) / 8) * ((f->screen_height + 3) / 4);
+	if (tiles > kMaxViewTiles)
+		return fail(c, HMRM_ERR_INVALID, "%d views of %dx%d are %lld tiles of 8x4 pixels, more than 2^26", n,
+		            f->screen_width, f->screen_height, tiles);
+	if (!c->skip_ready) return fail(c, HMRM_ERR_STATE, "the height range could not be quantised; use HMRM_TRAVERSAL_BRUTE");
+	RenderParams P;
+	skip_params(c, f, &P);
+	if (P.fx_bits < 1 || !std::isfinite(P.fx_scale))
+		return fail(c, HMRM_ERR_INVALID, "grid_width %g is too small for the skip traversal; views have no FP64 fallback",
+		            f->grid_width);
+	return HMRM_OK;
+}
+
+// A launch slot's pieces of a batch: the view records, the schedule and (spherical) each view's tables, back to back
+// from `base`; from base 0 they are only counted.
+struct ViewPieces {
+	ViewConst *rec;
+	uint32_t *rows;
+	double *sph;
+	size_t bytes;
+};
+
+ViewPieces view_pieces(uintptr_t base, int n, int rows, size_t sph) {
+	Carve k = {base, 0};
+	ViewPieces p;
+	p.rec = k.take<ViewConst>((unsigned long long)n);
+	p.rows = k.take<uint32_t>((unsigned long long)rows);
+	p.sph = k.take<double>(sph);
+	p.bytes = k.bytes;
+	return p;
+}
+
+// Enqueue n views of f (check_views has passed) on `stream` into d_out, view j at byte j * W * H * C.  The records,
+// schedule and spherical tables are written into the slot's pinned staging and go to the device in one copy.
+int enqueue_views(hmrm_ctx *c, const hmrm_frame *f, const hmrm_camera *cams, int n, uint8_t *d_out, cudaStream_t stream) {
+	HMRM_CUDA(c, cudaSetDevice(c->device));
+	const int W = f->screen_width, H = f->screen_height;
+	int rc = ensure_tables(c, W, H);
+	if (rc) return rc;
+	int ls = 0;
+	if ((rc = take_slot(c, -1, &ls)) != HMRM_OK) return rc;
+	LaunchSlot &slot = c->slots[ls];
+
+	const int ty_view = (H + 3) / 4;             // tile rows of one view
+	const int rows = n * ty_view;
+	const bool spherical = f->projection == HMRM_SPHERICAL;
+	const size_t sph_view = spherical ? (size_t)(2 * W + 2 * H) : 0;
+	const size_t need = view_pieces(0, n, rows, sph_view * (size_t)n).bytes;
+	if (need > slot.view_cap) {
+		if (slot.view_host) cudaFreeHost(slot.view_host);
+		cudaFree(slot.d_view);
+		slot.view_host = NULL;
+		slot.d_view = NULL;
+		slot.view_cap = 0;
+		HMRM_CUDA(c, cudaMallocHost(&slot.view_host, need));
+		HMRM_CUDA(c, cudaMalloc(&slot.d_view, need));
+		slot.view_cap = need;
+	}
+	const ViewPieces h = view_pieces((uintptr_t)slot.view_host, n, rows, sph_view * (size_t)n);
+	const ViewPieces d = view_pieces((uintptr_t)slot.d_view, n, rows, sph_view * (size_t)n);
+
+	hmrm_frame sf = *f;
+	set_camera(&sf, cams[0]);
+	RenderParams P;
+	frame_params(c, &sf, build_plane(sf), &P);
+	skip_params(c, &sf, &P);
+
+	// Per view: its record and its tables.
+	for (int j = 0; j < n; ++j) {
+		set_camera(&sf, cams[j]);
+		const PlaneConst pc = build_plane(sf);
+		ViewConst &v = h.rec[j];
+		const Vec3 *src[5] = {&pc.cam, &pc.ul, &pc.pr, &pc.pd, &pc.look};
+		double *dst[5] = {v.cam, v.ul, v.pr, v.pd, v.look};
+		for (int i = 0; i < 5; ++i) {
+			dst[i][0] = src[i]->x;
+			dst[i][1] = src[i]->y;
+			dst[i][2] = src[i]->z;
+		}
+		v.cos_ha = v.sin_ha = v.sin_va = v.cos_va = NULL;
+		if (spherical) {
+			fill_spherical_tables(pc, W, H, c->wtab, c->htab, &c->sph);
+			std::memcpy(h.sph + (size_t)j * sph_view, c->sph.data(), sph_view * 8);
+			const double *t = d.sph + (size_t)j * sph_view;
+			v.cos_ha = t;
+			v.sin_ha = t + W;
+			v.sin_va = t + 2 * W;
+			v.cos_va = t + 2 * W + H;
+		}
+	}
+	// Per view: its tile rows costliest first (row_schedule), orders[view_order[j] * ty_view ...], of which the first
+	// sky[j] march terrain and the rest look above the horizon from above the box.  The order depends on vang and not on
+	// hang or position, so views with one vang share it: the views are sorted by vang once (O(n log n)) and each run of
+	// equal vang gets one schedule.
+	const bool ordered = f->projection != HMRM_ORTHOGRAPHIC && ty_view > 1 && !c->knobs.no_row_order;
+	std::vector<int> view_order((size_t)n, -1), sky((size_t)n, ty_view);
+	std::vector<int> orders, identity((size_t)ty_view);
+	for (int t = 0; t < ty_view; ++t) identity[(size_t)t] = t;
+	if (ordered) {
+		std::vector<int> by_vang((size_t)n), order_sky;
+		for (int j = 0; j < n; ++j) by_vang[(size_t)j] = j;
+		std::sort(by_vang.begin(), by_vang.end(), [&](int a, int b) {
+			return cams[a].vang < cams[b].vang || (cams[a].vang == cams[b].vang && a < b);
+		});
+		std::vector<std::pair<double, int> > cost;
+		const double box_top = std::fmax(P.c0[2], P.c1[2]);
+		for (int i = 0; i < n; ++i) {
+			const int j = by_vang[(size_t)i];
+			if (i == 0 || cams[j].vang != cams[by_vang[(size_t)i - 1]].vang) {
+				set_camera(&sf, cams[j]);
+				orders.resize(orders.size() + (size_t)ty_view);
+				order_sky.push_back(0);
+				row_schedule(build_plane(sf), H, 0, 0, 1, ty_view, orders.data() + orders.size() - (size_t)ty_view,
+				             &order_sky.back(), &cost);
+			}
+			const int g = (int)order_sky.size() - 1;
+			view_order[(size_t)j] = g;
+			// (only when the camera is above the terrain: from below, rows that look up are the expensive ones)
+			if (cams[j].cam_pos[2] > box_top && !c->knobs.no_batch) sky[(size_t)j] = order_sky[(size_t)g];
+		}
+	}
+	// Global schedule, rank-major: the costliest terrain row of every view, then the second costliest of every view,
+	// ...; then every view's sky rows, grabbed sky_batch tiles at a time.  (HMRM_VIEWS_VIEW_MAJOR: view by view.)
+	auto row_of = [&](int j, int r) -> uint32_t {
+		const int g = view_order[(size_t)j];
+		const int t = g < 0 ? identity[(size_t)r] : orders[(size_t)g * (size_t)ty_view + (size_t)r];
+		return ((uint32_t)j << 14) | (uint32_t)t;
+	};
+	size_t at = 0;
+	if (c->knobs.views_view_major) {
+		for (int j = 0; j < n; ++j)
+			for (int r = 0; r < sky[(size_t)j]; ++r) h.rows[at++] = row_of(j, r);
+	}
+	else {
+		for (int r = 0; r < ty_view; ++r)
+			for (int j = 0; j < n; ++j)
+				if (r < sky[(size_t)j]) h.rows[at++] = row_of(j, r);
+	}
+	if (ordered) P.batch_from_tile = (unsigned)at * (unsigned)P.tiles_x;
+	for (int j = 0; j < n; ++j)
+		for (int r = sky[(size_t)j]; r < ty_view; ++r) h.rows[at++] = row_of(j, r);
+	HMRM_CUDA(c, cudaMemcpyAsync(slot.d_view, slot.view_host, need, cudaMemcpyHostToDevice, stream));
+
+	P.row_begin = 0;
+	P.row_end = H;
+	P.cycle = 0;
+	P.period = 1;
+	P.tile_y_first = 0;
+	P.tile_y_step = 1;
+	P.tiles_y = rows;
+	P.view_rows = d.rows;
+	P.views = d.rec;
+	P.n_views = n;
+	P.view_bytes = (unsigned long long)W * (unsigned long long)H * (f->pixel_format == HMRM_PIXEL_RGB8 ? 3ULL : 4ULL);
+	P.fb = (uint32_t *)d_out;                    // (each view's alignment is decided in the kernel)
+	P.stats = slot.d_stats;
+	P.tile_counter = slot.d_tile_counter;
+	if ((rc = reset_slot(c, slot, -1, stream)) != HMRM_OK) return rc;
+	const bool want_stats = (f->flags & HMRM_FLAG_STATS) != 0;
+	HMRM_CUDA(c, cudaEventRecord(slot.ev_begin, stream));
+	if ((rc = launch_lin<true>(c, P, want_stats, stream)) != HMRM_OK) return rc;
+	HMRM_CUDA(c, cudaGetLastError());
+	HMRM_CUDA(c, cudaEventRecord(slot.ev_end, stream));
+	slot.used = true;
+	c->launch_last = ls;
+	c->last_stream = stream;
+	c->last_had_stats = want_stats;
+	c->last_had_step_index = false;
+	c->last_had_ray_dump = false;
+	c->timing_valid = true;
+	c->last_w = W;
+	c->last_h = H;
+	return HMRM_OK;
+}
+
 } // namespace
 
 extern "C" {
@@ -1290,6 +1534,7 @@ int hmrm_create(int device, hmrm_ctx **out) {
 		else k.peer_memops = probe_memops();
 		k.no_batch = std::getenv("HMRM_NO_BATCH") != NULL;
 		k.debug_sched = std::getenv("HMRM_DEBUG_SCHED") != NULL;
+		k.views_view_major = std::getenv("HMRM_VIEWS_VIEW_MAJOR") != NULL;
 		k.lmin_bias = (e = std::getenv("HMRM_LMIN_BIAS")) ? std::atoi(e) : 0;
 		k.lstride = (e = std::getenv("HMRM_LSTRIDE")) ? std::atoi(e) : 1;
 		k.lstart = (e = std::getenv("HMRM_LSTART")) ? std::atoi(e) : 6;
@@ -1348,6 +1593,8 @@ int hmrm_create(int device, hmrm_ctx **out) {
 	std::memset(c->scratch_cap, 0, sizeof c->scratch_cap);
 	c->d_pixels = NULL;
 	c->pixels_cap = 0;
+	c->d_views = NULL;
+	c->views_cap = 0;
 	std::memset(c->sub, 0, sizeof c->sub);
 	c->sub_next = 0;
 	c->blur_n = 0;
@@ -1399,6 +1646,7 @@ void hmrm_destroy(hmrm_ctx *c) {
 
 	if (c->copy_stream) cudaStreamSynchronize(c->copy_stream);
 	cudaFree(c->d_pixels);
+	cudaFree(c->d_views);
 	for (int i = 0; i < kFrameRing; ++i) {
 		cudaFree(c->d_scratch[i]);
 		cudaFree(c->d_fb[i]);
@@ -1422,6 +1670,8 @@ void hmrm_destroy(hmrm_ctx *c) {
 		cudaFree(sl.d_sph);
 		cudaFree(sl.d_row_order);
 		if (sl.sph_host) cudaFreeHost(sl.sph_host);
+		cudaFree(sl.d_view);
+		if (sl.view_host) cudaFreeHost(sl.view_host);
 		if (sl.ev_begin) cudaEventDestroy(sl.ev_begin);
 		if (sl.ev_end) cudaEventDestroy(sl.ev_end);
 	}
@@ -1688,6 +1938,27 @@ int hmrm_render_device(hmrm_ctx *c, const hmrm_frame *f, void *d_rgba_out, void 
 	if (!d_rgba_out) return fail(c, HMRM_ERR_INVALID, "d_rgba_out is NULL");
 	if (!f) return fail(c, HMRM_ERR_INVALID, "frame is NULL");
 	return enqueue_frame(c, f, (uint32_t *)d_rgba_out, stream ? (cudaStream_t)stream : c->stream);
+}
+
+int hmrm_render_views_device(hmrm_ctx *c, const hmrm_frame *f, const hmrm_camera *cams, int32_t n, void *d_out,
+                             void *stream) {
+	if (!c) return HMRM_ERR_INVALID;
+	if (int rc = check_views(c, f, cams, n, d_out)) return rc;
+	return enqueue_views(c, f, cams, n, (uint8_t *)d_out, stream ? (cudaStream_t)stream : c->stream);
+}
+
+int hmrm_render_views(hmrm_ctx *c, const hmrm_frame *f, const hmrm_camera *cams, int32_t n, uint8_t *out) {
+	if (!c) return HMRM_ERR_INVALID;
+	if (int rc = check_views(c, f, cams, n, out)) return rc;
+	HMRM_CUDA(c, cudaSetDevice(c->device));
+	const size_t bytes = (size_t)n * (size_t)f->screen_width * (size_t)f->screen_height *
+	                     (f->pixel_format == HMRM_PIXEL_RGB8 ? 3 : 4);
+	// the buffer is idle: the call that used it last synchronised before it returned
+	if (int rc = grow(c, &c->d_views, &c->views_cap, bytes)) return rc;
+	if (int rc = enqueue_views(c, f, cams, n, c->d_views, c->stream)) return rc;
+	HMRM_CUDA(c, cudaMemcpyAsync(out, c->d_views, bytes, cudaMemcpyDefault, c->stream));
+	HMRM_CUDA(c, cudaStreamSynchronize(c->stream));
+	return HMRM_OK;
 }
 
 int hmrm_render_async(hmrm_ctx *c, const hmrm_frame *f, uint8_t *rgba_out) {

@@ -427,7 +427,10 @@ next_sample:
 	tally.fetches = fetches;
 }
 
-template <bool kStats, int kLayout, int kCtas>
+// kViews (hmrm_render_views): the queue runs over the tile rows of P.n_views views of one frame, in the order of the
+// host's schedule P.view_rows.  Only the camera (generate_ray's ViewConst) and the pixel destination differ per view;
+// the march, the shading and the statistics are those of a single frame.
+template <bool kStats, int kLayout, int kCtas, bool kViews = false>
 __global__ void __launch_bounds__(HMRM_LIN_THREADS, kCtas) k2_render_lin(const __grid_constant__ RenderParams P) {
 	const int lane = threadIdx.x & 31;
 	const unsigned n_tiles = (unsigned)(P.tiles_x * P.tiles_y);
@@ -454,7 +457,13 @@ __global__ void __launch_bounds__(HMRM_LIN_THREADS, kCtas) k2_render_lin(const _
 		int ty_seq, tx;
 		tile_row_col(P, tile, ty_seq, tx);
 		// longest-processing-time-first: a few grazing tiles take ~50x the mean, so they must start early
-		const int ty = P.row_order ? __ldg(P.row_order + HMRM_CHECKED(P, ty_seq, P.tiles_y)) : ty_seq;
+		int ty, view = 0;
+		if (kViews) {
+			const unsigned vr = __ldg(P.view_rows + HMRM_CHECKED(P, ty_seq, P.tiles_y));
+			view = (int)HMRM_CHECKED(P, vr >> 14, (unsigned)P.n_views);
+			ty = (int)(vr & 0x3FFFu);
+		}
+		else ty = P.row_order ? __ldg(P.row_order + HMRM_CHECKED(P, ty_seq, P.tiles_y)) : ty_seq;
 		const int px = tx * 8 + (lane & 7);
 		const int py = P.row_begin + (P.tile_y_first + ty * P.tile_y_step) * 4 + (lane >> 3);
 		const bool active = pixel_selected(P, px, py);
@@ -465,7 +474,7 @@ __global__ void __launch_bounds__(HMRM_LIN_THREADS, kCtas) k2_render_lin(const _
 			bool real_hit = false;
 			int first_hit = -1;
 			unsigned hit_cell = 0u;
-			const Ray ray = generate_ray(P, px, py);
+			const Ray ray = kViews ? generate_ray(P, P.views[view], px, py) : generate_ray(P, px, py);
 			double ex, ey, ez, lo = 0.0;
 			const bool entered = box_entry(P, ray, ex, ey, ez, lo);
 			if (kStats && P.ray_dump) dump_ray(P, px, py, ray, entered, lo, ex, ey, ez);
@@ -481,7 +490,15 @@ __global__ void __launch_bounds__(HMRM_LIN_THREADS, kCtas) k2_render_lin(const _
 			}
 			if (P.step_index) P.step_index[(size_t)py * (size_t)P.W + (size_t)px] = first_hit;
 		}
-		store_pixel(P, px, py, active, rgba);       // main/hmap.cpp:139-154 (RGBA8), or packed RGB8
+		if (kViews) {
+			// view j starts at byte j * W * H * C: with RGB8 and W * H * 3 not a multiple of 4, views differ in alignment
+			ViewDst dst;
+			dst.fb = (uint32_t *)((uint8_t *)P.fb + (size_t)view * P.view_bytes);
+			dst.fb_unaligned = ((uintptr_t)dst.fb & 3u) != 0u ? 1 : 0;
+			dst.rgb_words = (P.W % 4) == 0 && !dst.fb_unaligned ? 1 : 0;
+			store_pixel_to(P, dst, px, py, active, rgba);
+		}
+		else store_pixel(P, px, py, active, rgba);       // main/hmap.cpp:139-154 (RGBA8), or packed RGB8
 		commit_tally<kStats>(P, active, tally);
 	}
 }

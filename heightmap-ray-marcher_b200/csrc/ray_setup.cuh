@@ -21,39 +21,49 @@ struct Ray {
 	double dx, dy, dz;
 };
 
-__device__ __forceinline__ Ray generate_ray(const RenderParams &P, int px, int py) {
+// The camera comes from V: RenderParams itself for a single frame, or a ViewConst record of a batch of views; both have
+// the same field names.  The screen (projection, wtab, htab) always comes from P.
+template <class V>
+__device__ __forceinline__ Ray generate_ray_from(const RenderParams &P, const V &v, int px, int py) {
 	Ray r;
 	if (P.projection == 2) {
-		const double sv = __ldg(P.sin_va + py);
-		r.ox = P.cam[0]; r.oy = P.cam[1]; r.oz = P.cam[2];
-		r.dx = fmul(sv, __ldg(P.cos_ha + px));
-		r.dy = fmul(sv, __ldg(P.sin_ha + px));
-		r.dz = __ldg(P.cos_va + py);
+		const double sv = __ldg(v.sin_va + HMRM_CHECKED(P, py, P.H));
+		r.ox = v.cam[0]; r.oy = v.cam[1]; r.oz = v.cam[2];
+		r.dx = fmul(sv, __ldg(v.cos_ha + HMRM_CHECKED(P, px, P.W)));
+		r.dy = fmul(sv, __ldg(v.sin_ha + HMRM_CHECKED(P, px, P.W)));
+		r.dz = __ldg(v.cos_va + HMRM_CHECKED(P, py, P.H));
 		return r;
 	}
 	const double w = __ldg(P.wtab + px);
 	const double h = __ldg(P.htab + py);
 	// (upper_left + w * plane_right) + h * plane_down
-	const double qx = fadd(fadd(P.ul[0], fmul(w, P.pr[0])), fmul(h, P.pd[0]));
-	const double qy = fadd(fadd(P.ul[1], fmul(w, P.pr[1])), fmul(h, P.pd[1]));
-	const double qz = fadd(fadd(P.ul[2], fmul(w, P.pr[2])), fmul(h, P.pd[2]));
+	const double qx = fadd(fadd(v.ul[0], fmul(w, v.pr[0])), fmul(h, v.pd[0]));
+	const double qy = fadd(fadd(v.ul[1], fmul(w, v.pr[1])), fmul(h, v.pd[1]));
+	const double qz = fadd(fadd(v.ul[2], fmul(w, v.pr[2])), fmul(h, v.pd[2]));
 	if (P.projection == 1) {
-		const double vx = fsub(qx, P.cam[0]);
-		const double vy = fsub(qy, P.cam[1]);
-		const double vz = fsub(qz, P.cam[2]);
+		const double vx = fsub(qx, v.cam[0]);
+		const double vy = fsub(qy, v.cam[1]);
+		const double vz = fsub(qz, v.cam[2]);
 		// glm::normalize: v * (1 / sqrt(dot(v, v))), dot = (x*x + y*y) + z*z
 		const double len2 = fadd(fadd(fmul(vx, vx), fmul(vy, vy)), fmul(vz, vz));
 		const double inv = frcp(fsqrt(len2));
-		r.ox = P.cam[0]; r.oy = P.cam[1]; r.oz = P.cam[2];
+		r.ox = v.cam[0]; r.oy = v.cam[1]; r.oz = v.cam[2];
 		r.dx = fmul(vx, inv);
 		r.dy = fmul(vy, inv);
 		r.dz = fmul(vz, inv);
 	}
 	else {
 		r.ox = qx; r.oy = qy; r.oz = qz;
-		r.dx = P.look[0]; r.dy = P.look[1]; r.dz = P.look[2];
+		r.dx = v.look[0]; r.dy = v.look[1]; r.dz = v.look[2];
 	}
 	return r;
+}
+
+__device__ __forceinline__ Ray generate_ray(const RenderParams &P, int px, int py) { return generate_ray_from(P, P, px, py); }
+
+// view `v` of a batch (k2_render_lin<..., kViews = true>)
+__device__ __forceinline__ Ray generate_ray(const RenderParams &P, const ViewConst &v, int px, int py) {
+	return generate_ray_from(P, v, px, py);
 }
 
 // One axis of the slab test; returns false when the ray misses (src/AABB.cpp:58-73).
@@ -150,8 +160,10 @@ __device__ __noinline__ void dump_ray(const RenderParams &P, int px, int py, con
 }
 
 // RGBA8 pixel `at` (index into [H][W]): one 32-bit store, or four byte stores into a destination that is not 4-byte
-// aligned (hmrm_render_device and the peer calls accept any device pointer).
-__device__ __forceinline__ void store_rgba8(const RenderParams &P, size_t at, uint32_t rgba) {
+// aligned (hmrm_render_device and the peer calls accept any device pointer).  D holds fb and fb_unaligned: RenderParams
+// itself for a single frame, a ViewDst for one view of a batch.
+template <class D>
+__device__ __forceinline__ void store_rgba8(const D &P, size_t at, uint32_t rgba) {
 	if (!P.fb_unaligned) {
 		P.fb[at] = rgba;
 		return;
@@ -168,18 +180,20 @@ __device__ __forceinline__ void store_rgba8(const RenderParams &P, size_t at, ui
 // byte is always 255 in the reference, so it is dead weight on PCIe / NVLink): a tile row is 24 contiguous bytes;
 // when all 8 pixels of the row are written and rows are 4-byte aligned, lanes 0..5 of the row assemble them as six
 // 32-bit words from their neighbours' colours (two shuffles), otherwise every lane stores its 3 bytes.
-__device__ __forceinline__ void store_pixel(const RenderParams &P, int px, int py, bool active, uint32_t rgba) {
+// The destination (fb, fb_unaligned, rgb_words) is D's: the frame's (store_pixel), or one view's of a batch.
+template <class D>
+__device__ __forceinline__ void store_pixel_to(const RenderParams &P, const D &dst, int px, int py, bool active, uint32_t rgba) {
 	if (P.pixel_format == 0) {
-		if (active) store_rgba8(P, HMRM_CHECKED(P, (size_t)py * (size_t)P.W + (size_t)px, (size_t)P.W * (size_t)P.H), rgba);
+		if (active) store_rgba8(dst, HMRM_CHECKED(P, (size_t)py * (size_t)P.W + (size_t)px, (size_t)P.W * (size_t)P.H), rgba);
 		return;
 	}
 	const int lane = threadIdx.x & 31, i = lane & 7;
 	const unsigned full = __ballot_sync(0xFFFFFFFFu, active);
-	const bool row_full = ((full >> (lane & 24)) & 0xFFu) == 0xFFu && P.rgb_words;
+	const bool row_full = ((full >> (lane & 24)) & 0xFFu) == 0xFFu && dst.rgb_words;
 	const int a = (i * 4) / 3;                         // first pixel contributing to word i (i < 6): 0 1 2 4 5 6
 	const uint32_t A = __shfl_sync(0xFFFFFFFFu, rgba, (lane & 24) | min(a, 7)) & 0xFFFFFFu;
 	const uint32_t B = __shfl_sync(0xFFFFFFFFu, rgba, (lane & 24) | min(a + 1, 7)) & 0xFFFFFFu;
-	uint8_t *fb8 = (uint8_t *)P.fb;
+	uint8_t *fb8 = (uint8_t *)dst.fb;
 	if (row_full) {
 		if (i < 6) {
 			const int sh = 8 * ((i * 4) % 3);
@@ -195,6 +209,17 @@ __device__ __forceinline__ void store_pixel(const RenderParams &P, int px, int p
 		o[2] = (uint8_t)(rgba >> 16);
 	}
 }
+
+__device__ __forceinline__ void store_pixel(const RenderParams &P, int px, int py, bool active, uint32_t rgba) {
+	store_pixel_to(P, P, px, py, active, rgba);
+}
+
+// Where one view of a batch goes: its base has its own alignment (k2_render_lin<..., kViews = true>)
+struct ViewDst {
+	uint32_t *fb;
+	uint8_t fb_unaligned;
+	int rgb_words;
+};
 
 } // namespace hmrm
 

@@ -77,6 +77,18 @@ struct RenderParams {
 	uint32_t bg_rgba;              // bg colour with alpha 255
 	uint8_t bg[3];
 	uint8_t fb_unaligned;          // fb is not 4-byte aligned (a caller's device pointer): RGBA8 pixels go out as 4 bytes
+	// ---- k2_render_lin<..., kViews = true> (hmrm_render_views): n_views cameras of one frame in one launch.  Appended
+	// after every field above, so that the kernels of single frames see the parameter block they always saw. ----
+	const uint32_t *view_rows;     // [tiles_y]: launch tile row t is tile row (view_rows[t] & 0x3FFF) of view view_rows[t] >> 14
+	const struct ViewConst *views; // [n_views]
+	int n_views;
+	unsigned long long view_bytes; // W * H * C: view j's pixels start at byte j * view_bytes of fb (each view has its own alignment)
+};
+
+// The camera-dependent constants of one view of a batch: what generate_ray reads of RenderParams for a single frame.
+struct ViewConst {
+	double cam[3], ul[3], pr[3], pd[3], look[3];
+	const double *cos_ha, *sin_ha, *sin_va, *cos_va;   // spherical only: this view's tables (hang and vang differ per view)
 };
 
 } // namespace hmrm

@@ -215,6 +215,30 @@ int hmrm_wait(hmrm_ctx *ctx);
  * in its host buffer (so n + 1 host buffers are rotated); hmrm_wait_pending(ctx, 0) == hmrm_wait. */
 int hmrm_wait_pending(hmrm_ctx *ctx, int max_pending);
 
+/* ---- many cameras in one launch (kernel K2, csrc/k2_render_lin.cuh with kViews) ----
+ * n views of f in one launch.  View j is exactly the frame hmrm_render would produce for f with cam_pos, hang and vang
+ * replaced by cams[j] (set_camera's rule, as for motion blur); every other field comes from f, and f's own camera is
+ * not used.  Output: [n][screen_height][screen_width][C], C = 4 (HMRM_PIXEL_RGBA8) or 3 (HMRM_PIXEL_RGB8); view j
+ * starts at byte j * H * W * C.  cams is copied before the call returns.
+ * Limits: 1 <= n <= 65536; f passes hmrm_render's frame checks; the batch has at most 2^26 tiles of 8x4 pixels
+ * (n * ceil(W/8) * ceil(H/4)).  Outside them: HMRM_ERR_INVALID.
+ * Refused with HMRM_ERR_INVALID, nothing written and the context left usable: what a motion-blurred frame refuses
+ * (cycle_period != 1, band_count > 1, a partial row band, HMRM_FLAG_STEP_INDEX or HMRM_FLAG_RAY_DUMP); a supersample
+ * field other than 0; a context with motion blur set; a non-finite value in any camera; NULL cams or output; a traversal
+ * other than HMRM_TRAVERSAL_AUTO or HMRM_TRAVERSAL_SKIP; a grid_width so small that the skip traversal would fall back
+ * to FP64 (views have no fallback path).  Maps whose height range could not be quantised: HMRM_ERR_STATE.
+ * With HMRM_FLAG_STATS, hmrm_get_stats describes the batch: rays = n*W*H; box_hits, surf_hits, steps and fetches are
+ * sums over the views, max_steps the maximum, status the OR of the views, kernel_ms the one launch.  Afterwards
+ * hmrm_get_step_index and hmrm_get_ray_dump return HMRM_ERR_STATE.
+ * d_out may have any alignment, as for hmrm_render_device; each view's base address has its own (with RGB8 and W*H*3
+ * not a multiple of 4, consecutive views start at different offsets modulo 4) and is written accordingly. */
+int hmrm_render_views_device(hmrm_ctx *ctx, const hmrm_frame *f, const hmrm_camera *cams, int32_t n,
+                             void *d_out, void *stream);            /* stream-ordered; NULL = ctx's stream */
+/* the same into any host memory, through a device buffer of the context on ctx's stream; synchronous.  Frames of
+ * hmrm_render_async still in flight are not disturbed. */
+int hmrm_render_views(hmrm_ctx *ctx, const hmrm_frame *f, const hmrm_camera *cams, int32_t n,
+                      uint8_t *out);
+
 /* ---- PNG frames, deflated on the device (kernel K3, csrc/k3_png.cuh) ----
  * The file is 8-bit, not interlaced, colour type 6 for 4 channels and 2 for 3; the decoded pixels are the frame's, byte
  * for byte.  The file is exactly this function of the pixels (C channels, W x H):
